@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the PSGLA / PnP-ULA hot path on B200, next to the reference's CPU path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -24,6 +24,15 @@ steps, W warm-up steps, barrier + synchronize on both sides, max over ranks.  `v
 HBM; `e2e` goes through the public Python API with pinned-host inputs and outputs (copies inside the timed region).
 `--impl reference` times the reference's own CPU algorithm (the unmodified reference when /root/reference exists,
 else the oracle port) on all host cores.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step of four blocks computed for rank 0's chains:
+the 2D headline block's chain states (`gmm2d_state`, after step --steps; --only-image forces --steps to 1) and, for the
+three image blocks, the iterate and the running first and second moments (`image_X`, `image_mean`, `image_mean2`, the
+same for `image_deblur_*` and `image_drunet_*`, after the --image-steps / --drunet-steps steps of those blocks).  The
+strong-scaling, config0, e2e, image-set and GPU-reference timings are not dumped.  Files are DIR/<name>.npy in the array's
+own float32 / float64.  An array of more than 2^20 elements is written as the flattened array at a fixed set of 2^20
+indices (seeded, sorted; for `gmm2d_state` these are single coordinates, not whole chains), so the ten arrays stay under
+64 MB.  Every input is seeded: two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -183,6 +192,37 @@ class Timer:
         ms = [a.elapsed_time(b) for a, b in self.pairs]
         self.pairs = []
         return sum(ms), ms
+
+
+DUMP_MAX_ELEMENTS = 1 << 20
+_OUTPUTS = {}
+
+
+def keep_output(args, name, t):
+    """Copies (a fixed seeded sample of) a timed block's result to the host for --dump-outputs; a no-op without it."""
+    if not args.dump_outputs:
+        return
+    import numpy as np
+    import torch
+    a = t.detach()
+    if a.numel() > DUMP_MAX_ELEMENTS:
+        idx = np.sort(np.random.default_rng(0).choice(a.numel(), DUMP_MAX_ELEMENTS, replace=False))
+        a = a.reshape(-1)[torch.from_numpy(idx).to(a.device)]
+    _OUTPUTS[name] = (a if a.dtype == torch.float64 else a.float()).cpu().numpy()
+
+
+def keep_run_outputs(args, block, run):
+    """An image sampler's state after its last timed iteration: the iterate and the running moments its windows return."""
+    for field in ("X", "mean", "mean2"):
+        keep_output(args, "%s_%s" % (block, field), getattr(run, field))
+
+
+def write_outputs(path):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in _OUTPUTS.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+    log("--dump-outputs: %s written to %s" % (", ".join(sorted(_OUTPUTS)), path))
 
 
 def barrier(torch, dist_mod):
@@ -370,6 +410,7 @@ def bench_gmm2d(args, P, torch, rank, ws, dev):
         timer.step(lambda: ch.run(n_steps))
         flop += FLOP_PER_CHAIN_STEP[CELLS[k % len(CELLS)][2]] * float(n_chains) * n_steps
     total_ms, per_step = timer.total_ms()
+    keep_output(args, "gmm2d_state", ch.state)
     launches_per_step = int(P._lib.lib().psgla_gmm2d_last_launches())
     barrier(torch, P.dist)
     total_ms = P.dist.max_over_ranks(total_ms, dev)
@@ -446,6 +487,7 @@ def bench_image(args, P, torch, rank, ws, dev, peaks):
     for i in range(W, W + K):
         timer.step(lambda: run.step(i))
     total_ms, per_step = timer.total_ms()
+    keep_run_outputs(args, "image", run)
     barrier(torch, P.dist)
     total_ms = P.dist.max_over_ranks(total_ms, dev)
     finite = bool(torch.isfinite(run.X).all().item())
@@ -631,6 +673,7 @@ def bench_image_deblur(args, P, torch, rank, ws, dev, peaks):
     for i in range(W, W + K):
         timer.step(lambda: run.step(i))
     total_ms, per_step = timer.total_ms()
+    keep_run_outputs(args, "image_deblur", run)
     barrier(torch, P.dist)
     total_ms = P.dist.max_over_ranks(total_ms, dev)
     finite = bool(torch.isfinite(run.X).all().item())
@@ -686,6 +729,7 @@ def bench_image_drunet(args, P, torch, rank, ws, dev, peaks):
     for i in range(W, W + K):
         timer.step(lambda: run.step(i))
     total_ms, per_step = timer.total_ms()
+    keep_run_outputs(args, "image_drunet", run)
     barrier(torch, P.dist)
     total_ms = P.dist.max_over_ranks(total_ms, dev)
     finite = bool(torch.isfinite(run.X).all().item())
@@ -1016,7 +1060,13 @@ def main():
     ap.add_argument("--only-image", action="store_true", help="profiling aid: shrink the 2D part to a token run")
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of the 2D block and of the image blocks computed to "
+                                                        "DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path, not to --impl reference")
     args.warmup = max(args.warmup, 0)
     capture_stdout()
     if args.only_image:
@@ -1031,6 +1081,8 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: the product has no CPU path (use --impl reference for the CPU arm)")
     rank, ws, local = P.dist.init_from_env("nccl")
+    if rank != 0:
+        args.dump_outputs = None  # only rank 0 writes its chains' outputs, so the other ranks keep none
     if ws != max(args.gpus, 1):
         log("warning: --gpus %d but WORLD_SIZE %d; using WORLD_SIZE" % (args.gpus, ws))
     torch.cuda.set_device(local)
@@ -1164,6 +1216,8 @@ def main():
         if "gpu_reference" in img and "B1" in img["gpu_reference"]:
             summ["gpu_reference_B1_image_iterations_per_sec"] = img["gpu_reference"]["B1"]["value"]
         line["image_summary"] = summ
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs)
     emit(line)
     if ws > 1:
         import torch.distributed as dist
