@@ -299,6 +299,14 @@ int psgla_drunet_denoise_post_next(const void* packed_dev, psgla_img_shape shape
                                    size_t workspace_bytes, const float* base_dev, const psgla_post_params* post,
                                    float* x_out_dev, float* sample_dev, float* mean_dev, float* mean2_dev,
                                    const psgla_next_pre* next, void* stream);
+/* One layer of that network, exposed for parity tests like psgla_conv3x3_layer: exactly the kernel, ReLU and residual adds
+ * psgla_drunet_denoise_post runs for it.  layer: 0..63 in the state-dict order above; shape: the network's image shape (H, W
+ * multiples of 8); the layer works at its own scale of it.  in_dev: bf16 NHWC16 (layer 0, channel 3 = sigma) or bf16 NHWC.
+ * out_dev: bf16 NHWC, or for layer 63 the raw conv as fp32 NCHW [B][3][H][W].  res1_dev (the residual block's input) must
+ * be given exactly for the second conv of a residual block, res2_dev (the U-Net skip) exactly for the last such conv of the
+ * body and of each decoder stage; both are bf16 NHWC of the output's shape. */
+int psgla_drunet_layer(const void* packed_dev, psgla_img_shape shape, int layer, const void* in_dev, const void* res1_dev,
+                       const void* res2_dev, void* out_dev, void* stream);
 
 /* One general convolution layer of the DRUNet denoiser (deepinv.models.DRUNet, sampling_images.py:136) as implicit GEMM:
  *   mode 0: 3x3 stride 1 zero-pad 1 (Cin -> Cout); 1: 2x2 stride 2 (downsampling); 2: 2x2 stride 2 transposed (upsampling).

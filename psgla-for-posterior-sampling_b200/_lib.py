@@ -100,6 +100,7 @@ SIGNATURES = {
     "psgla_drunet_denoise_post": (_int, [_vp, ImgShape, _vp, _vp, _sz, _vp, C.POINTER(PostParams), _vp, _vp, _vp, _vp, _vp]),
     "psgla_drunet_denoise_post_next": (_int, [_vp, ImgShape, _vp, _vp, _sz, _vp, C.POINTER(PostParams), _vp, _vp, _vp, _vp,
                                               C.POINTER(NextPre), _vp]),
+    "psgla_drunet_layer": (_int, [_vp, ImgShape, _int, _vp, _vp, _vp, _vp, _vp]),
     "psgla_selftest_umma": (_int, [_vp, _vp, _vp, _int, _int, _vp]),
     "psgla_selftest_umma2": (_int, [_vp, _vp, _vp, _int, _vp]),
     "psgla_convg_layer": (_int, [_int, _int, _int, _int, _int, _int, _vp, _vp, _vp, _vp, _vp, _int, _vp]),

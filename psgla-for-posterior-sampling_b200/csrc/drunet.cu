@@ -20,6 +20,9 @@ enum DruKind { DRU_HEAD, DRU_C64, DRU_GEMM3, DRU_DOWN, DRU_UP, DRU_TAIL };
 struct DruLayer {
   DruKind kind;
   int cin, cout;
+  int scale;  // the layer's input is (H >> scale) x (W >> scale)
+  int relu;   // ReLU after the sum
+  int nres;   // residual inputs added before the ReLU: 1 = the block input (second conv of a residual block), 2 = and the U-Net skip
   size_t w_off, bytes;
 };
 
@@ -43,23 +46,28 @@ static const std::vector<DruLayer>& dru_plan() {
   if (!plan.empty()) return plan;
   std::vector<DruLayer> v;
   size_t off = 0;
-  auto add = [&](DruKind k, int cin, int cout) {
+  auto add = [&](DruKind k, int cin, int cout, int scale, int relu, int nres) {
     const size_t b = dru_layer_bytes(k, cin, cout);
-    v.push_back({k, cin, cout, off, b});
+    v.push_back({k, cin, cout, scale, relu, nres, off, b});
     off += b;
   };
   const int nc[4] = {64, 128, 256, 512};
-  add(DRU_HEAD, 4, 64);
-  for (int s = 0; s < 3; ++s) {
-    for (int i = 0; i < 8; ++i) add(s == 0 ? DRU_C64 : DRU_GEMM3, nc[s], nc[s]);
-    add(DRU_DOWN, nc[s], nc[s + 1]);
+  // four residual blocks x -> x + conv(relu(conv(x))); with `skip`, the last one also adds the U-Net skip connection
+  auto blocks = [&](int s, bool skip) {
+    for (int i = 0; i < 8; ++i)
+      add(s == 0 ? DRU_C64 : DRU_GEMM3, nc[s], nc[s], s, i % 2 == 0, i % 2 == 0 ? 0 : (skip && i == 7 ? 2 : 1));
+  };
+  add(DRU_HEAD, 4, 64, 0, 0, 0);
+  for (int s = 0; s < 3; ++s) {  // encoder
+    blocks(s, false);
+    add(DRU_DOWN, nc[s], nc[s + 1], s, 0, 0);
   }
-  for (int i = 0; i < 8; ++i) add(DRU_GEMM3, 512, 512);
-  for (int s = 2; s >= 0; --s) {
-    add(DRU_UP, nc[s + 1], nc[s]);
-    for (int i = 0; i < 8; ++i) add(s == 0 ? DRU_C64 : DRU_GEMM3, nc[s], nc[s]);
+  blocks(3, true);  // body, + x4
+  for (int s = 2; s >= 0; --s) {  // decoder, + x3 / x2 / x1
+    add(DRU_UP, nc[s + 1], nc[s], s + 1, 0, 0);
+    blocks(s, true);
   }
-  add(DRU_TAIL, 64, 3);
+  add(DRU_TAIL, 64, 3, 0, 0, 0);
   plan.swap(v);
   return plan;
 }
@@ -83,6 +91,47 @@ static size_t dru_workspace_bytes(int B, int H, int W) {
   size_t t = 0;
   for (int s = 0; s < 4; ++s) t += 4 * dru_scale_bytes(B, H, W, s);
   return t + 1024;
+}
+
+// What the tail does with its conv output: the fused Langevin post (the network) or nothing (base == NULL: x_out = the raw
+// fp32 NCHW conv, psgla_drunet_layer).
+struct DruPost {
+  const float* base;
+  float base_scale, gain, w_old, w_new;
+  float* x_out;
+  float* sample;
+  float* mean;
+  float* mean2;
+  const psgla_next_pre* next;
+};
+
+// Layer l of the plan as the network runs it: the kernel its kind selects, its ReLU, and its residual inputs (res1 = the block
+// input, res2 = the U-Net skip; null where the plan has none).  in / out / res are bf16 NHWC except the head's input (NHWC16)
+// and the tail's output, which goes through `post`.
+static int dru_layer(const uint8_t* packed, int l, int B, int H, int W, const void* in, const void* res1, const void* res2,
+                     void* out, const DruPost& post, cudaStream_t st) {
+  const DruLayer& L = dru_plan()[l];
+  const uint8_t* w = packed + L.w_off;
+  const int h = H >> L.scale, wd = W >> L.scale;
+  auto bias = [&](int nout_pad, int cin_pad) { return reinterpret_cast<const float*>(w + (size_t)9 * nout_pad * cin_pad * 2); };
+  switch (L.kind) {
+    case DRU_HEAD: return conv_first16(in, out, w, bias(64, 16), B, H, W, L.relu, st);
+    case DRU_C64: return conv64_hidden(in, out, w, bias(64, 64), B, h, wd, L.relu, res1, res2, st);
+    case DRU_GEMM3: return conv_gemm_layer(0, B, h, wd, L.cin, L.cout, w, in, res1, res2, out, L.relu, st);
+    case DRU_DOWN: return conv_gemm_layer(1, B, h, wd, L.cin, L.cout, w, in, res1, res2, out, L.relu, st);
+    case DRU_UP: return conv_gemm_layer(2, B, h, wd, L.cin, L.cout, w, in, res1, res2, out, L.relu, st);
+    case DRU_TAIL:
+      return conv_last_post(in, w, bias(16, 64), B, H, W, post.base, post.base_scale, post.gain, post.w_old, post.w_new,
+                            post.x_out, post.sample, post.mean, post.mean2, post.next, st);
+  }
+  return set_error(PSGLA_E_BADARG, "DRUNet layer %d: unknown kind", l);
+}
+
+static int dru_check_shape(const psgla_img_shape& shape) {
+  PSGLA_REQUIRE(shape.B > 0 && shape.C == 3 && shape.H > 0 && shape.W > 0, "image shape must be [B>0][3][H>0][W>0]");
+  PSGLA_REQUIRE(shape.H % 8 == 0 && shape.W % 8 == 0, "DRUNet needs H and W to be multiples of 8 (got %d x %d): crop or pad "
+                "the image (the reference's deepinv pads internally by an unverifiable rule)", shape.H, shape.W);
+  return PSGLA_OK;
 }
 
 }  // namespace psgla
@@ -154,15 +203,15 @@ extern "C" int psgla_drunet_denoise_post_next(const void* packed_dev, psgla_img_
     if (rcn) return rcn;
   }
   PSGLA_REQUIRE((mean_dev == nullptr) == (mean2_dev == nullptr), "mean and mean2 must be given together");
-  PSGLA_REQUIRE(shape.B > 0 && shape.C == 3 && shape.H > 0 && shape.W > 0, "image shape must be [B>0][3][H>0][W>0]");
-  PSGLA_REQUIRE(shape.H % 8 == 0 && shape.W % 8 == 0, "DRUNet needs H and W to be multiples of 8 (got %d x %d): crop or pad "
-                "the image (the reference's deepinv pads internally by an unverifiable rule)", shape.H, shape.W);
+  {
+    const int rcs = dru_check_shape(shape);
+    if (rcs) return rcs;
+  }
   const int B = shape.B, H = shape.H, W = shape.W;
   if (workspace_bytes < dru_workspace_bytes(B, H, W))
     return set_error(PSGLA_E_WORKSPACE, "workspace of %zu bytes is smaller than the %zu needed", workspace_bytes,
                      dru_workspace_bytes(B, H, W));
   cudaStream_t st = (cudaStream_t)stream;
-  const auto& plan = dru_plan();
   const uint8_t* packed = (const uint8_t*)packed_dev;
   DruBuffers bufs;
   {
@@ -173,15 +222,15 @@ extern "C" int psgla_drunet_denoise_post_next(const void* packed_dev, psgla_img_
         pp += dru_scale_bytes(B, H, W, s);
       }
   }
-  size_t li = 0;
+  int li = 0;
   int rc = 0;
-  auto wptr = [&](size_t l) { return packed + plan[l].w_off; };
-  auto bias_of = [&](size_t l, int nout_pad, int cin_pad) {
-    return reinterpret_cast<const float*>(packed + plan[l].w_off + (size_t)9 * nout_pad * cin_pad * 2);
+  const DruPost no_post{};
+  auto run = [&](const void* in, const void* res1, const void* res2, void* out) {
+    if (!rc) rc = dru_layer(packed, li, B, H, W, in, res1, res2, out, no_post, st);
+    ++li;
   };
   // four residual blocks at scale s starting from `cur`; the last block also adds `skip` (U-Net skip connection)
   auto resblocks = [&](int s, uint8_t* cur, const uint8_t* skip) -> uint8_t* {
-    const int C = 64 << s, h = H >> s, w = W >> s;
     for (int blk = 0; blk < 4 && !rc; ++blk) {
       uint8_t* scratch[2];
       int n = 0;
@@ -189,43 +238,46 @@ extern "C" int psgla_drunet_denoise_post_next(const void* packed_dev, psgla_img_
         if (bufs.buf[s][j] != cur) scratch[n++] = bufs.buf[s][j];
       uint8_t* tmp = scratch[0];
       uint8_t* nxt = scratch[1];
-      const uint8_t* extra = (blk == 3) ? skip : nullptr;
-      if (s == 0) {
-        rc = conv64_hidden(cur, tmp, wptr(li), bias_of(li, 64, 64), B, h, w, 1, nullptr, nullptr, st);
-        if (!rc) rc = conv64_hidden(tmp, nxt, wptr(li + 1), bias_of(li + 1, 64, 64), B, h, w, 0, cur, extra, st);
-      } else {
-        rc = conv_gemm_layer(0, B, h, w, C, C, wptr(li), cur, nullptr, nullptr, tmp, 1, st);
-        if (!rc) rc = conv_gemm_layer(0, B, h, w, C, C, wptr(li + 1), tmp, cur, extra, nxt, 0, st);
-      }
-      li += 2;
+      run(cur, nullptr, nullptr, tmp);
+      run(tmp, cur, blk == 3 ? skip : nullptr, nxt);
       cur = nxt;
     }
     return cur;
   };
 
-  // head: x1
-  rc = conv_first16(den_in_dev, bufs.buf[0][0], wptr(0), bias_of(0, 64, 16), B, H, W, 0, st);
-  if (rc) return rc;
-  li = 1;
+  run(den_in_dev, nullptr, nullptr, bufs.buf[0][0]);  // head: x1
   uint8_t* cur = bufs.buf[0][0];
   for (int s = 0; s < 3; ++s) {  // encoder
     cur = resblocks(s, cur, nullptr);
-    if (rc) return rc;
-    rc = conv_gemm_layer(1, B, H >> s, W >> s, 64 << s, 128 << s, wptr(li), cur, nullptr, nullptr, bufs.buf[s + 1][0], 0, st);
-    if (rc) return rc;
-    ++li;
+    run(cur, nullptr, nullptr, bufs.buf[s + 1][0]);
     cur = bufs.buf[s + 1][0];
   }
   cur = resblocks(3, cur, bufs.buf[3][0]);  // body, + x4
-  if (rc) return rc;
   for (int s = 2; s >= 0; --s) {  // decoder
-    rc = conv_gemm_layer(2, B, H >> (s + 1), W >> (s + 1), 128 << s, 64 << s, wptr(li), cur, nullptr, nullptr, bufs.buf[s][1], 0, st);
-    if (rc) return rc;
-    ++li;
+    run(cur, nullptr, nullptr, bufs.buf[s][1]);
     cur = resblocks(s, bufs.buf[s][1], bufs.buf[s][0]);  // + x3 / x2 / x1
-    if (rc) return rc;
   }
+  if (rc) return rc;
   // tail + fused Langevin post:  X+ = base_scale * base + gain * D
-  return conv_last_post(cur, wptr(li), bias_of(li, 16, 64), B, H, W, base_dev, post->base_scale, post->gain, post->w_old,
-                        post->w_new, x_out_dev, sample_dev, mean_dev, mean2_dev, next, st);
+  const DruPost tail{base_dev,  post->base_scale, post->gain, post->w_old, post->w_new,
+                     x_out_dev, sample_dev,       mean_dev,   mean2_dev,   next};
+  return dru_layer(packed, li, B, H, W, cur, nullptr, nullptr, nullptr, tail, st);
+}
+
+extern "C" int psgla_drunet_layer(const void* packed_dev, psgla_img_shape shape, int layer, const void* in_dev,
+                                  const void* res1_dev, const void* res2_dev, void* out_dev, void* stream) {
+  const auto& plan = dru_plan();
+  PSGLA_REQUIRE(layer >= 0 && layer < (int)plan.size(), "psgla_drunet_layer: layer %d is not in 0..%d", layer,
+                (int)plan.size() - 1);
+  PSGLA_REQUIRE(packed_dev && in_dev && out_dev, "psgla_drunet_layer: null pointer");
+  const int rc = dru_check_shape(shape);
+  if (rc) return rc;
+  const DruLayer& L = plan[layer];
+  PSGLA_REQUIRE((res1_dev != nullptr) == (L.nres >= 1) && (res2_dev != nullptr) == (L.nres >= 2),
+                "psgla_drunet_layer: layer %d takes %d residual input(s) (res1 = block input, res2 = U-Net skip), got res1 %s, "
+                "res2 %s", layer, L.nres, res1_dev ? "set" : "null", res2_dev ? "set" : "null");
+  DruPost raw{};
+  raw.x_out = (float*)out_dev;
+  return dru_layer((const uint8_t*)packed_dev, layer, shape.B, shape.H, shape.W, in_dev, res1_dev, res2_dev, out_dev, raw,
+                   (cudaStream_t)stream);
 }

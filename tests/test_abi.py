@@ -116,6 +116,37 @@ def test_next_pre_argument_errors_without_gpu(built):
     assert rc == -1 and b"mask_B" in lib.psgla_last_error()
 
 
+def test_drunet_layer_argument_errors_without_gpu(built):
+    """psgla_drunet_layer rejects, on the host before any CUDA call, a layer index out of range, null pointers, a shape the network
+    rejects, and every residual pattern the network would not pass for that layer: res1 (the block input) exactly on the second
+    conv of each residual block, res2 (the U-Net skip) exactly on the last such conv of the body and of each decoder stage."""
+    L = built._lib
+    lib = L.lib()
+    shape = L.ImgShape(1, 3, 16, 16)
+    fake = 0x1000  # never dereferenced: every call below is rejected first
+    for layer in (-1, 64, 1 << 20):
+        assert lib.psgla_drunet_layer(fake, shape, layer, fake, None, None, fake, None) == -1
+        assert b"layer" in lib.psgla_last_error()
+    assert lib.psgla_drunet_layer(None, shape, 0, fake, None, None, fake, None) == -1 and b"null" in lib.psgla_last_error()
+    assert lib.psgla_drunet_layer(fake, shape, 0, fake, None, None, None, None) == -1 and b"null" in lib.psgla_last_error()
+    for bad in (L.ImgShape(1, 3, 12, 16), L.ImgShape(1, 3, 16, 20), L.ImgShape(0, 3, 16, 16), L.ImgShape(1, 4, 16, 16)):
+        assert lib.psgla_drunet_layer(fake, bad, 1, fake, None, None, fake, None) == -1
+    keys = built.DRUNET_KEYS
+    assert len(keys) == lib.psgla_drunet_num_weights() == 64
+    n_roles = {0: 0, 1: 0, 2: 0}
+    for layer, key in enumerate(keys):
+        want = 0
+        if ".res.2." in key:
+            want = 2 if key.startswith("m_body.3.") or (key.startswith("m_up") and ".4.res." in key) else 1
+        n_roles[want] += 1
+        for r1, r2 in ((None, None), (fake, None), (fake, fake), (None, fake)):
+            if (r1 is not None) + (r2 is not None) == want and (r2 is None or r1 is not None):
+                continue  # what the network passes: not called here (it would launch)
+            assert lib.psgla_drunet_layer(fake, shape, layer, fake, r1, r2, fake, None) == -1, (layer, key, r1, r2)
+            assert b"residual" in lib.psgla_last_error(), key
+    assert n_roles == {0: 64 - 28, 1: 24, 2: 4}
+
+
 def _sass(obj):
     import shutil
     import subprocess

@@ -1,10 +1,11 @@
-"""GPU parity tests of the DRUNet path: the general tcgen05 conv layers against torch.nn.functional on bf16-rounded
-operands (fp32 accumulate on both sides), then the whole denoiser and the samplers against the fp32 oracle."""
+"""GPU parity tests of the DRUNet path: the general tcgen05 conv layers element by element against the fp64 sum of the same
+bf16 operands (tests/conv_reference.py), then the whole denoiser and the samplers against the fp32 oracle."""
 import numpy as np
 import pytest
 import torch
 import torch.nn.functional as F
 
+import conv_reference as CR
 import psgla_b200 as P
 
 pytestmark = pytest.mark.gpu
@@ -22,24 +23,21 @@ def _nhwc(x):
 
 
 def _run_layer(mode, x, w_taps, res1=None, res2=None, relu=False):
-    """x: bf16 NCHW; w_taps: bf16 [taps][Cout][Cin]; returns fp32 NCHW."""
+    """x: bf16 NCHW; w_taps: bf16 [taps][Cout][Cin]; returns the bf16 output as NCHW."""
     lib = P._lib.lib()
     B, Cin, H, W = x.shape
     Cout = w_taps.shape[1]
     Ho, Wo = {0: (H, W), 1: (H // 2, W // 2), 2: (2 * H, 2 * W)}[mode]
     xin = _nhwc(x)
-    out = torch.full((B, Ho, Wo, Cout), float("nan"), device="cuda", dtype=torch.bfloat16)
+    out = CR.Guarded((B, Ho, Wo, Cout), torch.bfloat16)
     r1 = _nhwc(res1) if res1 is not None else None
     r2 = _nhwc(res2) if res2 is not None else None
     P._lib.check(lib.psgla_convg_layer(mode, B, H, W, Cin, Cout, w_taps.data_ptr(), xin.data_ptr(),
                                        r1.data_ptr() if r1 is not None else None, r2.data_ptr() if r2 is not None else None,
-                                       out.data_ptr(), int(relu), None), "psgla_convg_layer")
+                                       out.ptr(), int(relu), None), "psgla_convg_layer")
     torch.cuda.synchronize()
-    return out.float().permute(0, 3, 1, 2)
-
-
-def _tol(ref):
-    return 2 ** -8 * max(1.0, ref.abs().max().item()) * 1.01  # one bf16 rounding of the output
+    assert out.intact()
+    return out.tensor.permute(0, 3, 1, 2)
 
 
 @pytest.mark.parametrize("B,H,W,Cin,Cout,res,relu", [
@@ -59,15 +57,10 @@ def test_conv3x3_general(B, H, W, Cin, Cout, res, relu):
     x = _bf(torch.randn(B, Cin, H, W, device="cuda", generator=g))
     w = _bf(torch.randn(Cout, Cin, 3, 3, device="cuda", generator=g) / np.sqrt(9 * Cin))
     rs = [_bf(torch.randn(B, Cout, H, W, device="cuda", generator=g)) for _ in range(res)]
-    ref = F.conv2d(x.float(), w.float(), padding=1)
-    for r in rs:
-        ref = ref + r.float()
-    if relu:
-        ref = ref.relu()
+    ref, S = CR.reference("conv3", x, w, None, rs, relu)
     w_taps = w.permute(2, 3, 0, 1).reshape(9, Cout, Cin).contiguous()
     got = _run_layer(0, x, w_taps, *(rs + [None, None])[:2], relu=relu)
-    assert torch.isfinite(got).all()
-    assert (got - ref).abs().max().item() <= _tol(ref)
+    CR.check("convg conv3x3 %s" % ((B, H, W, Cin, Cout, res, relu),), got, ref, S)
 
 
 @pytest.mark.parametrize("B,H,W,Cin,Cout", [(2, 16, 40, 64, 128), (1, 8, 8, 256, 512), (1, 2, 260, 128, 256)])
@@ -75,9 +68,9 @@ def test_strided_down_conv(B, H, W, Cin, Cout):
     g = torch.Generator(device="cuda").manual_seed(1)
     x = _bf(torch.randn(B, Cin, H, W, device="cuda", generator=g))
     w = _bf(torch.randn(Cout, Cin, 2, 2, device="cuda", generator=g) / np.sqrt(4 * Cin))
-    ref = F.conv2d(x.float(), w.float(), stride=2)
+    ref, S = CR.reference("down", x, w)
     got = _run_layer(1, x, w.permute(2, 3, 0, 1).reshape(4, Cout, Cin).contiguous())
-    assert (got - ref).abs().max().item() <= _tol(ref)
+    CR.check("convg down %s" % ((B, H, W, Cin, Cout),), got, ref, S)
 
 
 @pytest.mark.parametrize("B,H,W,Cin,Cout,res", [(2, 8, 20, 128, 64, 0), (1, 4, 4, 512, 256, 0), (1, 3, 130, 256, 128, 0),
@@ -86,9 +79,9 @@ def test_transposed_up_conv(B, H, W, Cin, Cout, res):
     g = torch.Generator(device="cuda").manual_seed(2)
     x = _bf(torch.randn(B, Cin, H, W, device="cuda", generator=g))
     w = _bf(torch.randn(Cin, Cout, 2, 2, device="cuda", generator=g) / np.sqrt(Cin))  # ConvTranspose2d layout
-    ref = F.conv_transpose2d(x.float(), w.float(), stride=2)
+    ref, S = CR.reference("up", x, w)
     got = _run_layer(2, x, w.permute(2, 3, 1, 0).reshape(4, Cout, Cin).contiguous())
-    assert (got - ref).abs().max().item() <= _tol(ref)
+    CR.check("convg up %s" % ((B, H, W, Cin, Cout),), got, ref, S)
 
 
 def test_convg_argument_errors():
