@@ -11,7 +11,7 @@ namespace psgla {
 int check_next_pre(const psgla_next_pre* next, const psgla_img_shape& shape);
 
 // Direction in which the next layer of a denoiser walks its work items: consecutive layers alternate, so that each starts on
-// the part of its input the previous layer wrote last (still in L2).  PSGLA_CONV_ALTERNATE=0 pins it to "forward".
+// the part of its input the previous layer wrote last (still in L2).
 int next_layer_direction();
 
 // conv_tc.cu -- layers whose weights stay resident in shared memory

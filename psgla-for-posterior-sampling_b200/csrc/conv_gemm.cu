@@ -1,8 +1,8 @@
 // General convolution layers of the DRUNet denoiser as implicit GEMM on tcgen05 tensor cores (sm_100a):
 //   CG_CONV3  3x3, stride 1, zero padding 1, C -> C      (the residual blocks at 128 / 256 / 512 channels)
 //   CG_DOWN2  2x2, stride 2, no padding,     C -> 2C     (KAIR "strideconv" downsampling)
-//   CG_UP2    2x2, stride 2 transposed,      C -> C/2    (KAIR "convtranspose" upsampling; four 1x1 GEMMs, one per
-//                                                          output quadrant (dy, dx))
+//   CG_UP2    2x2, stride 2 transposed,      C -> C/2    (KAIR "convtranspose" upsampling; one 1x1 GEMM with N = 4 C/2,
+//                                                          (output quadrant (dy, dx), channel))
 // Replaces the cuDNN fp32 convolutions behind deepinv.models.DRUNet.forward (constructed at sampling_images.py:136,
 // called at restoration_algorithms.py:238); architecture restated in oracle/image_oracle.py (KAIR UNetRes).
 //
@@ -29,25 +29,19 @@ enum { CG_CONV3 = 0, CG_DOWN2 = 1, CG_UP2 = 2 };
 
 constexpr int CG_EPI_WARPS = 8;
 constexpr int CG_NACC = 2;
-constexpr int CG_NA = 4;  // TS form: A tiles resident in tensor memory (32 columns each)
 
-// TS = true: four loader warps copy every A box from shared memory into tensor memory and the MMAs take A from there
-// (an M128 x N128 x K16 MMA then costs 73 instead of 106 cycles, profiles/r01b_mma_rate.txt); needs N_TILE <= 128 so that
-// two accumulator stages and the A ring fit the 512 TMEM columns.
-template <int N_TILE, bool TS>
+// The single-CTA kernel: N tiles of 64 columns, i.e. an output channel count that is an odd multiple of 64 (3x3 and stride-2
+// convs); every wider N tile runs on the CTA pair below.
+template <int N_TILE>
 struct CgCfg {
-  static constexpr int LOADER_WARPS = TS ? 8 : 0;  // two sets of four: set s copies the k-iterations with L % 2 == s
-  static constexpr int THREADS = 64 + 32 * LOADER_WARPS + 32 * CG_EPI_WARPS;
-  static constexpr int EPI_WARP0 = 2 + LOADER_WARPS;
-  static constexpr int A_COL0 = CG_NACC * N_TILE;
-  static_assert(!TS || CG_NACC * N_TILE + CG_NA * 32 <= 512, "TS form needs room for the A ring in tensor memory");
+  static constexpr int THREADS = 64 + 32 * CG_EPI_WARPS;
   static constexpr int A_BYTES = 128 * 128;     // 128 tile pixels x 64 channels bf16
   static constexpr int B_BYTES = N_TILE * 128;  // N_TILE output channels x 64 input channels bf16
   static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
   static constexpr int NSTAGE = (196608 / STAGE_BYTES) > 8 ? 8 : (196608 / STAGE_BYTES);
   static constexpr int OFF_BAR = NSTAGE * STAGE_BYTES;
   static constexpr int SMEM_BYTES = OFF_BAR + 256 + 1024;
-  static constexpr int TMEM_COLS = TS ? 512 : ((CG_NACC * N_TILE) < 32 ? 32 : CG_NACC * N_TILE);
+  static constexpr int TMEM_COLS = (CG_NACC * N_TILE) < 32 ? 32 : CG_NACC * N_TILE;
   static_assert(SMEM_BYTES <= 232448, "exceeds the 227 KB shared memory of one CTA");
   static_assert((TMEM_COLS & (TMEM_COLS - 1)) == 0 && TMEM_COLS <= 512, "TMEM columns must be a power of two <= 512");
 };
@@ -58,7 +52,7 @@ struct CgParams {
   int Hg, Wg;      // pixel grid the M tiles cover: the output grid (CONV3, DOWN2) or the input grid (UP2)
   int Hout, Wout;  // output tensor extent
   int PX, ROWS;    // tile = PX pixels x ROWS rows (PX * ROWS <= 128)
-  int tiles_x, tiles_y, n_tiles_n, quads, n_items;
+  int tiles_x, tiles_y, n_tiles_n, n_items;
   int reverse;  // pair kernels: walk the items back to front (alternates per layer, see conv_api.cuh)
   int relu;
   const __nv_bfloat16* res1;
@@ -67,15 +61,12 @@ struct CgParams {
 };
 
 struct CgItem {
-  int b, y0, x0, n0, q;
+  int b, y0, x0, n0;
 };
 __device__ __forceinline__ CgItem cg_decode(const CgParams& p, int item) {
   CgItem c;
-  const int inner = p.quads * p.n_tiles_n;
-  const int sub = item % inner;
-  int t = item / inner;
-  c.q = sub / p.n_tiles_n;
-  c.n0 = (sub % p.n_tiles_n);
+  c.n0 = item % p.n_tiles_n;
+  int t = item / p.n_tiles_n;
   const int tx = t % p.tiles_x;
   t /= p.tiles_x;
   const int ty = t % p.tiles_y;
@@ -102,10 +93,10 @@ __device__ __forceinline__ void cg_add_bf16x8(float (&f)[8], const uint4 r) {
   }
 }
 
-template <int N_TILE, bool TS>
-__global__ void __launch_bounds__((CgCfg<N_TILE, TS>::THREADS), 1)
+template <int N_TILE>
+__global__ void __launch_bounds__((CgCfg<N_TILE>::THREADS), 1)
 conv_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_w, const CgParams p) {
-  using Cfg = CgCfg<N_TILE, TS>;
+  using Cfg = CgCfg<N_TILE>;
   constexpr int NSTAGE = Cfg::NSTAGE;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -113,9 +104,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
   uint64_t* empty = full + NSTAGE;
   uint64_t* tfull = empty + NSTAGE;
   uint64_t* tempty = tfull + CG_NACC;
-  uint64_t* afull = tempty + CG_NACC;   // TS: the A box of this k-iteration is in tensor memory
-  uint64_t* aempty = afull + CG_NA;     // TS: the MMAs that read it have completed
-  uint32_t* tmem_ptr_s = reinterpret_cast<uint32_t*>(aempty + CG_NA);
+  uint32_t* tmem_ptr_s = reinterpret_cast<uint32_t*>(tempty + CG_NACC);
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -129,10 +118,6 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
     for (int i = 0; i < CG_NACC; ++i) {
       mbar_init(&tfull[i], 1);
       mbar_init(&tempty[i], 4);
-    }
-    for (int i = 0; i < CG_NA; ++i) {
-      mbar_init(&afull[i], 4);
-      mbar_init(&aempty[i], 1);
     }
     fence_barrier_init();
   }
@@ -165,13 +150,9 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
             if (p.mode == CG_CONV3) {
               tma_load_4d(sa, &map_a, &full[slot], kb * 64, c.x0 + (t % 3) - 1, c.y0 + (t / 3) - 1, c.b);
               tma_load_3d(sb, &map_w, &full[slot], kb * 64, c.n0 * N_TILE, t);
-            } else if (p.mode == CG_DOWN2) {
-              // input viewed as {C, 2 (dx), Win/2, 2 (dy), B * Hin/2}
+            } else {  // CG_DOWN2: input viewed as {C, 2 (dx), Win/2, 2 (dy), B * Hin/2}
               tma_load_5d(sa, &map_a, &full[slot], kb * 64, t & 1, c.x0, t >> 1, c.b * (p.Hin / 2) + c.y0);
               tma_load_3d(sb, &map_w, &full[slot], kb * 64, c.n0 * N_TILE, t);
-            } else {
-              tma_load_4d(sa, &map_a, &full[slot], kb * 64, c.x0, c.y0, c.b);
-              tma_load_3d(sb, &map_w, &full[slot], kb * 64, c.n0 * N_TILE, c.q);
             }
           }
         }
@@ -189,58 +170,25 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
       tc_fence_after();
       const uint32_t d_tmem = tmem_base + acc * N_TILE;
       for (int it = 0; it < kiters; ++it, ++L) {
-        const uint32_t slot = L % NSTAGE, as = L % CG_NA;
+        const uint32_t slot = L % NSTAGE;
         mbar_wait(&full[slot], (L / NSTAGE) & 1);
-        if (TS) mbar_wait(&afull[as], (L / CG_NA) & 1);
         tc_fence_after();
         if (elect_one()) {
           const uint32_t a_lo = smem_lo + slot * (uint32_t)(Cfg::STAGE_BYTES >> 4);
           const uint32_t b_lo = a_lo + (uint32_t)(Cfg::A_BYTES >> 4);
-          const uint32_t a_t = tmem_base + Cfg::A_COL0 + as * 32u;
 #pragma unroll
-          for (int k = 0; k < 4; ++k) {
-            if (TS)
-              umma_bf16_ts(d_tmem, a_t + k * 8, ((uint64_t)DESC_HI << 32) | (b_lo + k * 2), idesc, (it | k) != 0);
-            else
-              umma_bf16(d_tmem, ((uint64_t)DESC_HI << 32) | (a_lo + k * 2), ((uint64_t)DESC_HI << 32) | (b_lo + k * 2), idesc,
-                        (it | k) != 0);
-          }
+          for (int k = 0; k < 4; ++k)
+            umma_bf16(d_tmem, ((uint64_t)DESC_HI << 32) | (a_lo + k * 2), ((uint64_t)DESC_HI << 32) | (b_lo + k * 2), idesc,
+                      (it | k) != 0);
           umma_commit(&empty[slot]);
-          if (TS) umma_commit(&aempty[as]);
           if (it == kiters - 1) umma_commit(&tfull[acc]);
         }
         __syncwarp();
       }
     }
-  } else if (TS && warp < Cfg::EPI_WARP0) {
-    // ---------------------------------------------------------------- loaders (TS): smem A box -> registers -> TMEM
-    // One pass (wait, 8 shared-memory loads, tcgen05.st, wait::st, arrive) takes longer than the 4 MMAs of a k-iteration,
-    // so two sets of four warps alternate k-iterations.
-    const int set = (warp - 2) >> 2;
-    const int q4 = warp & 3;
-    const int m = q4 * 32 + lane;
-    const uint32_t smem_addr = smem_u32(smem);
-    const uint32_t lane_taddr = tmem_base + ((uint32_t)(q4 * 32) << 16) + Cfg::A_COL0;
-    uint32_t L = 0;
-    for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
-      for (int it = 0; it < kiters; ++it, ++L) {
-        if ((int)(L & 1) != set) continue;
-        const uint32_t slot = L % NSTAGE, as = L % CG_NA;
-        mbar_wait(&full[slot], (L / NSTAGE) & 1);
-        mbar_wait(&aempty[as], ((L / CG_NA) & 1) ^ 1);
-        tc_fence_after();
-        uint32_t v[32];
-        ld_swizzled_row128(smem_addr + slot * Cfg::STAGE_BYTES, m, v);
-        tmem_st_32x32b_x32(lane_taddr + as * 32u, v);
-        tmem_st_wait();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&afull[as]);
-      }
-    }
   } else {
     // ---------------------------------------------------------------- epilogue: 2 groups x 4 warps
-    const int ew = warp - Cfg::EPI_WARP0;
+    const int ew = warp - 2;
     const int grp = ew >> 2;
     const int q4 = warp & 3;
     const int m = q4 * 32 + lane;  // tile pixel
@@ -254,12 +202,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
       const uint32_t acc = T % CG_NACC;
       const int yg = c.y0 + r, xg = c.x0 + px;
       const bool valid = (m < p.PX * p.ROWS) && yg < p.Hg && xg < p.Wg;
-      int yo = yg, xo = xg;
-      if (p.mode == CG_UP2) {
-        yo = 2 * yg + (c.q >> 1);
-        xo = 2 * xg + (c.q & 1);
-      }
-      const size_t off = (((size_t)c.b * p.Hout + yo) * p.Wout + xo) * p.Cout + (size_t)c.n0 * N_TILE;
+      const size_t off = (((size_t)c.b * p.Hout + yg) * p.Wout + xg) * p.Cout + (size_t)c.n0 * N_TILE;
       mbar_wait(&tfull[acc], (T / CG_NACC) & 1);
       tc_fence_after();
       const uint32_t taddr = tmem_base + ((uint32_t)(q4 * 32) << 16) + acc * N_TILE;
@@ -308,7 +251,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
 // CTAs (one TPC) run one M = 256 MMA per K-step on two different pixel tiles, each streaming only N_TILE / 2 rows of
 // the weights.  Both producers signal the LEADER's "stage full" barrier (cp.async.bulk.tensor.cta_group::2), the leader
 // issues, and one multicast tcgen05.commit frees the stage in both CTAs.
-// Items: item = ((m_tile_pair * inner + sub) * 2 + rank), so the two CTAs of a cluster share (n tile, quadrant) and walk
+// Items: item = ((m_tile_pair * n_tiles_n + n_tile) * 2 + rank), so the two CTAs of a cluster share the n tile and walk
 // the same (tap, k-block) sequence on M tiles 2 i and 2 i + 1; an odd M-tile count is padded with a tile at b = B, whose
 // loads are out of bounds (zero fill) and whose stores are masked.
 //
@@ -345,13 +288,10 @@ struct CgCfg2 {
 __device__ __forceinline__ CgItem cg_decode2(const CgParams& p, int item) {
   if (p.reverse) item = p.n_items - 1 - item;  // items 2i, 2i+1 swap ranks and stay one pair
   CgItem c;
-  const int inner = p.quads * p.n_tiles_n;
   const int rank = item & 1;
   const int t = item >> 1;
-  const int sub = t % inner;
-  int mt = 2 * (t / inner) + rank;
-  c.q = sub / p.n_tiles_n;
-  c.n0 = sub % p.n_tiles_n;
+  int mt = 2 * (t / p.n_tiles_n) + rank;
+  c.n0 = t % p.n_tiles_n;
   const int tx = mt % p.tiles_x;
   mt /= p.tiles_x;
   const int ty = mt % p.tiles_y;
@@ -469,9 +409,9 @@ conv_gemm2_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
             } else if (p.mode == CG_DOWN2) {
               tma_load_5d_2sm(sa, &map_a, bar, kb * 64, t & 1, c.x0, t >> 1, c.b * (p.Hin / 2) + c.y0);
               tma_load_3d_2sm(sb, &map_w, bar, kb * 64, c.n0 * N_TILE + nrow0, t);
-            } else {
+            } else {  // CG_UP2: the weights are one [4 Cout][Cin] tap
               tma_load_4d_2sm(sa, &map_a, bar, kb * 64, c.x0, c.y0, c.b);
-              tma_load_3d_2sm(sb, &map_w, bar, kb * 64, c.n0 * N_TILE + nrow0, c.q);
+              tma_load_3d_2sm(sb, &map_w, bar, kb * 64, c.n0 * N_TILE + nrow0, 0);
             }
           }
         }
@@ -550,12 +490,12 @@ conv_gemm2_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
       const bool valid = (m < p.PX * p.ROWS) && yg < p.Hg && xg < p.Wg && c.b < p.B;
       int yo = yg, xo = xg;
       if (p.mode == CG_UP2) {
-        yo = 2 * yg + (c.q >> 1);
-        xo = 2 * xg + (c.q & 1);
+        yo = 2 * yg;
+        xo = 2 * xg;
       }
       const size_t off = (((size_t)c.b * p.Hout + yo) * p.Wout + xo) * p.Cout + (size_t)c.n0 * N_TILE;
-      // merged transposed conv (quads == 1): the N axis is (quadrant, channel), a 32-column chunk lies in one quadrant
-      const bool upm = p.mode == CG_UP2 && p.quads == 1;
+      // transposed conv: the N axis is (quadrant, channel), a 32-column chunk lies in one quadrant
+      const bool upm = p.mode == CG_UP2;
       auto chunk_off = [&](int ch) -> size_t {
         if (!upm) return off + (size_t)(ch * 32);
         const int n = c.n0 * N_TILE + ch * 32;
@@ -662,13 +602,13 @@ static int cg_cached_map(CUtensorMap* map, const CgMapKey& key, int rank, const 
   return PSGLA_OK;
 }
 
-template <int N_TILE, bool TS>
+template <int N_TILE>
 static int cg_launch(const CUtensorMap& ma, const CUtensorMap& mw, const CgParams& p, cudaStream_t st) {
-  using Cfg = CgCfg<N_TILE, TS>;
+  using Cfg = CgCfg<N_TILE>;
   static std::atomic<unsigned long long> attr_done{0};  // bit d: opted in on device d (a per-device function attribute)
   const unsigned long long dev_bit = 1ull << (current_device() & 63);
   if (!(attr_done.load(std::memory_order_acquire) & dev_bit)) {
-    PSGLA_CUDA_TRY(cudaFuncSetAttribute(conv_gemm_kernel<N_TILE, TS>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+    PSGLA_CUDA_TRY(cudaFuncSetAttribute(conv_gemm_kernel<N_TILE>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
     attr_done.fetch_or(dev_bit, std::memory_order_release);
   }
   const int grid = p.n_items < num_sms() ? p.n_items : num_sms();
@@ -682,7 +622,7 @@ static int cg_launch(const CUtensorMap& ma, const CUtensorMap& mw, const CgParam
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv_gemm_kernel<N_TILE, TS>, ma, mw, p));
+  PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv_gemm_kernel<N_TILE>, ma, mw, p));
   return PSGLA_OK;
 }
 
@@ -714,7 +654,7 @@ static int cg_launch2_t(const CUtensorMap& ma, const CUtensorMap& mw, CgParams p
     mc_slot.store(max_clusters, std::memory_order_release);
   }
   const int m_tiles = p.B * p.tiles_y * p.tiles_x;
-  const int pairs = ((m_tiles + 1) / 2) * p.quads * p.n_tiles_n;
+  const int pairs = ((m_tiles + 1) / 2) * p.n_tiles_n;
   p.n_items = 2 * pairs;
   cfg.gridDim = dim3((unsigned)(2 * std::min(pairs, max_clusters)));
   PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv_gemm2_kernel<N_TILE, REUSE, RES2, WRES>, ma, mw, p));
@@ -740,7 +680,6 @@ int conv_gemm_layer(int mode, int B, int Hin, int Win, int Cin, int Cout, const 
   CgParams p{};
   p.mode = mode;
   p.taps = mode == CG_CONV3 ? 9 : (mode == CG_DOWN2 ? 4 : 1);
-  p.quads = mode == CG_UP2 ? 4 : 1;  // (1 once the pair kernel merges the quadrants into the N axis, below)
   p.kblocks = Cin / 64;
   p.B = B, p.Hin = Hin, p.Win = Win, p.Cin = Cin, p.Cout = Cout;
   p.Hg = mode == CG_DOWN2 ? Hin / 2 : Hin;
@@ -751,47 +690,20 @@ int conv_gemm_layer(int mode, int B, int Hin, int Win, int Cin, int Cout, const 
   p.ROWS = std::max(1, std::min(128 / p.PX, p.Hg));
   p.tiles_x = (p.Wg + p.PX - 1) / p.PX;
   p.tiles_y = (p.Hg + p.ROWS - 1) / p.ROWS;
-  // PSGLA_CG_MODE: 0 (default) = both operands from shared memory with the widest N tile (256 / 128 / 64); 1 = A through
-  // tensor memory with N tiles of 128 / 64.  Measured on B200 (B = 16, 256^2, profiles/r01d_drunet_breakdown.txt): the TS
-  // form is 10-40 % SLOWER here -- every k-iteration's A box is used by only 4 MMAs (292 cycles), less than the
-  // smem -> register -> TMEM latency of one loader pass, so the loaders, not the MMAs, pace the pipeline.  Kept as an
-  // experiment; it needs software-pipelined loaders to pay off.
-  static int cg_mode = -1;
-  if (cg_mode < 0) {
-    const char* e = getenv("PSGLA_CG_MODE");
-    cg_mode = e ? atoi(e) : 0;
-  }
-  const bool ts = cg_mode == 1;
-  // PSGLA_CG_PAIR=0: single-CTA kernels everywhere (A/B runs); default: the CTA-pair kernel for N tiles of 128 and 256
-  static int cg_pair = -1;
-  if (cg_pair < 0) {
-    const char* e = getenv("PSGLA_CG_PAIR");
-    cg_pair = (e && e[0] == '0') ? 0 : 1;
-  }
-  // Transposed conv on the pair kernel: ONE GEMM with N = 4 Cout -- the weights [quadrant][Cout][Cin] are a [4 Cout][Cin]
-  // matrix as they lie, the epilogue scatters column n to quadrant n / Cout -- so an A tile is loaded once instead of once per
-  // quadrant and the 128 -> 64 layer gets 256-column tiles on the CTA pair instead of 64-column ones on one CTA.
-  // PSGLA_CG_UPMERGE=0: one GEMM per quadrant (A/B runs).
-  static int cg_upmerge = -1;
-  if (cg_upmerge < 0) {
-    const char* e = getenv("PSGLA_CG_UPMERGE");
-    cg_upmerge = (e && e[0] == '0') ? 0 : 1;
-  }
-  const bool upmerge = mode == CG_UP2 && cg_pair && !ts && cg_upmerge;
-  const int n_cols = upmerge ? 4 * Cout : Cout;
-  if (upmerge) p.quads = 1;
-  const int n_tile = (!ts && n_cols % 256 == 0) ? 256 : (n_cols % 128 == 0 ? 128 : 64);
-  const bool pair = cg_pair && !ts && n_tile >= 128;
+  // The transposed conv is ONE GEMM with N = 4 Cout -- the weights [quadrant][Cout][Cin] are a [4 Cout][Cin] matrix as they
+  // lie, the epilogue scatters column n to quadrant n / Cout -- so an A tile is loaded once instead of once per quadrant, and
+  // the 128 -> 64 layer gets 256-column tiles on the CTA pair.
+  const int n_cols = mode == CG_UP2 ? 4 * Cout : Cout;
+  // The widest N tile that divides the output columns.  Tiles of 128 and 256 columns run on the CTA-pair kernel (a single
+  // CTA reaches only 0.51 / 0.68 of the tensor peak, see above); 64-column tiles, i.e. Cout an odd multiple of 64 in a 3x3 or
+  // stride-2 conv (4 Cout is always a multiple of 256), on the single-CTA kernel.
+  const int n_tile = n_cols % 256 == 0 ? 256 : (n_cols % 128 == 0 ? 128 : 64);
+  const bool pair = n_tile >= 128;
   // one 130-pixel row box for the three horizontal taps (CgCfg2<., true>): 3x3 layers with rows of >= 128 pixels
-  static int cg_reuse = -1;
-  if (cg_reuse < 0) {
-    const char* e = getenv("PSGLA_CG_REUSE");
-    cg_reuse = (e && e[0] == '0') ? 0 : 1;
-  }
-  const bool reuse = pair && cg_reuse && mode == CG_CONV3 && p.PX == 128 && p.ROWS == 1;
+  const bool reuse = pair && mode == CG_CONV3 && p.PX == 128 && p.ROWS == 1;
   p.reverse = pair ? next_layer_direction() : 0;
   p.n_tiles_n = n_cols / n_tile;
-  p.n_items = B * p.tiles_y * p.tiles_x * p.quads * p.n_tiles_n;
+  p.n_items = B * p.tiles_y * p.tiles_x * p.n_tiles_n;
   p.relu = relu;
   p.res1 = (const __nv_bfloat16*)res1;
   p.res2 = (const __nv_bfloat16*)res2;
@@ -813,26 +725,18 @@ int conv_gemm_layer(int mode, int B, int Hin, int Win, int Cin, int Cout, const 
   }
   if (rc) return rc;
   {
-    const int taps_total = upmerge ? 1 : (mode == CG_UP2 ? 4 : p.taps);
-    const cuuint64_t dims[3] = {(cuuint64_t)Cin, (cuuint64_t)n_cols, (cuuint64_t)taps_total};
+    const cuuint64_t dims[3] = {(cuuint64_t)Cin, (cuuint64_t)n_cols, (cuuint64_t)p.taps};
     const cuuint64_t strides[2] = {(cuuint64_t)Cin * 2, (cuuint64_t)n_cols * Cin * 2};
     const int box_n = pair ? n_tile / 2 : n_tile;  // a CTA of a pair streams half of the N tile
     const cuuint32_t box[3] = {64, (cuuint32_t)box_n, reuse ? 3u : 1u};
-    rc = cg_cached_map(&mw, CgMapKey{w, 3, Cin, n_cols, taps_total, box_n, reuse ? 3 : 1}, 3, dims, strides, box);
+    rc = cg_cached_map(&mw, CgMapKey{w, 3, Cin, n_cols, p.taps, box_n, reuse ? 3 : 1}, 3, dims, strides, box);
   }
   if (rc) return rc;
-  // resident weights for the 128 -> 128 channel layers (CgCfg2<128, true, true>); PSGLA_CG_WRES=0: streamed (A/B runs)
-  static int cg_wres = -1;
-  if (cg_wres < 0) {
-    const char* e = getenv("PSGLA_CG_WRES");
-    cg_wres = (e && e[0] == '0') ? 0 : 1;
-  }
-  if (reuse && cg_wres && Cin == 128 && Cout == 128) return cg_launch2<128, true, true>(ma, mw, p, st);
+  // resident weights for the 128 -> 128 channel layers (CgCfg2<128, true, true>)
+  if (reuse && Cin == 128 && Cout == 128) return cg_launch2<128, true, true>(ma, mw, p, st);
   if (reuse) return n_tile == 256 ? cg_launch2<256, true>(ma, mw, p, st) : cg_launch2<128, true>(ma, mw, p, st);
   if (pair) return n_tile == 256 ? cg_launch2<256, false>(ma, mw, p, st) : cg_launch2<128, false>(ma, mw, p, st);
-  if (n_tile == 256) return cg_launch<256, false>(ma, mw, p, st);
-  if (n_tile == 128) return ts ? cg_launch<128, true>(ma, mw, p, st) : cg_launch<128, false>(ma, mw, p, st);
-  return ts ? cg_launch<64, true>(ma, mw, p, st) : cg_launch<64, false>(ma, mw, p, st);
+  return cg_launch<64>(ma, mw, p, st);
 }
 
 }  // namespace psgla

@@ -6,17 +6,16 @@
 //
 // GEMM view per 128-pixel output row segment:  D[128 x NOUT] = sum over 9 taps  A_tap[128 x CIN] * W_tap[NOUT x CIN]^T.
 // A work item is a (chain, 128-pixel strip, block of R rows); every input row (130 pixels = 128 + halo, TMA out-of-bounds
-// zero fill = the convolution's padding) is loaded ONCE and serves the three output rows around it.  Kernels in this file:
-//   conv3x3_kernel<CIN,NOUT,EPI>   SS form: A_tap = window into the shared-memory row ring (tap dx = descriptor start + dx rows,
-//                                  tap dy = ring slot).  Used for the 3(16)-channel first layer; A/B variant for 64 channels.
-//   conv3x3_ts_kernel<NOUT,EPI>    TS form: four loader warps copy each row into TENSOR MEMORY three times (shifted by dx) and
-//                                  the MMAs take A from there (N/2 instead of 32 + N/4 cycles per MMA at N = 64).  Last layer
-//                                  (NOUT = 16, fused Langevin post / next pre epilogue); single-CTA form of the hidden layers.
+// zero fill = the convolution's padding) is loaded ONCE and serves the three output rows around it.  One kernel per layer role:
+//   conv3x3_kernel<16,64>          the first layer (3, padded to 16, -> 64 channels).  SS form: A_tap = window into the
+//                                  shared-memory row ring (tap dx = descriptor start + dx rows, tap dy = ring slot).
+//   conv3x3_ts_kernel<16>          the last layer (64 -> 3, padded to 16, fused Langevin post / next pre epilogue).  TS form:
+//                                  four loader warps copy each row into TENSOR MEMORY three times (shifted by dx) and the MMAs
+//                                  take A from there (N/2 instead of 32 + N/4 cycles per MMA at N = 64).
 //   conv3x3_ts2_kernel<NOUT,RES>   the hidden layers: a CTA PAIR (cta_group::2, M = 256) on two adjacent strips, weights split
 //                                  32 / 32 output channels between the two shared memories; RES = 0 plain (no residual code in
 //                                  the epilogue at all), 1 = residual input by TMA, 2 = and a second one (U-Net skip tensor).
-//   (conv_fused2.cu: two hidden layers per launch when the work is a single wave of pairs; experiments.cu: the 18-layer
-//   persistent chain kernel with a grid barrier, off by default.)
+//   (conv_fused2.cu: two hidden layers per launch when the work is a single wave of pairs.)
 // Warp roles: warp 0 = TMA producer, warp 1 = MMA issuer (+ TMEM alloc), [warps 2..5 = loaders (TS forms)], 8 epilogue warps
 // in two groups (TMEM -> bias / residual / ReLU -> bf16 -> swizzled staging box -> TMA store; or the fused Langevin step,
 // restoration_algorithms.py:238-262, for the last layer).  Consecutive layers walk their items in opposite directions
@@ -36,10 +35,10 @@ namespace psgla {
 using namespace sm100;
 
 // ------------------------------------------------------------------------------------------------ SS kernel (A from smem)
-template <int CIN, int NOUT, int EPI>
+template <int CIN, int NOUT>
 __global__ void __launch_bounds__(CONV_THREADS, 1)
 conv3x3_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_out, const ConvParams p) {
-  using Cfg = ConvCfg<CIN, NOUT, EPI>;
+  using Cfg = ConvCfg<CIN, NOUT>;
   constexpr int NSTAGE = Cfg::NSTAGE;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -161,13 +160,8 @@ conv3x3_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__
   } else {
     // ------------------------------------------------------------------ epilogue: 2 groups x 4 warps
     const int ew = warp - 2;
-    uint32_t T = 0;
-    if (EPI == EPI_HIDDEN)
-      epilogue_hidden<NOUT, NACC, true, CIN != 16>(p, &tmap_out, smem + Cfg::OFF_STAGE + ew * Cfg::STAGE_BYTES, bias_s, tfull,
-                                                   tempty, tmem_base, ew >> 2, warp & 3, lane, T, 0,
-                                                   Cfg::STAGE_BUFS);  // the 3-channel first layers have no residual input
-    else
-      epilogue_post<NOUT, NACC>(p, bias_s, tfull, tempty, tmem_base, ew >> 2, warp & 3, lane);
+    epilogue_hidden<NOUT, NACC>(p, &tmap_out, smem + Cfg::OFF_STAGE + ew * Cfg::STAGE_BYTES, bias_s, tfull, tempty, tmem_base,
+                                ew >> 2, warp & 3, lane);
   }
   tc_fence_before();
   __syncthreads();
@@ -177,10 +171,10 @@ conv3x3_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__
   }
 }
 
-template <int NOUT, int EPI>
+template <int NOUT>
 __global__ void __launch_bounds__(TS_THREADS, 1)
-conv3x3_ts_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_out, const ConvParams p) {
-  using Cfg = ConvTsCfg<NOUT, EPI>;
+conv3x3_ts_kernel(const __grid_constant__ CUtensorMap tmap, const ConvParams p) {
+  using Cfg = ConvTsCfg<NOUT>;
   constexpr int NST = Cfg::NSTAGE;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -329,12 +323,7 @@ conv3x3_ts_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
   } else {
     // ---------------------------------------------------------------- epilogue: 2 groups x 4 warps
     const int ew = warp - 6;
-    uint32_t T = 0;
-    if (EPI == EPI_HIDDEN)
-      epilogue_hidden<NOUT, TS_NACC>(p, &tmap_out, smem + Cfg::OFF_STAGE + ew * Cfg::STAGE_BYTES, bias_s, tfull, tempty,
-                                     tmem_base, ew >> 2, warp & 3, lane, T, 0, Cfg::STAGE_BUFS);
-    else
-      epilogue_post<NOUT, TS_NACC>(p, bias_s, tfull, tempty, tmem_base, ew >> 2, warp & 3, lane);
+    epilogue_post<NOUT, TS_NACC>(p, bias_s, tfull, tempty, tmem_base, ew >> 2, warp & 3, lane);
   }
   tc_fence_before();
   __syncthreads();
@@ -473,101 +462,53 @@ conv3x3_ts2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
       mbar_wait(wbar, 0);
       mbar_wait_cluster(wready, 0);
       tc_fence_after();
-      if (p.lean_issue) {
-        // ONE thread runs the whole issue loop, barrier waits included: the tensor pipe's queue is shallow, so whatever the
-        // issuing thread executes between two MMAs beyond a few dozen cycles is a bubble in the pipe (the warp-uniform wait /
-        // elect / syncwarp boundary below costs ~160 cycles per row: conv_fused2.cu has the measurement).  A source row is
-        // awaited right before the first 12 MMAs that read it.
-        if (elect_one()) {
-          uint32_t L0 = 0, T = 0;
-#pragma unroll 1
-          for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
-            const ItemCoord c = decode_item(p, item);
-            int waited = 0;
-            const int ylast = c.y0 + c.rcur - 1;
-#pragma unroll 1
-            for (int y = c.y0; y <= ylast; ++y, ++T) {
-              const uint32_t acc = T % TS_NACC;
-              mbar_wait_spin(&tempty[acc], ((T / TS_NACC) & 1) ^ 1);
-              const uint32_t d_tmem = tmem_base + acc * NOUT;
-              uint32_t accumulate = 0;
-#pragma unroll
-              for (int dy = 0; dy < 3; ++dy) {
-                const int yy = y + dy - 1;
-                if (yy < 0 || yy >= p.H) continue;
-                const int rel = yy - c.ylo;
-                const uint32_t q = L0 + (uint32_t)rel;
-                if (rel == waited) {
-                  mbar_wait_spin(&afull[q % TS_NA], (q / TS_NA) & 1);
-                  ++waited;
-                }
-                tc_fence_after();
-                const uint32_t a_t = tmem_base + TS_A_COL0 + (q % TS_NA) * 96u;
-#pragma unroll
-                for (int dx = 0; dx < 3; ++dx) {
-#pragma unroll
-                  for (int k = 0; k < 4; ++k) {
-                    const uint32_t bl = w_lo + (uint32_t)(((dy * 3 + dx) * Cfg::TAP_BYTES + k * 32) >> 4);
-                    umma_bf16_ts2(d_tmem, a_t + dx * 32 + k * 8, ((uint64_t)DESC_HI << 32) | bl, idesc, accumulate | (uint32_t)(dx | k));
-                  }
-                }
-                accumulate = 1;
-                if ((dy == 0 && y - 1 >= c.ylo) || y == ylast) umma_commit2(&aempty[q % TS_NA], 3);
-              }
-              umma_commit2(&tfull[acc], 3);
-            }
-            L0 += (uint32_t)(c.yhi - c.ylo + 1);
-          }
-          umma_commit2(done, 3);
-        }
-        __syncwarp();
-      } else {
+      // ONE thread runs the whole issue loop, barrier waits included: the tensor pipe's queue is shallow, so whatever the
+      // issuing thread executes between two MMAs beyond a few dozen cycles is a bubble in the pipe (a warp-uniform wait /
+      // elect / syncwarp boundary per row cost ~160 cycles: conv_fused2.cu has the measurement).  A source row is awaited
+      // right before the first 12 MMAs that read it.
+      if (elect_one()) {
         uint32_t L0 = 0, T = 0;
+#pragma unroll 1
         for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
           const ItemCoord c = decode_item(p, item);
           int waited = 0;
           const int ylast = c.y0 + c.rcur - 1;
+#pragma unroll 1
           for (int y = c.y0; y <= ylast; ++y, ++T) {
-            const int need = min(y + 1, c.yhi) - c.ylo + 1;
-            while (waited < need) {
-              const uint32_t q = L0 + waited;
-              mbar_wait(&afull[q % TS_NA], (q / TS_NA) & 1);
-              ++waited;
-            }
             const uint32_t acc = T % TS_NACC;
-            mbar_wait(&tempty[acc], ((T / TS_NACC) & 1) ^ 1);
-            tc_fence_after();
+            mbar_wait_spin(&tempty[acc], ((T / TS_NACC) & 1) ^ 1);
             const uint32_t d_tmem = tmem_base + acc * NOUT;
-            if (elect_one()) {
-              uint32_t accumulate = 0;
+            uint32_t accumulate = 0;
 #pragma unroll
-              for (int dy = 0; dy < 3; ++dy) {
-                const int yy = y + dy - 1;
-                if (yy < 0 || yy >= p.H) continue;
-                const uint32_t q = L0 + (uint32_t)(yy - c.ylo);
-                const uint32_t a_t = tmem_base + TS_A_COL0 + (q % TS_NA) * 96u;
-#pragma unroll
-                for (int dx = 0; dx < 3; ++dx) {
-#pragma unroll
-                  for (int k = 0; k < 4; ++k) {
-                    const uint32_t bl = w_lo + (uint32_t)(((dy * 3 + dx) * Cfg::TAP_BYTES + k * 32) >> 4);
-                    umma_bf16_ts2(d_tmem, a_t + dx * 32 + k * 8, ((uint64_t)DESC_HI << 32) | bl, idesc, accumulate);
-                    accumulate = 1;
-                  }
-                }
-                if (dy == 0 && y - 1 >= c.ylo) umma_commit2(&aempty[(L0 + (uint32_t)(y - 1 - c.ylo)) % TS_NA], 3);
+            for (int dy = 0; dy < 3; ++dy) {
+              const int yy = y + dy - 1;
+              if (yy < 0 || yy >= p.H) continue;
+              const int rel = yy - c.ylo;
+              const uint32_t q = L0 + (uint32_t)rel;
+              if (rel == waited) {
+                mbar_wait_spin(&afull[q % TS_NA], (q / TS_NA) & 1);
+                ++waited;
               }
-              umma_commit2(&tfull[acc], 3);
-              if (y == ylast)
-                for (int yy = y; yy <= c.yhi; ++yy) umma_commit2(&aempty[(L0 + (uint32_t)(yy - c.ylo)) % TS_NA], 3);
+              tc_fence_after();
+              const uint32_t a_t = tmem_base + TS_A_COL0 + (q % TS_NA) * 96u;
+#pragma unroll
+              for (int dx = 0; dx < 3; ++dx) {
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                  const uint32_t bl = w_lo + (uint32_t)(((dy * 3 + dx) * Cfg::TAP_BYTES + k * 32) >> 4);
+                  umma_bf16_ts2(d_tmem, a_t + dx * 32 + k * 8, ((uint64_t)DESC_HI << 32) | bl, idesc, accumulate | (uint32_t)(dx | k));
+                }
+              }
+              accumulate = 1;
+              if ((dy == 0 && y - 1 >= c.ylo) || y == ylast) umma_commit2(&aempty[q % TS_NA], 3);
             }
-            __syncwarp();
+            umma_commit2(&tfull[acc], 3);
           }
           L0 += (uint32_t)(c.yhi - c.ylo + 1);
         }
-        if (elect_one()) umma_commit2(done, 3);
-        __syncwarp();
+        umma_commit2(done, 3);
       }
+      __syncwarp();
     }
     mbar_wait(done, 0);  // both CTAs: no MMA still reads this CTA's shared / tensor memory, no commit is still in flight
   } else if (warp < 6) {
@@ -605,13 +546,12 @@ conv3x3_ts2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
   } else {
     // ---------------------------------------------------------------- epilogue: 2 groups x 4 warps
     const int ew = warp - 6;
-    uint32_t T = 0;
     if (RES)
       epilogue_hidden_tmares<NOUT, TS_NACC, RES == 2>(p, &tmap_out, &tmap_res, smem + Cfg::OFF_STAGE + ew * Cfg::STAGE_BYTES,
                                             rbar + 2 * ew, bias_s, tfull, tempty, tmem_base, ew >> 2, warp & 3, lane, tempty_c);
     else
-      epilogue_hidden<NOUT, TS_NACC, true, false>(p, &tmap_out, smem + Cfg::OFF_STAGE + ew * Cfg::STAGE_BYTES, bias_s, tfull, tempty,
-                                                  tmem_base, ew >> 2, warp & 3, lane, T, tempty_c, Cfg::STAGE_BUFS);
+      epilogue_hidden<NOUT, TS_NACC>(p, &tmap_out, smem + Cfg::OFF_STAGE + ew * Cfg::STAGE_BYTES, bias_s, tfull, tempty,
+                                     tmem_base, ew >> 2, warp & 3, lane, tempty_c);
   }
   tc_fence_before();
   cluster_sync();  // neither CTA may exit (or free tensor memory) while its partner can still signal or read it
@@ -672,7 +612,7 @@ int get_act_tensor_map(CUtensorMap* map, const void* ptr, int B, int H, int W, i
 // Work items = (chain, 128-pixel strip, block of R output rows), dealt round-robin to one persistent CTA per SM.
 // R trades the 2 halo rows an item re-reads against the tail when items do not divide by the CTA count:
 // pick the R that minimises (items per CTA) * (R + 1).
-void plan_items(ConvParams* p) {
+static void plan_items(ConvParams* p) {
   p->strips = (p->W + TILE_M - 1) / TILE_M;
   const int sms = num_sms();
   int best = 1;
@@ -693,22 +633,18 @@ void plan_items(ConvParams* p) {
   p->n_items = p->B * p->strips * p->row_blocks;
 }
 
-template <int CIN, int NOUT, int EPI>
-static int launch_conv(const void* in, void* out_bf16, ConvParams p, cudaStream_t st) {
-  using Cfg = ConvCfg<CIN, NOUT, EPI>;
+// The first layer: bf16 NHWC16 input (3 channels padded to 16) -> bf16 NHWC 64-channel output
+static int launch_first(const void* in, void* out_bf16, ConvParams p, cudaStream_t st) {
+  using Cfg = ConvCfg<16, 64>;
   CUtensorMap map, map_out;
-  int rc = get_act_tensor_map(&map, in, p.B, p.H, p.W, CIN, BOX_W);
+  int rc = get_act_tensor_map(&map, in, p.B, p.H, p.W, 16, BOX_W);
   if (rc) return rc;
-  if (EPI == EPI_HIDDEN) {
-    rc = get_act_tensor_map(&map_out, out_bf16, p.B, p.H, p.W, NOUT, 32);
-    if (rc) return rc;
-  } else {
-    map_out = map;  // unused by the fused-post epilogue
-  }
+  rc = get_act_tensor_map(&map_out, out_bf16, p.B, p.H, p.W, 64, 32);
+  if (rc) return rc;
   static std::atomic<unsigned long long> attr_done{0};  // bit d: opted in on device d (a per-device function attribute)
   const unsigned long long dev_bit = 1ull << (current_device() & 63);
   if (!(attr_done.load(std::memory_order_acquire) & dev_bit)) {
-    PSGLA_CUDA_TRY(cudaFuncSetAttribute(conv3x3_kernel<CIN, NOUT, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    PSGLA_CUDA_TRY(cudaFuncSetAttribute(conv3x3_kernel<16, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                         Cfg::SMEM_BYTES));
     attr_done.fetch_or(dev_bit, std::memory_order_release);
   }
@@ -724,26 +660,20 @@ static int launch_conv(const void* in, void* out_bf16, ConvParams p, cudaStream_
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv3x3_kernel<CIN, NOUT, EPI>, map, map_out, p));
+  PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv3x3_kernel<16, 64>, map, map_out, p));
   return PSGLA_OK;
 }
 
-template <int NOUT, int EPI>
-static int launch_conv_ts(const void* in, void* out_bf16, ConvParams p, cudaStream_t st) {
-  using Cfg = ConvTsCfg<NOUT, EPI>;
-  CUtensorMap map, map_out;
+// The last layer: bf16 NHWC 64-channel input -> the fused Langevin post epilogue (fp32 NCHW outputs named in p)
+static int launch_last(const void* in, ConvParams p, cudaStream_t st) {
+  using Cfg = ConvTsCfg<16>;
+  CUtensorMap map;
   int rc = get_act_tensor_map(&map, in, p.B, p.H, p.W, 64, BOX_W);
   if (rc) return rc;
-  if (EPI == EPI_HIDDEN) {
-    rc = get_act_tensor_map(&map_out, out_bf16, p.B, p.H, p.W, NOUT, 32);
-    if (rc) return rc;
-  } else {
-    map_out = map;
-  }
   static std::atomic<unsigned long long> attr_done{0};  // bit d: opted in on device d (a per-device function attribute)
   const unsigned long long dev_bit = 1ull << (current_device() & 63);
   if (!(attr_done.load(std::memory_order_acquire) & dev_bit)) {
-    PSGLA_CUDA_TRY(cudaFuncSetAttribute(conv3x3_ts_kernel<NOUT, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    PSGLA_CUDA_TRY(cudaFuncSetAttribute(conv3x3_ts_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                         Cfg::SMEM_BYTES));
     attr_done.fetch_or(dev_bit, std::memory_order_release);
   }
@@ -759,12 +689,10 @@ static int launch_conv_ts(const void* in, void* out_bf16, ConvParams p, cudaStre
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv3x3_ts_kernel<NOUT, EPI>, map, map_out, p));
+  PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv3x3_ts_kernel<16>, map, p));
   return PSGLA_OK;
 }
 
-// A-operand source of the 64-input-channel layers: tensor memory (default) or shared memory (PSGLA_CONV_SS=1, kept for
-// A/B measurements and as the path of the 3-channel first layer).
 // Work items of the pair kernel: (chain, row block, strip) with the strip count padded to even and the strip index
 // fastest, so that items 2i and 2i + 1 -- the two CTAs of a cluster -- share chain and rows.
 static void plan_items_pair(ConvParams* p, int n_clusters) {
@@ -827,15 +755,6 @@ static int launch_conv_ts2_t(const void* in, void* out_bf16, ConvParams p, cudaS
     if (getenv("PSGLA_VERBOSE")) fprintf(stderr, "psgla_b200: conv3x3_ts2_kernel: %d co-resident CTA pairs (occupancy query %d)\n", max_clusters, n);
   }
   plan_items_pair(&p, max_clusters);
-  {
-    // PSGLA_CONV_ISSUE=0: the warp-uniform issue loop (A/B runs); default: the single-thread one
-    static int lean = -1;
-    if (lean < 0) {
-      const char* e = getenv("PSGLA_CONV_ISSUE");
-      lean = (e && e[0] == '0') ? 0 : 1;
-    }
-    p.lean_issue = lean;
-  }
   const int pairs = p.n_items / 2;
   cfg.gridDim = dim3((unsigned)(2 * std::min(pairs, max_clusters)));
   if (getenv("PSGLA_VERBOSE")) fprintf(stderr, "psgla_b200: pair conv B=%d H=%d W=%d: R=%d items=%d grid=%u\n", p.B, p.H, p.W, p.R, p.n_items, cfg.gridDim.x);
@@ -843,48 +762,10 @@ static int launch_conv_ts2_t(const void* in, void* out_bf16, ConvParams p, cudaS
   return PSGLA_OK;
 }
 
-template <int NOUT>
-static int launch_conv_ts2(const void* in, void* out_bf16, const ConvParams& p, cudaStream_t st) {
-  if (!p.res1) return launch_conv_ts2_t<NOUT, 0>(in, out_bf16, p, st);
-  return p.res2 ? launch_conv_ts2_t<NOUT, 2>(in, out_bf16, p, st) : launch_conv_ts2_t<NOUT, 1>(in, out_bf16, p, st);
-}
-
-// PSGLA_CONV_PAIR=0 falls back to the single-CTA TS kernel (A/B runs)
-static bool conv_use_pair() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("PSGLA_CONV_PAIR");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v != 0;
-}
-
-static bool conv_use_ts() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("PSGLA_CONV_SS");
-    v = (e && atoi(e) != 0) ? 0 : 1;
-  }
-  return v == 1;
-}
+// The hidden 64 -> 64 channel layers, with up to two residual inputs
 static int launch_hidden64(const void* in, void* out, const ConvParams& p, cudaStream_t st) {
-  if (!conv_use_ts()) return launch_conv<64, 64, EPI_HIDDEN>(in, out, p, st);
-  return conv_use_pair() ? launch_conv_ts2<64>(in, out, p, st) : launch_conv_ts<64, EPI_HIDDEN>(in, out, p, st);
-}
-static int launch_last(const void* in, const ConvParams& p, cudaStream_t st) {
-  return conv_use_ts() ? launch_conv_ts<16, EPI_POST>(in, nullptr, p, st) : launch_conv<64, 16, EPI_POST>(in, nullptr, p, st);
-}
-
-// Measured on B200 (1-16 chains of 256 x 256): the chain is NOT faster than the per-layer launches (181.7 vs 187.8 us per
-// DnCNN application at one chain in round 1; 174.6 vs 176.9 us in round 2, and 8-20 % SLOWER at 4-16 chains).  Round 2 also
-// tried replacing the grid barrier by per-item flags (an item waits only for the <= 9 items whose rows / halo pixels it
-// reads): 224 us -- the acquire-polls of the neighbours' flags cost more than the barrier's single counter.  A layer's ~8 us at that size is pipeline fill and drain inside the CTA -- TMA load
-// latency, three rows through the loader warps before the first MMA, the last row's epilogue and store -- not launch
-// overhead, which PDL already overlaps; the grid barrier costs what the kernel boundary cost.  The kernel stays as a
-// tested alternative (PSGLA_CHAIN=1) and as the base for keeping a CTA's own rows on chip between layers.
-static bool use_chain(const ConvParams&) {
-  const char* e = getenv("PSGLA_CHAIN");  // read per call: tests and A/B scripts switch it inside one process
-  return conv_use_ts() && e && atoi(e) == 1;
+  if (!p.res1) return launch_conv_ts2_t<64, 0>(in, out, p, st);
+  return p.res2 ? launch_conv_ts2_t<64, 2>(in, out, p, st) : launch_conv_ts2_t<64, 1>(in, out, p, st);
 }
 
 // ---- packed weight layout: per layer [weights (9 taps, swizzled) | bias fp32], each layer 1024 B aligned
@@ -948,24 +829,14 @@ extern "C" int psgla_dncnn_pack_weights(int depth, const float* const* weights_h
 }
 
 extern "C" size_t psgla_dncnn_workspace_bytes(psgla_img_shape s) {
-  // two ping-pong activation buffers (each rounded up to 1 KB) + 4 KB holding the layer-chain kernel's barrier / item flags
-  return 2 * (((size_t)s.B * s.H * s.W * 64 * 2 + 1023) / 1024 * 1024) + 4096 + 1024;
+  // two ping-pong activation buffers, each rounded up to 1 KB
+  return 2 * (((size_t)s.B * s.H * s.W * 64 * 2 + 1023) / 1024 * 1024);
 }
 
 static int check_shape(const psgla_img_shape& s) {
   PSGLA_REQUIRE(s.B > 0 && s.H > 0 && s.W > 0 && s.C == 3, "image shape must be [B>0][3][H>0][W>0], got [%d][%d][%d][%d]",
                 s.B, s.C, s.H, s.W);
   return PSGLA_OK;
-}
-
-// PSGLA_CONV_ALTERNATE=0: every layer walks its items front to back (A/B runs)
-static bool alternate_items() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("PSGLA_CONV_ALTERNATE");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v != 0;
 }
 
 static ConvParams base_params(const psgla_img_shape& s, const uint8_t* packed, const LayerInfo& li) {
@@ -993,7 +864,7 @@ static int last_layer_post(int depth, const uint8_t* packed, const psgla_img_sha
   p.base_scale = 1.0f;  // DnCNN is a residual denoiser: X+ = base + gain * R
   p.w_old = post->w_old;
   p.w_new = post->w_new;
-  p.reverse = alternate_items() ? ((depth - 1) & 1) : 0;
+  p.reverse = (depth - 1) & 1;
   int rc = set_next_pre(&p, next);
   if (rc) return rc;
   return launch_last(hidden, p, st);
@@ -1013,7 +884,7 @@ extern "C" int psgla_conv3x3_layer(const void* packed_dev, int depth, int layer,
     p.x_out = (float*)out_dev;
     return launch_last(in_dev, p, st);
   }
-  return layer == 0 ? launch_conv<16, 64, EPI_HIDDEN>(in_dev, out_dev, p, st) : launch_hidden64(in_dev, out_dev, p, st);
+  return layer == 0 ? launch_first(in_dev, out_dev, p, st) : launch_hidden64(in_dev, out_dev, p, st);
 }
 
 extern "C" int psgla_dncnn_residual_post(int depth, const void* packed_dev, psgla_img_shape shape,
@@ -1046,46 +917,31 @@ extern "C" int psgla_dncnn_residual_post_next(int depth, const void* packed_dev,
   uint8_t* ws[2] = {(uint8_t*)workspace_dev, (uint8_t*)workspace_dev + half};
   const uint8_t* packed = (const uint8_t*)packed_dev;
   const void* cur = den_in_dev;
-  {
-    ConvParams p = base_params(shape, packed, layer_info(depth, 0));
-    if (depth > 3 && use_chain(p)) {
-      // first layer, then all hidden layers in one persistent launch
-      p.relu = 1;
-      rc = launch_conv<16, 64, EPI_HIDDEN>(cur, ws[0], p, st);
+  int wsel = 0;  // the buffer the next layer writes
+  for (int l = 0; l < depth - 1; ++l) {
+    const LayerInfo li = layer_info(depth, l);
+    if (l >= 1 && l + 1 < depth - 1) {
+      // few chains: two hidden layers per launch (conv_fused2.cu), the intermediate rows never leave the SM pair
+      const LayerInfo l2 = layer_info(depth, l + 1);
+      int fused = 0;
+      rc = conv64_hidden_fused2(cur, ws[wsel], packed + li.w_off, reinterpret_cast<const float*>(packed + li.b_off),
+                                packed + l2.w_off, reinterpret_cast<const float*>(packed + l2.b_off), shape.B, shape.H, shape.W,
+                                &fused, st);
       if (rc) return rc;
-      const LayerInfo l1 = layer_info(depth, 1);
-      unsigned int* barrier = reinterpret_cast<unsigned int*>((uint8_t*)workspace_dev + 2 * half);
-      rc = launch_hidden_chain(ws[0], ws[1], depth - 2, packed + l1.w_off, barrier, base_params(shape, packed, l1), st);
-      if (rc) return rc;
-      cur = ws[(depth - 2) & 1];
-    } else {
-      int wsel = 0;  // the buffer the next layer writes
-      for (int l = 0; l < depth - 1; ++l) {
-        const LayerInfo li = layer_info(depth, l);
-        if (l >= 1 && l + 1 < depth - 1 && conv_use_ts() && conv_use_pair()) {
-          // few chains: two hidden layers per launch (conv_fused2.cu), the intermediate rows never leave the SM pair
-          const LayerInfo l2 = layer_info(depth, l + 1);
-          int fused = 0;
-          rc = conv64_hidden_fused2(cur, ws[wsel], packed + li.w_off, reinterpret_cast<const float*>(packed + li.b_off),
-                                    packed + l2.w_off, reinterpret_cast<const float*>(packed + l2.b_off), shape.B, shape.H, shape.W,
-                                    &fused, st);
-          if (rc) return rc;
-          if (fused) {
-            cur = ws[wsel];
-            wsel ^= 1;
-            ++l;
-            continue;
-          }
-        }
-        ConvParams pl = base_params(shape, packed, li);
-        pl.relu = 1;
-        pl.reverse = alternate_items() ? (l & 1) : 0;
-        rc = (l == 0) ? launch_conv<16, 64, EPI_HIDDEN>(cur, ws[wsel], pl, st) : launch_hidden64(cur, ws[wsel], pl, st);
-        if (rc) return rc;
+      if (fused) {
         cur = ws[wsel];
         wsel ^= 1;
+        ++l;
+        continue;
       }
     }
+    ConvParams pl = base_params(shape, packed, li);
+    pl.relu = 1;
+    pl.reverse = l & 1;
+    rc = (l == 0) ? launch_first(cur, ws[wsel], pl, st) : launch_hidden64(cur, ws[wsel], pl, st);
+    if (rc) return rc;
+    cur = ws[wsel];
+    wsel ^= 1;
   }
   return last_layer_post(depth, packed, shape, cur, base_dev, post, x_out_dev, sample_dev, mean_dev, mean2_dev, next, st);
 }
@@ -1127,7 +983,6 @@ void pack_conv3x3_swizzled(const float* w, int nout_real, int cin_real, int nout
 
 int next_layer_direction() {
   static thread_local int dir = 0;
-  if (!alternate_items()) return 0;
   dir ^= 1;
   return dir;
 }
@@ -1152,7 +1007,7 @@ int conv_first16(const void* in16, void* out, const uint8_t* w, const float* bia
   p.weights = w;
   p.bias = bias;
   p.relu = relu;
-  return launch_conv<16, 64, EPI_HIDDEN>(in16, out, p, st);
+  return launch_first(in16, out, p, st);
 }
 
 int check_next_pre(const psgla_next_pre* next, const psgla_img_shape& s) {

@@ -1,5 +1,5 @@
-// Shared device code of the resident-weight 3x3 convolution kernels (conv_tc.cu: the production kernels; experiments.cu: the
-// persistent layer-chain experiment): configurations, the parameter block, work-item decoding, the epilogues.
+// Shared device code of the resident-weight 3x3 convolution kernels (conv_tc.cu: one kernel per layer role; conv_fused2.cu:
+// two hidden layers per launch): configurations, the parameter block, work-item decoding, the epilogues.
 #pragma once
 #include <cuda_bf16.h>
 
@@ -16,14 +16,11 @@ using namespace sm100;
 
 constexpr int TILE_M = 128;
 constexpr int BOX_W = TILE_M + 2;
-constexpr int NSTAGE_64 = 6;   // input-row ring slots, 64-channel rows (17 KB each); 16-channel rows: ConvCfg::NSTAGE
 constexpr int NACC = 4;       // TMEM accumulator stages; stage s is drained by epilogue group s & 1
 constexpr int EPI_WARPS = 8;  // two groups of four warps (one warp per TMEM lane quarter)
 constexpr int CONV_THREADS = 64 + 32 * EPI_WARPS;
 
 constexpr int round_up_c(int v, int a) { return (v + a - 1) / a * a; }
-
-enum { EPI_HIDDEN = 0, EPI_POST = 2 };
 
 // f[0..7] += eight bf16 values packed in a 16-byte vector
 __device__ __forceinline__ void add_bf16x8(float (&f)[8], const uint4 r) {
@@ -38,44 +35,38 @@ __device__ __forceinline__ void add_bf16x8(float (&f)[8], const uint4 r) {
 // The 8 biases of 16-byte output chunk j.  The epilogues fetch them ONE CHUNK AHEAD with explicit shared-space loads: through a
 // generic pointer they compile to LD.E, and placed after the previous chunk's staging store (a "memory"-clobbering asm
 // statement keeps program order) every chunk paid a long-scoreboard round trip -- the first layer, whose epilogue is its
-// critical path, ran at 1 240 cycles per row (profiles/r02_first_last_layer_full.txt).  SMEM = false: bias in global memory
-// (the layer-chain experiment).
+// critical path, ran at 1 240 cycles per row (profiles/r02_first_last_layer_full.txt).
 struct BiasPair {
   float4 b0, b1;
 };
-template <bool SMEM>
-__device__ __forceinline__ BiasPair load_bias_pair(const float* bias, uint32_t bias_saddr, int j) {
+__device__ __forceinline__ BiasPair load_bias_pair(uint32_t bias_saddr, int j) {
   BiasPair r;
-  if (SMEM) {
-    r.b0 = ld_shared_f4_nc(bias_saddr + 32u * (uint32_t)j);
-    r.b1 = ld_shared_f4_nc(bias_saddr + 32u * (uint32_t)j + 16u);
-  } else {
-    const float4* b4 = reinterpret_cast<const float4*>(bias);
-    r.b0 = b4[2 * j];
-    r.b1 = b4[2 * j + 1];
-  }
+  r.b0 = ld_shared_f4_nc(bias_saddr + 32u * (uint32_t)j);
+  r.b1 = ld_shared_f4_nc(bias_saddr + 32u * (uint32_t)j + 16u);
   return r;
 }
 
-template <int CIN, int NOUT, int EPI>
+// The SS kernel (A from shared memory), i.e. the first layer: 16 (3 padded) input channels, 64 output channels
+template <int CIN, int NOUT>
 struct ConvCfg {
+  static_assert(CIN == 16, "ring depth, swizzle and staging are sized for the 16-channel rows of the first layer");
   static constexpr int ROW_BYTES = CIN * 2;
   static constexpr int BOX_BYTES = BOX_W * ROW_BYTES;
   static constexpr int SLOT_BYTES = round_up_c(BOX_BYTES, 1024);
-  static constexpr uint32_t LAYOUT = (CIN == 64) ? LAYOUT_SW128 : LAYOUT_SW32;
+  static constexpr uint32_t LAYOUT = LAYOUT_SW32;
   static constexpr uint32_t SBO = 8 * ROW_BYTES;
   static constexpr int KSTEPS = CIN / 16;
   static constexpr int TAP_BYTES = NOUT * ROW_BYTES;
   static constexpr int W_BYTES = 9 * TAP_BYTES;
   static constexpr int OFF_RING = round_up_c(W_BYTES, 1024);
-  // 32-pixel output boxes per epilogue warp: two (the warp fills one while the TMA store of the previous row still reads
-  // the other) where shared memory allows, i.e. not next to 72 KB of weights and a 64-channel ring
   // Ring depth.  A slot stays occupied for three output rows, so NSTAGE - 3 rows are in flight ahead of the MMAs; the
   // 16-channel first layer consumes a row in ~430 cycles against ~2 us of TMA latency from HBM and needs a deep ring
   // (6 slots: 1 560 cycles per row measured), its rows are only 5 KB.
-  static constexpr int NSTAGE = (CIN == 16) ? 20 : NSTAGE_64;
-  static constexpr int STAGE_BUFS = (CIN == 16) ? 2 : 1;
-  static constexpr int STAGE_BYTES = (EPI == EPI_HIDDEN) ? STAGE_BUFS * 32 * NOUT * 2 : 0;
+  static constexpr int NSTAGE = 20;
+  // two 32-pixel output boxes per epilogue warp: the warp fills one while the TMA store of the previous row still reads
+  // the other
+  static constexpr int STAGE_BUFS = 2;
+  static constexpr int STAGE_BYTES = STAGE_BUFS * 32 * NOUT * 2;
   static constexpr int OFF_STAGE = OFF_RING + NSTAGE * SLOT_BYTES;
   static constexpr int OFF_BIAS = OFF_STAGE + EPI_WARPS * STAGE_BYTES;
   static constexpr int OFF_BAR = OFF_BIAS + 256;
@@ -91,21 +82,20 @@ struct ConvParams {
   int B, H, W;
   int R, strips, row_blocks, n_items;
   int reverse;  // walk the work items back to front (see decode_item)
-  int lean_issue;  // pair kernel: one thread runs the MMA issue loop incl. its barrier waits (conv_tc.cu)
   const uint8_t* weights;  // 9 taps, swizzled
   const float* bias;       // NOUT floats
   int relu;
-  // EPI_HIDDEN: optional bf16 NHWC tensors of the output's shape added before the ReLU (DRUNet residual / skip adds)
+  // hidden layers: optional bf16 NHWC tensors of the output's shape added before the ReLU (DRUNet residual / skip adds)
   const __nv_bfloat16* res1;
   const __nv_bfloat16* res2;
-  // EPI_POST
+  // last layer
   const float* base;
   float* x_out;
   float* sample;
   float* mean;
   float* mean2;
   float gain, base_scale, w_old, w_new;
-  // EPI_POST, optional: the "pre" step of the NEXT iteration applied to the iterate this epilogue produces (inpainting):
+  // last layer, optional: the "pre" step of the NEXT iteration applied to the iterate this epilogue produces (inpainting):
   // nx_base = langevin_base(X+), nx_den_in = bf16 NHWC16 of it (PSGLA) or of X+ (PnP-ULA); nx_base may alias base.
   int nx_enable;
   PreArgs nx;
@@ -155,41 +145,26 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float a, float b, bool relu) {
 // Eight epilogue warps form two groups of four (one warp per TMEM lane quarter q4); group g drains the output rows
 // with T % 2 == g, where T counts the CTA's output rows in issue order and accumulator stage = T % NACC_.
 
-// Hidden layers: TMEM -> +bias -> ReLU -> bf16 -> 128B-swizzled staging box in shared memory -> one TMA store of
-// 32 pixels x NOUT channels per warp and row (clipped at the image edge by the tensor map).
-// ALLOW_RES = false: the caller never has residual inputs (the pair kernel's plain instantiation, i.e. every hidden layer of
-// DnCNN): the per-thread residual path, a divergent branch per chunk inside the unrolled loop, is compiled out.
-template <int NOUT, int NACC_, bool BIAS_SMEM = true, bool ALLOW_RES = true>
+// Hidden layers without a residual input: TMEM -> +bias -> ReLU -> bf16 -> 128B-swizzled staging box in shared memory -> one
+// TMA store of 32 pixels x NOUT channels per warp and row (clipped at the image edge by the tensor map).  The warp alternates
+// between two staging boxes, so a row is staged while the previous row's TMA store is still reading its box (the store's
+// read latency otherwise serialises with the warp's work on every row).
+template <int NOUT, int NACC_>
 __device__ __forceinline__ void epilogue_hidden(const ConvParams& p, const CUtensorMap* tmap_out, uint8_t* stage,
                                                 const float* bias_s, uint64_t* tfull, uint64_t* tempty,
-                                                uint32_t tmem_base, int grp, int q4, int lane, uint32_t& T,
-                                                uint32_t tempty_cluster = 0, int stage_bufs = 1) {
+                                                uint32_t tmem_base, int grp, int q4, int lane, uint32_t tempty_cluster = 0) {
   // tempty_cluster != 0 (CTA-pair kernel): the accumulator-free barriers live in the leader CTA, at this cluster address.
-  // T: the CTA's running output-row counter (accumulator stage and mbarrier phase); it carries over when one kernel
-  // runs several layers back to back.  bias_s may point to shared or global memory.
-  // stage_bufs == 2: the warp alternates between two staging boxes, so a row is staged while the previous row's TMA
-  // store is still reading its box (the store's read latency otherwise serialises with the warp's work on every row)
-  uint32_t nrow = 0;
-  const uint32_t bias_sa = BIAS_SMEM ? smem_u32(bias_s) : 0u;
+  // T: the CTA's running output-row counter (accumulator stage and mbarrier phase).
+  uint32_t nrow = 0, T = 0;
+  const uint32_t bias_sa = smem_u32(bias_s);
   const bool relu = p.relu != 0;
   if (lane == 0) tma_prefetch_desc(tmap_out);
-  // the residual tensors come from earlier kernels and are now read ahead of the accumulator (i.e. before anything in this
-  // warp depends on the producer's own griddepcontrol.wait)
-  if (ALLOW_RES && p.res1 != nullptr) griddep_wait();
   for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
     const ItemCoord c = decode_item(p, item);
     const int xw = c.x0 + q4 * 32;  // first pixel of this warp's 32-pixel box
     for (int y = c.y0; y < c.y0 + c.rcur; ++y, ++T) {
       if ((int)(T & 1) != grp) continue;
       const uint32_t acc = T % NACC_;
-      // residual inputs (DRUNet) are fetched while the row's MMAs are still in flight
-      const bool has_res = ALLOW_RES && p.res1 != nullptr && xw + lane < p.W;
-      const size_t roff = (((size_t)c.b * p.H + y) * p.W + (xw + lane)) * NOUT;
-      uint4 rr[NOUT / 8];
-      if (has_res) {
-#pragma unroll
-        for (int j = 0; j < NOUT / 8; ++j) rr[j] = *reinterpret_cast<const uint4*>(p.res1 + roff + 8 * j);
-      }
       mbar_wait(&tfull[acc], (T / NACC_) & 1);
       tc_fence_after();
       const uint32_t taddr = tmem_base + ((uint32_t)(q4 * 32) << 16) + acc * NOUT;
@@ -199,33 +174,26 @@ __device__ __forceinline__ void epilogue_hidden(const ConvParams& p, const CUten
       tmem_ld_wait();
       tc_fence_before();
       // the staging box of the previous row must have been read by its TMA store before it is overwritten
-      uint8_t* stage_cur = stage + (stage_bufs == 2 ? (nrow & 1u) * (32 * NOUT * 2) : 0);
+      uint8_t* stage_cur = stage + (nrow & 1u) * (32 * NOUT * 2);
       const uint32_t stage_row = smem_u32(stage_cur) + lane * (NOUT * 2);
       ++nrow;
       if (lane == 0) {
-        if (stage_bufs == 2)
-          bulk_wait_group_read1();
-        else
-          bulk_wait_group_read0();
+        bulk_wait_group_read1();
         if (tempty_cluster)
           mbar_arrive_remote(tempty_cluster + acc * 8u);
         else
           mbar_arrive(&tempty[acc]);
       }
       __syncwarp();
-      BiasPair bp = load_bias_pair<BIAS_SMEM>(bias_s, bias_sa, 0);
+      BiasPair bp = load_bias_pair(bias_sa, 0);
 #pragma unroll
       for (int j = 0; j < NOUT / 8; ++j) {  // 16-byte chunk j = channels 8j..8j+7
         const float4 b0 = bp.b0, b1 = bp.b1;
-        if (j + 1 < NOUT / 8) bp = load_bias_pair<BIAS_SMEM>(bias_s, bias_sa, j + 1);
+        if (j + 1 < NOUT / 8) bp = load_bias_pair(bias_sa, j + 1);
         float f[8] = {__uint_as_float(v[8 * j + 0]) + b0.x, __uint_as_float(v[8 * j + 1]) + b0.y,
                       __uint_as_float(v[8 * j + 2]) + b0.z, __uint_as_float(v[8 * j + 3]) + b0.w,
                       __uint_as_float(v[8 * j + 4]) + b1.x, __uint_as_float(v[8 * j + 5]) + b1.y,
                       __uint_as_float(v[8 * j + 6]) + b1.z, __uint_as_float(v[8 * j + 7]) + b1.w};
-        if (ALLOW_RES && has_res) {
-          add_bf16x8(f, rr[j]);
-          if (p.res2) add_bf16x8(f, *reinterpret_cast<const uint4*>(p.res2 + roff + 8 * j));
-        }
         uint4 o;
         o.x = pack_bf16x2(f[0], f[1], relu);
         o.y = pack_bf16x2(f[2], f[3], relu);
@@ -242,8 +210,7 @@ __device__ __forceinline__ void epilogue_hidden(const ConvParams& p, const CUten
     }
   }
   // Before the CTA exits its stores must have READ their staging boxes; their writes are complete and visible when the grid
-  // completes, which is what a dependent launch's griddepcontrol.wait awaits.  (A kernel that publishes its rows to other CTAs
-  // of the same grid must wait for the writes itself: experiments.cu.)
+  // completes, which is what a dependent launch's griddepcontrol.wait awaits.
   if (lane == 0) bulk_wait_group_read0();
 }
 
@@ -360,11 +327,11 @@ __device__ __forceinline__ void epilogue_hidden_tmares(const ConvParams& p, cons
       else
         mbar_arrive(&tempty[acc]);
     }
-    BiasPair bp = load_bias_pair<true>(bias_s, bias_sa, 0);
+    BiasPair bp = load_bias_pair(bias_sa, 0);
 #pragma unroll
     for (int j = 0; j < NOUT / 8; ++j) {
       const float4 b0 = bp.b0, b1 = bp.b1;
-      if (j + 1 < NOUT / 8) bp = load_bias_pair<true>(bias_s, bias_sa, j + 1);
+      if (j + 1 < NOUT / 8) bp = load_bias_pair(bias_sa, j + 1);
       float f[8] = {__uint_as_float(v[8 * j + 0]) + b0.x, __uint_as_float(v[8 * j + 1]) + b0.y,
                     __uint_as_float(v[8 * j + 2]) + b0.z, __uint_as_float(v[8 * j + 3]) + b0.w,
                     __uint_as_float(v[8 * j + 4]) + b1.x, __uint_as_float(v[8 * j + 5]) + b1.y,
@@ -561,27 +528,25 @@ __device__ __forceinline__ void epilogue_post(const ConvParams& p, const float* 
 //   TMEM columns [0, NACC_TS * NOUT)            accumulators (one stage per epilogue group)
 //                [128 + s*96 + dx*32 + k*8 ...)  A ring: slot s = input row mod 4, shift dx, K-step k (8 columns = 16 bf16)
 // Warps: 0 TMA producer, 1 MMA issuer, 2-5 loaders (TMEM lane quarter = warp & 3), 6-13 epilogue (two groups).
-constexpr int TS_NSTAGE = 4;   // shared-memory staging slots of the TMA ring
 constexpr int TS_NA = 4;       // input rows resident in TMEM
 constexpr int TS_NACC = 2;
 constexpr int TS_A_COL0 = 128;
 constexpr int TS_THREADS = 64 + 128 + 32 * EPI_WARPS;
 
-template <int NOUT, int EPI>
+// The single-CTA TS kernel, i.e. the last layer: 64 input channels, 16 (3 padded) output channels, fused Langevin epilogue
+template <int NOUT>
 struct ConvTsCfg {
+  static_assert(NOUT == 16, "ring depth and shared-memory plan are sized for the last layer");
   static constexpr int ROW_BYTES = 128;
   static constexpr int BOX_BYTES = BOX_W * ROW_BYTES;
   static constexpr int SLOT_BYTES = round_up_c(BOX_BYTES, 1024);
   static constexpr int TAP_BYTES = NOUT * ROW_BYTES;
   static constexpr int W_BYTES = 9 * TAP_BYTES;
   static constexpr int OFF_RING = round_up_c(W_BYTES, 1024);
-  static constexpr int STAGE_BUFS = 2;
-  static constexpr int STAGE_BYTES = (EPI == EPI_HIDDEN) ? STAGE_BUFS * 32 * NOUT * 2 : 0;
   // staging ring depth: the last layer (N = 16: 9 x 4 MMAs of ~9 cycles per row, no output staging) outruns a 4-slot
   // ring by far and has the shared memory for a deep one
-  static constexpr int NSTAGE = (NOUT == 16) ? 10 : TS_NSTAGE;
-  static constexpr int OFF_STAGE = OFF_RING + NSTAGE * SLOT_BYTES;
-  static constexpr int OFF_BIAS = OFF_STAGE + EPI_WARPS * STAGE_BYTES;
+  static constexpr int NSTAGE = 10;
+  static constexpr int OFF_BIAS = OFF_RING + NSTAGE * SLOT_BYTES;
   static constexpr int OFF_BAR = OFF_BIAS + 256;
   static constexpr int BAR_BYTES = 512;
   static_assert((2 * NSTAGE + 2 * TS_NA + 2 * TS_NACC + 3) * 8 + 4 <= BAR_BYTES, "barrier block overflows");
@@ -590,15 +555,11 @@ struct ConvTsCfg {
   static_assert(SMEM_BYTES <= 232448, "exceeds the 227 KB shared memory of one CTA");
 };
 
-// host helpers defined in conv_tc.cu
+// host helper defined in conv_tc.cu
 int get_act_tensor_map(CUtensorMap* map, const void* ptr, int B, int H, int W, int C, int box_w);
-void plan_items(ConvParams* p);
 // conv_fused2.cu: two hidden layers (both conv + bias + ReLU) in one launch when the shape is a single wave of CTA pairs
 // (few chains); *applicable = 0 and nothing launched otherwise
 int conv64_hidden_fused2(const void* in, void* out, const uint8_t* w1, const float* b1, const uint8_t* w2, const float* b2, int B,
                          int H, int W, int* applicable, cudaStream_t st);
-// experiments.cu: the 18 hidden layers of DnCNN as one persistent launch (PSGLA_CHAIN=1)
-int launch_hidden_chain(void* buf0, void* buf1, int n_layers, const uint8_t* weights0, unsigned int* barrier, ConvParams p,
-                        cudaStream_t st);
 
 }  // namespace psgla

@@ -1,270 +1,14 @@
-// Experiments and development probes of the tcgen05 path, kept OUT of the production kernels' file (conv_tc.cu): the persistent
-// 18-layer chain kernel (PSGLA_CHAIN=1; measured, not faster -- see launch_hidden_chain's note in conv_tc.cu), the UMMA descriptor / TMEM
-// self-tests the gpu tests run (tests/test_image_gpu.py::test_umma_descriptor_selftest), the CTA-pair (cta_group::2)
-// self-test, and the MMA issue-rate probes whose measurements DESIGN.md section 4 quotes (profiles/r01b_mma_rate.txt,
+// Development probes of the tcgen05 path, kept OUT of the production kernels' files: the UMMA descriptor / TMEM self-tests
+// the gpu tests run (tests/test_image_gpu.py::test_umma_descriptor_selftest), the CTA-pair (cta_group::2) self-test, and
+// the MMA issue-rate probes whose measurements DESIGN.md section 4 quotes (profiles/r01b_mma_rate.txt,
 // profiles/r01e_mma_rate.txt).  Nothing here is on a sampler's path.
-#include <cuda_bf16.h>
-
-#include <algorithm>
 #include <atomic>
-#include <cstring>
 
-#include "conv_tc.cuh"
+#include "common.cuh"
+#include "sm100.cuh"
 
 namespace psgla {
-
-// ------------------------------------------------------------------------------------------------ layer-chain kernel
-// With few chains a layer is ~3 us of MMAs wrapped in ~5 us of launch, prologue, first-load latency and drain, so the 18
-// hidden layers of DnCNN are also available as ONE persistent launch: every CTA walks the layers, ping-ponging between
-// the two activation buffers, reloading the 73.7 KB of weights per layer (prefetched as soon as the previous layer's MMAs
-// retire) and meeting the other CTAs at a grid-wide barrier between layers (layer l+1 needs halo rows and neighbouring
-// strips produced by other CTAs).  grid <= #SMs with one CTA per SM, so all CTAs are co-resident and the barrier cannot
-// deadlock.  Same roles and pipelines as conv3x3_ts_kernel; counters and mbarrier phases simply run on across layers.
-constexpr int HIDDEN_LAYER_STRIDE = 9 * 64 * 128 + 1024;  // packed weights (73 728 B) + bias, rounded to 1 KB
-
-struct ChainParams {
-  int n_layers;
-  const uint8_t* weights0;   // packed weights of the first layer of the chain; layer l at + l * HIDDEN_LAYER_STRIDE
-  unsigned int* barrier;     // zero-initialised counter in global memory
-};
-
-__device__ __forceinline__ void grid_barrier_arrive_wait(unsigned int* counter, unsigned int target) {
-  __threadfence();  // publish this CTA's completed stores (already awaited by their issuers) at gpu scope
-  atomicAdd(counter, 1u);
-  unsigned int v;
-  long long t0 = clock64();
-  do {
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(counter) : "memory");
-    if (v < target && clock64() - t0 > 20000000000LL) {  // ~10 s: a protocol bug must not hang the GPU
-      printf("psgla_b200: grid barrier timed out (block %d, %u of %u)\n", (int)blockIdx.x, v, target);
-      __trap();
-    }
-  } while (v < target);
-  fence_proxy_async_global();  // order the TMA (async proxy) loads that follow after the acquire
-}
-
-__global__ void __launch_bounds__(TS_THREADS, 1)
-conv3x3_ts_chain_kernel(const __grid_constant__ CUtensorMap map_ld0, const __grid_constant__ CUtensorMap map_ld1,
-                        const __grid_constant__ CUtensorMap map_st0, const __grid_constant__ CUtensorMap map_st1,
-                        const ConvParams p, const ChainParams cp) {
-  // layer l reads buffer (l & 1) through map_ld{l&1} and writes buffer ((l + 1) & 1) through map_st{(l+1)&1}
-  constexpr int NOUT = 64;
-  using Cfg = ConvTsCfg<NOUT, EPI_HIDDEN>;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  uint8_t* smem_w = smem;
-  uint8_t* ring = smem + Cfg::OFF_RING;
-  uint64_t* full = reinterpret_cast<uint64_t*>(smem + Cfg::OFF_BAR);
-  uint64_t* empty = full + TS_NSTAGE;
-  uint64_t* afull = empty + TS_NSTAGE;
-  uint64_t* aempty = afull + TS_NA;
-  uint64_t* tfull = aempty + TS_NA;
-  uint64_t* tempty = tfull + TS_NACC;
-  uint64_t* wbar = tempty + TS_NACC;   // weights of the current layer have landed
-  uint64_t* wfree = wbar + 1;          // every MMA of the layer that used them has completed
-  uint64_t* ldone = wfree + 1;         // the eight epilogue warps have finished (and flushed) their rows of the layer
-  uint32_t* tmem_ptr_s = reinterpret_cast<uint32_t*>(ldone + 1);
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  griddep_launch_dependents();
-
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < TS_NSTAGE; ++i) {
-      mbar_init(&full[i], 1);
-      mbar_init(&empty[i], 4);
-    }
-    for (int i = 0; i < TS_NA; ++i) {
-      mbar_init(&afull[i], 4);
-      mbar_init(&aempty[i], 1);
-    }
-    for (int i = 0; i < TS_NACC; ++i) {
-      mbar_init(&tfull[i], 1);
-      mbar_init(&tempty[i], 4);
-    }
-    mbar_init(wbar, 1);
-    mbar_init(wfree, 1);
-    mbar_init(ldone, EPI_WARPS);
-    fence_barrier_init();
-  }
-  if (warp == 1) {
-    tmem_alloc(tmem_ptr_s, 512);
-    tmem_relinquish();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr_s;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      // ---------------------------------------------------------------- TMA producer (+ the CTA's voice at the grid barrier)
-      tma_prefetch_desc(&map_ld0);
-      tma_prefetch_desc(&map_ld1);
-      uint32_t L = 0;
-      for (int l = 0; l < cp.n_layers; ++l) {
-        if (l > 0) mbar_wait(wfree, (l - 1) & 1);  // the previous layer's MMAs no longer read the weight buffer
-        mbar_expect_tx(wbar, Cfg::W_BYTES);
-        bulk_load(smem_w, cp.weights0 + (size_t)l * HIDDEN_LAYER_STRIDE, Cfg::W_BYTES, wbar);
-        if (l == 0) {
-          griddep_wait();
-        } else {
-          mbar_wait(ldone, (l - 1) & 1);  // this CTA's outputs of layer l-1 are complete in global memory
-          grid_barrier_arrive_wait(cp.barrier, (unsigned)l * gridDim.x);
-        }
-        const CUtensorMap* map = (l & 1) ? &map_ld1 : &map_ld0;
-        for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
-          const ItemCoord c = decode_item(p, item);
-          for (int y = c.ylo; y <= c.yhi; ++y, ++L) {
-            const uint32_t slot = L % TS_NSTAGE;
-            mbar_wait(&empty[slot], ((L / TS_NSTAGE) & 1) ^ 1);
-            mbar_expect_tx(&full[slot], Cfg::BOX_BYTES);
-            tma_load_4d(ring + slot * Cfg::SLOT_BYTES, map, &full[slot], 0, c.x0 - 1, y, c.b);
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ---------------------------------------------------------------- MMA issuer
-    constexpr uint32_t idesc = make_idesc_bf16(TILE_M, NOUT);
-    constexpr uint32_t DESC_HI = (1024u >> 4) | (1u << 14) | (LAYOUT_SW128 << 29);
-    const uint32_t w_lo = (smem_u32(smem_w) >> 4) | 0x10000u;
-    uint32_t L0 = 0, T = 0;
-    for (int l = 0; l < cp.n_layers; ++l) {
-      mbar_wait(wbar, l & 1);
-      tc_fence_after();
-      for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
-        const ItemCoord c = decode_item(p, item);
-        int waited = 0;
-        const int ylast = c.y0 + c.rcur - 1;
-        for (int y = c.y0; y <= ylast; ++y, ++T) {
-          const int need = min(y + 1, c.yhi) - c.ylo + 1;
-          while (waited < need) {
-            const uint32_t q = L0 + waited;
-            mbar_wait(&afull[q % TS_NA], (q / TS_NA) & 1);
-            ++waited;
-          }
-          const uint32_t acc = T % TS_NACC;
-          mbar_wait(&tempty[acc], ((T / TS_NACC) & 1) ^ 1);
-          tc_fence_after();
-          const uint32_t d_tmem = tmem_base + acc * NOUT;
-          if (elect_one()) {
-            uint32_t accumulate = 0;
-#pragma unroll
-            for (int dy = 0; dy < 3; ++dy) {
-              const int yy = y + dy - 1;
-              if (yy < 0 || yy >= p.H) continue;
-              const uint32_t q = L0 + (uint32_t)(yy - c.ylo);
-              const uint32_t a_t = tmem_base + TS_A_COL0 + (q % TS_NA) * 96u;
-#pragma unroll
-              for (int dx = 0; dx < 3; ++dx) {
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                  const uint32_t bl = w_lo + (uint32_t)(((dy * 3 + dx) * Cfg::TAP_BYTES + k * 32) >> 4);
-                  umma_bf16_ts(d_tmem, a_t + dx * 32 + k * 8, ((uint64_t)DESC_HI << 32) | bl, idesc, accumulate);
-                  accumulate = 1;
-                }
-              }
-            }
-            umma_commit(&tfull[acc]);
-            if (y - 1 >= c.ylo) umma_commit(&aempty[(L0 + (uint32_t)(y - 1 - c.ylo)) % TS_NA]);
-            if (y == ylast)
-              for (int yy = y; yy <= c.yhi; ++yy) umma_commit(&aempty[(L0 + (uint32_t)(yy - c.ylo)) % TS_NA]);
-          }
-          __syncwarp();
-        }
-        L0 += (uint32_t)(c.yhi - c.ylo + 1);
-      }
-      if (elect_one()) umma_commit(wfree);  // arrives once every MMA issued so far has completed
-      __syncwarp();
-    }
-  } else if (warp < 6) {
-    // ---------------------------------------------------------------- loaders: staging ring -> registers -> TMEM
-    const int q4 = warp & 3;
-    const int m = q4 * 32 + lane;
-    const uint32_t ring_addr = smem_u32(ring);
-    const uint32_t lane_taddr = tmem_base + ((uint32_t)(q4 * 32) << 16) + TS_A_COL0;
-    uint32_t L = 0;
-    for (int l = 0; l < cp.n_layers; ++l) {
-      for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
-        const ItemCoord c = decode_item(p, item);
-        for (int y = c.ylo; y <= c.yhi; ++y, ++L) {
-          const uint32_t slot = L % TS_NSTAGE, as = L % TS_NA;
-          mbar_wait(&full[slot], (L / TS_NSTAGE) & 1);
-          mbar_wait(&aempty[as], ((L / TS_NA) & 1) ^ 1);
-          tc_fence_after();
-          const uint32_t tile = ring_addr + slot * Cfg::SLOT_BYTES;
-#pragma unroll
-          for (int dx = 0; dx < 3; ++dx) {
-            uint32_t v[32];
-            ld_swizzled_row128(tile, m + dx, v);
-            tmem_st_32x32b_x32(lane_taddr + as * 96u + dx * 32u, v);
-          }
-          tmem_st_wait();
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) {
-            mbar_arrive(&empty[slot]);
-            mbar_arrive(&afull[as]);
-          }
-        }
-      }
-    }
-  } else {
-    // ---------------------------------------------------------------- epilogue: 2 groups x 4 warps
-    const int ew = warp - 6;
-    uint32_t T = 0;
-    for (int l = 0; l < cp.n_layers; ++l) {
-      const float* bias = reinterpret_cast<const float*>(cp.weights0 + (size_t)l * HIDDEN_LAYER_STRIDE + Cfg::W_BYTES);
-      epilogue_hidden<NOUT, TS_NACC, false>(p, ((l + 1) & 1) ? &map_st1 : &map_st0, smem + Cfg::OFF_STAGE + ew * Cfg::STAGE_BYTES, bias,
-                                     tfull, tempty, tmem_base, ew >> 2, warp & 3, lane, T, 0, Cfg::STAGE_BUFS);
-      // other CTAs of this grid read these rows after the barrier: wait for the stores' WRITES, not only their reads
-      if (lane == 0) bulk_wait_group0();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(ldone);
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 512);
-  }
-}
-
-// The 18 hidden layers as one persistent launch (conv3x3_ts_chain_kernel).  buf0 holds the input of the first layer of the
-// chain; layers alternate buf0 -> buf1 -> buf0 ...; the result is in buf[n_layers & 1].
-int launch_hidden_chain(void* buf0, void* buf1, int n_layers, const uint8_t* weights0, unsigned int* barrier,
-                               ConvParams p, cudaStream_t st) {
-  using Cfg = ConvTsCfg<64, EPI_HIDDEN>;
-  CUtensorMap ld0, ld1, st0, st1;
-  int rc = get_act_tensor_map(&ld0, buf0, p.B, p.H, p.W, 64, BOX_W);
-  if (!rc) rc = get_act_tensor_map(&ld1, buf1, p.B, p.H, p.W, 64, BOX_W);
-  if (!rc) rc = get_act_tensor_map(&st0, buf0, p.B, p.H, p.W, 64, 32);
-  if (!rc) rc = get_act_tensor_map(&st1, buf1, p.B, p.H, p.W, 64, 32);
-  if (rc) return rc;
-  static std::atomic<unsigned long long> attr_done{0};  // bit d: opted in on device d (a per-device function attribute)
-  const unsigned long long dev_bit = 1ull << (current_device() & 63);
-  if (!(attr_done.load(std::memory_order_acquire) & dev_bit)) {
-    PSGLA_CUDA_TRY(cudaFuncSetAttribute(conv3x3_ts_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-    attr_done.fetch_or(dev_bit, std::memory_order_release);
-  }
-  plan_items(&p);
-  p.relu = 1;
-  const int grid = p.n_items < num_sms() ? p.n_items : num_sms();
-  PSGLA_CUDA_TRY(cudaMemsetAsync(barrier, 0, sizeof(unsigned int), st));
-  ChainParams cp{n_layers, weights0, barrier};
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(TS_THREADS);
-  cfg.dynamicSmemBytes = Cfg::SMEM_BYTES;
-  cfg.stream = st;
-  cfg.attrs = nullptr;  // plain stream order: the memset above must be complete, and every CTA must be free to start
-  cfg.numAttrs = 0;
-  PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv3x3_ts_chain_kernel, ld0, ld1, st0, st1, p, cp));
-  return PSGLA_OK;
-}
-
+using namespace sm100;
 }  // namespace psgla
 
 using namespace psgla;
