@@ -41,7 +41,7 @@ enum {
 const char* psgla_last_error(void);
 int psgla_abi_version(void);
 /* sizeof() of the structs below as the library was compiled (0: psgla_gmm2d_problem, 1: psgla_img_shape, 2: psgla_pre_params,
- * 3: psgla_post_params, 4: psgla_next_pre; -1 otherwise) -- lets a binding verify its struct layout. */
+ * 3: psgla_post_params, 4: psgla_next_pre, 5: psgla_tv_params; -1 otherwise) -- lets a binding verify its struct layout. */
 int psgla_struct_size(int which);
 /* Philox4x32-10 (Salmon et al., SC'11) block function as the kernels use it: counter[4], key[2] -> out[4].  Host code,
  * no GPU needed; the tests pin it to the Random123 known-answer vectors. */
@@ -264,6 +264,29 @@ int psgla_img_to_nhwc16(psgla_img_shape shape, const float* x_dev, float c3, voi
  * inputs whose sides are not multiples of 8).  The samplers call it on the denoiser input before every DRUNet application of a
  * problem that was padded to multiples of 8. */
 int psgla_img_pad_replicate_nhwc16(psgla_img_shape padded, int H, int W, void* img_dev, void* stream);
+
+/* Total-variation denoiser (deepinv.models.TVDenoiser, sampling_images.py:139-140; the PSGLA-TV runs of :181-184): the prox
+ *   D(y) = argmin_x 1/2 ||x - y||^2 + ths * sum_{c,p} ||(grad x)_{c,p}||_2     (isotropic per channel and pixel)
+ * by over-relaxed Chambolle-Pock, tau, rho, sigma = 1 / (8 tau), iterated until ||x_prev - x2|| / ||x2 + 1e-12|| < crit after
+ * the third iteration or n_it_max iterations.  The norms run per chain, so a chain's result does not depend on the other
+ * chains of the batch.  fp32 state and arithmetic; one cooperative launch per call, fused with the post:
+ *   x_out = post->base_scale * y + post->gain * D(y), thinning and moments as in psgla_dncnn_residual_post.
+ * state_dev (psgla_tv_state_bytes): x2 fp32 [B][3][H][W], then u2 fp32 [B][3][H][W][2]; restart = 0 continues from it (warm
+ * start), restart = 1 starts from x2 = y, u2 = 0.  On return it holds each chain's final x2 / u2.
+ * workspace_dev (psgla_tv_workspace_bytes): the second ping-pong copy of the state, per-tile partial sums, per-chain counters.
+ * x_out_dev may alias y_dev; state_dev may not.  iters_dev: NULL or int32 [B], each chain's CP iteration count.
+ * Any H, W >= 1. */
+typedef struct psgla_tv_params {
+  float ths, tau, rho, crit;   /* ths > 0; tau > 0; 0 < rho < 2; crit >= 0 (0: run n_it_max) */
+  int32_t n_it_max;            /* >= 1 */
+  int32_t restart;             /* 1: x2 = y, u2 = 0 first; 0: continue from state_dev */
+} psgla_tv_params;             /* psgla_struct_size(5) */
+size_t psgla_tv_state_bytes(psgla_img_shape shape);      /* x2 fp32 [B][3][H][W], then u2 fp32 [B][3][H][W][2]; 0: bad shape */
+size_t psgla_tv_workspace_bytes(psgla_img_shape shape);  /* ping-pong copy, tile partials, counters; 0: bad shape */
+int psgla_tv_prox_post(const psgla_tv_params* tv, psgla_img_shape shape, const float* y_dev, void* state_dev,
+                       size_t state_bytes, void* workspace_dev, size_t workspace_bytes, const psgla_post_params* post,
+                       float* x_out_dev, float* sample_dev, float* mean_dev, float* mean2_dev, int32_t* iters_dev,
+                       void* stream);
 
 /* tcgen05 descriptor self-test (development aid): runs a 128 x 64 x 64 GEMM tile whose A operand starts `row_shift`
  * rows into a 128B-swizzled shared-memory buffer.  mode 0: A from shared memory, shift = descriptor start address;

@@ -11,7 +11,7 @@ from . import metrics  # noqa: F401
 from . import image_set  # noqa: F401
 from .image_set import load_image, run_image_set  # noqa: F401
 from .metrics import posterior_summary, psnr_ssim  # noqa: F401
-from .denoisers import (DRUNET_KEYS, DRUNet, DnCNN, lipschitz_dncnn_state_dict, random_dncnn_state_dict,  # noqa: F401
+from .denoisers import (DRUNET_KEYS, DRUNet, DnCNN, TVDenoiser, lipschitz_dncnn_state_dict, random_dncnn_state_dict,  # noqa: F401
                         random_drunet_state_dict, smoothing_dncnn_state_dict)  # noqa: F401
 from .operators import (DeblurDataGrad, InpaintingDataGrad, PriorGrad, blur_taps, make_deblurring,  # noqa: F401
                         make_inpainting)

@@ -54,6 +54,12 @@ class NextPre(C.Structure):
                 ("y_B", C.c_int32), ("base_dev", C.c_void_p), ("den_in_dev", C.c_void_p)]
 
 
+class TVParams(C.Structure):
+    """psgla_tv_params"""
+    _fields_ = [("ths", C.c_float), ("tau", C.c_float), ("rho", C.c_float), ("crit", C.c_float), ("n_it_max", C.c_int32),
+                ("restart", C.c_int32)]
+
+
 _vp, _i64, _u64, _int, _sz = C.c_void_p, C.c_int64, C.c_uint64, C.c_int, C.c_size_t
 
 # name -> (restype, argtypes); every symbol include/psgla_b200.h declares
@@ -101,6 +107,10 @@ SIGNATURES = {
     "psgla_drunet_denoise_post_next": (_int, [_vp, ImgShape, _vp, _vp, _sz, _vp, C.POINTER(PostParams), _vp, _vp, _vp, _vp,
                                               C.POINTER(NextPre), _vp]),
     "psgla_drunet_layer": (_int, [_vp, ImgShape, _int, _vp, _vp, _vp, _vp, _vp]),
+    "psgla_tv_state_bytes": (_sz, [ImgShape]),
+    "psgla_tv_workspace_bytes": (_sz, [ImgShape]),
+    "psgla_tv_prox_post": (_int, [C.POINTER(TVParams), ImgShape, _vp, _vp, _sz, _vp, _sz, C.POINTER(PostParams), _vp, _vp, _vp,
+                                  _vp, _vp, _vp]),
     "psgla_selftest_umma": (_int, [_vp, _vp, _vp, _int, _int, _vp]),
     "psgla_selftest_umma2": (_int, [_vp, _vp, _vp, _int, _vp]),
     "psgla_convg_layer": (_int, [_int, _int, _int, _int, _int, _int, _vp, _vp, _vp, _vp, _vp, _int, _vp]),
@@ -129,7 +139,7 @@ def lib() -> C.CDLL:
                     fn = getattr(handle, name)  # AttributeError if the header and the library disagree
                     fn.restype = res
                     fn.argtypes = args
-                for which, struct in enumerate((GmmProblem, ImgShape, PreParams, PostParams, NextPre)):
+                for which, struct in enumerate((GmmProblem, ImgShape, PreParams, PostParams, NextPre, TVParams)):
                     if handle.psgla_struct_size(which) != C.sizeof(struct):
                         raise RuntimeError("ctypes layout of %s (%d bytes) disagrees with libpsgla_b200.so (%d bytes): "
                                            "rebuild the library" % (struct.__name__, C.sizeof(struct), handle.psgla_struct_size(which)))

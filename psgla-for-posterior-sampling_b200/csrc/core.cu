@@ -32,7 +32,7 @@ extern "C" int psgla_device_arch(void) {
 }
 
 // sizeof() of the ABI structs as this library was compiled, for binding self-checks (0: gmm2d_problem, 1: img_shape,
-// 2: pre_params, 3: post_params).
+// 2: pre_params, 3: post_params, 4: next_pre, 5: tv_params).
 extern "C" int psgla_struct_size(int which) {
   switch (which) {
     case 0: return (int)sizeof(psgla_gmm2d_problem);
@@ -40,6 +40,7 @@ extern "C" int psgla_struct_size(int which) {
     case 2: return (int)sizeof(psgla_pre_params);
     case 3: return (int)sizeof(psgla_post_params);
     case 4: return (int)sizeof(psgla_next_pre);
+    case 5: return (int)sizeof(psgla_tv_params);
     default: return -1;
   }
 }

@@ -1,6 +1,7 @@
-"""DnCNN denoiser running as tcgen05 implicit-GEMM convolutions (csrc/conv_tc.cu).
+"""The image denoisers: DnCNN and DRUNet as tcgen05 implicit-GEMM convolutions (csrc/conv_tc.cu, csrc/conv_gemm.cu), and
+the TV proximal operator (csrc/tv_prox.cu).
 
-Mirrors ``deepinv.models.DnCNN(in_channels=3, out_channels=3, pretrained=..., device=...)`` as the reference constructs
+``DnCNN`` mirrors ``deepinv.models.DnCNN(in_channels=3, out_channels=3, pretrained=..., device=...)`` as the reference constructs
 it (sampling_images.py:130) and calls it (``denoiser.forward(x, sigma)``, restoration_algorithms.py:238): depth 20,
 64 features, 3x3, bias, ReLU, residual output, ``sigma`` ignored.  Weights come from a deepinv-style state dict
 (keys ``in_conv``, ``conv_list.i``, ``out_conv``) -- a checkpoint path, a dict, or ``None`` for seeded random init.
@@ -15,7 +16,7 @@ import torch
 
 from . import _lib
 
-__all__ = ["DnCNN", "DRUNet", "random_dncnn_state_dict", "lipschitz_dncnn_state_dict", "smoothing_dncnn_state_dict",
+__all__ = ["DnCNN", "DRUNet", "TVDenoiser", "random_dncnn_state_dict", "lipschitz_dncnn_state_dict", "smoothing_dncnn_state_dict",
            "random_drunet_state_dict", "DRUNET_KEYS"]
 
 
@@ -302,5 +303,106 @@ class DRUNet:
                        "psgla_img_to_nhwc16")
         self.apply_post(shape, den_in, x, _lib.PostParams(1.0, 0.0, 0.0, 1.0), out)  # out = 0 * x + 1 * D(x)
         return out[:, :, :H0, :W0].contiguous() if (ph or pw) else out
+
+    __call__ = forward
+
+
+# ----------------------------------------------------------------------------------------------------- TV
+class TVDenoiser:
+    """``deepinv.models.TVDenoiser(verbose=False, tau=0.01, rho=1.99, n_it_max=1000, crit=1e-5)`` (sampling_images.py:139-140)
+    on one cooperative CUDA launch per call (csrc/tv_prox.cu): the prox of ths * isotropic total variation (per channel and
+    pixel) by over-relaxed Chambolle-Pock, fp32.  ``forward(y, ths)`` warm-starts from the previous call's primal / dual state
+    like deepinv's: it restarts (x2 = y, u2 = 0) on the first call, after ``reset()`` or ``restart = True``, and when y's shape
+    changes.  One difference: the stopping test ||x_prev - x2|| / ||x2|| < crit is evaluated per chain (per batch entry) and
+    each chain stops on its own, so a chain's result does not depend on the chains next to it; for a single chain -- every
+    run the reference makes -- this is deepinv's rule.  Any image size.
+
+    ``x2`` / ``u2``: views of the state ([B,3,H,W] and [B,3,H,W,2]); ``last_iterations``: device int32 [B], the CP iteration
+    count of each chain in the last call (no host synchronisation)."""
+
+    is_residual = False  # D(y) itself: the samplers form (1 - alpha) Y + alpha D(Y)
+
+    def __init__(self, verbose=False, tau=0.01, rho=1.99, n_it_max=1000, crit=1e-5, device=None):
+        torch_ = _lib.require_cuda()
+        self.device = torch_.device("cuda", torch_.cuda.current_device()) if device is None else torch_.device(device)
+        self.verbose = bool(verbose)
+        self.tau, self.rho, self.n_it_max, self.crit = float(tau), float(rho), int(n_it_max), float(crit)
+        self.restart = True
+        self._shape = None
+        self._state = None
+        self._ws = None
+        self._den_in = None
+        self.last_iterations = None
+
+    def reset(self):
+        """The next call starts from x2 = y, u2 = 0."""
+        self.restart = True
+
+    @property
+    def x2(self):
+        if self._shape is None:
+            return None
+        B, _, H, W = self._shape
+        return self._state[:B * 3 * H * W].view(B, 3, H, W)
+
+    @property
+    def u2(self):
+        if self._shape is None:
+            return None
+        B, _, H, W = self._shape
+        return self._state[B * 3 * H * W:].view(B, 3, H, W, 2)
+
+    def buffers(self, shape: "_lib.ImgShape"):
+        """(workspace, denoiser input): the samplers' "pre" writes the bf16 input every denoiser takes; the prox reads the
+        fp32 base instead, so the second buffer is only written."""
+        lib = _lib.lib()
+        need = lib.psgla_tv_workspace_bytes(shape)
+        if need == 0:
+            raise ValueError("bad image shape for the TV prox")
+        if self._ws is None or self._ws.numel() < need:
+            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        n_in = shape.B * shape.H * shape.W * 16
+        if self._den_in is None or self._den_in.numel() < n_in:
+            self._den_in = torch.empty(n_in, dtype=torch.bfloat16, device=self.device)
+        return self._ws, self._den_in
+
+    def apply_post(self, shape, den_in, base, post, x_out, sample=None, mean=None, mean2=None, next_pre=None, ths=None):
+        """x_out = post.base_scale * base + post.gain * TV_prox(base; ths), thinning and moments (the samplers' post).
+        ``den_in`` is not read; the fused next-iteration pre is a conv-epilogue feature and is not offered."""
+        if next_pre is not None:
+            raise ValueError("the TV prox does not fuse the next iteration's pre")
+        if ths is None:
+            raise ValueError("the TV prox needs ths")
+        ws, _ = self.buffers(shape)
+        key = (shape.B, 3, shape.H, shape.W)
+        restart = self.restart or self._shape != key
+        if restart and self._shape != key:
+            self._state = torch.empty(_lib.lib().psgla_tv_state_bytes(shape) // 4, dtype=torch.float32, device=self.device)
+            self._shape = key
+        if self.last_iterations is None or self.last_iterations.numel() != shape.B:
+            self.last_iterations = torch.empty(shape.B, dtype=torch.int32, device=self.device)
+        prm = _lib.TVParams(float(ths), self.tau, self.rho, self.crit, self.n_it_max, int(restart))
+        with torch.cuda.device(self.device):
+            rc = _lib.lib().psgla_tv_prox_post(C.byref(prm), shape, _lib.ptr(base), _lib.ptr(self._state), self._state.numel() * 4,
+                                               _lib.ptr(ws), ws.numel(), C.byref(post), _lib.ptr(x_out), _lib.ptr(sample),
+                                               _lib.ptr(mean), _lib.ptr(mean2), _lib.ptr(self.last_iterations),
+                                               _lib.stream_ptr(self.device))
+        _lib.check(rc, "psgla_tv_prox_post")
+        self.restart = False
+        if self.verbose:
+            print("TV prox: %s Chambolle-Pock iterations" % self.last_iterations.tolist())
+
+    def forward(self, y, ths):
+        """TV_prox(y; ths), fp32 [B,3,H,W] in and out (``ths``: a number or a one-element tensor)."""
+        if not y.is_cuda:
+            raise RuntimeError("TVDenoiser.forward needs a CUDA tensor: there is no CPU path")
+        if y.dim() != 4 or y.shape[1] != 3:
+            raise ValueError("expected a [B,3,H,W] colour batch, got %s" % (tuple(y.shape),))
+        ths = float(ths.reshape(-1)[0]) if isinstance(ths, torch.Tensor) else float(ths)
+        y = y.to(self.device, torch.float32).contiguous()
+        shape = _lib.ImgShape(int(y.shape[0]), 3, int(y.shape[2]), int(y.shape[3]))
+        out = torch.empty_like(y)
+        self.apply_post(shape, None, y, _lib.PostParams(1.0, 0.0, 0.0, 1.0), out, ths=ths)  # out = 0 * y + 1 * D(y)
+        return out
 
     __call__ = forward

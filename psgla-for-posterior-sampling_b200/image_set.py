@@ -14,7 +14,7 @@ import torch
 
 from . import dist as _dist
 from . import metrics as _metrics
-from .denoisers import DnCNN
+from .denoisers import DnCNN, TVDenoiser
 from .operators import PriorGrad, make_deblurring, make_inpainting
 from .params import as_pnpula_kwargs, as_psgla_kwargs, sampler_params
 from .restoration_algorithms import pnpula, psgla
@@ -59,6 +59,10 @@ def _sample_image(index, im, denoiser, problem, alg, n_chains, prm, seed, seed_i
     else:
         raise ValueError("problem must be 'inpainting' or 'deblurring'")
     kw = dict(n_chains=n_chains, chain_id0=index * n_chains, store="stats", rng="philox")
+    if isinstance(denoiser, TVDenoiser):
+        # every image starts the prox from x2 = y, u2 = 0, so a row does not depend on which images this rank ran before
+        # it (the reference warm-starts across the images of its loop)
+        denoiser.reset()
     if alg == "psgla":
         _, M, M2 = psgla(init, dg, denoiser, **as_psgla_kwargs(prm, seed=seed), **kw)
     elif alg in ("pnp_ula", "pnpula"):
@@ -93,7 +97,8 @@ def run_image_set(images, denoiser=None, problem="inpainting", alg="psgla", n_ch
     """Posterior sampling of a SET of images, ``n_chains`` independent chains each, sharded over the process group.
 
     images     list of [3, H, W] / [1, 3, H, W] float tensors in [0, 1] (sizes may differ), the same list on every rank
-    denoiser   this rank's ``psgla_b200.DnCNN`` / ``DRUNet`` (default: a DnCNN with the library's seeded weights)
+    denoiser   this rank's ``psgla_b200.DnCNN`` / ``DRUNet`` / ``TVDenoiser`` (default: a DnCNN with the library's seeded
+               weights; TV: psgla only, table row ``den="TV"``, the prox state is reset before each image)
     params     the dict of ``psgla_b200.sampler_params`` (default: the script's table for ``alg`` / the denoiser family, with
                ``N = n_iter`` when given)
     Returns, on rank 0, a list of dicts (one per image, in input order) with the keys of ``ROW_FIELDS`` (+ ``xmmse`` / ``std``
@@ -102,7 +107,7 @@ def run_image_set(images, denoiser=None, problem="inpainting", alg="psgla", n_ch
     if _sample is None:
         if denoiser is None:
             denoiser = DnCNN()
-        den_name = "DnCNN" if isinstance(denoiser, DnCNN) else "DRUNet"
+        den_name = "DnCNN" if isinstance(denoiser, DnCNN) else ("TV" if isinstance(denoiser, TVDenoiser) else "DRUNet")
         prm = dict(params) if params is not None else sampler_params("pnp_ula" if alg in ("pnp_ula", "pnpula") else alg, den=den_name,
                                                                      sigma=sigma, N=n_iter)
         if n_iter is not None:

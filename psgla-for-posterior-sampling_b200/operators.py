@@ -14,6 +14,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .denoisers import TVDenoiser
 
 __all__ = ["InpaintingDataGrad", "DeblurDataGrad", "PriorGrad", "make_inpainting", "make_deblurring", "blur_taps"]
 
@@ -92,6 +93,8 @@ class PriorGrad:
     """``prior_grad(x) = alpha * (D(x; s1) - x) / s2`` (sampling_images.py:156-157)."""
 
     def __init__(self, denoiser, alpha, s1, s2):
+        if isinstance(denoiser, TVDenoiser):
+            raise TypeError("PriorGrad supports a psgla_b200.DnCNN or psgla_b200.DRUNet denoiser, not the TV prox")
         self.denoiser, self.alpha, self.s1, self.s2 = denoiser, float(alpha), float(s1), float(s2)
 
     def __call__(self, x):

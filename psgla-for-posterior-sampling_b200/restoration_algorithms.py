@@ -20,8 +20,11 @@ Extra keyword-only arguments:
                  device, so ``Xlist_mmse`` / ``Xlist_mmse2`` hold ONE tensor each: the mean over windows the reference's
                  post-processing forms anyway, sampling_images.py:427,436).  What batched runs (64 chains per image) need:
                  memory independent of n_iter.
-The data term must be an ``InpaintingDataGrad`` / ``DeblurDataGrad`` and the denoiser a ``psgla_b200.DnCNN``
+The data term must be an ``InpaintingDataGrad`` / ``DeblurDataGrad`` and the denoiser a ``psgla_b200.DnCNN`` / ``DRUNet``
 (``prior_grad`` a ``PriorGrad`` wrapping one); opaque callables raise ``TypeError`` -- there is no eager fallback.
+``psgla`` / ``psgla_run`` / ``pnp`` also take a ``psgla_b200.TVDenoiser`` (PSGLA-TV): each iteration is then the "pre" launch and
+one cooperative launch of the TV prox with the post fused (csrc/tv_prox.cu), at any image size.  ``pnpula`` and ``red`` feed
+the denoiser X instead of the fp32 base and reject it.
 """
 from __future__ import annotations
 
@@ -33,7 +36,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .denoisers import DRUNet, DnCNN
+from .denoisers import DRUNet, DnCNN, TVDenoiser
 from .operators import DeblurDataGrad, InpaintingDataGrad, PriorGrad
 
 __all__ = ["psgla", "pnpula", "pnp_ula", "psgla_run", "pnpula_run", "pnp", "red"]
@@ -55,8 +58,8 @@ class _Run:
         if not isinstance(data_grad, (InpaintingDataGrad, DeblurDataGrad)):
             raise TypeError("data_grad must be an InpaintingDataGrad or DeblurDataGrad (structured callable); an opaque "
                             "callable cannot be fused into the CUDA kernels and there is no eager fallback")
-        if not isinstance(denoiser, (DnCNN, DRUNet)):
-            raise TypeError("denoiser must be a psgla_b200.DnCNN or psgla_b200.DRUNet")
+        if not isinstance(denoiser, (DnCNN, DRUNet, TVDenoiser)):
+            raise TypeError("denoiser must be a psgla_b200.DnCNN, psgla_b200.DRUNet or (psgla / pnp only) psgla_b200.TVDenoiser")
         if seed is None and noise is None:
             raise ValueError("seed=None: the reference fails with UnboundLocalError here "
                              "(restoration_algorithms.py:211-213,232); pass a seed or a noise tensor")
@@ -165,7 +168,9 @@ class _Run:
 
     def configure(self, pre, gain, base_scale=1.0):
         self.pre_params, self.gain, self.base_scale = pre, float(gain), float(base_scale)
-        self.fuse_next_pre, self._pre_done_for = os.environ.get("PSGLA_FUSE_PRE", "1") != "0", None
+        # the fused next-iteration pre is a conv-epilogue feature: the TV prox runs one pre launch per iteration
+        self.fuse_next_pre = os.environ.get("PSGLA_FUSE_PRE", "1") != "0" and not isinstance(self.den, TVDenoiser)
+        self._pre_done_for = None
         self._next_params = _lib.PreParams()
 
     def step(self, i):
@@ -237,7 +242,11 @@ class _Run:
             with torch.cuda.device(self.device):
                 _lib.check(_lib.lib().psgla_img_pad_replicate_nhwc16(self.shape, self.crop[0], self.crop[1], _lib.ptr(self.den_in),
                                                                      _lib.stream_ptr(self.device)), "psgla_img_pad_replicate_nhwc16")
-        self.den.apply_post(self.shape, self.den_in, self.base, post, self.X, sample, self.mean, self.mean2, next_pre=nxt)
+        if isinstance(self.den, TVDenoiser):  # ths = the level the pre carries for non-residual denoisers (pnp anneals it)
+            self.den.apply_post(self.shape, self.den_in, self.base, post, self.X, sample, self.mean, self.mean2,
+                                ths=self.pre_params.den_in_c3)
+        else:
+            self.den.apply_post(self.shape, self.den_in, self.base, post, self.X, sample, self.mean, self.mean2, next_pre=nxt)
         if sample is not None:
             self.Xlist.append(self._out(sample))
         # window bookkeeping exactly as restoration_algorithms.py:128-144 / :255-271
@@ -300,7 +309,7 @@ def psgla_run(init, data_grad, denoiser, alpha, lambd, sig_float=0.0055, delta=4
     if denoiser.is_residual:  # DnCNN: (1-alpha) Y + alpha (Y + R(Y)) = Y + alpha R(Y)
         pre.den_in_c3 = 0.0
         run.configure(pre, _f(alpha))
-    else:  # DRUNet: (1-alpha) Y + alpha D(Y; sig) with the noise-level map sig in channel 3 (restoration_algorithms.py:238)
+    else:  # DRUNet / TV: (1-alpha) Y + alpha D(Y; sig), sig = the noise-level map in channel 3 resp. ths (restoration_algorithms.py:238)
         pre.den_in_c3 = sig32
         run.configure(pre, _f(alpha), 1.0 - _f(alpha))
     return run
@@ -327,6 +336,8 @@ def pnpula_run(init, data_grad, prior_grad, delta, lambd, n_iter=5000, n_inter=1
     """The stepping object behind ``pnpula`` (see ``psgla_run``)."""
     if not isinstance(prior_grad, PriorGrad):
         raise TypeError("prior_grad must be a PriorGrad(denoiser, alpha, s1, s2) structured callable")
+    if isinstance(prior_grad.denoiser, TVDenoiser):
+        raise TypeError("pnpula supports a psgla_b200.DnCNN or psgla_b200.DRUNet prior, not the TV prox")
     run = _Run(init, data_grad, prior_grad.denoiser, n_iter, n_inter, n_inter_mmse, seed, noise, rng, n_chains, chain_id0,
                store)
     delta_f, lambd_f = _f(delta), _f(lambd)
