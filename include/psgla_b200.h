@@ -331,6 +331,36 @@ int psgla_drunet_denoise_post_next(const void* packed_dev, psgla_img_shape shape
 int psgla_drunet_layer(const void* packed_dev, psgla_img_shape shape, int layer, const void* in_dev, const void* res1_dev,
                        const void* res2_dev, void* out_dev, void* stream);
 
+/* Gradient-step DRUNet (deepinv.models.GSDRUNet(alpha, in_channels=3, out_channels=3, nb=2, nc=[64,128,256,512],
+ * act_mode="E"), sampling_images.py:129-140; Prox-DRUNet is the same network from another checkpoint):
+ *   N = KAIR UNetRes with nb = 2 residual blocks x + conv(elu(conv(x))) per stage, no biases, sigma map as fourth input channel
+ *   D(x) = x - alpha (v - J^T v),  v = x - N(x),  J^T v = the vector-Jacobian product of N at x (sigma's gradient dropped).
+ * weights_host: psgla_gsdrunet_num_weights() = 36 fp32 tensors in state-dict order (m_head, m_down1.{0,1}.res.{0,2}, m_down1.2,
+ * m_down2.*, m_down3.*, m_body.{0,1}.res.{0,2}, m_up3.0, m_up3.{1,2}.res.{0,2}, m_up2.*, m_up1.*, m_tail; torch layouts); the
+ * packed buffer holds them for the forward and, repacked as adjoints, for the backward.  H and W must be multiples of 8.
+ * psgla_gsdrunet_denoise_post_next: X+ = post->base_scale * base + post->gain * D(x), thinning, moments and the optional next
+ * pre as in psgla_drunet_denoise_post_next.  den_in_dev: bf16 NHWC16 of x with channel 3 = sigma (a "pre" call's output);
+ * x_dev: x itself, fp32 [B][3][H][W], or NULL when x is base_dev (PSGLA; PnP-ULA and RED evaluate D at the chain state X,
+ * which may be x_out_dev).  alpha: finite.  One call is 72 conv launches and one element-wise launch; the workspace holds
+ * the forward activations, the 14 ELU outputs the backward's gates read and the four held skip gradients (~2 KB per pixel). */
+int psgla_gsdrunet_num_weights(void);
+size_t psgla_gsdrunet_packed_bytes(void);
+int psgla_gsdrunet_pack_weights(const float* const* weights_host, void* packed_dev, void* stream);
+size_t psgla_gsdrunet_workspace_bytes(psgla_img_shape shape); /* 0: bad shape */
+int psgla_gsdrunet_denoise_post_next(const void* packed_dev, psgla_img_shape shape, const void* den_in_dev, const float* x_dev,
+                                     void* workspace_dev, size_t workspace_bytes, const float* base_dev, float alpha,
+                                     const psgla_post_params* post, float* x_out_dev, float* sample_dev, float* mean_dev,
+                                     float* mean2_dev, const psgla_next_pre* next, void* stream);
+/* One layer of that call, for tests: backward = 0: forward layer 0..35 (state-dict order); backward = 1: backward layer b =
+ * the adjoint of forward layer 35 - b.  in_dev: bf16 NHWC16 (forward 0, channel 3 = sigma; backward 0, the cotangent in
+ * channels 0..2) or bf16 NHWC; out_dev: bf16 NHWC, or the raw conv as fp32 NCHW [B][3][H][W] for forward 35 and backward 35.
+ * res1_dev / res2_dev exactly where the layer adds them (forward: as psgla_drunet_layer; backward: res1 = the gradient of
+ * the block's output on each first conv's adjoint, res2 = the held skip gradient on the first block's of the body and of
+ * each encoder stage); gate_dev exactly for the adjoint of each block's second conv: the forward's ELU output of that block,
+ * the conv is multiplied by elu'(z) (1 where gate > 0, else gate + 1).  All bf16 NHWC of the output's shape. */
+int psgla_gsdrunet_layer(const void* packed_dev, psgla_img_shape shape, int backward, int layer, const void* in_dev,
+                         const void* res1_dev, const void* res2_dev, const void* gate_dev, void* out_dev, void* stream);
+
 /* One general convolution layer of the DRUNet denoiser (deepinv.models.DRUNet, sampling_images.py:136) as implicit GEMM:
  *   mode 0: 3x3 stride 1 zero-pad 1 (Cin -> Cout); 1: 2x2 stride 2 (downsampling); 2: 2x2 stride 2 transposed (upsampling).
  * in_dev bf16 NHWC [B][Hin][Win][Cin]; w_dev bf16 [taps][Cout][Cin] (taps = 9 / 4 / 4, tap = ky * kw + kx);

@@ -11,8 +11,9 @@ from . import metrics  # noqa: F401
 from . import image_set  # noqa: F401
 from .image_set import load_image, run_image_set  # noqa: F401
 from .metrics import posterior_summary, psnr_ssim  # noqa: F401
-from .denoisers import (DRUNET_KEYS, DRUNet, DnCNN, TVDenoiser, lipschitz_dncnn_state_dict, random_dncnn_state_dict,  # noqa: F401
-                        random_drunet_state_dict, smoothing_dncnn_state_dict)  # noqa: F401
+from .denoisers import (DRUNET_KEYS, GSDRUNET_KEYS, DRUNet, DnCNN, GSDRUNet, TVDenoiser, lipschitz_dncnn_state_dict,  # noqa: F401
+                        random_dncnn_state_dict, random_drunet_state_dict, random_gsdrunet_state_dict,  # noqa: F401
+                        smoothing_dncnn_state_dict)  # noqa: F401
 from .operators import (DeblurDataGrad, InpaintingDataGrad, PriorGrad, blur_taps, make_deblurring,  # noqa: F401
                         make_inpainting)
 from .params import as_pnpula_kwargs, as_psgla_kwargs, sampler_params  # noqa: F401

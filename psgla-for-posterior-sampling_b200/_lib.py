@@ -107,6 +107,13 @@ SIGNATURES = {
     "psgla_drunet_denoise_post_next": (_int, [_vp, ImgShape, _vp, _vp, _sz, _vp, C.POINTER(PostParams), _vp, _vp, _vp, _vp,
                                               C.POINTER(NextPre), _vp]),
     "psgla_drunet_layer": (_int, [_vp, ImgShape, _int, _vp, _vp, _vp, _vp, _vp]),
+    "psgla_gsdrunet_num_weights": (_int, []),
+    "psgla_gsdrunet_packed_bytes": (_sz, []),
+    "psgla_gsdrunet_pack_weights": (_int, [C.POINTER(C.POINTER(C.c_float)), _vp, _vp]),
+    "psgla_gsdrunet_workspace_bytes": (_sz, [ImgShape]),
+    "psgla_gsdrunet_denoise_post_next": (_int, [_vp, ImgShape, _vp, _vp, _vp, _sz, _vp, C.c_float, C.POINTER(PostParams), _vp,
+                                                _vp, _vp, _vp, C.POINTER(NextPre), _vp]),
+    "psgla_gsdrunet_layer": (_int, [_vp, ImgShape, _int, _int, _vp, _vp, _vp, _vp, _vp, _vp]),
     "psgla_tv_state_bytes": (_sz, [ImgShape]),
     "psgla_tv_workspace_bytes": (_sz, [ImgShape]),
     "psgla_tv_prox_post": (_int, [C.POINTER(TVParams), ImgShape, _vp, _vp, _sz, _vp, _sz, C.POINTER(PostParams), _vp, _vp, _vp,

@@ -92,6 +92,22 @@ __device__ __forceinline__ void cg_add_bf16x8(float (&f)[8], const uint4 r) {
     f[2 * i + 1] += __uint_as_float(w[i] & 0xffff0000u);
   }
 }
+// The gradient-step DRUNet's epilogues (conv_tc.cuh has the same two for the 64-channel kernel): ELU after the sum, and the
+// backward's gate f *= elu'(z), with t = the bf16 ELU output the forward stored: 1 for t > 0, else t + 1 = exp(z).
+__device__ __forceinline__ void cg_elu8(float (&f)[8]) {  // exp by MUFU, as elu8 in conv_tc.cuh explains
+#pragma unroll
+  for (int i = 0; i < 8; ++i) f[i] = f[i] > 0.f ? f[i] : __expf(f[i]) - 1.f;
+}
+__device__ __forceinline__ void cg_gate_bf16x8(float (&f)[8], const uint4 r) {
+  const uint32_t w[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const float t0 = __uint_as_float(w[i] << 16), t1 = __uint_as_float(w[i] & 0xffff0000u);
+    f[2 * i] *= t0 > 0.f ? 1.f : t0 + 1.f;
+    f[2 * i + 1] *= t1 > 0.f ? 1.f : t1 + 1.f;
+  }
+}
+enum { CG_EPI_SUM = 0, CG_EPI_ELU = 1, CG_EPI_GATE = 2 };
 
 template <int N_TILE>
 __global__ void __launch_bounds__((CgCfg<N_TILE>::THREADS), 1)
@@ -302,8 +318,10 @@ __device__ __forceinline__ CgItem cg_decode2(const CgParams& p, int item) {
 }
 
 // RES2: a second residual tensor (U-Net skip, one layer per scale) is prefetched like the first; its own instantiation,
-// so that its 64 extra registers do not weigh on the other layers.
-template <int N_TILE, bool REUSE, bool RES2, bool WRES = false>
+// so that its 64 extra registers do not weigh on the other layers.  EPI: CG_EPI_SUM (residual adds, optional ReLU),
+// CG_EPI_ELU (ELU instead of ReLU) or CG_EPI_GATE (res1 is a stored ELU output t; multiply by elu'(t) instead of adding it),
+// the last two for the gradient-step DRUNet in instantiations of their own.
+template <int N_TILE, bool REUSE, bool RES2, bool WRES = false, int EPI = CG_EPI_SUM>
 __global__ void __launch_bounds__((CgCfg2<N_TILE, REUSE, WRES>::THREADS), 1)
 conv_gemm2_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_w, const CgParams p) {
   using Cfg = CgCfg2<N_TILE, REUSE, WRES>;
@@ -540,8 +558,13 @@ conv_gemm2_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
                 float f[8];
 #pragma unroll
                 for (int i = 0; i < 8; ++i) f[i] = __uint_as_float(v[8 * j + i]);
-                if (has_res) cg_add_bf16x8(f, rr[c4 * 4 + j]);
+                if (EPI == CG_EPI_GATE) {
+                  if (has_res) cg_gate_bf16x8(f, rr[c4 * 4 + j]);
+                } else if (has_res) {
+                  cg_add_bf16x8(f, rr[c4 * 4 + j]);
+                }
                 if (RES2 && has_res2) cg_add_bf16x8(f, rr2[RES2 ? c4 * 4 + j : 0]);
+                if (EPI == CG_EPI_ELU) cg_elu8(f);
                 w[h].x = cg_pack(f[0], f[1], relu);
                 w[h].y = cg_pack(f[2], f[3], relu);
                 w[h].z = cg_pack(f[4], f[5], relu);
@@ -626,7 +649,7 @@ static int cg_launch(const CUtensorMap& ma, const CUtensorMap& mw, const CgParam
   return PSGLA_OK;
 }
 
-template <int N_TILE, bool REUSE, bool RES2, bool WRES = false>
+template <int N_TILE, bool REUSE, bool RES2, bool WRES = false, int EPI = CG_EPI_SUM>
 static int cg_launch2_t(const CUtensorMap& ma, const CUtensorMap& mw, CgParams p, cudaStream_t st) {
   using Cfg = CgCfg2<N_TILE, REUSE, WRES>;
   cudaLaunchConfig_t cfg{};
@@ -646,10 +669,10 @@ static int cg_launch2_t(const CUtensorMap& ma, const CUtensorMap& mw, CgParams p
   std::atomic<int>& mc_slot = max_clusters_dev[current_device() % kMaxDevices];
   int max_clusters = mc_slot.load(std::memory_order_acquire);
   if (!max_clusters) {
-    PSGLA_CUDA_TRY(cudaFuncSetAttribute(conv_gemm2_kernel<N_TILE, REUSE, RES2, WRES>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+    PSGLA_CUDA_TRY(cudaFuncSetAttribute(conv_gemm2_kernel<N_TILE, REUSE, RES2, WRES, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
     cfg.gridDim = dim3((unsigned)(num_sms() & ~1));
     int n = 0;
-    PSGLA_CUDA_TRY(cudaOccupancyMaxActiveClusters(&n, conv_gemm2_kernel<N_TILE, REUSE, RES2, WRES>, &cfg));
+    PSGLA_CUDA_TRY(cudaOccupancyMaxActiveClusters(&n, conv_gemm2_kernel<N_TILE, REUSE, RES2, WRES, EPI>, &cfg));
     max_clusters = n > 0 ? std::min(n, num_sms() / 2) : num_sms() / 2;
     mc_slot.store(max_clusters, std::memory_order_release);
   }
@@ -657,19 +680,22 @@ static int cg_launch2_t(const CUtensorMap& ma, const CUtensorMap& mw, CgParams p
   const int pairs = ((m_tiles + 1) / 2) * p.n_tiles_n;
   p.n_items = 2 * pairs;
   cfg.gridDim = dim3((unsigned)(2 * std::min(pairs, max_clusters)));
-  PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv_gemm2_kernel<N_TILE, REUSE, RES2, WRES>, ma, mw, p));
+  PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv_gemm2_kernel<N_TILE, REUSE, RES2, WRES, EPI>, ma, mw, p));
   return PSGLA_OK;
 }
 
 template <int N_TILE, bool REUSE, bool WRES = false>
-static int cg_launch2(const CUtensorMap& ma, const CUtensorMap& mw, const CgParams& p, cudaStream_t st) {
+static int cg_launch2(const CUtensorMap& ma, const CUtensorMap& mw, const CgParams& p, cudaStream_t st, int act) {
+  if (act == ACT_ELU) return cg_launch2_t<N_TILE, REUSE, false, WRES, CG_EPI_ELU>(ma, mw, p, st);
+  if (act == ACT_GATE) return cg_launch2_t<N_TILE, REUSE, false, WRES, CG_EPI_GATE>(ma, mw, p, st);
   return p.res2 ? cg_launch2_t<N_TILE, REUSE, true, WRES>(ma, mw, p, st) : cg_launch2_t<N_TILE, REUSE, false, WRES>(ma, mw, p, st);
 }
 
 // One layer.  in: bf16 NHWC [B][Hin][Win][Cin]; w: bf16 [taps][Cout][Cin]; out: bf16 NHWC (CONV3: same extent, DOWN2:
-// half, UP2: double); res1 / res2: optional tensors of the output's shape added before the optional ReLU.
+// half, UP2: double); res1 / res2: optional tensors of the output's shape added before the optional ReLU.  act: ConvAct;
+// ACT_ELU and ACT_GATE (res1 = the gate's ELU output, no res2) run on the 3x3 CTA-pair kernels only.
 int conv_gemm_layer(int mode, int B, int Hin, int Win, int Cin, int Cout, const void* w, const void* in, const void* res1,
-                    const void* res2, void* out, int relu, cudaStream_t st) {
+                    const void* res2, void* out, int act, cudaStream_t st) {
   PSGLA_REQUIRE(mode >= CG_CONV3 && mode <= CG_UP2, "conv_gemm_layer: unknown mode %d", mode);
   PSGLA_REQUIRE(B > 0 && Hin > 0 && Win > 0 && Cin >= 64 && Cin % 64 == 0 && Cout >= 64 && Cout % 64 == 0,
                 "conv_gemm_layer: channels must be multiples of 64 (got %d -> %d), extents positive", Cin, Cout);
@@ -677,6 +703,8 @@ int conv_gemm_layer(int mode, int B, int Hin, int Win, int Cin, int Cout, const 
   PSGLA_REQUIRE(((uintptr_t)out | (uintptr_t)res1 | (uintptr_t)res2) % 32 == 0 && (uintptr_t)in % 16 == 0 && (uintptr_t)w % 16 == 0,
                 "conv_gemm_layer: out / residual tensors must be 32-byte aligned, in / weights 16-byte aligned");
   PSGLA_REQUIRE(mode != CG_DOWN2 || (Hin % 2 == 0 && Win % 2 == 0), "stride-2 conv needs even extents (got %d x %d)", Hin, Win);
+  PSGLA_REQUIRE(act == ACT_NONE || act == ACT_RELU || (mode == CG_CONV3 && Cout % 128 == 0 && !res2 && (act == ACT_ELU ? !res1 : act == ACT_GATE && res1)),
+                "conv_gemm_layer: the ELU / gate epilogues are for 3x3 layers of 128k channels (ELU: no residual; gate: res1 only)");
   CgParams p{};
   p.mode = mode;
   p.taps = mode == CG_CONV3 ? 9 : (mode == CG_DOWN2 ? 4 : 1);
@@ -704,7 +732,7 @@ int conv_gemm_layer(int mode, int B, int Hin, int Win, int Cin, int Cout, const 
   p.reverse = pair ? next_layer_direction() : 0;
   p.n_tiles_n = n_cols / n_tile;
   p.n_items = B * p.tiles_y * p.tiles_x * p.n_tiles_n;
-  p.relu = relu;
+  p.relu = act == ACT_RELU;
   p.res1 = (const __nv_bfloat16*)res1;
   p.res2 = (const __nv_bfloat16*)res2;
   p.out = (__nv_bfloat16*)out;
@@ -733,9 +761,9 @@ int conv_gemm_layer(int mode, int B, int Hin, int Win, int Cin, int Cout, const 
   }
   if (rc) return rc;
   // resident weights for the 128 -> 128 channel layers (CgCfg2<128, true, true>)
-  if (reuse && Cin == 128 && Cout == 128) return cg_launch2<128, true, true>(ma, mw, p, st);
-  if (reuse) return n_tile == 256 ? cg_launch2<256, true>(ma, mw, p, st) : cg_launch2<128, true>(ma, mw, p, st);
-  if (pair) return n_tile == 256 ? cg_launch2<256, false>(ma, mw, p, st) : cg_launch2<128, false>(ma, mw, p, st);
+  if (reuse && Cin == 128 && Cout == 128) return cg_launch2<128, true, true>(ma, mw, p, st, act);
+  if (reuse) return n_tile == 256 ? cg_launch2<256, true>(ma, mw, p, st, act) : cg_launch2<128, true>(ma, mw, p, st, act);
+  if (pair) return n_tile == 256 ? cg_launch2<256, false>(ma, mw, p, st, act) : cg_launch2<128, false>(ma, mw, p, st, act);
   return cg_launch<64>(ma, mw, p, st);
 }
 
@@ -745,5 +773,6 @@ using namespace psgla;
 
 extern "C" int psgla_convg_layer(int mode, int B, int Hin, int Win, int Cin, int Cout, const void* w_dev, const void* in_dev,
                                  const void* res1_dev, const void* res2_dev, void* out_dev, int relu, void* stream) {
-  return conv_gemm_layer(mode, B, Hin, Win, Cin, Cout, w_dev, in_dev, res1_dev, res2_dev, out_dev, relu, (cudaStream_t)stream);
+  return conv_gemm_layer(mode, B, Hin, Win, Cin, Cout, w_dev, in_dev, res1_dev, res2_dev, out_dev, relu ? ACT_RELU : ACT_NONE,
+                         (cudaStream_t)stream);
 }

@@ -369,7 +369,10 @@ struct ConvTs2Cfg {
 
 // RES: the layer has a residual input and fetches it by TMA (epilogue_hidden_tmares), RES = 2: and a second one (the U-Net
 // skip tensor, per-thread loads); separate instantiations so that the plain layers (all of DnCNN) keep their own register
-// allocation and code (sharing one kernel cost them 5 %, ncu), and the single-residual layers theirs.
+// allocation and code (sharing one kernel cost them 5 %, ncu), and the single-residual layers theirs.  The gradient-step
+// DRUNet adds two more: TS_GATE (the TMA-fetched tensor is an ELU output t and the sum is multiplied by elu'(t)) and TS_ELU
+// (no residual, ELU instead of ReLU).
+constexpr int TS_GATE = 3, TS_ELU = 4;
 template <int NOUT, int RES>
 __global__ void __launch_bounds__(TS_THREADS, 1)
 conv3x3_ts2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_out,
@@ -413,7 +416,7 @@ conv3x3_ts2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
     mbar_init(wbar, 1);
     mbar_init(wready, 1);
     mbar_init(done, 1);
-    if (RES)
+    if (RES && RES != TS_ELU)
       for (int i = 0; i < 2 * EPI_WARPS; ++i) mbar_init(&rbar[i], 1);
     fence_barrier_init();
   }
@@ -546,12 +549,13 @@ conv3x3_ts2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
   } else {
     // ---------------------------------------------------------------- epilogue: 2 groups x 4 warps
     const int ew = warp - 6;
-    if (RES)
-      epilogue_hidden_tmares<NOUT, TS_NACC, RES == 2>(p, &tmap_out, &tmap_res, smem + Cfg::OFF_STAGE + ew * Cfg::STAGE_BYTES,
+    if (RES && RES != TS_ELU)
+      epilogue_hidden_tmares<NOUT, TS_NACC, RES == 2, RES == TS_GATE>(p, &tmap_out, &tmap_res,
+                                            smem + Cfg::OFF_STAGE + ew * Cfg::STAGE_BYTES,
                                             rbar + 2 * ew, bias_s, tfull, tempty, tmem_base, ew >> 2, warp & 3, lane, tempty_c);
     else
-      epilogue_hidden<NOUT, TS_NACC>(p, &tmap_out, smem + Cfg::OFF_STAGE + ew * Cfg::STAGE_BYTES, bias_s, tfull, tempty,
-                                     tmem_base, ew >> 2, warp & 3, lane, tempty_c);
+      epilogue_hidden<NOUT, TS_NACC, RES == TS_ELU>(p, &tmap_out, smem + Cfg::OFF_STAGE + ew * Cfg::STAGE_BYTES, bias_s, tfull,
+                                                    tempty, tmem_base, ew >> 2, warp & 3, lane, tempty_c);
   }
   tc_fence_before();
   cluster_sync();  // neither CTA may exit (or free tensor memory) while its partner can still signal or read it
@@ -762,8 +766,11 @@ static int launch_conv_ts2_t(const void* in, void* out_bf16, ConvParams p, cudaS
   return PSGLA_OK;
 }
 
-// The hidden 64 -> 64 channel layers, with up to two residual inputs
-static int launch_hidden64(const void* in, void* out, const ConvParams& p, cudaStream_t st) {
+// The hidden 64 -> 64 channel layers, with up to two residual inputs, or (act ACT_ELU / ACT_GATE) the gradient-step DRUNet's
+// ELU and gate epilogues
+static int launch_hidden64(const void* in, void* out, const ConvParams& p, cudaStream_t st, int act = ACT_NONE) {
+  if (act == ACT_ELU) return launch_conv_ts2_t<64, TS_ELU>(in, out, p, st);
+  if (act == ACT_GATE) return launch_conv_ts2_t<64, TS_GATE>(in, out, p, st);
   if (!p.res1) return launch_conv_ts2_t<64, 0>(in, out, p, st);
   return p.res2 ? launch_conv_ts2_t<64, 2>(in, out, p, st) : launch_conv_ts2_t<64, 1>(in, out, p, st);
 }
@@ -987,17 +994,17 @@ int next_layer_direction() {
   return dir;
 }
 
-int conv64_hidden(const void* in, void* out, const uint8_t* w, const float* bias, int B, int H, int W, int relu,
+int conv64_hidden(const void* in, void* out, const uint8_t* w, const float* bias, int B, int H, int W, int act,
                   const void* res1, const void* res2, cudaStream_t st) {
   ConvParams p{};
   p.B = B, p.H = H, p.W = W;
   p.reverse = next_layer_direction();
   p.weights = w;
   p.bias = bias;
-  p.relu = relu;
+  p.relu = act == ACT_RELU;
   p.res1 = (const __nv_bfloat16*)res1;
   p.res2 = (const __nv_bfloat16*)res2;
-  return launch_hidden64(in, out, p, st);
+  return launch_hidden64(in, out, p, st, act);
 }
 
 int conv_first16(const void* in16, void* out, const uint8_t* w, const float* bias, int B, int H, int W, int relu,

@@ -31,6 +31,24 @@ __device__ __forceinline__ void add_bf16x8(float (&f)[8], const uint4 r) {
     f[2 * i + 1] += __uint_as_float(w[i] & 0xffff0000u);
   }
 }
+// ELU (alpha = 1) in place: z for z > 0, exp(z) - 1 otherwise (the gradient-step DRUNet's block activation).  exp by the
+// MUFU approximation: its ~1e-7 absolute error near 0 is far below the bf16 output's rounding and the conv's own error bound;
+// expm1f, inlined per element, made the forward's ELU layers slower than the whole backward.
+__device__ __forceinline__ void elu8(float (&f)[8]) {
+#pragma unroll
+  for (int i = 0; i < 8; ++i) f[i] = f[i] > 0.f ? f[i] : __expf(f[i]) - 1.f;
+}
+// f *= elu'(z) with t = bf16 ELU(z) as the forward stored it: elu'(z) = 1 for t > 0, else exp(z) = t + 1.  The backward of a
+// residual block's activation, so that no pre-activation has to be kept.
+__device__ __forceinline__ void gate_bf16x8(float (&f)[8], const uint4 r) {
+  const uint32_t w[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const float t0 = __uint_as_float(w[i] << 16), t1 = __uint_as_float(w[i] & 0xffff0000u);
+    f[2 * i] *= t0 > 0.f ? 1.f : t0 + 1.f;
+    f[2 * i + 1] *= t1 > 0.f ? 1.f : t1 + 1.f;
+  }
+}
 
 // The 8 biases of 16-byte output chunk j.  The epilogues fetch them ONE CHUNK AHEAD with explicit shared-space loads: through a
 // generic pointer they compile to LD.E, and placed after the previous chunk's staging store (a "memory"-clobbering asm
@@ -149,7 +167,8 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float a, float b, bool relu) {
 // TMA store of 32 pixels x NOUT channels per warp and row (clipped at the image edge by the tensor map).  The warp alternates
 // between two staging boxes, so a row is staged while the previous row's TMA store is still reading its box (the store's
 // read latency otherwise serialises with the warp's work on every row).
-template <int NOUT, int NACC_>
+// ELU: apply ELU instead of the optional ReLU (gradient-step DRUNet forward, its own instantiation).
+template <int NOUT, int NACC_, bool ELU = false>
 __device__ __forceinline__ void epilogue_hidden(const ConvParams& p, const CUtensorMap* tmap_out, uint8_t* stage,
                                                 const float* bias_s, uint64_t* tfull, uint64_t* tempty,
                                                 uint32_t tmem_base, int grp, int q4, int lane, uint32_t tempty_cluster = 0) {
@@ -194,6 +213,7 @@ __device__ __forceinline__ void epilogue_hidden(const ConvParams& p, const CUten
                       __uint_as_float(v[8 * j + 2]) + b0.z, __uint_as_float(v[8 * j + 3]) + b0.w,
                       __uint_as_float(v[8 * j + 4]) + b1.x, __uint_as_float(v[8 * j + 5]) + b1.y,
                       __uint_as_float(v[8 * j + 6]) + b1.z, __uint_as_float(v[8 * j + 7]) + b1.w};
+        if (ELU) elu8(f);
         uint4 o;
         o.x = pack_bf16x2(f[0], f[1], relu);
         o.y = pack_bf16x2(f[2], f[3], relu);
@@ -221,7 +241,9 @@ __device__ __forceinline__ void epilogue_hidden(const ConvParams& p, const CUten
 // ahead; the lanes then read-modify-write the box in shared memory and the TMA store ships it.  Box ownership: the load for
 // row n + 1 into box b' is issued after cp.async.bulk.wait_group.read 1, i.e. once the store of row n - 1 has finished
 // reading b'; generic writes precede the store by fence.proxy.async as before.
-template <int NOUT, int NACC_, bool RES2>
+// GATE (gradient-step DRUNet backward, its own instantiation, no RES2): the box holds a stored ELU output t and the sum is
+// multiplied by elu'(t) instead of added to it.
+template <int NOUT, int NACC_, bool RES2, bool GATE = false>
 __device__ __forceinline__ void epilogue_hidden_tmares(const ConvParams& p, const CUtensorMap* tmap_out,
                                                        const CUtensorMap* tmap_res, uint8_t* stage, uint64_t* rbar,
                                                        const float* bias_s, uint64_t* tfull, uint64_t* tempty,
@@ -340,7 +362,11 @@ __device__ __forceinline__ void epilogue_hidden_tmares(const ConvParams& p, cons
 #pragma unroll
         for (int i = 0; i < RB; ++i) rr[i] = ld_shared_v4_nc(stage_row + ((uint32_t)((j + i) ^ (lane & 7)) << 4));
       }
-      if (row_has) add_bf16x8(f, rr[j % RB]);
+      if (GATE) {
+        if (row_has) gate_bf16x8(f, rr[j % RB]);
+      } else if (row_has) {
+        add_bf16x8(f, rr[j % RB]);
+      }
       if (RES2 && has_res2) add_bf16x8(f, rr2[RES2 ? j : 0]);
       uint4 o;
       o.x = pack_bf16x2(f[0], f[1], relu);

@@ -15,8 +15,6 @@
 
 namespace psgla {
 
-enum DruKind { DRU_HEAD, DRU_C64, DRU_GEMM3, DRU_DOWN, DRU_UP, DRU_TAIL };
-
 struct DruLayer {
   DruKind kind;
   int cin, cout;
@@ -26,7 +24,7 @@ struct DruLayer {
   size_t w_off, bytes;
 };
 
-static size_t dru_layer_bytes(DruKind k, int cin, int cout) {
+size_t dru_layer_bytes(DruKind k, int cin, int cout) {
   size_t b = 0;
   switch (k) {
     case DRU_HEAD: b = (size_t)9 * 64 * 16 * 2 + 64 * 4; break;   // swizzled weights + (zero) bias
@@ -78,6 +76,32 @@ static inline uint16_t dru_bf16(float f) {
   if ((u & 0x7fffffffu) > 0x7f800000u) return (uint16_t)((u >> 16) | 0x40);
   u += 0x7fffu + ((u >> 16) & 1u);
   return (uint16_t)(u >> 16);
+}
+
+void dru_pack_layer(DruKind kind, const float* w, int cin, int cout, uint8_t* dst) {
+  switch (kind) {
+    case DRU_HEAD: pack_conv3x3_swizzled(w, 64, cin, 64, 16, dst); break;
+    case DRU_C64: pack_conv3x3_swizzled(w, 64, 64, 64, 64, dst); break;
+    case DRU_TAIL: pack_conv3x3_swizzled(w, cout, 64, 16, 64, dst); break;
+    case DRU_GEMM3:  // OIHW [cout][cin][3][3] -> [tap][cout][cin]
+    case DRU_DOWN: {  // OIHW [cout][cin][2][2] -> [tap][cout][cin]
+      const int taps = kind == DRU_GEMM3 ? 9 : 4;
+      uint16_t* d = reinterpret_cast<uint16_t*>(dst);
+      for (int n = 0; n < cout; ++n)
+        for (int k = 0; k < cin; ++k)
+          for (int t = 0; t < taps; ++t)
+            d[((size_t)t * cout + n) * cin + k] = dru_bf16(w[((size_t)n * cin + k) * taps + t]);
+      break;
+    }
+    case DRU_UP: {  // ConvTranspose2d weight [cin][cout][2][2] -> [quadrant][cout][cin]
+      uint16_t* d = reinterpret_cast<uint16_t*>(dst);
+      for (int k = 0; k < cin; ++k)
+        for (int n = 0; n < cout; ++n)
+          for (int t = 0; t < 4; ++t)
+            d[((size_t)t * cout + n) * cin + k] = dru_bf16(w[((size_t)k * cout + n) * 4 + t]);
+      break;
+    }
+  }
 }
 
 struct DruBuffers {
@@ -153,30 +177,7 @@ extern "C" int psgla_drunet_pack_weights(const float* const* weights_host, void*
     const DruLayer& L = plan[l];
     const float* w = weights_host[l];
     PSGLA_REQUIRE(w != nullptr, "DRUNet weight tensor %zu is null", l);
-    uint8_t* dst = host.data() + L.w_off;
-    switch (L.kind) {
-      case DRU_HEAD: pack_conv3x3_swizzled(w, 64, 4, 64, 16, dst); break;
-      case DRU_C64: pack_conv3x3_swizzled(w, 64, 64, 64, 64, dst); break;
-      case DRU_TAIL: pack_conv3x3_swizzled(w, 3, 64, 16, 64, dst); break;
-      case DRU_GEMM3:  // OIHW [cout][cin][3][3] -> [tap][cout][cin]
-      case DRU_DOWN: {  // OIHW [cout][cin][2][2] -> [tap][cout][cin]
-        const int taps = L.kind == DRU_GEMM3 ? 9 : 4;
-        uint16_t* d = reinterpret_cast<uint16_t*>(dst);
-        for (int n = 0; n < L.cout; ++n)
-          for (int k = 0; k < L.cin; ++k)
-            for (int t = 0; t < taps; ++t)
-              d[((size_t)t * L.cout + n) * L.cin + k] = dru_bf16(w[((size_t)n * L.cin + k) * taps + t]);
-        break;
-      }
-      case DRU_UP: {  // ConvTranspose2d weight [cin][cout][2][2] -> [quadrant][cout][cin]
-        uint16_t* d = reinterpret_cast<uint16_t*>(dst);
-        for (int k = 0; k < L.cin; ++k)
-          for (int n = 0; n < L.cout; ++n)
-            for (int t = 0; t < 4; ++t)
-              d[((size_t)t * L.cout + n) * L.cin + k] = dru_bf16(w[((size_t)k * L.cout + n) * 4 + t]);
-        break;
-      }
-    }
+    dru_pack_layer(L.kind, w, L.cin, L.cout, host.data() + L.w_off);
   }
   PSGLA_CUDA_TRY(cudaMemcpyAsync(packed_dev, host.data(), host.size(), cudaMemcpyHostToDevice, (cudaStream_t)stream));
   PSGLA_CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));  // `host` dies at return

@@ -1,5 +1,6 @@
-"""The image denoisers: DnCNN and DRUNet as tcgen05 implicit-GEMM convolutions (csrc/conv_tc.cu, csrc/conv_gemm.cu), and
-the TV proximal operator (csrc/tv_prox.cu).
+"""The image denoisers: DnCNN, DRUNet and the gradient-step DRUNet (its network and the network's vector-Jacobian product,
+csrc/gsdrunet.cu) as tcgen05 implicit-GEMM convolutions (csrc/conv_tc.cu, csrc/conv_gemm.cu), and the TV proximal operator
+(csrc/tv_prox.cu).
 
 ``DnCNN`` mirrors ``deepinv.models.DnCNN(in_channels=3, out_channels=3, pretrained=..., device=...)`` as the reference constructs
 it (sampling_images.py:130) and calls it (``denoiser.forward(x, sigma)``, restoration_algorithms.py:238): depth 20,
@@ -16,8 +17,8 @@ import torch
 
 from . import _lib
 
-__all__ = ["DnCNN", "DRUNet", "TVDenoiser", "random_dncnn_state_dict", "lipschitz_dncnn_state_dict", "smoothing_dncnn_state_dict",
-           "random_drunet_state_dict", "DRUNET_KEYS"]
+__all__ = ["DnCNN", "DRUNet", "GSDRUNet", "TVDenoiser", "random_dncnn_state_dict", "lipschitz_dncnn_state_dict",
+           "smoothing_dncnn_state_dict", "random_drunet_state_dict", "random_gsdrunet_state_dict", "DRUNET_KEYS", "GSDRUNET_KEYS"]
 
 
 def random_dncnn_state_dict(seed=0, depth=20, nf=64, scale=1.0):
@@ -187,6 +188,7 @@ def _drunet_keys(nb=4):
 
 
 DRUNET_KEYS = _drunet_keys()  # the 64 weight tensors of drunet_color.pth in state-dict order
+GSDRUNET_KEYS = _drunet_keys(2)  # the 36 of the gradient-step DRUNet's network (nb = 2)
 
 
 def _drunet_shape(key, nc=(64, 128, 256, 512)):
@@ -204,12 +206,13 @@ def _drunet_shape(key, nc=(64, 128, 256, 512)):
     return (nc[s], nc[s - 1], 2, 2)      # transposed conv: [Cin][Cout][2][2]
 
 
-def random_drunet_state_dict(seed=0, gain=0.5):
+def random_drunet_state_dict(seed=0, gain=0.5, nb=4):
     """Seeded random-init DRUNet state dict on the CPU (checkpoints are unreachable offline): uniform
-    +-gain*sqrt(3/fan_in), second conv of every residual block halved, tail quartered, so activations stay O(1)."""
+    +-gain*sqrt(3/fan_in), second conv of every residual block halved, tail quartered, so activations stay O(1).
+    ``nb``: residual blocks per stage (2: the gradient-step DRUNet's network)."""
     g = torch.Generator().manual_seed(seed)
     sd = {}
-    for k in DRUNET_KEYS:
+    for k in _drunet_keys(nb):
         shp = _drunet_shape(k)
         is_up = k.startswith("m_up") and ".res." not in k
         fan_in = shp[0] * 4 if is_up else shp[1] * shp[2] * shp[3]
@@ -303,6 +306,122 @@ class DRUNet:
                        "psgla_img_to_nhwc16")
         self.apply_post(shape, den_in, x, _lib.PostParams(1.0, 0.0, 0.0, 1.0), out)  # out = 0 * x + 1 * D(x)
         return out[:, :, :H0, :W0].contiguous() if (ph or pw) else out
+
+    __call__ = forward
+
+
+# ----------------------------------------------------------------------------------------------------- GSDRUNet
+def random_gsdrunet_state_dict(seed=0, gain=0.5):
+    """Seeded random-init state dict of the gradient-step DRUNet's network (``random_drunet_state_dict`` with nb = 2)."""
+    return random_drunet_state_dict(seed, gain, nb=2)
+
+
+_GS_PREFIX = "student_grad.model."
+
+
+def gsdrunet_weights(sd):
+    """The 36 fp32 CPU tensors of GSDRUNET_KEYS from a state dict with KAIR keys.  A ``{"state_dict": ...}`` wrapper and
+    the ``student_grad.model.`` prefix of deepinv's GSDRUNet module are stripped (both forms recalled, not verified against a
+    deepinv checkpoint)."""
+    if "state_dict" in sd and isinstance(sd["state_dict"], dict):
+        sd = sd["state_dict"]
+    sd = {(k[len(_GS_PREFIX):] if k.startswith(_GS_PREFIX) else k): v for k, v in sd.items()}
+    missing = [k for k in GSDRUNET_KEYS if k not in sd]
+    if missing:
+        raise KeyError("state dict lacks %s" % missing[:3])
+    ws = []
+    for k in GSDRUNET_KEYS:
+        w = sd[k].detach().to("cpu", torch.float32).contiguous()
+        if tuple(w.shape) != _drunet_shape(k):
+            raise ValueError("%s has shape %s, expected %s" % (k, tuple(w.shape), _drunet_shape(k)))
+        ws.append(w)
+    return ws
+
+
+class GSDRUNet:
+    """``deepinv.models.GSDRUNet(alpha=1.0, in_channels=3, out_channels=3, nb=2, nc=[64,128,256,512], act_mode="E",
+    pretrained=..., device=...)``, the gradient-step denoiser (Prox-DRUNet is the same class from another checkpoint):
+    ``D(x; sigma) = x - alpha grad g(x)`` with ``g(x) = 1/2 ||x - N(x)||^2`` and N the KAIR U-Net with 2 residual blocks per
+    stage, ELU inside the blocks and no biases.  Each call runs N and its vector-Jacobian product on tcgen05 convolutions
+    (csrc/gsdrunet.cu).  ``pretrained``: None (seeded random init), a checkpoint path or a state dict.  H, W multiples of 8."""
+
+    is_residual = False  # D(x) itself
+
+    def __init__(self, alpha=1.0, in_channels=3, out_channels=3, nb=2, nc=(64, 128, 256, 512), act_mode="E", pretrained=None,
+                 device=None):
+        if in_channels != 3 or out_channels != 3 or nb != 2 or list(nc) != [64, 128, 256, 512] or act_mode != "E":
+            raise ValueError("the sm_100a GSDRUNet path is built for in = out = 3 channels, nb = 2, nc = [64, 128, 256, 512], "
+                             "act_mode = 'E'")
+        self.alpha = float(alpha)
+        if not math.isfinite(self.alpha):
+            raise ValueError("alpha must be finite")
+        torch_ = _lib.require_cuda()
+        self.device = torch_.device("cuda", torch_.cuda.current_device()) if device is None else torch_.device(device)
+        if pretrained is None:
+            sd = random_gsdrunet_state_dict(0)
+        elif isinstance(pretrained, str):
+            sd = torch_.load(pretrained, map_location="cpu")
+        else:
+            sd = pretrained
+        ws = gsdrunet_weights(sd)
+        self.state_dict_fp32 = dict(zip(GSDRUNET_KEYS, ws))
+        lib = _lib.lib()
+        assert lib.psgla_gsdrunet_num_weights() == len(ws)
+        self.packed = torch_.empty(lib.psgla_gsdrunet_packed_bytes(), dtype=torch_.uint8, device=self.device)
+        FP = C.POINTER(C.c_float)
+        warr = (FP * len(ws))(*[C.cast(w.data_ptr(), FP) for w in ws])
+        with torch_.cuda.device(self.device):
+            _lib.check(lib.psgla_gsdrunet_pack_weights(warr, _lib.ptr(self.packed), _lib.stream_ptr(self.device)),
+                       "psgla_gsdrunet_pack_weights")
+        self._ws = None
+        self._den_in = None
+
+    @staticmethod
+    def check_size(H, W):
+        if H % 8 or W % 8:
+            raise ValueError("GSDRUNet needs H and W to be multiples of 8 (got %d x %d): crop the image; the gradient through "
+                             "a padded input is not implemented" % (H, W))
+
+    def buffers(self, shape: "_lib.ImgShape"):
+        need = _lib.lib().psgla_gsdrunet_workspace_bytes(shape)
+        if need == 0:
+            raise ValueError("bad image shape for GSDRUNet")
+        if self._ws is None or self._ws.numel() < need:
+            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        n_in = shape.B * shape.H * shape.W * 16
+        if self._den_in is None or self._den_in.numel() < n_in:
+            self._den_in = torch.empty(n_in, dtype=torch.bfloat16, device=self.device)
+        return self._ws, self._den_in
+
+    def apply_post(self, shape, den_in, base, post, x_out, sample=None, mean=None, mean2=None, next_pre=None, x=None):
+        """x_out = post.base_scale * base + post.gain * D(x), thinning, moments, optional fused next pre.  ``den_in``: bf16
+        NHWC16 of x with the sigma map in channel 3; ``x``: x in fp32, None when it is ``base`` (PSGLA)."""
+        ws, _ = self.buffers(shape)
+        with torch.cuda.device(self.device):
+            rc = _lib.lib().psgla_gsdrunet_denoise_post_next(_lib.ptr(self.packed), shape, _lib.ptr(den_in), _lib.ptr(x),
+                                                             _lib.ptr(ws), ws.numel(), _lib.ptr(base), self.alpha, C.byref(post),
+                                                             _lib.ptr(x_out), _lib.ptr(sample), _lib.ptr(mean), _lib.ptr(mean2),
+                                                             C.byref(next_pre) if next_pre is not None else None,
+                                                             _lib.stream_ptr(self.device))
+        _lib.check(rc, "psgla_gsdrunet_denoise_post_next")
+
+    def forward(self, x, sigma):
+        """D(x; sigma), fp32 [B,3,H,W] in and out, H and W multiples of 8."""
+        if not x.is_cuda:
+            raise RuntimeError("GSDRUNet.forward needs a CUDA tensor: there is no CPU path")
+        if x.dim() != 4 or x.shape[1] != 3:
+            raise ValueError("expected a [B,3,H,W] colour batch, got %s" % (tuple(x.shape),))
+        self.check_size(int(x.shape[2]), int(x.shape[3]))
+        sigma = float(sigma.reshape(-1)[0]) if isinstance(sigma, torch.Tensor) else float(sigma)
+        x = x.to(self.device, torch.float32).contiguous()
+        shape = _lib.ImgShape(int(x.shape[0]), 3, int(x.shape[2]), int(x.shape[3]))
+        _, den_in = self.buffers(shape)
+        out = torch.empty_like(x)
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().psgla_img_to_nhwc16(shape, _lib.ptr(x), sigma, _lib.ptr(den_in), _lib.stream_ptr(self.device)),
+                       "psgla_img_to_nhwc16")
+        self.apply_post(shape, den_in, x, _lib.PostParams(1.0, 0.0, 0.0, 1.0), out)  # out = 0 * x + 1 * D(x)
+        return out
 
     __call__ = forward
 

@@ -14,7 +14,7 @@ import torch
 
 from . import dist as _dist
 from . import metrics as _metrics
-from .denoisers import DnCNN, TVDenoiser
+from .denoisers import DnCNN, GSDRUNet, TVDenoiser
 from .operators import PriorGrad, make_deblurring, make_inpainting
 from .params import as_pnpula_kwargs, as_psgla_kwargs, sampler_params
 from .restoration_algorithms import pnpula, psgla
@@ -97,7 +97,7 @@ def run_image_set(images, denoiser=None, problem="inpainting", alg="psgla", n_ch
     """Posterior sampling of a SET of images, ``n_chains`` independent chains each, sharded over the process group.
 
     images     list of [3, H, W] / [1, 3, H, W] float tensors in [0, 1] (sizes may differ), the same list on every rank
-    denoiser   this rank's ``psgla_b200.DnCNN`` / ``DRUNet`` / ``TVDenoiser`` (default: a DnCNN with the library's seeded
+    denoiser   this rank's ``psgla_b200.DnCNN`` / ``DRUNet`` / ``GSDRUNet`` / ``TVDenoiser`` (default: a DnCNN with the library's seeded
                weights; TV: psgla only, table row ``den="TV"``, the prox state is reset before each image)
     params     the dict of ``psgla_b200.sampler_params`` (default: the script's table for ``alg`` / the denoiser family, with
                ``N = n_iter`` when given)
@@ -107,7 +107,8 @@ def run_image_set(images, denoiser=None, problem="inpainting", alg="psgla", n_ch
     if _sample is None:
         if denoiser is None:
             denoiser = DnCNN()
-        den_name = "DnCNN" if isinstance(denoiser, DnCNN) else ("TV" if isinstance(denoiser, TVDenoiser) else "DRUNet")
+        den_name = ("DnCNN" if isinstance(denoiser, DnCNN) else "TV" if isinstance(denoiser, TVDenoiser)
+                    else "GSDRUNet" if isinstance(denoiser, GSDRUNet) else "DRUNet")
         prm = dict(params) if params is not None else sampler_params("pnp_ula" if alg in ("pnp_ula", "pnpula") else alg, den=den_name,
                                                                      sigma=sigma, N=n_iter)
         if n_iter is not None:

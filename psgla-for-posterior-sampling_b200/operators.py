@@ -94,7 +94,7 @@ class PriorGrad:
 
     def __init__(self, denoiser, alpha, s1, s2):
         if isinstance(denoiser, TVDenoiser):
-            raise TypeError("PriorGrad supports a psgla_b200.DnCNN or psgla_b200.DRUNet denoiser, not the TV prox")
+            raise TypeError("PriorGrad supports a psgla_b200.DnCNN, DRUNet or GSDRUNet denoiser, not the TV prox")
         self.denoiser, self.alpha, self.s1, self.s2 = denoiser, float(alpha), float(s1), float(s2)
 
     def __call__(self, x):

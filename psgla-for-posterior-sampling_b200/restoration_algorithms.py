@@ -20,8 +20,9 @@ Extra keyword-only arguments:
                  device, so ``Xlist_mmse`` / ``Xlist_mmse2`` hold ONE tensor each: the mean over windows the reference's
                  post-processing forms anyway, sampling_images.py:427,436).  What batched runs (64 chains per image) need:
                  memory independent of n_iter.
-The data term must be an ``InpaintingDataGrad`` / ``DeblurDataGrad`` and the denoiser a ``psgla_b200.DnCNN`` / ``DRUNet``
-(``prior_grad`` a ``PriorGrad`` wrapping one); opaque callables raise ``TypeError`` -- there is no eager fallback.
+The data term must be an ``InpaintingDataGrad`` / ``DeblurDataGrad`` and the denoiser a ``psgla_b200.DnCNN`` / ``DRUNet`` /
+``GSDRUNet`` (``prior_grad`` a ``PriorGrad`` wrapping one); opaque callables raise ``TypeError`` -- there is no eager fallback.
+``GSDRUNet`` needs image sides that are multiples of 8.
 ``psgla`` / ``psgla_run`` / ``pnp`` also take a ``psgla_b200.TVDenoiser`` (PSGLA-TV): each iteration is then the "pre" launch and
 one cooperative launch of the TV prox with the post fused (csrc/tv_prox.cu), at any image size.  ``pnpula`` and ``red`` feed
 the denoiser X instead of the fp32 base and reject it.
@@ -36,7 +37,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .denoisers import DRUNet, DnCNN, TVDenoiser
+from .denoisers import DRUNet, DnCNN, GSDRUNet, TVDenoiser
 from .operators import DeblurDataGrad, InpaintingDataGrad, PriorGrad
 
 __all__ = ["psgla", "pnpula", "pnp_ula", "psgla_run", "pnpula_run", "pnp", "red"]
@@ -58,8 +59,8 @@ class _Run:
         if not isinstance(data_grad, (InpaintingDataGrad, DeblurDataGrad)):
             raise TypeError("data_grad must be an InpaintingDataGrad or DeblurDataGrad (structured callable); an opaque "
                             "callable cannot be fused into the CUDA kernels and there is no eager fallback")
-        if not isinstance(denoiser, (DnCNN, DRUNet, TVDenoiser)):
-            raise TypeError("denoiser must be a psgla_b200.DnCNN, psgla_b200.DRUNet or (psgla / pnp only) psgla_b200.TVDenoiser")
+        if not isinstance(denoiser, (DnCNN, DRUNet, GSDRUNet, TVDenoiser)):
+            raise TypeError("denoiser must be a psgla_b200.DnCNN, DRUNet, GSDRUNet or (psgla / pnp only) TVDenoiser")
         if seed is None and noise is None:
             raise ValueError("seed=None: the reference fails with UnboundLocalError here "
                              "(restoration_algorithms.py:211-213,232); pass a seed or a noise tensor")
@@ -82,6 +83,8 @@ class _Run:
         # network application (psgla_img_pad_replicate_nhwc16) -- and every returned tensor is cropped.  Inpainting only: the
         # circular blur of the deblurring problem is defined on the true image size.
         self.crop = None
+        if isinstance(denoiser, GSDRUNet):
+            denoiser.check_size(int(x.shape[2]), int(x.shape[3]))
         if isinstance(denoiser, DRUNet) and (x.shape[2] % 8 or x.shape[3] % 8):
             if not isinstance(data_grad, InpaintingDataGrad):
                 raise RuntimeError("DRUNet needs H and W to be multiples of 8 for deblurring problems (crop the image, e.g. "
@@ -245,6 +248,9 @@ class _Run:
         if isinstance(self.den, TVDenoiser):  # ths = the level the pre carries for non-residual denoisers (pnp anneals it)
             self.den.apply_post(self.shape, self.den_in, self.base, post, self.X, sample, self.mean, self.mean2,
                                 ths=self.pre_params.den_in_c3)
+        elif isinstance(self.den, GSDRUNet):  # D is evaluated where the pre left the denoiser input: base (PSGLA) or X
+            x = self.X if self.pre_params.alg == _lib.ALG_PNPULA else None
+            self.den.apply_post(self.shape, self.den_in, self.base, post, self.X, sample, self.mean, self.mean2, next_pre=nxt, x=x)
         else:
             self.den.apply_post(self.shape, self.den_in, self.base, post, self.X, sample, self.mean, self.mean2, next_pre=nxt)
         if sample is not None:
@@ -397,8 +403,8 @@ def red(init, data_grad, Pb, denoiser, lambd, sig_float=0.0055, delta=1e-5, n_it
         save_images_online=False, name=None, *, n_chains=None):
     """RED (restoration_algorithms.py:465-529): X+ = X + delta data_grad(X) - delta lambd (X - D(X; sig_den)), sig_den =
     50/255 for the first 10 iterations of an inpainting problem.  Returns (all iterates, [last iterate], [])."""
-    if not isinstance(denoiser, (DnCNN, DRUNet)):
-        raise TypeError("denoiser must be a psgla_b200.DnCNN or psgla_b200.DRUNet")
+    if not isinstance(denoiser, (DnCNN, DRUNet, GSDRUNet)):
+        raise TypeError("denoiser must be a psgla_b200.DnCNN, DRUNet or GSDRUNet")
     run = _Run(init, data_grad, denoiser, n_iter, 1, max(int(n_iter), 1), 0, None, "philox", n_chains, 0)
     delta32 = float(np.float32(delta))
     g = delta32 * _f(lambd)
