@@ -11,7 +11,8 @@
  *     (torch allocates inputs, outputs and workspace); the library never frees caller memory.
  *   - every call is stream-ordered on `stream` (a cudaStream_t passed as void*), asynchronous, re-entrant.
  *   - return value: 0 = ok; >0 = cudaError_t; <0 = PSGLA_E_* below.  psgla_last_error() gives a thread-local message.
- *   - image tensors are fp32 NCHW [B][3][H][W] ("chains" = B); denoiser activations are bf16 NHWC, library-internal.
+ *   - image tensors are fp32 NCHW [B][C][H][W] ("chains" = B; C = 3 colour, or 1 grayscale where an entry says so);
+ *     denoiser activations are bf16 NHWC, library-internal.
  *   - noise: in-kernel Philox4x32-10 keyed by (seed; subsequence = global chain id; counter = step / element), or,
  *     when a replay pointer is given, the caller's N(0,1) draws (the reference's np.random.randn / torch.randn).
  */
@@ -113,15 +114,19 @@ int psgla_gmm2d_sliced_w2(const void* x_dev, int precision, int64_t n, const flo
 
 /* ------------------------------------------------------------------------------------------------------------
  * Image inverse problems.  One "iteration" of psgla (restoration_algorithms.py:232-238) or pnpula (:104-115) on a
- * batch of B independent chains of shape [3][H][W] is
+ * batch of B independent chains of shape [C][H][W] is
  *     pre   : data-fidelity gradient (+ projection term for PnP-ULA) + noise  -> base (fp32) and the denoiser input
  *     dncnn : 20 conv3x3 layers (tcgen05 implicit GEMM, bf16 in / fp32 accumulate)
  *     post  : fused into the last conv's epilogue: X+ = base + gain * (out_conv(h) + bias), thinning, E[X], E[X^2]
  * ---------------------------------------------------------------------------------------------------------- */
 
 typedef struct psgla_img_shape {
-  int32_t B, C, H, W; /* chains, channels (3), rows, cols */
+  int32_t B, C, H, W; /* chains, channels, rows, cols */
 } psgla_img_shape;
+/* Channels: the pre kernels, psgla_img_blur, psgla_img_noise, psgla_img_to_nhwc16, psgla_img_pad_replicate_nhwc16,
+ * psgla_img_psnr_ssim, psgla_dncnn_*, psgla_conv3x3_layer and psgla_drunet_* take C = 3 (colour) or C = 1 (grayscale); the
+ * TV prox and the gradient-step DRUNet take C = 3 only.  Any other C is rejected before any CUDA call.  The element index
+ * within a chain is c H W + pixel for both, so channel 0 of a colour chain and a grayscale chain draw the same Philox noise. */
 
 /* Inpainting "pre" (sampling_images.py:295 data_grad; restoration_algorithms.py:236 / :110-115):
  *   PSGLA  : base = X + gain_data * (-mask (X - y)) + noise_scale * Z        (gain_data = (delta/lambd)/sigma^2)
@@ -130,7 +135,8 @@ typedef struct psgla_img_shape {
  *            den_in = bf16(X)                                              (gain_data = delta/sigma^2)
  * mask_dev, y_dev: [1 or B][C][H][W] fp32 (mask_B / y_B say which; 1 = shared by all chains).
  * noise_dev: NULL (Philox: subsequence = chain_id0 + b, counter = (iteration, element)) or [B][C][H][W] fp32.
- * den_in_dev: bf16 NHWC [B][H][W][16] (channels 3..15 zero) -- the padded input of the first conv layer. */
+ * den_in_dev: bf16 NHWC [B][H][W][16] -- the padded input of the first conv layer: the C image channels from slot 0, slot 3 =
+ * den_in_c3, every other slot zero (grayscale: (v, 0, 0, den_in_c3, 0, ...)). */
 typedef struct psgla_pre_params {
   int32_t alg;        /* PSGLA_ALG_* */
   float gain_data;    /* multiplies -mask (X - y) resp. -A^T(A X - y) */
@@ -145,7 +151,7 @@ typedef struct psgla_pre_params {
   int64_t iteration;
   /* Which N(0,1) stream the kernel generates when noise_dev is NULL:
    *   PSGLA_NOISE_PHILOX     the library's own (subsequence = chain_id0 + b, counter = (iteration, element / 4));
-   *   PSGLA_NOISE_TORCH_CUDA the stream of torch.randn((B,3,H,W), generator=Generator("cuda").manual_seed(seed)) -- what
+   *   PSGLA_NOISE_TORCH_CUDA the stream of torch.randn((B,C,H,W), generator=Generator("cuda").manual_seed(seed)) -- what
    *                          the reference draws each iteration (restoration_algorithms.py:104,232) -- bit for bit:
    *                          torch_offset = the generator's Philox offset before that call and torch_threads = the
    *                          thread count of torch's launch, both from psgla_torch_cuda_randn_policy(). */
@@ -196,10 +202,15 @@ int psgla_img_noise(psgla_img_shape shape, uint64_t seed, int64_t chain_id0, int
  * sampling_images.py:156): depth conv3x3 layers, nf = 64 features, bias, ReLU, residual.
  * psgla_dncnn_pack_weights converts the fp32 OIHW state-dict tensors (host pointers, in layer order:
  * in_conv, conv_list[0..depth-3], out_conv) into the library's device layout (bf16, tap-major, K-major, 128B-swizzled
- * as the tcgen05 B operand wants it) inside packed_dev (psgla_dncnn_packed_bytes(depth) bytes). */
+ * as the tcgen05 B operand wants it) inside packed_dev (psgla_dncnn_packed_bytes(depth) bytes).
+ * psgla_dncnn_pack_weights_ch packs a network of `channels` = 3 or 1 image channels (in_conv [64][channels][3][3], out_conv
+ * [channels][64][3][3]); psgla_dncnn_pack_weights is it with 3.  The packed size does not depend on the channel count, but a
+ * packed buffer must be used with shapes of the channel count it was packed for. */
 size_t psgla_dncnn_packed_bytes(int depth);
 int psgla_dncnn_pack_weights(int depth, const float* const* weights_host, const float* const* biases_host,
                              void* packed_dev, void* stream);
+int psgla_dncnn_pack_weights_ch(int depth, int channels, const float* const* weights_host, const float* const* biases_host,
+                                void* packed_dev, void* stream);
 /* Bytes of activation workspace for B chains of H x W (two ping-pong bf16 NHWC [B][H][W][64] buffers). */
 size_t psgla_dncnn_workspace_bytes(psgla_img_shape shape);
 
@@ -241,7 +252,7 @@ int psgla_dncnn_residual_post_next(int depth, const void* packed_dev, psgla_img_
                                    const psgla_post_params* post, float* x_out_dev, float* sample_dev, float* mean_dev,
                                    float* mean2_dev, const psgla_next_pre* next, void* stream);
 
-/* The last layer of that chain alone (64 -> 3 channels + the fused post / next pre): hidden_dev = bf16 NHWC [B][H][W][64], the
+/* The last layer of that chain alone (64 -> C channels + the fused post / next pre): hidden_dev = bf16 NHWC [B][H][W][64], the
  * output of layer depth - 2.  What psgla_dncnn_residual_post_next launches last; exposed so that the fused epilogue can be
  * timed (bench.py's HBM roofline of this stage) and tested on its own. */
 int psgla_dncnn_last_layer_post_next(int depth, const void* packed_dev, psgla_img_shape shape, const void* hidden_dev,
@@ -250,13 +261,14 @@ int psgla_dncnn_last_layer_post_next(int depth, const void* packed_dev, psgla_im
                                      void* stream);
 
 /* Single conv3x3 layers, exposed for parity tests against torch.nn.functional.conv2d.
- *   cin_pad: 16 (first layer, channels 3..15 zero) or 64.   in_dev: bf16 NHWC [B][H][W][cin_pad].
- *   out_dev: bf16 NHWC [B][H][W][64], ReLU applied if relu != 0.   layer: index into the packed weights. */
+ *   cin_pad: 16 (first layer, channels C..15 zero) or 64.   in_dev: bf16 NHWC [B][H][W][cin_pad].
+ *   out_dev: bf16 NHWC [B][H][W][64], ReLU applied if relu != 0; the last layer: the raw conv as fp32 NCHW [B][C][H][W].
+ *   layer: index into the packed weights. */
 int psgla_conv3x3_layer(const void* packed_dev, int depth, int layer, psgla_img_shape shape, const void* in_dev,
                         void* out_dev, int relu, void* stream);
 
-/* Layout helper: fp32 NCHW [B][3][H][W] -> bf16 NHWC [B][H][W][16]; channel 3 = c3 (the DRUNet noise-level map, 0 for
- * DnCNN), channels 4..15 zero. */
+/* Layout helper: fp32 NCHW [B][C][H][W] -> bf16 NHWC [B][H][W][16]: the C channels from slot 0, slot 3 = c3 (the DRUNet
+ * noise-level map, 0 for DnCNN), every other slot zero. */
 int psgla_img_to_nhwc16(psgla_img_shape shape, const float* x_dev, float c3, void* out_dev, void* stream);
 
 /* In-place replication padding of a bf16 NHWC16 batch [B][padded.H][padded.W][16]: pixels with y >= H or x >= W copy the nearest
@@ -306,14 +318,19 @@ size_t psgla_img_metrics_workspace_bytes(int n);
 int psgla_img_psnr_ssim(psgla_img_shape shape, const float* stack_dev, const float* ref_dev, float data_range,
                         void* workspace_dev, size_t workspace_bytes, float* psnr_out_dev, float* ssim_out_dev, void* stream);
 
-/* DRUNet (deepinv.models.DRUNet(in_channels=3, out_channels=3), sampling_images.py:136; KAIR UNetRes nc = 64/128/256/512,
+/* DRUNet (deepinv.models.DRUNet(in_channels=C, out_channels=C), sampling_images.py:136; KAIR UNetRes nc = 64/128/256/512,
  * nb = 4, no biases).  weights_host: psgla_drunet_num_weights() = 64 fp32 tensors in state-dict order (m_head, m_down1.*,
  * m_down2.*, m_down3.*, m_body.*, m_up3.*, m_up2.*, m_up1.*, m_tail; torch layouts).  den_in_dev: bf16 NHWC16 as written by a
  * "pre" call with den_in_c3 = sigma.  H and W must be multiples of 8.
- * psgla_drunet_denoise_post: X+ = post->base_scale * base + post->gain * DRUNet(den_in), thinning and moments as above. */
+ * psgla_drunet_denoise_post: X+ = post->base_scale * base + post->gain * DRUNet(den_in), thinning and moments as above.
+ * psgla_drunet_pack_weights_ch packs a network of `channels` = 3 or 1 image channels: m_head [64][channels + 1][3][3] (the
+ * noise level last, as deepinv appends it), m_tail [channels][64][3][3]; psgla_drunet_pack_weights is it with 3.  The packed
+ * size does not depend on the channel count, but a packed buffer must be used with shapes of the channel count it was
+ * packed for. */
 int psgla_drunet_num_weights(void);
 size_t psgla_drunet_packed_bytes(void);
 int psgla_drunet_pack_weights(const float* const* weights_host, void* packed_dev, void* stream);
+int psgla_drunet_pack_weights_ch(int channels, const float* const* weights_host, void* packed_dev, void* stream);
 size_t psgla_drunet_workspace_bytes(psgla_img_shape shape);
 int psgla_drunet_denoise_post(const void* packed_dev, psgla_img_shape shape, const void* den_in_dev, void* workspace_dev,
                               size_t workspace_bytes, const float* base_dev, const psgla_post_params* post,
@@ -325,7 +342,7 @@ int psgla_drunet_denoise_post_next(const void* packed_dev, psgla_img_shape shape
 /* One layer of that network, exposed for parity tests like psgla_conv3x3_layer: exactly the kernel, ReLU and residual adds
  * psgla_drunet_denoise_post runs for it.  layer: 0..63 in the state-dict order above; shape: the network's image shape (H, W
  * multiples of 8); the layer works at its own scale of it.  in_dev: bf16 NHWC16 (layer 0, channel 3 = sigma) or bf16 NHWC.
- * out_dev: bf16 NHWC, or for layer 63 the raw conv as fp32 NCHW [B][3][H][W].  res1_dev (the residual block's input) must
+ * out_dev: bf16 NHWC, or for layer 63 the raw conv as fp32 NCHW [B][C][H][W].  res1_dev (the residual block's input) must
  * be given exactly for the second conv of a residual block, res2_dev (the U-Net skip) exactly for the last such conv of the
  * body and of each decoder stage; both are bf16 NHWC of the output's shape. */
 int psgla_drunet_layer(const void* packed_dev, psgla_img_shape shape, int layer, const void* in_dev, const void* res1_dev,

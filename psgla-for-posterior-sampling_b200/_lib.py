@@ -87,6 +87,8 @@ SIGNATURES = {
     "psgla_img_noise_torch_cuda": (_int, [_i64, _u64, _u64, C.c_uint32, _vp, _vp]),
     "psgla_dncnn_packed_bytes": (_sz, [_int]),
     "psgla_dncnn_pack_weights": (_int, [_int, C.POINTER(C.POINTER(C.c_float)), C.POINTER(C.POINTER(C.c_float)), _vp, _vp]),
+    "psgla_dncnn_pack_weights_ch": (_int, [_int, _int, C.POINTER(C.POINTER(C.c_float)), C.POINTER(C.POINTER(C.c_float)), _vp,
+                                           _vp]),
     "psgla_dncnn_workspace_bytes": (_sz, [ImgShape]),
     "psgla_dncnn_residual_post": (_int, [_int, _vp, ImgShape, _vp, _vp, _sz, _vp, C.POINTER(PostParams), _vp, _vp, _vp,
                                          _vp, _vp]),
@@ -102,6 +104,7 @@ SIGNATURES = {
     "psgla_drunet_num_weights": (_int, []),
     "psgla_drunet_packed_bytes": (_sz, []),
     "psgla_drunet_pack_weights": (_int, [C.POINTER(C.POINTER(C.c_float)), _vp, _vp]),
+    "psgla_drunet_pack_weights_ch": (_int, [_int, C.POINTER(C.POINTER(C.c_float)), _vp, _vp]),
     "psgla_drunet_workspace_bytes": (_sz, [ImgShape]),
     "psgla_drunet_denoise_post": (_int, [_vp, ImgShape, _vp, _vp, _sz, _vp, C.POINTER(PostParams), _vp, _vp, _vp, _vp, _vp]),
     "psgla_drunet_denoise_post_next": (_int, [_vp, ImgShape, _vp, _vp, _sz, _vp, C.POINTER(PostParams), _vp, _vp, _vp, _vp,

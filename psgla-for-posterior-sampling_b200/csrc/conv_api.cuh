@@ -25,15 +25,17 @@ int conv64_hidden(const void* in, void* out, const uint8_t* w, const float* bias
                   const void* res1, const void* res2, cudaStream_t st);
 int conv_first16(const void* in16, void* out, const uint8_t* w, const float* bias, int B, int H, int W, int relu,
                  cudaStream_t st);
-int conv_last_post(const void* in, const uint8_t* w, const float* bias, int B, int H, int W, const float* base,
+// the last layer (64 -> C = 3 or 1 image channels) and the fused post
+int conv_last_post(const void* in, const uint8_t* w, const float* bias, int B, int C, int H, int W, const float* base,
                    float base_scale, float gain, float w_old, float w_new, float* x_out, float* sample, float* mean,
                    float* mean2, const psgla_next_pre* next, cudaStream_t st);
 
 // drunet.cu -- the U-Net layer kinds (which kernel runs a layer) and their packed weights, shared with gsdrunet.cu
 enum DruKind { DRU_HEAD, DRU_C64, DRU_GEMM3, DRU_DOWN, DRU_UP, DRU_TAIL };
 size_t dru_layer_bytes(DruKind k, int cin, int cout);
-// fp32 torch-layout weight -> the kind's packed layout: HEAD / C64 / TAIL OIHW 3x3 (HEAD: cin <= 16 real input channels,
-// TAIL: cout <= 16 real outputs), GEMM3 / DOWN OIHW, UP ConvTranspose2d [cin][cout][2][2].  dst zero-initialised.
+// fp32 torch-layout weight -> the kind's packed layout: HEAD / C64 / TAIL OIHW 3x3 (HEAD: cin <= 16 real input channels; cin = 2
+// is the grayscale DRUNet head (image, noise level), whose noise level goes to K slot 3 as the colour head's does; TAIL: cout <= 16 real outputs), GEMM3
+// / DOWN OIHW, UP ConvTranspose2d [cin][cout][2][2].  dst zero-initialised.
 void dru_pack_layer(DruKind kind, const float* w, int cin, int cout, uint8_t* dst);
 
 // conv_gemm.cu -- layers with streamed weights (mode: 0 conv3x3, 1 2x2 stride-2 down, 2 2x2 transposed up)

@@ -7,9 +7,9 @@
 // GEMM view per 128-pixel output row segment:  D[128 x NOUT] = sum over 9 taps  A_tap[128 x CIN] * W_tap[NOUT x CIN]^T.
 // A work item is a (chain, 128-pixel strip, block of R rows); every input row (130 pixels = 128 + halo, TMA out-of-bounds
 // zero fill = the convolution's padding) is loaded ONCE and serves the three output rows around it.  One kernel per layer role:
-//   conv3x3_kernel<16,64>          the first layer (3, padded to 16, -> 64 channels).  SS form: A_tap = window into the
+//   conv3x3_kernel<16,64>          the first layer (3 or 1, padded to 16, -> 64 channels).  SS form: A_tap = window into the
 //                                  shared-memory row ring (tap dx = descriptor start + dx rows, tap dy = ring slot).
-//   conv3x3_ts_kernel<16>          the last layer (64 -> 3, padded to 16, fused Langevin post / next pre epilogue).  TS form:
+//   conv3x3_ts_kernel<16,C>        the last layer (64 -> C = 3 or 1, padded to 16, fused Langevin post / next pre epilogue).  TS form:
 //                                  four loader warps copy each row into TENSOR MEMORY three times (shifted by dx) and the MMAs
 //                                  take A from there (N/2 instead of 32 + N/4 cycles per MMA at N = 64).
 //   conv3x3_ts2_kernel<NOUT,RES>   the hidden layers: a CTA PAIR (cta_group::2, M = 256) on two adjacent strips, weights split
@@ -171,7 +171,7 @@ conv3x3_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__
   }
 }
 
-template <int NOUT>
+template <int NOUT, int C>  // C: image channels of the fused post, 3 or 1
 __global__ void __launch_bounds__(TS_THREADS, 1)
 conv3x3_ts_kernel(const __grid_constant__ CUtensorMap tmap, const ConvParams p) {
   using Cfg = ConvTsCfg<NOUT>;
@@ -323,7 +323,7 @@ conv3x3_ts_kernel(const __grid_constant__ CUtensorMap tmap, const ConvParams p) 
   } else {
     // ---------------------------------------------------------------- epilogue: 2 groups x 4 warps
     const int ew = warp - 6;
-    epilogue_post<NOUT, TS_NACC>(p, bias_s, tfull, tempty, tmem_base, ew >> 2, warp & 3, lane);
+    epilogue_post<NOUT, TS_NACC, C>(p, bias_s, tfull, tempty, tmem_base, ew >> 2, warp & 3, lane);
   }
   tc_fence_before();
   __syncthreads();
@@ -668,8 +668,9 @@ static int launch_first(const void* in, void* out_bf16, ConvParams p, cudaStream
   return PSGLA_OK;
 }
 
-// The last layer: bf16 NHWC 64-channel input -> the fused Langevin post epilogue (fp32 NCHW outputs named in p)
-static int launch_last(const void* in, ConvParams p, cudaStream_t st) {
+// The last layer: bf16 NHWC 64-channel input -> the fused Langevin post epilogue (fp32 NCHW outputs of C channels named in p)
+template <int C>
+static int launch_last_t(const void* in, ConvParams p, cudaStream_t st) {
   using Cfg = ConvTsCfg<16>;
   CUtensorMap map;
   int rc = get_act_tensor_map(&map, in, p.B, p.H, p.W, 64, BOX_W);
@@ -677,7 +678,7 @@ static int launch_last(const void* in, ConvParams p, cudaStream_t st) {
   static std::atomic<unsigned long long> attr_done{0};  // bit d: opted in on device d (a per-device function attribute)
   const unsigned long long dev_bit = 1ull << (current_device() & 63);
   if (!(attr_done.load(std::memory_order_acquire) & dev_bit)) {
-    PSGLA_CUDA_TRY(cudaFuncSetAttribute(conv3x3_ts_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    PSGLA_CUDA_TRY(cudaFuncSetAttribute(conv3x3_ts_kernel<16, C>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                         Cfg::SMEM_BYTES));
     attr_done.fetch_or(dev_bit, std::memory_order_release);
   }
@@ -693,8 +694,11 @@ static int launch_last(const void* in, ConvParams p, cudaStream_t st) {
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv3x3_ts_kernel<16>, map, p));
+  PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv3x3_ts_kernel<16, C>, map, p));
   return PSGLA_OK;
+}
+static int launch_last(const void* in, const ConvParams& p, int channels, cudaStream_t st) {
+  return channels == 1 ? launch_last_t<1>(in, p, st) : launch_last_t<3>(in, p, st);
 }
 
 // Work items of the pair kernel: (chain, row block, strip) with the strip count padded to even and the strip index
@@ -818,12 +822,20 @@ extern "C" size_t psgla_dncnn_packed_bytes(int depth) { return depth >= 2 ? pack
 
 extern "C" int psgla_dncnn_pack_weights(int depth, const float* const* weights_host, const float* const* biases_host,
                                         void* packed_dev, void* stream) {
+  return psgla_dncnn_pack_weights_ch(depth, 3, weights_host, biases_host, packed_dev, stream);
+}
+
+// Image channel k of a C-channel network (C = 3 or 1) is K slot k of the first layer and N slot k of the last: the denoiser
+// input is NHWC16 with the image from slot 0 whatever C (the DRUNet head's noise-level channel: dru_pack_layer).
+extern "C" int psgla_dncnn_pack_weights_ch(int depth, int channels, const float* const* weights_host,
+                                           const float* const* biases_host, void* packed_dev, void* stream) {
   PSGLA_REQUIRE(depth >= 2 && weights_host && packed_dev, "psgla_dncnn_pack_weights: bad argument");
+  PSGLA_REQUIRE(channels == 3 || channels == 1, "psgla_dncnn_pack_weights_ch: channels must be 3 or 1 (got %d)", channels);
   std::vector<uint8_t> host(packed_bytes(depth), 0);
   for (int l = 0; l < depth; ++l) {
     const LayerInfo li = layer_info(depth, l);
-    const int cin_real = (l == 0) ? 3 : 64;
-    const int nout_real = (l == depth - 1) ? 3 : 64;
+    const int cin_real = (l == 0) ? channels : 64;
+    const int nout_real = (l == depth - 1) ? channels : 64;
     const float* w = weights_host[l];  // OIHW [nout_real][cin_real][3][3]
     PSGLA_REQUIRE(w != nullptr, "layer %d: null weight pointer", l);
     pack_conv3x3_swizzled(w, nout_real, cin_real, li.nout, li.cin, host.data() + li.w_off);
@@ -841,8 +853,8 @@ extern "C" size_t psgla_dncnn_workspace_bytes(psgla_img_shape s) {
 }
 
 static int check_shape(const psgla_img_shape& s) {
-  PSGLA_REQUIRE(s.B > 0 && s.H > 0 && s.W > 0 && s.C == 3, "image shape must be [B>0][3][H>0][W>0], got [%d][%d][%d][%d]",
-                s.B, s.C, s.H, s.W);
+  PSGLA_REQUIRE(s.B > 0 && s.H > 0 && s.W > 0 && (s.C == 3 || s.C == 1),
+                "image shape must be [B>0][C = 1 or 3][H>0][W>0], got [%d][%d][%d][%d]", s.B, s.C, s.H, s.W);
   return PSGLA_OK;
 }
 
@@ -856,7 +868,7 @@ static ConvParams base_params(const psgla_img_shape& s, const uint8_t* packed, c
   return p;
 }
 
-// The last layer (64 -> 3) with the Langevin post (and optionally the next iteration's pre) in its epilogue.
+// The last layer (64 -> C) with the Langevin post (and optionally the next iteration's pre) in its epilogue.
 static int last_layer_post(int depth, const uint8_t* packed, const psgla_img_shape& shape, const void* hidden, const float* base_dev,
                            const psgla_post_params* post, float* x_out_dev, float* sample_dev, float* mean_dev,
                            float* mean2_dev, const psgla_next_pre* next, cudaStream_t st) {
@@ -872,9 +884,9 @@ static int last_layer_post(int depth, const uint8_t* packed, const psgla_img_sha
   p.w_old = post->w_old;
   p.w_new = post->w_new;
   p.reverse = (depth - 1) & 1;
-  int rc = set_next_pre(&p, next);
+  int rc = set_next_pre(&p, next, shape.C);
   if (rc) return rc;
-  return launch_last(hidden, p, st);
+  return launch_last(hidden, p, shape.C, st);
 }
 
 extern "C" int psgla_conv3x3_layer(const void* packed_dev, int depth, int layer, psgla_img_shape shape,
@@ -889,7 +901,7 @@ extern "C" int psgla_conv3x3_layer(const void* packed_dev, int depth, int layer,
   cudaStream_t st = (cudaStream_t)stream;
   if (layer == depth - 1) {  // raw conv + bias -> fp32 NCHW
     p.x_out = (float*)out_dev;
-    return launch_last(in_dev, p, st);
+    return launch_last(in_dev, p, shape.C, st);
   }
   return layer == 0 ? launch_first(in_dev, out_dev, p, st) : launch_hidden64(in_dev, out_dev, p, st);
 }
@@ -1027,12 +1039,12 @@ int check_next_pre(const psgla_next_pre* next, const psgla_img_shape& s) {
   return fill_pre(next->pre, &a);
 }
 
-int set_next_pre(ConvParams* p, const psgla_next_pre* next) {
+int set_next_pre(ConvParams* p, const psgla_next_pre* next, int channels) {
   p->nx_enable = 0;
   if (!next) return PSGLA_OK;
   int rc = fill_pre(next->pre, &p->nx);
   if (rc) return rc;
-  p->nx.chw = 3LL * p->H * p->W;
+  p->nx.chw = (long long)channels * p->H * p->W;
   p->nx_enable = 1;
   p->nx_mask = next->mask_dev;
   p->nx_y = next->y_dev;
@@ -1043,7 +1055,7 @@ int set_next_pre(ConvParams* p, const psgla_next_pre* next) {
   return PSGLA_OK;
 }
 
-int conv_last_post(const void* in, const uint8_t* w, const float* bias, int B, int H, int W, const float* base,
+int conv_last_post(const void* in, const uint8_t* w, const float* bias, int B, int C, int H, int W, const float* base,
                    float base_scale, float gain, float w_old, float w_new, float* x_out, float* sample, float* mean,
                    float* mean2, const psgla_next_pre* next, cudaStream_t st) {
   ConvParams p{};
@@ -1059,9 +1071,9 @@ int conv_last_post(const void* in, const uint8_t* w, const float* bias, int B, i
   p.sample = sample;
   p.mean = mean;
   p.mean2 = mean2;
-  int rc = set_next_pre(&p, next);
+  int rc = set_next_pre(&p, next, C);
   if (rc) return rc;
-  return launch_last(in, p, st);
+  return launch_last(in, p, C, st);
 }
 
 }  // namespace psgla

@@ -124,7 +124,7 @@ struct ConvParams {
   __nv_bfloat16* nx_den_in;
 };
 
-int set_next_pre(ConvParams* p, const psgla_next_pre* next);  // host: fills the nx_* fields (conv_tc.cu)
+int set_next_pre(ConvParams* p, const psgla_next_pre* next, int channels);  // host: fills the nx_* fields (conv_tc.cu)
 
 struct ItemCoord {
   int b, y0, rcur, x0, ylo, yhi;
@@ -397,18 +397,20 @@ __device__ __forceinline__ void epilogue_hidden_tmares(const ConvParams& p, cons
 // The layer is HBM-bound (128 B of activations in, ~70-140 B of fp32 state in and out per pixel) and its MMAs take only a few
 // hundred cycles per row, so nothing hides a DRAM round trip behind them: the epilogue therefore walks ITS rows with a
 // one-row-ahead register prefetch of everything it reads from global memory, and draws the row's noise before it waits
-// for the accumulator.
+// for the accumulator.  C: image channels, 3 (colour) or 1 (grayscale: output column 0 of the accumulator; the element index
+// within a chain is c H W + pixel either way, so channel 0 draws the same noise at C = 1 and C = 3).
 struct PostRowIter {
   int item, y, yend;
   uint32_t T;
   ItemCoord c;
   bool done;
 };
+template <int C>
 struct PostRowData {
-  float bse[3], m1[3], m2[3], nmask[3], nobs[3];
+  float bse[C], m1[C], m2[C], nmask[C], nobs[C];
 };
 
-template <int NOUT, int NACC_>
+template <int NOUT, int NACC_, int C>
 __device__ __forceinline__ void epilogue_post(const ConvParams& p, const float* bias_s, uint64_t* tfull, uint64_t* tempty,
                                               uint32_t tmem_base, int grp, int q4, int lane) {
   griddep_wait();  // base / running moments were written by earlier kernels
@@ -430,15 +432,15 @@ __device__ __forceinline__ void epilogue_post(const ConvParams& p, const float* 
   auto settle = [&](PostRowIter& r) {  // forward to the next row this epilogue group drains
     while (!r.done && (int)(r.T & 1) != grp) step(r);
   };
-  auto fetch = [&](const PostRowIter& r, PostRowData& d) {
+  auto fetch = [&](const PostRowIter& r, PostRowData<C>& d) {
     const int x = r.c.x0 + q4 * 32 + lane;
 #pragma unroll
-    for (int ch = 0; ch < 3; ++ch) d.bse[ch] = d.m1[ch] = d.m2[ch] = d.nmask[ch] = d.nobs[ch] = 0.f;
+    for (int ch = 0; ch < C; ++ch) d.bse[ch] = d.m1[ch] = d.m2[ch] = d.nmask[ch] = d.nobs[ch] = 0.f;
     if (r.done || x >= p.W) return;
     const size_t e0 = (size_t)r.y * p.W + x;
-    const size_t idx0 = ((size_t)r.c.b * 3) * plane + e0;
+    const size_t idx0 = ((size_t)r.c.b * C) * plane + e0;
 #pragma unroll
-    for (int ch = 0; ch < 3; ++ch) {
+    for (int ch = 0; ch < C; ++ch) {
       if (p.base) d.bse[ch] = p.base[idx0 + ch * plane];
       if (p.mean) {
         d.m1[ch] = p.mean[idx0 + ch * plane];
@@ -446,10 +448,10 @@ __device__ __forceinline__ void epilogue_post(const ConvParams& p, const float* 
       }
     }
     if (p.nx_enable) {
-      const size_t mi = ((size_t)(p.nx_mask_B > 1 ? r.c.b : 0) * 3) * plane + e0;
-      const size_t yi = ((size_t)(p.nx_y_B > 1 ? r.c.b : 0) * 3) * plane + e0;
+      const size_t mi = ((size_t)(p.nx_mask_B > 1 ? r.c.b : 0) * C) * plane + e0;
+      const size_t yi = ((size_t)(p.nx_y_B > 1 ? r.c.b : 0) * C) * plane + e0;
 #pragma unroll
-      for (int ch = 0; ch < 3; ++ch) {
+      for (int ch = 0; ch < C; ++ch) {
         d.nmask[ch] = p.nx_mask[mi + ch * plane];
         d.nobs[ch] = p.nx_y[yi + ch * plane];
       }
@@ -466,32 +468,35 @@ __device__ __forceinline__ void epilogue_post(const ConvParams& p, const float* 
     it.yend = it.c.y0 + it.c.rcur;
   }
   settle(it);
-  PostRowData cur;
+  PostRowData<C> cur;
   fetch(it, cur);
   while (!it.done) {
     PostRowIter nxt = it;
     step(nxt);
     settle(nxt);
-    PostRowData nd;
+    PostRowData<C> nd;
     fetch(nxt, nd);  // in flight while this row is processed
     const ItemCoord& c = it.c;
     const int y = it.y;
     const uint32_t T = it.T;
     const int x = c.x0 + q4 * 32 + lane;
     const bool valid = x < p.W;
-    const size_t idx0 = ((size_t)c.b * 3) * plane + (size_t)y * p.W + x;
-    float z[3] = {0.f, 0.f, 0.f};
+    const size_t idx0 = ((size_t)c.b * C) * plane + (size_t)y * p.W + x;
+    float z[C];
+#pragma unroll
+    for (int ch = 0; ch < C; ++ch) z[ch] = 0.f;
     if (p.nx_enable) {
       if (p.nx.noise_mode == PSGLA_NOISE_PHILOX && (p.W & 3) == 0) {
         // Library stream: one Philox call serves four consecutive elements, and lanes 4k .. 4k+3 hold four consecutive
         // pixels (x0, the warp offset and W are multiples of 4).  Lane 4k + ch draws channel ch's quad, the four lanes
-        // exchange components by shuffle: one Philox call per lane instead of three.
+        // exchange components by shuffle: one Philox call per lane instead of three.  Grayscale: lane 4k draws the quad
+        // of its four pixels and shares it.
         const int sub = lane & 3;
         float z4[4] = {0.f, 0.f, 0.f, 0.f};
-        if (sub < 3 && x - sub < p.W)
+        if (sub < C && x - sub < p.W)
           draw_quad(p.nx, c.b, (uint32_t)((size_t)sub * plane + (size_t)y * p.W + (size_t)(x - sub)), z4);
 #pragma unroll
-        for (int ch = 0; ch < 3; ++ch) {
+        for (int ch = 0; ch < C; ++ch) {
           const int src = (lane & ~3) + ch;
           const float t0 = __shfl_sync(0xffffffffu, z4[0], src), t1 = __shfl_sync(0xffffffffu, z4[1], src);
           const float t2 = __shfl_sync(0xffffffffu, z4[2], src), t3 = __shfl_sync(0xffffffffu, z4[3], src);
@@ -499,7 +504,7 @@ __device__ __forceinline__ void epilogue_post(const ConvParams& p, const float* 
         }
       } else if (valid) {
 #pragma unroll
-        for (int ch = 0; ch < 3; ++ch) z[ch] = draw_at(p.nx, c.b, (uint32_t)((size_t)ch * plane + (size_t)y * p.W + x));
+        for (int ch = 0; ch < C; ++ch) z[ch] = draw_at(p.nx, c.b, (uint32_t)((size_t)ch * plane + (size_t)y * p.W + x));
       }
     }
     const uint32_t acc = T % NACC_;
@@ -513,9 +518,9 @@ __device__ __forceinline__ void epilogue_post(const ConvParams& p, const float* 
     __syncwarp();
     if (lane == 0) mbar_arrive(&tempty[acc]);
     if (valid) {
-      float xnew[3];
+      float xnew[C];
 #pragma unroll
-      for (int ch = 0; ch < 3; ++ch) {
+      for (int ch = 0; ch < C; ++ch) {
         const size_t idx = idx0 + ch * plane;
         const float r = __uint_as_float(v[ch]) + bias_s[ch];
         const float xn = p.base ? fmaf(p.gain, r, p.base_scale * cur.bse[ch]) : r;
@@ -531,14 +536,15 @@ __device__ __forceinline__ void epilogue_post(const ConvParams& p, const float* 
       if (p.nx_enable) {
         // the next iteration's Langevin "pre" on the fresh iterate: same arithmetic and the same noise element as
         // pre_inpaint_kernel (img_elementwise.cu), so fused and unfused runs agree bit for bit
-        float din[3];
+        float din[C];
 #pragma unroll
-        for (int ch = 0; ch < 3; ++ch) {
+        for (int ch = 0; ch < C; ++ch) {
           const float bv = langevin_base(p.nx, xnew[ch], cur.nmask[ch] * (xnew[ch] - cur.nobs[ch]), z[ch]);
           p.nx_base[idx0 + ch * plane] = bv;
           din[ch] = (p.nx.alg == PSGLA_ALG_PNPULA) ? xnew[ch] : bv;
         }
-        store_nhwc16(p.nx_den_in + (((size_t)c.b * plane) + (size_t)y * p.W + x) * 16, din[0], din[1], din[2], p.nx.den_in_c3);
+        store_nhwc16(p.nx_den_in + (((size_t)c.b * plane) + (size_t)y * p.W + x) * 16, din[0], C > 1 ? din[1 % C] : 0.f,
+                     C > 2 ? din[2 % C] : 0.f, p.nx.den_in_c3);
       }
     }
     it = nxt;
@@ -559,7 +565,7 @@ constexpr int TS_NACC = 2;
 constexpr int TS_A_COL0 = 128;
 constexpr int TS_THREADS = 64 + 128 + 32 * EPI_WARPS;
 
-// The single-CTA TS kernel, i.e. the last layer: 64 input channels, 16 (3 padded) output channels, fused Langevin epilogue
+// The single-CTA TS kernel, i.e. the last layer: 64 input channels, 16 (3 or 1 padded) output channels, fused Langevin epilogue
 template <int NOUT>
 struct ConvTsCfg {
   static_assert(NOUT == 16, "ring depth and shared-memory plan are sized for the last layer");

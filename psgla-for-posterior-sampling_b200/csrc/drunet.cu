@@ -3,6 +3,8 @@
 // blocks per stage, stride-2 2x2 convs down, 2x2 transposed convs up, no biases, ReLU; the input is the image plus a
 // constant noise-level channel and the output is the denoised image (architecture restated in oracle/image_oracle.py).
 //
+// Colour (C = 3) or grayscale (C = 1) images: the head takes C + 1 channels, the tail gives C.
+//
 // Layer schedule (68 launches): head 4->64 (first-layer SS kernel on the NHWC16 input, channel 3 = sigma), the 16
 // full-resolution 64-channel convs on the weight-resident TS kernel (conv_tc.cu), every other layer on the streamed
 // implicit-GEMM kernel (conv_gemm.cu); residual and U-Net skip additions are folded into the epilogue of the conv that
@@ -65,7 +67,7 @@ static const std::vector<DruLayer>& dru_plan() {
     add(DRU_UP, nc[s + 1], nc[s], s + 1, 0, 0);
     blocks(s, true);
   }
-  add(DRU_TAIL, 64, 3, 0, 0, 0);
+  add(DRU_TAIL, 64, 3, 0, 0, 0);  // (colour; psgla_drunet_pack_weights_ch packs head and tail for the channel count)
   plan.swap(v);
   return plan;
 }
@@ -80,7 +82,23 @@ static inline uint16_t dru_bf16(float f) {
 
 void dru_pack_layer(DruKind kind, const float* w, int cin, int cout, uint8_t* dst) {
   switch (kind) {
-    case DRU_HEAD: pack_conv3x3_swizzled(w, 64, cin, 64, 16, dst); break;
+    case DRU_HEAD: {
+      // The NHWC16 denoiser input holds the image from slot 0 and the noise level in slot 3 whatever the channel count, so a
+      // grayscale head [64][2] (image, sigma) is packed as the colour head [64][4] with input channels 1 and 2 zero.  Every
+      // other cin is packed as it stands (colour: 4; the gradient-step DRUNet's adjoint of the tail: 3).
+      if (cin != 2) {
+        pack_conv3x3_swizzled(w, 64, cin, 64, 16, dst);
+        break;
+      }
+      std::vector<float> w4((size_t)64 * 4 * 9, 0.f);
+      for (int n = 0; n < 64; ++n)
+        for (int t = 0; t < 9; ++t) {
+          w4[((size_t)n * 4 + 0) * 9 + t] = w[((size_t)n * 2 + 0) * 9 + t];
+          w4[((size_t)n * 4 + 3) * 9 + t] = w[((size_t)n * 2 + 1) * 9 + t];
+        }
+      pack_conv3x3_swizzled(w4.data(), 64, 4, 64, 16, dst);
+      break;
+    }
     case DRU_C64: pack_conv3x3_swizzled(w, 64, 64, 64, 64, dst); break;
     case DRU_TAIL: pack_conv3x3_swizzled(w, cout, 64, 16, 64, dst); break;
     case DRU_GEMM3:  // OIHW [cout][cin][3][3] -> [tap][cout][cin]
@@ -132,7 +150,7 @@ struct DruPost {
 // Layer l of the plan as the network runs it: the kernel its kind selects, its ReLU, and its residual inputs (res1 = the block
 // input, res2 = the U-Net skip; null where the plan has none).  in / out / res are bf16 NHWC except the head's input (NHWC16)
 // and the tail's output, which goes through `post`.
-static int dru_layer(const uint8_t* packed, int l, int B, int H, int W, const void* in, const void* res1, const void* res2,
+static int dru_layer(const uint8_t* packed, int l, int B, int C, int H, int W, const void* in, const void* res1, const void* res2,
                      void* out, const DruPost& post, cudaStream_t st) {
   const DruLayer& L = dru_plan()[l];
   const uint8_t* w = packed + L.w_off;
@@ -145,14 +163,15 @@ static int dru_layer(const uint8_t* packed, int l, int B, int H, int W, const vo
     case DRU_DOWN: return conv_gemm_layer(1, B, h, wd, L.cin, L.cout, w, in, res1, res2, out, L.relu, st);
     case DRU_UP: return conv_gemm_layer(2, B, h, wd, L.cin, L.cout, w, in, res1, res2, out, L.relu, st);
     case DRU_TAIL:
-      return conv_last_post(in, w, bias(16, 64), B, H, W, post.base, post.base_scale, post.gain, post.w_old, post.w_new,
+      return conv_last_post(in, w, bias(16, 64), B, C, H, W, post.base, post.base_scale, post.gain, post.w_old, post.w_new,
                             post.x_out, post.sample, post.mean, post.mean2, post.next, st);
   }
   return set_error(PSGLA_E_BADARG, "DRUNet layer %d: unknown kind", l);
 }
 
 static int dru_check_shape(const psgla_img_shape& shape) {
-  PSGLA_REQUIRE(shape.B > 0 && shape.C == 3 && shape.H > 0 && shape.W > 0, "image shape must be [B>0][3][H>0][W>0]");
+  PSGLA_REQUIRE(shape.B > 0 && (shape.C == 3 || shape.C == 1) && shape.H > 0 && shape.W > 0,
+                "image shape must be [B>0][C = 1 or 3][H>0][W>0]");
   PSGLA_REQUIRE(shape.H % 8 == 0 && shape.W % 8 == 0, "DRUNet needs H and W to be multiples of 8 (got %d x %d): crop or pad "
                 "the image (the reference's deepinv pads internally by an unverifiable rule)", shape.H, shape.W);
   return PSGLA_OK;
@@ -170,14 +189,20 @@ extern "C" size_t psgla_drunet_packed_bytes(void) {
 }
 
 extern "C" int psgla_drunet_pack_weights(const float* const* weights_host, void* packed_dev, void* stream) {
+  return psgla_drunet_pack_weights_ch(3, weights_host, packed_dev, stream);
+}
+
+extern "C" int psgla_drunet_pack_weights_ch(int channels, const float* const* weights_host, void* packed_dev, void* stream) {
   PSGLA_REQUIRE(weights_host && packed_dev, "psgla_drunet_pack_weights: null pointer");
+  PSGLA_REQUIRE(channels == 3 || channels == 1, "psgla_drunet_pack_weights_ch: channels must be 3 or 1 (got %d)", channels);
   const auto& plan = dru_plan();
   std::vector<uint8_t> host(psgla_drunet_packed_bytes(), 0);
   for (size_t l = 0; l < plan.size(); ++l) {
     const DruLayer& L = plan[l];
     const float* w = weights_host[l];
     PSGLA_REQUIRE(w != nullptr, "DRUNet weight tensor %zu is null", l);
-    dru_pack_layer(L.kind, w, L.cin, L.cout, host.data() + L.w_off);
+    const int cin = L.kind == DRU_HEAD ? channels + 1 : L.cin, cout = L.kind == DRU_TAIL ? channels : L.cout;
+    dru_pack_layer(L.kind, w, cin, cout, host.data() + L.w_off);
   }
   PSGLA_CUDA_TRY(cudaMemcpyAsync(packed_dev, host.data(), host.size(), cudaMemcpyHostToDevice, (cudaStream_t)stream));
   PSGLA_CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));  // `host` dies at return
@@ -227,7 +252,7 @@ extern "C" int psgla_drunet_denoise_post_next(const void* packed_dev, psgla_img_
   int rc = 0;
   const DruPost no_post{};
   auto run = [&](const void* in, const void* res1, const void* res2, void* out) {
-    if (!rc) rc = dru_layer(packed, li, B, H, W, in, res1, res2, out, no_post, st);
+    if (!rc) rc = dru_layer(packed, li, B, shape.C, H, W, in, res1, res2, out, no_post, st);
     ++li;
   };
   // four residual blocks at scale s starting from `cur`; the last block also adds `skip` (U-Net skip connection)
@@ -262,7 +287,7 @@ extern "C" int psgla_drunet_denoise_post_next(const void* packed_dev, psgla_img_
   // tail + fused Langevin post:  X+ = base_scale * base + gain * D
   const DruPost tail{base_dev,  post->base_scale, post->gain, post->w_old, post->w_new,
                      x_out_dev, sample_dev,       mean_dev,   mean2_dev,   next};
-  return dru_layer(packed, li, B, H, W, cur, nullptr, nullptr, nullptr, tail, st);
+  return dru_layer(packed, li, B, shape.C, H, W, cur, nullptr, nullptr, nullptr, tail, st);
 }
 
 extern "C" int psgla_drunet_layer(const void* packed_dev, psgla_img_shape shape, int layer, const void* in_dev,
@@ -279,6 +304,6 @@ extern "C" int psgla_drunet_layer(const void* packed_dev, psgla_img_shape shape,
                 "res2 %s", layer, L.nres, res1_dev ? "set" : "null", res2_dev ? "set" : "null");
   DruPost raw{};
   raw.x_out = (float*)out_dev;
-  return dru_layer((const uint8_t*)packed_dev, layer, shape.B, shape.H, shape.W, in_dev, res1_dev, res2_dev, out_dev, raw,
+  return dru_layer((const uint8_t*)packed_dev, layer, shape.B, shape.C, shape.H, shape.W, in_dev, res1_dev, res2_dev, out_dev, raw,
                    (cudaStream_t)stream);
 }

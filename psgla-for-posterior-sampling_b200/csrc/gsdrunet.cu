@@ -171,7 +171,7 @@ static int gs_layer(const uint8_t* packed, int l, int B, int H, int W, const voi
     case DRU_DOWN: return conv_gemm_layer(1, B, h, wd, L.cin, L.cout, w, in, nullptr, nullptr, out, ACT_NONE, st);
     case DRU_UP: return conv_gemm_layer(2, B, h, wd, L.cin, L.cout, w, in, nullptr, nullptr, out, ACT_NONE, st);
     case DRU_TAIL:
-      return conv_last_post(in, w, bias(16, 64), B, H, W, post.base, post.base_scale, post.gain, post.w_old, post.w_new,
+      return conv_last_post(in, w, bias(16, 64), B, 3, H, W, post.base, post.base_scale, post.gain, post.w_old, post.w_new,
                             post.x_out, post.sample, post.mean, post.mean2, post.next, st);
   }
   return set_error(PSGLA_E_BADARG, "GSDRUNet layer %d: unknown kind", l);

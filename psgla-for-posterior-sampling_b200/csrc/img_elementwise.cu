@@ -18,8 +18,9 @@
 namespace psgla {
 
 // ------------------------------------------------------------------------------------------------ inpainting pre
-// One thread = 4 consecutive pixels of one row (all 3 channels) when W % 4 == 0, else 1 pixel.
-template <int VEC>
+// One thread = 4 consecutive pixels of one row (all C channels) when W % 4 == 0, else 1 pixel.  C = 3 (colour) or 1
+// (grayscale): the element index within a chain is e = c H W + pixel either way, so channel 0 draws the same noise.
+template <int VEC, int C>
 __global__ void __launch_bounds__(256)
 pre_inpaint_kernel(PreArgs a, int B, int H, int W, const float* __restrict__ x, const float* __restrict__ mask,
                    int mask_B, const float* __restrict__ y, int y_B, const float* __restrict__ noise,
@@ -30,13 +31,13 @@ pre_inpaint_kernel(PreArgs a, int B, int H, int W, const float* __restrict__ x, 
   if (g >= groups_per_chain * B) return;
   const int b = (int)(g / groups_per_chain);
   const long long pix = (g % groups_per_chain) * VEC;  // first pixel (row-major) of this thread
-  float outv[3][VEC];
+  float outv[C][VEC];
 #pragma unroll
-  for (int c = 0; c < 3; ++c) {
+  for (int c = 0; c < C; ++c) {
     const long long e = c * plane + pix;  // element index inside the chain
-    const long long gi = ((long long)b * 3) * plane + e;
-    const long long mi = ((long long)(mask_B > 1 ? b : 0) * 3) * plane + e;
-    const long long yi = ((long long)(y_B > 1 ? b : 0) * 3) * plane + e;
+    const long long gi = ((long long)b * C) * plane + e;
+    const long long mi = ((long long)(mask_B > 1 ? b : 0) * C) * plane + e;
+    const long long yi = ((long long)(y_B > 1 ? b : 0) * C) * plane + e;
     float xv[VEC], mv[VEC], yv[VEC], zv[VEC];
     if (VEC == 4) {
       const float4 t0 = *reinterpret_cast<const float4*>(x + gi);
@@ -73,7 +74,8 @@ pre_inpaint_kernel(PreArgs a, int B, int H, int W, const float* __restrict__ x, 
   }
 #pragma unroll
   for (int j = 0; j < VEC; ++j)
-    store_nhwc16(den_in + ((long long)b * plane + pix + j) * 16, outv[0][j], outv[1][j], outv[2][j], a.den_in_c3);
+    store_nhwc16(den_in + ((long long)b * plane + pix + j) * 16, outv[0][j], C > 1 ? outv[1 % C][j] : 0.f,
+                 C > 2 ? outv[2 % C][j] : 0.f, a.den_in_c3);
 }
 
 // ------------------------------------------------------------------------------------------------ blur / deblur pre
@@ -102,7 +104,7 @@ __device__ __forceinline__ int wrap(int i, int n) {
 }
 
 // All loops below are (row = warp, warp + 8, ...; column = lane, lane + 32, ...): no integer division in the hot path.
-template <bool FULL>  // FULL: Langevin pre; else: out = A x
+template <bool FULL, int C>  // FULL: Langevin pre; else: out = A x.  C: image channels (3 or 1)
 __global__ void __launch_bounds__(256)
 blur_kernel(PreArgs a, const Taps c_taps_arg, int B, int H, int W, int l, const float* __restrict__ x, const float* __restrict__ y, int y_B,
             const float* __restrict__ noise, float* __restrict__ out, __nv_bfloat16* __restrict__ den_in) {
@@ -121,12 +123,12 @@ blur_kernel(PreArgs a, const Taps c_taps_arg, int B, int H, int W, int l, const 
   const int prow = tid >> 3, pcol = (tid & 7) * 4;  // this thread's 4 pixels inside the tile
   const int nt = 2 * l + 1;
   const int w1 = SW - 2 * l, h1 = SW - 2 * l;  // extent after one pass of A
-  float res[3][4];
-  float xin[3][4];
+  float res[C][4];
+  float xin[C][4];
 
 #pragma unroll
-  for (int c = 0; c < 3; ++c) {
-    const float* xp = x + ((long long)b * 3 + c) * plane;
+  for (int c = 0; c < C; ++c) {
+    const float* xp = x + ((long long)b * C + c) * plane;
     __syncthreads();
     for (int r = warp; r < SW; r += 8) {
       const float* row = xp + (long long)wrap(y0 - halo + r, H) * W;
@@ -143,7 +145,7 @@ blur_kernel(PreArgs a, const Taps c_taps_arg, int B, int H, int W, int l, const 
       }
     __syncthreads();
     // vertical pass of A (minus the observation for the Langevin step): s0[r][cc], r in [0, h1)
-    const float* yp = FULL ? y + ((long long)(y_B > 1 ? b : 0) * 3 + c) * plane : nullptr;
+    const float* yp = FULL ? y + ((long long)(y_B > 1 ? b : 0) * C + c) * plane : nullptr;
     for (int r = warp; r < h1; r += 8) {
       const long long yrow = FULL ? (long long)wrap(y0 - l + r, H) * W : 0;
       for (int cc = lane; cc < w1; cc += 32) {
@@ -161,7 +163,7 @@ blur_kernel(PreArgs a, const Taps c_taps_arg, int B, int H, int W, int l, const 
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         const int gx = x0 + pcol + j;
-        if (gy < H && gx < W) out[((long long)b * 3 + c) * plane + (long long)gy * W + gx] = s0[prow * SW + pcol + j];
+        if (gy < H && gx < W) out[((long long)b * C + c) * plane + (long long)gy * W + gx] = s0[prow * SW + pcol + j];
       }
       continue;
     }
@@ -186,8 +188,8 @@ blur_kernel(PreArgs a, const Taps c_taps_arg, int B, int H, int W, int l, const 
   const int gy = y0 + prow;
   if (gy >= H) return;
 #pragma unroll
-  for (int c = 0; c < 3; ++c) {
-    const long long rowoff = ((long long)b * 3 + c) * plane + (long long)gy * W;
+  for (int c = 0; c < C; ++c) {
+    const long long rowoff = ((long long)b * C + c) * plane + (long long)gy * W;
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       const int gx = x0 + pcol + j;
@@ -204,7 +206,8 @@ blur_kernel(PreArgs a, const Taps c_taps_arg, int B, int H, int W, int l, const 
   for (int j = 0; j < 4; ++j) {
     const int gx = x0 + pcol + j;
     if (gx < W)
-      store_nhwc16(den_in + ((long long)b * plane + (long long)gy * W + gx) * 16, xin[0][j], xin[1][j], xin[2][j], a.den_in_c3);
+      store_nhwc16(den_in + ((long long)b * plane + (long long)gy * W + gx) * 16, xin[0][j], C > 1 ? xin[1 % C][j] : 0.f,
+                   C > 2 ? xin[2 % C][j] : 0.f, a.den_in_c3);
   }
 }
 
@@ -222,7 +225,7 @@ struct BlurCfg {
   static constexpr size_t SMEM = (size_t)(2 * SW * SW + (FULL ? W1 * W1 : 0)) * sizeof(float);
 };
 
-template <bool FULL, int L>
+template <bool FULL, int L, int C>
 __global__ void __launch_bounds__(256, 3)
 blur_kernel_t(PreArgs a, const Taps c_taps_arg, int B, int H, int W, const float* __restrict__ x, const float* __restrict__ y, int y_B,
               const float* __restrict__ noise, float* __restrict__ out, __nv_bfloat16* __restrict__ den_in) {
@@ -254,7 +257,7 @@ blur_kernel_t(PreArgs a, const Taps c_taps_arg, int B, int H, int W, const float
     gxs[i] = wrap(x0 - HALO + lane + 32 * i, W);
     gys[i] = wrap(x0 - L + lane + 32 * i, W);
   }
-  float res[3][4], xc[3][4];
+  float res[C][4], xc[C][4];
   // Global -> register staging of one channel's tile: every load of the channel is issued before the first dependent
   // store (an in-order warp otherwise pays one DRAM round trip per staged row), and channel c + 1 is fetched while
   // channel c runs its four passes.
@@ -262,7 +265,7 @@ blur_kernel_t(PreArgs a, const Taps c_taps_arg, int B, int H, int W, const float
   constexpr int XI = (SW + 31) / 32, YI = (W1 + 31) / 32;    // staged columns per lane
   float xv[XR][XI], yv[FULL ? YR : 1][FULL ? YI : 1];
   auto fetch = [&](int c) {
-    const float* xp = x + ((long long)b * 3 + c) * plane;
+    const float* xp = x + ((long long)b * C + c) * plane;
 #pragma unroll
     for (int k = 0; k < XR; ++k) {
       const int r = warp + 8 * k;
@@ -271,7 +274,7 @@ blur_kernel_t(PreArgs a, const Taps c_taps_arg, int B, int H, int W, const float
       for (int i = 0; i < XI; ++i) xv[k][i] = (r < SW && lane + 32 * i < SW) ? row[gxs[i]] : 0.f;
     }
     if (FULL) {
-      const float* yp = y + ((long long)(y_B > 1 ? b : 0) * 3 + c) * plane;
+      const float* yp = y + ((long long)(y_B > 1 ? b : 0) * C + c) * plane;
 #pragma unroll
       for (int k = 0; k < YR; ++k) {
         const int r = warp + 8 * k;
@@ -284,7 +287,7 @@ blur_kernel_t(PreArgs a, const Taps c_taps_arg, int B, int H, int W, const float
   fetch(0);
 
 #pragma unroll
-  for (int c = 0; c < 3; ++c) {
+  for (int c = 0; c < C; ++c) {
     __syncthreads();  // previous channel's readers of s0 / s1 are done
 #pragma unroll
     for (int k = 0; k < XR; ++k) {
@@ -302,7 +305,7 @@ blur_kernel_t(PreArgs a, const Taps c_taps_arg, int B, int H, int W, const float
           if (r < W1 && lane + 32 * i < W1) sy[r * W1 + lane + 32 * i] = yv[k][i];
       }
     }
-    if (c < 2) fetch(c + 1);
+    if (c < C - 1) fetch(c + 1);
     __syncthreads();
     {
       const float4 v = *reinterpret_cast<const float4*>(s0 + (HALO + prow) * SW + HALO + pcol);  // x at the owned pixels
@@ -394,11 +397,11 @@ blur_kernel_t(PreArgs a, const Taps c_taps_arg, int B, int H, int W, const float
   const int gx0 = x0 + pcol;
   if (gx0 >= W) return;
   const bool full_quad = gx0 + 3 < W;
-  float xin[3][4];
+  float xin[C][4];
 #pragma unroll
-  for (int c = 0; c < 3; ++c) {
+  for (int c = 0; c < C; ++c) {
     const long long e0 = (long long)c * plane + (long long)gy * W + gx0;  // element index inside the chain
-    const long long gi0 = (long long)b * 3 * plane + e0;
+    const long long gi0 = (long long)b * C * plane + e0;
     if (!FULL) {
 #pragma unroll
       for (int j = 0; j < 4; ++j)
@@ -433,7 +436,8 @@ blur_kernel_t(PreArgs a, const Taps c_taps_arg, int B, int H, int W, const float
 #pragma unroll
     for (int j = 0; j < 4; ++j)
       if (gx0 + j < W)
-        store_nhwc16(den_in + ((long long)b * plane + (long long)gy * W + gx0 + j) * 16, xin[0][j], xin[1][j], xin[2][j], a.den_in_c3);
+        store_nhwc16(den_in + ((long long)b * plane + (long long)gy * W + gx0 + j) * 16, xin[0][j], C > 1 ? xin[1 % C][j] : 0.f,
+                     C > 2 ? xin[2 % C][j] : 0.f, a.den_in_c3);
   }
 }
 
@@ -451,7 +455,10 @@ blur_kernel_t(PreArgs a, const Taps c_taps_arg, int B, int H, int W, const float
 //     columns in registers (the row loop is unrolled by 4l + 1 so that the ring is statically indexed);
 //   * the Langevin step, the noise draw and the fp32 base store happen in the thread that owns the pixel; the bf16 NHWC16
 //     denoiser input needs the three channels of a pixel together and is written one row late by the channel-0 threads from
-//     a double-buffered shared-memory row.
+//     a double-buffered shared-memory row;
+//   * grayscale (C = 1): the three thread groups that take the three channels of a colour image take three bands of RH rows
+//     of the one channel instead (a block covers 3 RH rows), so the block stays full; each thread stores its own pixels'
+//     denoiser input.
 // Per pixel-channel: 2 (4l + 1) FMAs against the 4-pass kernel's ~50 at l = 4 -- but what the 4-pass kernel really lost its
 // time on was five block-wide barriers per channel-tile and a 2.25x read amplification; here it is two barriers per ROW and
 // (RH + 4l) / RH.  Results differ from the two-pass-of-A formulation by fp32 rounding only (tests: 2e-5 relative).
@@ -492,7 +499,7 @@ __device__ __forceinline__ void ata_vpass(float (&hring)[NT][4], const float (&o
 
 // Two blocks per SM (156 registers).  A 96-register build with three resident blocks spills part of the window: 86 us
 // instead of 58 (measured, scripts/blur_sweep.py).
-template <int K2>  // K2 = 2 l: half-width of A^T A
+template <int K2, int C>  // K2 = 2 l: half-width of A^T A;  C: image channels (3 or 1)
 __global__ void __launch_bounds__(ATA_THREADS, 2)
 deblur_ata_kernel(PreArgs a, const Taps2 k, int B, int H, int W, int RH, const float* __restrict__ x,
                   const float* __restrict__ aty, int aty_B, const float* __restrict__ noise, float* __restrict__ out,
@@ -505,14 +512,16 @@ deblur_ata_kernel(PreArgs a, const Taps2 k, int B, int H, int W, int RH, const f
   float* aring = ring + NBUF * ROWSET;           // [NABUF][3][ATA_COLS]: every thread stages and reads its own 4 floats
   float* xin_s = aring + NABUF * 3 * ATA_COLS;   // [2][3][ATA_COLS]
   const int tid = threadIdx.x;
-  const int ch = tid >> 6, q = tid & 63;
+  const int ch = tid >> 6, q = tid & 63;  // ch: the thread group's channel (C = 3) or row band (C = 1)
   const int b = blockIdx.z;
-  const int x0 = blockIdx.x * ATA_COLS, y0 = blockIdx.y * RH;
-  const int rh = min(RH, H - y0);        // output rows of this block
+  const int x0 = blockIdx.x * ATA_COLS, y0 = blockIdx.y * RH * (3 / C);
+  const int yb = C == 3 ? y0 : y0 + ch * RH;  // first output row of this thread group
+  const int rh = min(RH, H - y0);        // output rows of this block (C = 1: of its first band, the longest)
+  const int rhb = min(RH, H - yb);       // output rows of this thread group's band (C = 1)
   const int nrows = rh + 2 * K2;         // input rows it walks
   const long long plane = (long long)H * W;
-  const float* xb = x + (long long)b * 3 * plane;
-  const float* ab = aty + (long long)(aty_B > 1 ? b : 0) * 3 * plane + (long long)ch * plane;
+  const float* xb = x + (long long)b * C * plane;
+  const float* ab = aty + (long long)(aty_B > 1 ? b : 0) * C * plane + (long long)(C == 3 ? ch : 0) * plane;
   const int gx0 = x0 + 4 * q;
   const bool vec_ok = (W % 4 == 0) && gx0 + 3 < W;
   // this thread's staged elements: e = tid + 192 i  ->  (channel, staged column); global offset without the row term.
@@ -521,11 +530,13 @@ deblur_ata_kernel(PreArgs a, const Taps2 k, int B, int H, int W, int RH, const f
   constexpr int NQ = (ROWSET / 4 + ATA_THREADS - 1) / ATA_THREADS;
   const bool vstage = (K2 % 4 == 0) && (W % 4 == 0);
   unsigned goff[NE];
+  int grow[NE];  // C = 1: the staged element's band, as its first input row minus K2
 #pragma unroll
   for (int i = 0; i < NE; ++i) {
     const int e = vstage ? 4 * (tid + ATA_THREADS * i) : tid + ATA_THREADS * i;  // first element of the quad / the element
     const int c = e / SROW, col = e - c * SROW;
-    goff[i] = (e < ROWSET) ? (unsigned)((long long)c * plane + wrap(x0 - K2 + col, W)) : 0u;
+    goff[i] = (e < ROWSET) ? (unsigned)((long long)(C == 3 ? c : 0) * plane + wrap(x0 - K2 + col, W)) : 0u;
+    grow[i] = y0 + c * RH - K2;
   }
   // One commit group per input row r: the row itself and the A^T y values of the output row it completes (r - 2 K2).
   auto stage = [&](int r) {
@@ -538,7 +549,8 @@ deblur_ata_kernel(PreArgs a, const Taps2 k, int B, int H, int W, int RH, const f
           const int e = 4 * (tid + ATA_THREADS * i);
           if (e < ROWSET) {
             const unsigned saddr = (unsigned)__cvta_generic_to_shared(dst + e);
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(saddr), "l"(xb + rowoff + goff[i]) : "memory");
+            const long long ro = C == 3 ? rowoff : (long long)wrap(grow[i] + r, H) * W;
+            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(saddr), "l"(xb + ro + goff[i]) : "memory");
           }
         }
       } else {
@@ -547,13 +559,14 @@ deblur_ata_kernel(PreArgs a, const Taps2 k, int B, int H, int W, int RH, const f
           const int e = tid + ATA_THREADS * i;
           if (e < ROWSET) {
             const unsigned saddr = (unsigned)__cvta_generic_to_shared(dst + e);
-            asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(saddr), "l"(xb + rowoff + goff[i]) : "memory");
+            const long long ro = C == 3 ? rowoff : (long long)wrap(grow[i] + r, H) * W;
+            asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(saddr), "l"(xb + ro + goff[i]) : "memory");
           }
         }
       }
       const int orow = r - 2 * K2;
-      if (orow >= 0 && gx0 < W) {
-        const float* src = ab + (long long)(y0 + orow) * W + gx0;
+      if (orow >= 0 && gx0 < W && (C == 3 || orow < rhb)) {
+        const float* src = ab + (long long)(yb + orow) * W + gx0;
         float* adst = aring + ((orow % NABUF) * 3 + ch) * ATA_COLS + 4 * q;
         const unsigned saddr = (unsigned)__cvta_generic_to_shared(adst);
         if (vec_ok) {
@@ -576,7 +589,7 @@ deblur_ata_kernel(PreArgs a, const Taps2 k, int B, int H, int W, int RH, const f
 #pragma unroll
     for (int j = 0; j < 4; ++j) hring[t][j] = 0.f;
 
-  // den_in of output row `orow` (tile-local), written by the channel-0 threads once all three channels are in xin_s
+  // den_in of output row `orow` (tile-local), written by the channel-0 threads once all three channels are in xin_s (C = 3)
   auto flush_den_in = [&](int orow) {
     if (ch == 0 && gx0 < W) {
       const int gy = y0 + orow;
@@ -594,7 +607,7 @@ deblur_ata_kernel(PreArgs a, const Taps2 k, int B, int H, int W, int RH, const f
     asm volatile("cp.async.wait_group %0;" ::"n"(ATA_AHEAD - 1) : "memory");  // this thread's part of row r has landed
     __syncthreads();           // row r is visible to all; every thread has finished iteration r - 1
     stage(r + ATA_AHEAD);      // into the slot of row r - K2 - 1, whose last reader was iteration r - 1 (the centre row)
-    if (r > 2 * K2) flush_den_in(r - 2 * K2 - 1);  // the previous output row's xin_s is complete
+    if (C == 3 && r > 2 * K2) flush_den_in(r - 2 * K2 - 1);  // the previous output row's xin_s is complete
     // ---- horizontal pass on row r
     float o[4];
     {
@@ -631,11 +644,11 @@ deblur_ata_kernel(PreArgs a, const Taps2 k, int B, int H, int W, int RH, const f
     // ---- Langevin step
     if (emit) {
       const int orow = r - 2 * K2;
-      const int gy = y0 + orow;
+      const int gy = yb + orow;
       float xin[4] = {0.f, 0.f, 0.f, 0.f};
-      if (gx0 < W) {
-        const long long e0 = (long long)ch * plane + (long long)gy * W + gx0;  // element index inside the chain
-        const long long gi0 = (long long)b * 3 * plane + e0;
+      if (gx0 < W && (C == 3 || orow < rhb)) {
+        const long long e0 = (long long)(C == 3 ? ch : 0) * plane + (long long)gy * W + gx0;  // element index inside the chain
+        const long long gi0 = (long long)b * C * plane + e0;
         float xv[4], av[4], z[4];
         const float* xc = ring + ((r - K2) % NBUF) * ROWSET + ch * SROW + K2 + 4 * q;  // the output row itself, still staged
         const float* ac = aring + ((orow % NABUF) * 3 + ch) * ATA_COLS + 4 * q;
@@ -663,12 +676,20 @@ deblur_ata_kernel(PreArgs a, const Taps2 k, int B, int H, int W, int RH, const f
           for (int j = 0; j < 4; ++j)
             if (gx0 + j < W) out[gi0 + j] = bv[j];
         }
+        if (C == 1) {
+#pragma unroll
+          for (int j = 0; j < 4; ++j)
+            if (gx0 + j < W) store_nhwc16(den_in + ((long long)b * plane + (long long)gy * W + gx0 + j) * 16, xin[j], 0.f, 0.f, a.den_in_c3);
+        }
       }
-      *reinterpret_cast<float4*>(xin_s + ((orow & 1) * 3 + ch) * ATA_COLS + 4 * q) = make_float4(xin[0], xin[1], xin[2], xin[3]);
+      if (C == 3)
+        *reinterpret_cast<float4*>(xin_s + ((orow & 1) * 3 + ch) * ATA_COLS + 4 * q) = make_float4(xin[0], xin[1], xin[2], xin[3]);
     }
   }
-  __syncthreads();
-  flush_den_in(rh - 1);
+  if (C == 3) {
+    __syncthreads();
+    flush_den_in(rh - 1);
+  }
 }
 
 __global__ void __launch_bounds__(256)
@@ -693,14 +714,15 @@ noise_torch_cuda_kernel(long long numel, unsigned long long seed, unsigned long 
   if (g < numel) out[g] = torch_cuda_normal_at(seed, offset, T, (uint64_t)g);
 }
 
+template <int C>
 __global__ void __launch_bounds__(256)
 to_nhwc16_kernel(int B, int H, int W, const float* __restrict__ x, float c3, __nv_bfloat16* __restrict__ out) {
   const long long plane = (long long)H * W;
   const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= plane * B) return;
   const long long b = g / plane, pix = g % plane;
-  const float* xp = x + b * 3 * plane + pix;
-  store_nhwc16(out + g * 16, xp[0], xp[plane], xp[2 * plane], c3);
+  const float* xp = x + b * C * plane + pix;
+  store_nhwc16(out + g * 16, xp[0], C > 1 ? xp[plane] : 0.f, C > 2 ? xp[2 * plane] : 0.f, c3);
 }
 
 // Replication padding of a bf16 NHWC16 image batch in place: pixels with y >= H or x >= W (the pad a U-Net needs to reach a
@@ -756,9 +778,10 @@ int fill_pre(const psgla_pre_params* p, PreArgs* a) {
   return PSGLA_OK;
 }
 
+// C = 3 (colour) or 1 (grayscale): the kernels take the channel count as a template parameter
 static int check_img(const psgla_img_shape& s) {
-  PSGLA_REQUIRE(s.B > 0 && s.H > 0 && s.W > 0 && s.C == 3, "image shape must be [B>0][3][H>0][W>0], got [%d][%d][%d][%d]",
-                s.B, s.C, s.H, s.W);
+  PSGLA_REQUIRE(s.B > 0 && s.H > 0 && s.W > 0 && (s.C == 3 || s.C == 1),
+                "image shape must be [B>0][C = 1 or 3][H>0][W>0], got [%d][%d][%d][%d]", s.B, s.C, s.H, s.W);
   PSGLA_REQUIRE((long long)s.C * s.H * s.W < (1LL << 32), "one chain must have fewer than 2^32 elements");
   return PSGLA_OK;
 }
@@ -785,56 +808,51 @@ extern "C" int psgla_img_pre_inpaint(const psgla_pre_params* p, psgla_img_shape 
   PSGLA_REQUIRE(x_dev && mask_dev && y_dev && base_dev && den_in_dev, "psgla_img_pre_inpaint: null pointer");
   PSGLA_REQUIRE((mask_B == 1 || mask_B == s.B) && (y_B == 1 || y_B == s.B), "mask_B / y_B must be 1 or B");
   const long long plane = (long long)s.H * s.W;
-  a.chw = 3 * plane;
+  a.chw = s.C * plane;
   cudaStream_t st = (cudaStream_t)stream;
-  if (plane % 4 == 0) {
-    const long long n = plane / 4 * s.B;
-    pre_inpaint_kernel<4><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(a, s.B, s.H, s.W, x_dev, mask_dev, mask_B, y_dev,
-                                                                      y_B, noise_dev, base_dev,
-                                                                      (__nv_bfloat16*)den_in_dev);
-  } else {
-    const long long n = plane * s.B;
-    pre_inpaint_kernel<1><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(a, s.B, s.H, s.W, x_dev, mask_dev, mask_B, y_dev,
-                                                                      y_B, noise_dev, base_dev,
-                                                                      (__nv_bfloat16*)den_in_dev);
-  }
+  const int vec = plane % 4 == 0 ? 4 : 1;
+  const long long n = plane / vec * s.B;
+  auto kern = vec == 4 ? (s.C == 3 ? pre_inpaint_kernel<4, 3> : pre_inpaint_kernel<4, 1>)
+                       : (s.C == 3 ? pre_inpaint_kernel<1, 3> : pre_inpaint_kernel<1, 1>);
+  kern<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(a, s.B, s.H, s.W, x_dev, mask_dev, mask_B, y_dev, y_B, noise_dev, base_dev,
+                                                    (__nv_bfloat16*)den_in_dev);
   PSGLA_CUDA_TRY(cudaGetLastError());
   return PSGLA_OK;
 }
 
-template <bool FULL, int L>
+template <bool FULL, int L, int C>
 static int launch_blur_t(const PreArgs& a, const Taps& taps, psgla_img_shape s, const float* x, const float* y, int y_B,
                          const float* noise, float* out, void* den_in, cudaStream_t st) {
   constexpr size_t smem = BlurCfg<FULL, L>::SMEM;
   static std::atomic<unsigned long long> attr_done{0};  // bit d: opted in on device d (a per-device function attribute)
   const unsigned long long dev_bit = 1ull << (current_device() & 63);
   if (smem > 48 * 1024 && !(attr_done.load(std::memory_order_acquire) & dev_bit)) {
-    PSGLA_CUDA_TRY(cudaFuncSetAttribute(blur_kernel_t<FULL, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    PSGLA_CUDA_TRY(cudaFuncSetAttribute(blur_kernel_t<FULL, L, C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_done.fetch_or(dev_bit, std::memory_order_release);
   }
   const int tiles = ((s.W + BT - 1) / BT) * ((s.H + BT - 1) / BT);
-  blur_kernel_t<FULL, L><<<dim3(tiles, s.B), 256, smem, st>>>(a, taps, s.B, s.H, s.W, x, y, y_B, noise, out, (__nv_bfloat16*)den_in);
+  blur_kernel_t<FULL, L, C><<<dim3(tiles, s.B), 256, smem, st>>>(a, taps, s.B, s.H, s.W, x, y, y_B, noise, out, (__nv_bfloat16*)den_in);
   PSGLA_CUDA_TRY(cudaGetLastError());
   return PSGLA_OK;
 }
 
-template <bool FULL>
+template <bool FULL, int C>
 static int launch_blur(const PreArgs& a, const Taps& taps, psgla_img_shape s, int l, const float* x, const float* y, int y_B,
                        const float* noise, float* out, void* den_in, cudaStream_t st) {
   switch (l) {  // compile-time even half-widths (the reference's default is l = 4); anything else takes the generic kernel
-    case 2: return launch_blur_t<FULL, 2>(a, taps, s, x, y, y_B, noise, out, den_in, st);
-    case 4: return launch_blur_t<FULL, 4>(a, taps, s, x, y, y_B, noise, out, den_in, st);
-    case 6: return launch_blur_t<FULL, 6>(a, taps, s, x, y, y_B, noise, out, den_in, st);
-    case 8: return launch_blur_t<FULL, 8>(a, taps, s, x, y, y_B, noise, out, den_in, st);
+    case 2: return launch_blur_t<FULL, 2, C>(a, taps, s, x, y, y_B, noise, out, den_in, st);
+    case 4: return launch_blur_t<FULL, 4, C>(a, taps, s, x, y, y_B, noise, out, den_in, st);
+    case 6: return launch_blur_t<FULL, 6, C>(a, taps, s, x, y, y_B, noise, out, den_in, st);
+    case 8: return launch_blur_t<FULL, 8, C>(a, taps, s, x, y, y_B, noise, out, den_in, st);
     default: break;
   }
   const int halo = FULL ? 2 * l : l;
   const int SW = BT + 2 * halo;
   const size_t smem = (size_t)2 * SW * SW * sizeof(float);
   if (smem > 48 * 1024)  // a per-device attribute of the function, cheap to set: no process-wide cache
-    PSGLA_CUDA_TRY(cudaFuncSetAttribute(blur_kernel<FULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    PSGLA_CUDA_TRY(cudaFuncSetAttribute(blur_kernel<FULL, C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int tiles = ((s.W + BT - 1) / BT) * ((s.H + BT - 1) / BT);
-  blur_kernel<FULL><<<dim3(tiles, s.B), 256, smem, st>>>(a, taps, s.B, s.H, s.W, l, x, y, y_B, noise, out,
+  blur_kernel<FULL, C><<<dim3(tiles, s.B), 256, smem, st>>>(a, taps, s.B, s.H, s.W, l, x, y, y_B, noise, out,
                                                         (__nv_bfloat16*)den_in);
   PSGLA_CUDA_TRY(cudaGetLastError());
   return PSGLA_OK;
@@ -851,11 +869,12 @@ extern "C" int psgla_img_pre_deblur(const psgla_pre_params* p, psgla_img_shape s
   PSGLA_REQUIRE(x_dev && y_dev && base_dev && den_in_dev, "psgla_img_pre_deblur: null pointer");
   PSGLA_REQUIRE(x_dev != base_dev, "psgla_img_pre_deblur: base must not alias x (the stencil reads neighbours)");
   PSGLA_REQUIRE(y_B == 1 || y_B == s.B, "y_B must be 1 or B");
-  a.chw = 3LL * s.H * s.W;
+  a.chw = (long long)s.C * s.H * s.W;
   Taps taps;
   rc = make_taps(h1d_host, l, &taps);
   if (rc) return rc;
-  return launch_blur<true>(a, taps, s, l, x_dev, y_dev, y_B, noise_dev, base_dev, den_in_dev, (cudaStream_t)stream);
+  return (s.C == 3 ? launch_blur<true, 3> : launch_blur<true, 1>)(a, taps, s, l, x_dev, y_dev, y_B, noise_dev, base_dev,
+                                                                  den_in_dev, (cudaStream_t)stream);
 }
 
 // k = h * h (full 1-D convolution, 4 l + 1 taps) in double, rounded once.
@@ -870,17 +889,19 @@ static void ata_taps(const float* h, int l, Taps2* k) {
   }
 }
 
-template <int K2>
+template <int K2, int C>
 static int launch_ata(const PreArgs& a, const Taps2& k, psgla_img_shape s, const float* x, const float* aty, int aty_B,
                       const float* noise, float* out, void* den_in, cudaStream_t st) {
   // rows per block: two blocks are resident per SM (registers) and hide each other's latencies, so the launch takes about
   // ceil(blocks / (2 SMs)) rounds of RH + 2 K2 row steps (measured at 32 chains of 256 x 256, l = 4: RH = 8 / 16 / 32 / 64 / 128
-  // -> 83 / 66 / 59 / 82 / 152 us; the four-pass kernel 84 us)
+  // -> 83 / 66 / 59 / 82 / 152 us; the four-pass kernel 84 us).  A grayscale block covers `bands` = 3 bands of RH rows in the
+  // same RH + 2 K2 row steps, so the cost model holds for it with three times the rows per block.
+  const int bands = 3 / C;
   const int strips = (s.W + ATA_COLS - 1) / ATA_COLS, sms = 2 * num_sms();
   int best_rh = 16;
   long long best = -1;
   for (int rh = 8; rh <= 128; rh *= 2) {
-    const long long blocks = (long long)strips * ((s.H + rh - 1) / rh) * s.B;
+    const long long blocks = (long long)strips * ((s.H + bands * rh - 1) / (bands * rh)) * s.B;
     const long long cost = ((blocks + sms - 1) / sms) * (rh + 2 * K2);
     if (best < 0 || cost < best) best = cost, best_rh = rh;
   }
@@ -888,15 +909,16 @@ static int launch_ata(const PreArgs& a, const Taps2& k, psgla_img_shape s, const
     const int v = std::atoi(e);
     if (v >= 1) best_rh = v;
   }
-  PSGLA_REQUIRE(s.B <= 65535 && (s.H + best_rh - 1) / best_rh <= 65535, "too many chains / rows for one launch");
+  const int row_blocks = (s.H + bands * best_rh - 1) / (bands * best_rh);
+  PSGLA_REQUIRE(s.B <= 65535 && row_blocks <= 65535, "too many chains / rows for one launch");
   constexpr size_t smem = AtaCfg<K2>::SMEM;
   static std::atomic<unsigned long long> attr_done{0};  // bit d: opted in on device d (a per-device function attribute)
   const unsigned long long dev_bit = 1ull << (current_device() & 63);
   if (smem > 48 * 1024 && !(attr_done.load(std::memory_order_acquire) & dev_bit)) {
-    PSGLA_CUDA_TRY(cudaFuncSetAttribute(deblur_ata_kernel<K2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    PSGLA_CUDA_TRY(cudaFuncSetAttribute(deblur_ata_kernel<K2, C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_done.fetch_or(dev_bit, std::memory_order_release);
   }
-  deblur_ata_kernel<K2><<<dim3(strips, (s.H + best_rh - 1) / best_rh, s.B), ATA_THREADS, smem, st>>>(
+  deblur_ata_kernel<K2, C><<<dim3(strips, row_blocks, s.B), ATA_THREADS, smem, st>>>(
       a, k, s.B, s.H, s.W, best_rh, x, aty, aty_B, noise, out, (__nv_bfloat16*)den_in);
   PSGLA_CUDA_TRY(cudaGetLastError());
   return PSGLA_OK;
@@ -914,15 +936,16 @@ extern "C" int psgla_img_pre_deblur_ata(const psgla_pre_params* p, psgla_img_sha
   PSGLA_REQUIRE(x_dev != base_dev, "psgla_img_pre_deblur_ata: base must not alias x (the stencil reads neighbours)");
   PSGLA_REQUIRE(aty_B == 1 || aty_B == s.B, "aty_B must be 1 or B");
   PSGLA_REQUIRE(l >= 1 && l <= 4, "psgla_img_pre_deblur_ata serves half-widths 1..4 (got %d); use psgla_img_pre_deblur", l);
-  a.chw = 3LL * s.H * s.W;
+  a.chw = (long long)s.C * s.H * s.W;
   Taps2 k;
   ata_taps(h1d_host, l, &k);
   cudaStream_t st = (cudaStream_t)stream;
+  const bool gray = s.C == 1;
   switch (l) {
-    case 1: return launch_ata<2>(a, k, s, x_dev, aty_dev, aty_B, noise_dev, base_dev, den_in_dev, st);
-    case 2: return launch_ata<4>(a, k, s, x_dev, aty_dev, aty_B, noise_dev, base_dev, den_in_dev, st);
-    case 3: return launch_ata<6>(a, k, s, x_dev, aty_dev, aty_B, noise_dev, base_dev, den_in_dev, st);
-    default: return launch_ata<8>(a, k, s, x_dev, aty_dev, aty_B, noise_dev, base_dev, den_in_dev, st);
+    case 1: return (gray ? launch_ata<2, 1> : launch_ata<2, 3>)(a, k, s, x_dev, aty_dev, aty_B, noise_dev, base_dev, den_in_dev, st);
+    case 2: return (gray ? launch_ata<4, 1> : launch_ata<4, 3>)(a, k, s, x_dev, aty_dev, aty_B, noise_dev, base_dev, den_in_dev, st);
+    case 3: return (gray ? launch_ata<6, 1> : launch_ata<6, 3>)(a, k, s, x_dev, aty_dev, aty_B, noise_dev, base_dev, den_in_dev, st);
+    default: return (gray ? launch_ata<8, 1> : launch_ata<8, 3>)(a, k, s, x_dev, aty_dev, aty_B, noise_dev, base_dev, den_in_dev, st);
   }
 }
 
@@ -935,7 +958,8 @@ extern "C" int psgla_img_blur(psgla_img_shape s, const float* x_dev, const float
   rc = make_taps(h1d_host, l, &taps);
   if (rc) return rc;
   PreArgs a{};
-  return launch_blur<false>(a, taps, s, l, x_dev, nullptr, 1, nullptr, out_dev, nullptr, (cudaStream_t)stream);
+  return (s.C == 3 ? launch_blur<false, 3> : launch_blur<false, 1>)(a, taps, s, l, x_dev, nullptr, 1, nullptr, out_dev, nullptr,
+                                                                    (cudaStream_t)stream);
 }
 
 extern "C" int psgla_img_noise(psgla_img_shape s, uint64_t seed, int64_t chain_id0, int64_t iteration, float* out_dev,
@@ -999,8 +1023,8 @@ extern "C" int psgla_img_to_nhwc16(psgla_img_shape s, const float* x_dev, float 
   if (rc) return rc;
   PSGLA_REQUIRE(x_dev && out_dev, "psgla_img_to_nhwc16: null pointer");
   const long long n = (long long)s.H * s.W * s.B;
-  to_nhwc16_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(s.B, s.H, s.W, x_dev, c3,
-                                                                                 (__nv_bfloat16*)out_dev);
+  (s.C == 3 ? to_nhwc16_kernel<3> : to_nhwc16_kernel<1>)<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+      s.B, s.H, s.W, x_dev, c3, (__nv_bfloat16*)out_dev);
   PSGLA_CUDA_TRY(cudaGetLastError());
   return PSGLA_OK;
 }

@@ -3,7 +3,7 @@ csrc/gsdrunet.cu) as tcgen05 implicit-GEMM convolutions (csrc/conv_tc.cu, csrc/c
 (csrc/tv_prox.cu).
 
 ``DnCNN`` mirrors ``deepinv.models.DnCNN(in_channels=3, out_channels=3, pretrained=..., device=...)`` as the reference constructs
-it (sampling_images.py:130) and calls it (``denoiser.forward(x, sigma)``, restoration_algorithms.py:238): depth 20,
+it (sampling_images.py:130), and its one-channel form ``in_channels=out_channels=1`` for grayscale images and calls it (``denoiser.forward(x, sigma)``, restoration_algorithms.py:238): depth 20,
 64 features, 3x3, bias, ReLU, residual output, ``sigma`` ignored.  Weights come from a deepinv-style state dict
 (keys ``in_conv``, ``conv_list.i``, ``out_conv``) -- a checkpoint path, a dict, or ``None`` for seeded random init.
 Activations are bf16 with fp32 accumulation; the input / output images stay fp32.
@@ -21,8 +21,9 @@ __all__ = ["DnCNN", "DRUNet", "GSDRUNet", "TVDenoiser", "random_dncnn_state_dict
            "smoothing_dncnn_state_dict", "random_drunet_state_dict", "random_gsdrunet_state_dict", "DRUNET_KEYS", "GSDRUNET_KEYS"]
 
 
-def random_dncnn_state_dict(seed=0, depth=20, nf=64, scale=1.0):
-    """Deterministic random-init DnCNN state dict (uniform +-1/sqrt(fan_in) like nn.Conv2d's default), on the CPU."""
+def random_dncnn_state_dict(seed=0, depth=20, nf=64, scale=1.0, channels=3):
+    """Deterministic random-init DnCNN state dict (uniform +-1/sqrt(fan_in) like nn.Conv2d's default), on the CPU.
+    ``channels``: image channels, 3 (colour) or 1 (grayscale)."""
     g = torch.Generator().manual_seed(seed)
     sd = {}
 
@@ -31,10 +32,10 @@ def random_dncnn_state_dict(seed=0, depth=20, nf=64, scale=1.0):
         sd[name + ".weight"] = (torch.rand((cout, cin, 3, 3), generator=g) * 2 - 1) * bound
         sd[name + ".bias"] = (torch.rand((cout,), generator=g) * 2 - 1) * 0.01
 
-    conv("in_conv", nf, 3)
+    conv("in_conv", nf, channels)
     for i in range(depth - 2):
         conv("conv_list.%d" % i, nf, nf)
-    conv("out_conv", 3, nf)
+    conv("out_conv", channels, nf)
     return sd
 
 
@@ -54,11 +55,12 @@ def _conv_operator_norm(w, spatial=16, n_power_iter=40):
     return float(lam.max().sqrt())
 
 
-def lipschitz_dncnn_state_dict(seed=0, depth=20, nf=64, lipschitz=0.9, spatial=16):
+def lipschitz_dncnn_state_dict(seed=0, depth=20, nf=64, lipschitz=0.9, spatial=16, channels=3):
     """Seeded random-init DnCNN whose residual branch has Lipschitz bound ``lipschitz`` < 1 (the stand-in BASELINE.json
     prescribes for the unavailable ``dncnn_sigma2_lipschitz_color.pth``, README.md:28-29): every conv is divided by
-    its exact circular operator norm and the layers share the bound evenly.  Set-up code, runs once on the CPU."""
-    sd = random_dncnn_state_dict(seed, depth, nf)
+    its exact circular operator norm and the layers share the bound evenly.  Set-up code, runs once on the CPU.
+    ``channels``: image channels, 3 (colour) or 1 (grayscale)."""
+    sd = random_dncnn_state_dict(seed, depth, nf, channels=channels)
     per_layer = lipschitz ** (1.0 / depth)
     for name in ["in_conv"] + ["conv_list.%d" % i for i in range(depth - 2)] + ["out_conv"]:
         w = sd[name + ".weight"]
@@ -66,14 +68,15 @@ def lipschitz_dncnn_state_dict(seed=0, depth=20, nf=64, lipschitz=0.9, spatial=1
     return sd
 
 
-def smoothing_dncnn_state_dict(eps=0.5, n_smooth=6, depth=20, nf=64):
+def smoothing_dncnn_state_dict(eps=0.5, n_smooth=6, depth=20, nf=64, channels=3):
     """A DnCNN-architecture state dict, written down by hand, that IS a (weak) denoiser: its residual is
     ``R(x) = eps * (G x - x)`` with G = ``n_smooth`` passes of the 3 x 3 binomial kernel [1 2 1]^T [1 2 1] / 16.  The checkpoint the
     reference uses cannot be fetched offline and a random-init network restores nothing (unobserved pixels random-walk), so
     this is the stand-in for runs whose PSNR should MEAN something: PSGLA with it is diffusion inpainting / smoothing-regularised
     deblurring, stable at any length, and ||R||_Lip <= eps < 1.  Construction (ReLU networks compute linear maps on
     x = relu(x) - relu(-x)): features 0-2 / 3-5 carry relu(+-x) and are smoothed by layers 1..n_smooth, features 6-8 / 9-11
-    carry relu(+-x) unchanged, every other feature is zero; the last layer forms eps ((f0-2 - f3-5) - (f6-8 - f9-11))."""
+    carry relu(+-x) unchanged, every other feature is zero; the last layer forms eps ((f0-2 - f3-5) - (f6-8 - f9-11)).
+    ``channels``: image channels, 3 (colour) or 1 (grayscale: features 0, 3, 6, 9 carry the one channel)."""
     if depth < n_smooth + 2 or nf < 12:
         raise ValueError("needs depth >= n_smooth + 2 and nf >= 12")
     g1 = torch.tensor([1.0, 2.0, 1.0]) / 4.0
@@ -81,8 +84,8 @@ def smoothing_dncnn_state_dict(eps=0.5, n_smooth=6, depth=20, nf=64):
     ident = torch.zeros(3, 3)
     ident[1, 1] = 1.0
     sd = {}
-    w = torch.zeros(nf, 3, 3, 3)
-    for c in range(3):
+    w = torch.zeros(nf, channels, 3, 3)
+    for c in range(channels):
         for base, sign in ((0, 1.0), (3, -1.0), (6, 1.0), (9, -1.0)):
             w[base + c, c, 1, 1] = sign
     sd["in_conv.weight"], sd["in_conv.bias"] = w, torch.zeros(nf)
@@ -91,26 +94,31 @@ def smoothing_dncnn_state_dict(eps=0.5, n_smooth=6, depth=20, nf=64):
         for f in range(12):
             w[f, f] = G if (f < 6 and i < n_smooth) else ident
         sd["conv_list.%d.weight" % i], sd["conv_list.%d.bias" % i] = w, torch.zeros(nf)
-    w = torch.zeros(3, nf, 3, 3)
-    for c in range(3):
+    w = torch.zeros(channels, nf, 3, 3)
+    for c in range(channels):
         w[c, c, 1, 1], w[c, 3 + c, 1, 1], w[c, 6 + c, 1, 1], w[c, 9 + c, 1, 1] = eps, -eps, -eps, eps
-    sd["out_conv.weight"], sd["out_conv.bias"] = w, torch.zeros(3)
+    sd["out_conv.weight"], sd["out_conv.bias"] = w, torch.zeros(channels)
     return sd
 
 
 class DnCNN:
+    """``channels`` (= in_channels = out_channels): 3 for colour images, 1 for grayscale ones.  The weights are packed for that
+    channel count, and the samplers take images of that many channels only."""
+
     is_residual = True  # D(x) = x + R(x): the samplers add gain * R to their base
 
     def __init__(self, in_channels=3, out_channels=3, depth=20, bias=True, nf=64, pretrained=None, device=None):
         torch_ = _lib.require_cuda()
-        if in_channels != 3 or out_channels != 3 or nf != 64:
-            raise ValueError("the sm_100a conv path is built for colour DnCNN: in=out=3 channels, nf=64")
+        if in_channels != out_channels or in_channels not in (1, 3) or nf != 64:
+            raise ValueError("the sm_100a conv path is built for DnCNN with in = out = 3 (colour) or 1 (grayscale) channels, "
+                             "nf = 64")
         if depth < 2:
             raise ValueError("depth must be >= 2")
+        self.channels = int(in_channels)
         self.depth = int(depth)
         self.device = torch_.device("cuda", torch_.cuda.current_device()) if device is None else torch_.device(device)
         if pretrained is None:
-            sd = random_dncnn_state_dict(0, depth, nf)
+            sd = random_dncnn_state_dict(0, depth, nf, channels=self.channels)
         elif isinstance(pretrained, str):
             sd = torch_.load(pretrained, map_location="cpu")
         else:
@@ -121,7 +129,7 @@ class DnCNN:
             raise KeyError("state dict lacks %s" % missing[:3])
         self.state_dict_fp32 = {k: v.detach().to("cpu", torch_.float32).contiguous() for k, v in sd.items()}
         ws = [self.state_dict_fp32[n + ".weight"] for n in names]
-        expect = [(nf, 3, 3, 3)] + [(nf, nf, 3, 3)] * (depth - 2) + [(3, nf, 3, 3)]
+        expect = [(nf, self.channels, 3, 3)] + [(nf, nf, 3, 3)] * (depth - 2) + [(self.channels, nf, 3, 3)]
         for w, e, n in zip(ws, expect, names):
             if tuple(w.shape) != e:
                 raise ValueError("%s.weight has shape %s, expected %s" % (n, tuple(w.shape), e))
@@ -132,8 +140,8 @@ class DnCNN:
         warr = (FP * depth)(*[C.cast(w.data_ptr(), FP) for w in ws])
         barr = (FP * depth)(*[C.cast(b.data_ptr(), FP) if b is not None else FP() for b in bs])
         with torch_.cuda.device(self.device):
-            _lib.check(lib.psgla_dncnn_pack_weights(self.depth, warr, barr, _lib.ptr(self.packed),
-                                                    _lib.stream_ptr(self.device)), "psgla_dncnn_pack_weights")
+            _lib.check(lib.psgla_dncnn_pack_weights_ch(self.depth, self.channels, warr, barr, _lib.ptr(self.packed),
+                                                       _lib.stream_ptr(self.device)), "psgla_dncnn_pack_weights_ch")
         self._ws = None
         self._den_in = None
 
@@ -159,11 +167,12 @@ class DnCNN:
         _lib.check(rc, "psgla_dncnn_residual_post_next")
 
     def forward(self, x, sigma=None):
-        """D(x) = x + R(x), fp32 [B,3,H,W] in and out (``sigma`` ignored, as in deepinv's DnCNN)."""
+        """D(x) = x + R(x), fp32 [B,C,H,W] in and out, C = ``channels`` (``sigma`` ignored, as in deepinv's DnCNN)."""
         if not x.is_cuda:
             raise RuntimeError("DnCNN.forward needs a CUDA tensor: there is no CPU path")
+        _check_channels(x, self.channels, "DnCNN")
         x = x.to(torch.float32).contiguous()
-        shape = _lib.ImgShape(int(x.shape[0]), 3, int(x.shape[2]), int(x.shape[3]))
+        shape = _lib.ImgShape(int(x.shape[0]), self.channels, int(x.shape[2]), int(x.shape[3]))
         _, den_in = self.buffers(shape)
         out = torch.empty_like(x)
         with torch.cuda.device(self.device):
@@ -174,6 +183,12 @@ class DnCNN:
 
     __call__ = forward
     apply_post = residual_post  # common name used by the samplers for both denoiser families
+
+
+def _check_channels(x, channels, name):
+    if x.dim() != 4 or x.shape[1] != channels:
+        raise ValueError("%s was built for %d-channel images: expected a [B,%d,H,W] batch, got %s" %
+                         (name, channels, channels, tuple(x.shape)))
 
 
 # ----------------------------------------------------------------------------------------------------- DRUNet
@@ -191,11 +206,11 @@ DRUNET_KEYS = _drunet_keys()  # the 64 weight tensors of drunet_color.pth in sta
 GSDRUNET_KEYS = _drunet_keys(2)  # the 36 of the gradient-step DRUNet's network (nb = 2)
 
 
-def _drunet_shape(key, nc=(64, 128, 256, 512)):
+def _drunet_shape(key, nc=(64, 128, 256, 512), channels=3):
     if key == "m_head.weight":
-        return (nc[0], 4, 3, 3)
+        return (nc[0], channels + 1, 3, 3)  # the image channels, then the noise-level map
     if key == "m_tail.weight":
-        return (3, nc[0], 3, 3)
+        return (channels, nc[0], 3, 3)
     if key.startswith("m_body"):
         return (nc[3], nc[3], 3, 3)
     s = int(key[len("m_down")]) if key.startswith("m_down") else int(key[len("m_up")])
@@ -206,14 +221,14 @@ def _drunet_shape(key, nc=(64, 128, 256, 512)):
     return (nc[s], nc[s - 1], 2, 2)      # transposed conv: [Cin][Cout][2][2]
 
 
-def random_drunet_state_dict(seed=0, gain=0.5, nb=4):
+def random_drunet_state_dict(seed=0, gain=0.5, nb=4, channels=3):
     """Seeded random-init DRUNet state dict on the CPU (checkpoints are unreachable offline): uniform
     +-gain*sqrt(3/fan_in), second conv of every residual block halved, tail quartered, so activations stay O(1).
-    ``nb``: residual blocks per stage (2: the gradient-step DRUNet's network)."""
+    ``nb``: residual blocks per stage (2: the gradient-step DRUNet's network).  ``channels``: image channels, 3 or 1."""
     g = torch.Generator().manual_seed(seed)
     sd = {}
     for k in _drunet_keys(nb):
-        shp = _drunet_shape(k)
+        shp = _drunet_shape(k, channels=channels)
         is_up = k.startswith("m_up") and ".res." not in k
         fan_in = shp[0] * 4 if is_up else shp[1] * shp[2] * shp[3]
         bound = gain * math.sqrt(3.0 / fan_in)
@@ -229,17 +244,20 @@ class DRUNet:
     """``deepinv.models.DRUNet(in_channels=3, out_channels=3, pretrained=..., device=...)`` (sampling_images.py:136) on
     tcgen05 convolutions: the DPIR U-Net (KAIR UNetRes, nc = 64/128/256/512, 4 residual blocks per stage, no biases).
     ``forward(x, sigma)`` appends the constant noise-level channel and returns the denoised image.  ``pretrained``: a
-    ``drunet_color.pth``-style state dict / path, or None for seeded random init.  H, W multiples of 8."""
+    ``drunet_color.pth``-style state dict / path, or None for seeded random init.  H, W multiples of 8.
+    ``channels`` (= in_channels = out_channels): 3 for colour images, 1 for grayscale ones (``drunet_gray.pth``-style: m_head
+    takes the image and the noise-level map, m_tail gives one channel); the samplers take images of that many channels only."""
 
     is_residual = False  # the network outputs D(x) itself
 
     def __init__(self, in_channels=3, out_channels=3, pretrained=None, device=None):
         torch_ = _lib.require_cuda()
-        if in_channels != 3 or out_channels != 3:
-            raise ValueError("the sm_100a DRUNet path is built for colour images: in = out = 3 channels")
+        if in_channels != out_channels or in_channels not in (1, 3):
+            raise ValueError("the sm_100a DRUNet path is built for in = out = 3 (colour) or 1 (grayscale) channels")
+        self.channels = int(in_channels)
         self.device = torch_.device("cuda", torch_.cuda.current_device()) if device is None else torch_.device(device)
         if pretrained is None:
-            sd = random_drunet_state_dict(0)
+            sd = random_drunet_state_dict(0, channels=self.channels)
         elif isinstance(pretrained, str):
             sd = torch_.load(pretrained, map_location="cpu")
         else:
@@ -250,8 +268,9 @@ class DRUNet:
         ws = []
         for k in DRUNET_KEYS:
             w = sd[k].detach().to("cpu", torch_.float32).contiguous()
-            if tuple(w.shape) != _drunet_shape(k):
-                raise ValueError("%s has shape %s, expected %s" % (k, tuple(w.shape), _drunet_shape(k)))
+            want = _drunet_shape(k, channels=self.channels)
+            if tuple(w.shape) != want:
+                raise ValueError("%s has shape %s, expected %s" % (k, tuple(w.shape), want))
             ws.append(w)
         self.state_dict_fp32 = dict(zip(DRUNET_KEYS, ws))
         lib = _lib.lib()
@@ -260,8 +279,8 @@ class DRUNet:
         FP = C.POINTER(C.c_float)
         warr = (FP * len(ws))(*[C.cast(w.data_ptr(), FP) for w in ws])
         with torch_.cuda.device(self.device):
-            _lib.check(lib.psgla_drunet_pack_weights(warr, _lib.ptr(self.packed), _lib.stream_ptr(self.device)),
-                       "psgla_drunet_pack_weights")
+            _lib.check(lib.psgla_drunet_pack_weights_ch(self.channels, warr, _lib.ptr(self.packed), _lib.stream_ptr(self.device)),
+                       "psgla_drunet_pack_weights_ch")
         self._ws = None
         self._den_in = None
 
@@ -285,20 +304,21 @@ class DRUNet:
         _lib.check(rc, "psgla_drunet_denoise_post_next")
 
     def forward(self, x, sigma):
-        """D(x; sigma), fp32 [B,3,H,W] in and out.  The U-Net halves the resolution three times, so H and W must be multiples
+        """D(x; sigma), fp32 [B,C,H,W] in and out, C = ``channels``.  The U-Net halves the resolution three times, so H and W must be multiples
         of 8; other sizes (CBSD68's 481 x 321) are replication-padded at the bottom / right to the next multiple, denoised and
         cropped -- KAIR's ``test_pad`` rule, which is what deepinv applies to small inputs (its rule for large ones, a 4-way
         overlapping split, cannot be verified offline: a documented deviation).  The samplers apply the same per-call padding to
         inpainting problems (restoration_algorithms._Run); deblurring problems must be cropped to multiples of 8."""
         if not x.is_cuda:
             raise RuntimeError("DRUNet.forward needs a CUDA tensor: there is no CPU path")
+        _check_channels(x, self.channels, "DRUNet")
         sigma = float(sigma.reshape(-1)[0]) if isinstance(sigma, torch.Tensor) else float(sigma)
         x = x.to(torch.float32).contiguous()
         H0, W0 = int(x.shape[2]), int(x.shape[3])
         ph, pw = (-H0) % 8, (-W0) % 8
         if ph or pw:
             x = torch.nn.functional.pad(x, (0, pw, 0, ph), mode="replicate").contiguous()
-        shape = _lib.ImgShape(int(x.shape[0]), 3, int(x.shape[2]), int(x.shape[3]))
+        shape = _lib.ImgShape(int(x.shape[0]), self.channels, int(x.shape[2]), int(x.shape[3]))
         _, den_in = self.buffers(shape)
         out = torch.empty_like(x)
         with torch.cuda.device(self.device):
@@ -346,6 +366,7 @@ class GSDRUNet:
     (csrc/gsdrunet.cu).  ``pretrained``: None (seeded random init), a checkpoint path or a state dict.  H, W multiples of 8."""
 
     is_residual = False  # D(x) itself
+    channels = 3  # colour-only
 
     def __init__(self, alpha=1.0, in_channels=3, out_channels=3, nb=2, nc=(64, 128, 256, 512), act_mode="E", pretrained=None,
                  device=None):
@@ -440,6 +461,7 @@ class TVDenoiser:
     count of each chain in the last call (no host synchronisation)."""
 
     is_residual = False  # D(y) itself: the samplers form (1 - alpha) Y + alpha D(Y)
+    channels = 3  # colour-only
 
     def __init__(self, verbose=False, tau=0.01, rho=1.99, n_it_max=1000, crit=1e-5, device=None):
         torch_ = _lib.require_cuda()

@@ -26,11 +26,21 @@ ROW_FIELDS = ("index", "psnr_mmse", "ssim_mmse", "psnr_chain_mean", "psnr_chain_
               "psnr_observation", "std_mean", "std_max", "n_chains", "n_windows", "H", "W")
 
 
-def load_image(path, device=None):
-    """A colour image file as the reference reads it (sampling_images.py:268-276: ``imread_uint`` -> RGB uint8 -> float32 / 255
-    -> [1, 3, H, W])."""
+def load_image(path, device=None, n_channels=3):
+    """An image file as the reference reads it (sampling_images.py:268-276: ``imread_uint`` -> uint8 -> float32 / 255 ->
+    [1, n_channels, H, W]).  ``n_channels=3``: RGB.  ``n_channels=1`` (the reference's ``--grayscale`` runs): the file is read
+    as ``cv2.imread(path, 0)``, which is KAIR's ``imread_uint(path, n_channels=1)`` as recalled -- that rule cannot be checked
+    against KAIR here, so a colour file's conversion to gray may differ from the reference's."""
     import cv2
     import numpy as np
+    if n_channels not in (1, 3):
+        raise ValueError("n_channels must be 1 or 3")
+    if n_channels == 1:
+        gray = cv2.imread(path, 0)
+        if gray is None:
+            raise FileNotFoundError(path)
+        t = torch.from_numpy(np.ascontiguousarray(np.float32(gray / 255.0))).float()[None, None]
+        return t if device is None else t.to(device)
     bgr = cv2.imread(path, cv2.IMREAD_COLOR)
     if bgr is None:
         raise FileNotFoundError(path)
@@ -74,7 +84,7 @@ def _sample_image(index, im, denoiser, problem, alg, n_chains, prm, seed, seed_i
         raise ValueError("alg must be 'psgla' or 'pnp_ula'")
     if not M:
         raise ValueError("no statistics window closed: n_iter = %d must exceed n_inter_mmse = %d" % (prm["N"], prm["n_inter_mmse"]))
-    M, M2 = M[0], M2[0]  # [n_chains, 3, H, W]: per-chain mean of the window means / second moments
+    M, M2 = M[0], M2[0]  # [n_chains, C, H, W]: per-chain mean of the window means / second moments
     xmmse = M.mean(0)    # chains are exchangeable: the pooled posterior mean (sampling_images.py:427 over chains as well)
     var = M2.mean(0) - xmmse ** 2
     std = torch.sqrt(torch.clamp(var, min=0.0))  # :436-439
@@ -96,7 +106,8 @@ def run_image_set(images, denoiser=None, problem="inpainting", alg="psgla", n_ch
                   seed_ip=0, prop=0.5, sigma=1.0, l=4, blur_type="uniform", si=1.0, keep_maps=False, _sample=None):
     """Posterior sampling of a SET of images, ``n_chains`` independent chains each, sharded over the process group.
 
-    images     list of [3, H, W] / [1, 3, H, W] float tensors in [0, 1] (sizes may differ), the same list on every rank
+    images     list of [C, H, W] / [1, C, H, W] float tensors in [0, 1] (sizes may differ), the same list on every rank; C = the
+               denoiser's channel count (1: grayscale images with a one-channel DnCNN / DRUNet)
     denoiser   this rank's ``psgla_b200.DnCNN`` / ``DRUNet`` / ``GSDRUNet`` / ``TVDenoiser`` (default: a DnCNN with the library's seeded
                weights; TV: psgla only, table row ``den="TV"``, the prox state is reset before each image)
     params     the dict of ``psgla_b200.sampler_params`` (default: the script's table for ``alg`` / the denoiser family, with

@@ -20,15 +20,15 @@ __all__ = ["InpaintingDataGrad", "DeblurDataGrad", "PriorGrad", "make_inpainting
 
 
 def _shape_of(x) -> "_lib.ImgShape":
-    if x.dim() != 4 or x.shape[1] != 3:
-        raise ValueError("expected a [B,3,H,W] tensor, got %s" % (tuple(x.shape),))
-    return _lib.ImgShape(int(x.shape[0]), 3, int(x.shape[2]), int(x.shape[3]))
+    if x.dim() != 4 or x.shape[1] not in (1, 3):
+        raise ValueError("expected a [B,3,H,W] (colour) or [B,1,H,W] (grayscale) tensor, got %s" % (tuple(x.shape),))
+    return _lib.ImgShape(int(x.shape[0]), int(x.shape[1]), int(x.shape[2]), int(x.shape[3]))
 
 
 class InpaintingDataGrad:
     """``data_grad(x) = -mask * (x - y) / sigma2`` (sampling_images.py:295).
 
-    mask, y: tensors broadcastable to [B,3,H,W] (the reference uses [1,3,H,W]); sigma2: float."""
+    mask, y: tensors broadcastable to [B,C,H,W] (the reference uses [1,C,H,W]; C = 3, or 1 for grayscale); sigma2: float."""
 
     kind = "inpainting"
 

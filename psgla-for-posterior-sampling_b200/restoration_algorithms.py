@@ -23,6 +23,8 @@ Extra keyword-only arguments:
 The data term must be an ``InpaintingDataGrad`` / ``DeblurDataGrad`` and the denoiser a ``psgla_b200.DnCNN`` / ``DRUNet`` /
 ``GSDRUNet`` (``prior_grad`` a ``PriorGrad`` wrapping one); opaque callables raise ``TypeError`` -- there is no eager fallback.
 ``GSDRUNet`` needs image sides that are multiples of 8.
+Images have the denoiser's channel count: 3 (colour), or 1 (grayscale, the reference's ``--grayscale`` runs) with a
+``DnCNN`` / ``DRUNet`` built with ``in_channels = out_channels = 1``.  ``TVDenoiser`` and ``GSDRUNet`` are colour-only.
 ``psgla`` / ``psgla_run`` / ``pnp`` also take a ``psgla_b200.TVDenoiser`` (PSGLA-TV): each iteration is then the "pre" launch and
 one cooperative launch of the TV prox with the post fused (csrc/tv_prox.cu), at any image size.  ``pnpula`` and ``red`` feed
 the denoiser X instead of the fp32 base and reject it.
@@ -71,9 +73,11 @@ class _Run:
         x = init.detach().to(torch.float32)
         if x.dim() == 3:
             x = x[None]
-        if x.dim() != 4 or x.shape[1] != 3:
-            raise ValueError("init must be a [B,3,H,W] (or [3,H,W]) colour image batch, got %s: the kernels index three "
-                             "planes per chain (the reference's --grayscale runs are out of scope)" % (tuple(init.shape),))
+        Cn = int(denoiser.channels)  # 3, or 1 for a grayscale DnCNN / DRUNet
+        if x.dim() != 4 or x.shape[1] != Cn:
+            raise ValueError("init must be a [B,%d,H,W] (or [%d,H,W]) %s image batch to match the %d-channel %s%s, got %s" %
+                             (Cn, Cn, "colour" if Cn == 3 else "grayscale", Cn, type(denoiser).__name__,
+                              " (colour-only)" if isinstance(denoiser, (TVDenoiser, GSDRUNet)) else "", tuple(init.shape)))
         self.squeeze = n_chains is None and x.shape[0] == 1
         B = int(n_chains) if n_chains is not None else int(x.shape[0])
         # DRUNet halves the resolution three times.  Sides that are not multiples of 8 (CBSD68: 481 x 321) are handled like KAIR's
@@ -93,10 +97,10 @@ class _Run:
             ph, pw = (-x.shape[2]) % 8, (-x.shape[3]) % 8
             x = torch.nn.functional.pad(x, (0, pw, 0, ph), mode="replicate")
             if noise is not None:
-                noise = torch.nn.functional.pad(noise.reshape((noise.shape[0], -1, 3) + self.crop).to(self.device, torch.float32),
+                noise = torch.nn.functional.pad(noise.reshape((noise.shape[0], -1, Cn) + self.crop).to(self.device, torch.float32),
                                                 (0, pw, 0, ph))
         self.X = x.expand(B, -1, -1, -1).contiguous().clone() if x.shape[0] != B else x.contiguous().clone()
-        self.shape = _lib.ImgShape(B, 3, int(x.shape[2]), int(x.shape[3]))
+        self.shape = _lib.ImgShape(B, Cn, int(x.shape[2]), int(x.shape[3]))
         self.base = torch.empty_like(self.X)
         _, self.den_in = denoiser.buffers(self.shape)
         self.n_iter, self.n_inter = int(n_iter), int(n_inter)
@@ -155,10 +159,10 @@ class _Run:
                                  (what, tuple(t.shape), B, "/".join(str(c) for c in channels), want[0], want[1]))
             if self.crop is not None:  # zero pad: the pad region is unobserved
                 t = torch.nn.functional.pad(t, (0, W - want[1], 0, H - want[0]))
-            return t.expand(-1, 3, -1, -1).contiguous()
+            return t.expand(-1, Cn, -1, -1).contiguous()
 
         if isinstance(data_grad, DeblurDataGrad):
-            self.y = operand(data_grad.y, "the blurred observation y", (3,))
+            self.y = operand(data_grad.y, "the blurred observation y", (Cn,))
             self.mask = None
             # A^T(A x - y) = (A^T A) x - A^T y: A^T y is blurred once here, the iterations run the two-pass A^T A kernel
             # (PSGLA_BLUR_4PASS=1 keeps the four-pass kernel for A/B runs; half-widths above 4 always take it)
@@ -166,8 +170,8 @@ class _Run:
             if 1 <= data_grad.l <= 4 and os.environ.get("PSGLA_BLUR_4PASS", "0") != "1":
                 self.aty = data_grad.AT(self.y)
         else:
-            self.y = operand(data_grad.y, "the observation y", (1, 3))
-            self.mask = operand(data_grad.mask, "the mask", (1, 3))
+            self.y = operand(data_grad.y, "the observation y", (1, Cn))
+            self.mask = operand(data_grad.mask, "the mask", (1, Cn))
 
     def configure(self, pre, gain, base_scale=1.0):
         self.pre_params, self.gain, self.base_scale = pre, float(gain), float(base_scale)
@@ -191,7 +195,10 @@ class _Run:
     def _out(self, t):
         if self.crop is not None:
             t = t[..., :self.crop[0], :self.crop[1]]
-        return t[0] if self.squeeze else t
+        if not self.squeeze:
+            return t
+        # the reference appends torch.squeeze(X): [3, H, W] for colour, [H, W] for a grayscale chain
+        return t[0, 0] if self.shape.C == 1 else t[0]
 
     def z_for(self, i):
         if self.noise is not None:
