@@ -19,7 +19,6 @@
 // quadratic in v; r > 2: online log-sum-exp over the components held in shared memory).
 #include <algorithm>
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 
 #include "common.cuh"
@@ -28,10 +27,8 @@ namespace psgla {
 
 constexpr int RMAX = PSGLA_GMM_MAX_COMPONENTS;
 
-// default launch geometry of the fp32, r == 2 Philox path: cpt, nb, block, pack, dynamic (see launch_run)
-#ifndef PSGLA_GMM_DEFAULT_GEOM
-#define PSGLA_GMM_DEFAULT_GEOM 4, 64, 16, 1, 2
-#endif
+// gmm2d_lean_kernel's geometry: 4 Philox counter blocks (8 steps) per round, 64-thread blocks, 16 of them resident per SM.
+constexpr int LEAN_NB = 4, LEAN_BLOCK = 64, LEAN_MINB = 16;
 
 template <typename T>
 struct Gmm2dConsts {
@@ -137,12 +134,11 @@ __device__ __forceinline__ void langevin_step(const Gmm2dConsts<T>& c, const Gmm
 }
 
 // ------------------------------------------------------------------------------------------------ packed fp32 pairs
-// sm_100 issues two fp32 FMAs per lane as ONE instruction (FFMA2, PTX fma.rn.f32x2).  The chain kernel is issue-bound, so
-// the r == 2 fp32 path carries chains in PAIRS: every state / noise / intermediate register pair holds the same quantity of
-// chains 2p and 2p+1, the constants are duplicated into both halves on the host (Gmm2dConstsPk), and the affine maps, the
-// quadratic logit, the component means and the Box-Muller arithmetic cost one instruction per pair instead of two.  The
-// operations and their order per chain are those of langevin_step<float>: results are bit-identical to the scalar path.
-typedef unsigned long long pk2;  // {lo: chain 2p, hi: chain 2p+1}
+// sm_100 issues two fp32 FMAs per lane as ONE instruction (FFMA2, PTX fma.rn.f32x2).  The lean kernel is issue-bound, so it
+// runs the Box-Muller arithmetic of two Philox counter blocks as pairs: each 64-bit register holds the same quantity of both
+// blocks and costs one instruction instead of two.  The operations and their order per value are those of box_muller
+// (common.cuh): results are bit-identical to the scalar path.
+typedef unsigned long long pk2;  // {lo, hi}
 __device__ __forceinline__ pk2 pk(float lo, float hi) {
   pk2 r;
   asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
@@ -159,48 +155,7 @@ __device__ __forceinline__ pk2 mul2(pk2 a, pk2 b) {
   asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
   return r;
 }
-__device__ __forceinline__ pk2 add2(pk2 a, pk2 b) {
-  pk2 r;
-  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-  return r;
-}
-
-struct Gmm2dConstsPk {  // Gmm2dConsts<float> with every constant duplicated into both halves of a 64-bit word
-  pk2 P[4], q[2], cn, cp, tq[6], M1[4], b1[2], dM[4], db[2], one;
-};
-
-__device__ __forceinline__ void denoise_r2_pk(const Gmm2dConstsPk& c, pk2 v0, pk2 v1, pk2& d0, pk2& d1) {
-  const pk2 t = fma2(v0, fma2(c.tq[3], v0, fma2(c.tq[4], v1, c.tq[1])), fma2(v1, fma2(c.tq[5], v1, c.tq[2]), c.tq[0]));
-  float ta, tb;
-  unpk(t, ta, tb);
-  float sa, sb;
-  unpk(add2(c.one, pk(fast_exp2(ta), fast_exp2(tb))), sa, sb);
-  const pk2 w0 = pk(fast_rcp(sa), fast_rcp(sb));
-  const pk2 m0 = fma2(c.M1[0], v0, fma2(c.M1[1], v1, c.b1[0]));
-  const pk2 m1 = fma2(c.M1[2], v0, fma2(c.M1[3], v1, c.b1[1]));
-  const pk2 e0 = fma2(c.dM[0], v0, fma2(c.dM[1], v1, c.db[0]));
-  const pk2 e1 = fma2(c.dM[2], v0, fma2(c.dM[3], v1, c.db[1]));
-  d0 = fma2(w0, e0, m0);
-  d1 = fma2(w0, e1, m1);
-}
-
-template <int ALG>
-__device__ __forceinline__ void langevin_step_pk(const Gmm2dConstsPk& c, pk2& x0, pk2& x1, pk2 z0, pk2 z1) {
-  const pk2 l0 = fma2(c.P[0], x0, fma2(c.P[1], x1, fma2(c.cn, z0, c.q[0])));
-  const pk2 l1 = fma2(c.P[2], x0, fma2(c.P[3], x1, fma2(c.cn, z1, c.q[1])));
-  pk2 d0, d1;
-  if (ALG == PSGLA_ALG_PSGLA) {
-    denoise_r2_pk(c, l0, l1, d0, d1);
-    x0 = d0;
-    x1 = d1;
-  } else {
-    denoise_r2_pk(c, x0, x1, d0, d1);
-    x0 = fma2(c.cp, d0, l0);
-    x1 = fma2(c.cp, d1, l1);
-  }
-}
-
-// box_muller (common.cuh) on the same word of two chains at once: (a, b) of chain 2p and of chain 2p+1.
+// box_muller (common.cuh) on the same word of two counter blocks at once: (a, b) of block A and of block B.
 __device__ __forceinline__ void box_muller_pk(uint32_t aA, uint32_t bA, uint32_t aB, uint32_t bB, pk2& z0, pk2& z1) {
   const pk2 u1 = fma2(pk((float)aA, (float)aB), pk(2.3283064365386963e-10f, 2.3283064365386963e-10f),
                       pk(1.1641532182693481e-10f, 1.1641532182693481e-10f));
@@ -227,15 +182,13 @@ __device__ __forceinline__ void box_muller_pk(uint32_t aA, uint32_t bA, uint32_t
 // Philox mode draws NB counter blocks (= 2 NB steps) of every owned chain at once: the 10-round integer pipeline of the NB x CPT
 // independent blocks is where the instruction-level parallelism comes from, so a thread that owns ONE chain (small populations,
 // and the 1-warp blocks of the dynamically scheduled launch) still keeps the pipes busy between the dependent Langevin steps.
-template <typename T, int ALG, bool R2, int CPT, int NB, int BLOCK, bool PACK>
+template <typename T, int ALG, bool R2, int CPT, int NB, int BLOCK>
 __global__ void __launch_bounds__(BLOCK, (sizeof(T) == 4 && R2) ? 1024 / BLOCK : 1)
-gmm2d_kernel(const Gmm2dConsts<T> c, const Gmm2dConstsPk cpk, const Gmm2dComponents<T>* __restrict__ comps_gmem,
-             T* __restrict__ x, long long n_chains, long long chain_lo, long long n_launch, unsigned long long chain_id0,
-             long long n_steps, long long step0, const PhiloxKeys keys, const T* __restrict__ noise, T* __restrict__ traj,
-             long long thin) {
+gmm2d_kernel(const Gmm2dConsts<T> c, const Gmm2dComponents<T>* __restrict__ comps_gmem, T* __restrict__ x,
+             long long n_chains, long long chain_lo, long long n_launch, unsigned long long chain_id0, long long n_steps,
+             long long step0, const PhiloxKeys keys, const T* __restrict__ noise, T* __restrict__ traj, long long thin) {
   // This launch owns chains [chain_lo, chain_lo + n_launch) of the call's n_chains (the stride of noise / traj rows).
   using V2 = typename Vec2<T>::type;
-  static_assert(!PACK || (sizeof(T) == 4 && R2 && CPT % 2 == 0), "the packed path is fp32, r == 2, chains in pairs");
   __shared__ Gmm2dComponents<T> comps_smem;
   const Gmm2dComponents<T>* comps = nullptr;
   if (!R2) {
@@ -315,73 +268,27 @@ gmm2d_kernel(const Gmm2dConsts<T> c, const Gmm2dConstsPk cpk, const Gmm2dCompone
       }
     };
     if (t < t_end && (t & 1)) one_block(false, true);  // a segment that starts on the second half of a counter block
-    if constexpr (PACK) {
-      pk2 X0[CPT / 2], X1[CPT / 2];
+    while (t + 2 * NB <= t_end) {
+      float z[NB][CPT][4];
+      const unsigned long long pair = (unsigned long long)t >> 1;
 #pragma unroll
-      for (int p = 0; p < CPT / 2; ++p) {
-        X0[p] = pk(x0[2 * p], x0[2 * p + 1]);
-        X1[p] = pk(x1[2 * p], x1[2 * p + 1]);
-      }
-      auto sync_scalars = [&](void) {
+      for (int b = 0; b < NB; ++b)
 #pragma unroll
-        for (int p = 0; p < CPT / 2; ++p) {
-          unpk(X0[p], x0[2 * p], x0[2 * p + 1]);
-          unpk(X1[p], x1[2 * p], x1[2 * p + 1]);
+        for (int j = 0; j < CPT; ++j) {
+          const unsigned long long pr = pair + b;
+          philox_normal4_keyed(keys, sub[j], (uint32_t)pr, (uint32_t)(pr >> 32), z[b][j][0], z[b][j][1], z[b][j][2], z[b][j][3]);
         }
-      };
-      while (t + 2 * NB <= t_end) {
-        pk2 z[NB][CPT / 2][4];
-        const unsigned long long pair = (unsigned long long)t >> 1;
 #pragma unroll
-        for (int b = 0; b < NB; ++b)
+      for (int b = 0; b < NB; ++b) {
 #pragma unroll
-          for (int p = 0; p < CPT / 2; ++p) {
-            const unsigned long long pr = pair + b;
-            uint32_t a0 = (uint32_t)pr, a1 = (uint32_t)(pr >> 32), a2 = (uint32_t)sub[2 * p], a3 = (uint32_t)(sub[2 * p] >> 32);
-            uint32_t b0 = a0, b1 = a1, b2 = (uint32_t)sub[2 * p + 1], b3 = (uint32_t)(sub[2 * p + 1] >> 32);
-            philox4x32_10_keyed(a0, a1, a2, a3, keys);
-            philox4x32_10_keyed(b0, b1, b2, b3, keys);
-            box_muller_pk(a0, a1, b0, b1, z[b][p][0], z[b][p][1]);
-            box_muller_pk(a2, a3, b2, b3, z[b][p][2], z[b][p][3]);
-          }
+        for (int h = 0; h < 2; ++h) {
 #pragma unroll
-        for (int b = 0; b < NB; ++b) {
-#pragma unroll
-          for (int h = 0; h < 2; ++h) {
-#pragma unroll
-            for (int p = 0; p < CPT / 2; ++p) langevin_step_pk<ALG>(cpk, X0[p], X1[p], z[b][p][2 * h], z[b][p][2 * h + 1]);
-            if (traj != nullptr) {
-              sync_scalars();
-              after_step();
-            }
-          }
+          for (int j = 0; j < CPT; ++j)
+            langevin_step<T, ALG, R2>(c, comps, x0[j], x1[j], T(z[b][j][2 * h]), T(z[b][j][2 * h + 1]));
+          after_step();
         }
-        t += 2 * NB;
       }
-      sync_scalars();
-    } else {
-      while (t + 2 * NB <= t_end) {
-        float z[NB][CPT][4];
-        const unsigned long long pair = (unsigned long long)t >> 1;
-#pragma unroll
-        for (int b = 0; b < NB; ++b)
-#pragma unroll
-          for (int j = 0; j < CPT; ++j) {
-            const unsigned long long pr = pair + b;
-            philox_normal4_keyed(keys, sub[j], (uint32_t)pr, (uint32_t)(pr >> 32), z[b][j][0], z[b][j][1], z[b][j][2], z[b][j][3]);
-          }
-#pragma unroll
-        for (int b = 0; b < NB; ++b) {
-#pragma unroll
-          for (int h = 0; h < 2; ++h) {
-#pragma unroll
-            for (int j = 0; j < CPT; ++j)
-              langevin_step<T, ALG, R2>(c, comps, x0[j], x1[j], T(z[b][j][2 * h]), T(z[b][j][2 * h + 1]));
-            after_step();
-          }
-        }
-        t += 2 * NB;
-      }
+      t += 2 * NB;
     }
     while (t < t_end) one_block(true, t + 1 < t_end);  // fewer than 2 NB steps left
   }
@@ -443,78 +350,44 @@ static int constants_structure(const Gmm2dConsts<float>& c) {
 // ------------------------------------------------------------------------------------------------ the lean kernel
 // fp32, r == 2, in-kernel Philox, no trajectory: the throughput path and nothing else, so that it fits a register budget
 // that keeps more warps resident than the general kernel's 64 registers allow (the general kernel spends ~20 registers on
-// 64-bit bookkeeping of the optional replay / trajectory paths).  One chain per thread; each round draws NB counter blocks
-// (2 NB steps), with the Box-Muller arithmetic of two blocks packed into FFMA2 / FMUL2 when PK.  Same Philox counters, same
-// arithmetic per chain as gmm2d_kernel: bit-identical results.
-// MODE bit 0: Box-Muller arithmetic of two counter blocks packed (FFMA2 / FMUL2); bit 1: software pipelining -- the Philox
-// words of round r + 1 are computed in the same loop body as the Box-Muller transform and the Langevin steps of round r, so
-// that every warp offers the scheduler IMAD.WIDE (FMA pipe), MUFU (XU pipe) and FFMA work at the same time instead of in
-// three phases.
-template <int ALG, int STRUCT, int NB, int BLOCK, int MINB, int MODE>
-__global__ void __launch_bounds__(BLOCK, MINB)
+// 64-bit bookkeeping of the optional replay / trajectory paths).  One chain per thread; each round draws LEAN_NB counter
+// blocks (2 LEAN_NB steps), with the Box-Muller arithmetic of two blocks packed into FFMA2 / FMUL2.  Same Philox counters,
+// same arithmetic per chain as gmm2d_kernel: bit-identical results.
+template <int ALG, int STRUCT>
+__global__ void __launch_bounds__(LEAN_BLOCK, LEAN_MINB)
 gmm2d_lean_kernel(const Gmm2dConsts<float> c, float2* __restrict__ x, unsigned n_launch, unsigned long long sub0,
                   unsigned long long pair0, int n_rounds, const PhiloxKeys keys) {
-  constexpr bool PK = (MODE & 1) != 0 && NB % 2 == 0, PIPE = (MODE & 2) != 0;
-  const unsigned g = blockIdx.x * BLOCK + threadIdx.x;
+  static_assert(LEAN_NB % 2 == 0, "Box-Muller packs counter blocks in pairs");
+  const unsigned g = blockIdx.x * LEAN_BLOCK + threadIdx.x;
   if (g >= n_launch) return;
   float2 v = x[g];
   float x0 = v.x, x1 = v.y;
   const unsigned long long sub = sub0 + g;
   const uint32_t s_lo = (uint32_t)sub, s_hi = (uint32_t)(sub >> 32);
   unsigned long long pair = pair0;
-  auto words = [&](unsigned long long pr0, uint32_t (&w)[NB][4]) {  // Philox4x32-10 of counter blocks pr0 .. pr0 + NB - 1
+  for (int r = 0; r < n_rounds; ++r, pair += LEAN_NB) {
+    uint32_t w[LEAN_NB][4];  // Philox4x32-10 of counter blocks pair .. pair + LEAN_NB - 1
 #pragma unroll
-    for (int b = 0; b < NB; ++b) {
-      const unsigned long long pr = pr0 + b;
+    for (int b = 0; b < LEAN_NB; ++b) {
+      const unsigned long long pr = pair + b;
       w[b][0] = (uint32_t)pr, w[b][1] = (uint32_t)(pr >> 32), w[b][2] = s_lo, w[b][3] = s_hi;
       philox4x32_10_keyed(w[b][0], w[b][1], w[b][2], w[b][3], keys);
     }
-  };
-  auto normals = [&](const uint32_t (&w)[NB][4], float (&z)[NB][4]) {
-    if constexpr (PK) {
+    float z[LEAN_NB][4];
 #pragma unroll
-      for (int b = 0; b < NB; b += 2) {
-        pk2 q0, q1, q2, q3;
-        box_muller_pk(w[b][0], w[b][1], w[b + 1][0], w[b + 1][1], q0, q1);
-        box_muller_pk(w[b][2], w[b][3], w[b + 1][2], w[b + 1][3], q2, q3);
-        unpk(q0, z[b][0], z[b + 1][0]);
-        unpk(q1, z[b][1], z[b + 1][1]);
-        unpk(q2, z[b][2], z[b + 1][2]);
-        unpk(q3, z[b][3], z[b + 1][3]);
-      }
-    } else {
-#pragma unroll
-      for (int b = 0; b < NB; ++b) {
-        box_muller(w[b][0], w[b][1], z[b][0], z[b][1]);
-        box_muller(w[b][2], w[b][3], z[b][2], z[b][3]);
-      }
+    for (int b = 0; b < LEAN_NB; b += 2) {
+      pk2 q0, q1, q2, q3;
+      box_muller_pk(w[b][0], w[b][1], w[b + 1][0], w[b + 1][1], q0, q1);
+      box_muller_pk(w[b][2], w[b][3], w[b + 1][2], w[b + 1][3], q2, q3);
+      unpk(q0, z[b][0], z[b + 1][0]);
+      unpk(q1, z[b][1], z[b + 1][1]);
+      unpk(q2, z[b][2], z[b + 1][2]);
+      unpk(q3, z[b][3], z[b + 1][3]);
     }
-  };
-  uint32_t w[NB][4];
-  if (PIPE) words(pair, w);
-  for (int r = 0; r < n_rounds; ++r, pair += NB) {
-    float z[NB][4];
-    if (PIPE) {
-      uint32_t wn[NB][4];
-      words(pair + NB, wn);  // one round ahead (the last iteration's are unused)
-      normals(w, z);
 #pragma unroll
-      for (int b = 0; b < NB; ++b) {
-        langevin_step_s<ALG, STRUCT>(c, x0, x1, z[b][0], z[b][1]);
-        langevin_step_s<ALG, STRUCT>(c, x0, x1, z[b][2], z[b][3]);
-      }
-#pragma unroll
-      for (int b = 0; b < NB; ++b)
-#pragma unroll
-        for (int i = 0; i < 4; ++i) w[b][i] = wn[b][i];
-    } else {
-      words(pair, w);
-      normals(w, z);
-#pragma unroll
-      for (int b = 0; b < NB; ++b) {
-        langevin_step_s<ALG, STRUCT>(c, x0, x1, z[b][0], z[b][1]);
-        langevin_step_s<ALG, STRUCT>(c, x0, x1, z[b][2], z[b][3]);
-      }
+    for (int b = 0; b < LEAN_NB; ++b) {
+      langevin_step_s<ALG, STRUCT>(c, x0, x1, z[b][0], z[b][1]);
+      langevin_step_s<ALG, STRUCT>(c, x0, x1, z[b][2], z[b][3]);
     }
   }
   x[g] = float2{x0, x1};
@@ -655,9 +528,7 @@ static int fold_problem(const psgla_gmm2d_problem* p, double eps, bool linear_pa
 
 template <typename T>
 static void narrow(const Folded& f, Gmm2dConsts<T>* c, Gmm2dComponents<T>* k) {
-  const double* src = reinterpret_cast<const double*>(&f.c);
   // Gmm2dConsts<double> is all doubles followed by one int: copy field by field
-  (void)src;
   for (int i = 0; i < 4; ++i) c->P[i] = (T)f.c.P[i];
   for (int i = 0; i < 2; ++i) c->q[i] = (T)f.c.q[i];
   c->cn = (T)f.c.cn;
@@ -689,35 +560,14 @@ static int upload_components(const Gmm2dComponents<T>& k, cudaStream_t st, Gmm2d
   return PSGLA_OK;
 }
 
-static Gmm2dConstsPk pack_consts(const Gmm2dConsts<float>& c) {
-  Gmm2dConstsPk r;
-  auto dup = [](float v) {
-    uint32_t u;
-    std::memcpy(&u, &v, 4);
-    return (pk2)u | ((pk2)u << 32);
-  };
-  for (int i = 0; i < 4; ++i) r.P[i] = dup(c.P[i]), r.M1[i] = dup(c.M1[i]), r.dM[i] = dup(c.dM[i]);
-  for (int i = 0; i < 2; ++i) r.q[i] = dup(c.q[i]), r.b1[i] = dup(c.b1[i]), r.db[i] = dup(c.db[i]);
-  for (int i = 0; i < 6; ++i) r.tq[i] = dup(c.tq[i]);
-  r.cn = dup(c.cn);
-  r.cp = dup(c.cp);
-  r.one = dup(1.0f);
-  return r;
-}
-
-// Launch geometry.  The kernel is issue-bound and its warps do identical work, but the SM's warp arbiter is not fair: of the
+// Launch policy.  The kernel is issue-bound and its warps do identical work, but the SM's warp arbiter is not fair: of the
 // warps resident on a scheduler some finish long before others (ncu: 5.4 of 8 warps active on average over a launch whose
-// grid is exactly one resident wave), and what they leave behind is an under-filled tail.  Two ways to launch:
-//   waves   (the round-1 policy) full waves of (resident threads) x CPT chains + one remainder wave of 1..CPT chains per thread;
-//   dynamic ONE launch of small blocks (1 warp), many more blocks than fit: the hardware block scheduler back-fills every slot
-//           a finished warp frees, so all SMs stay full until the population is exhausted and the tail is one short block.
-struct Geom {
-  int cpt, nb, block, pack, dynamic;
-};
-
+// grid is exactly one resident wave), and what they leave behind is an under-filled tail.  So the fp32, r == 2 Philox path,
+// the throughput path, is ONE launch of small blocks, many more blocks than fit: the hardware block scheduler back-fills
+// every slot a finished warp frees, so all SMs stay full until the population is exhausted and the tail is one short block.
+// The other paths (fp64, replay, r != 2: parity paths, not throughput paths) keep the round-1 policy: occupancy-sized waves.
 struct Launch {  // everything a launch needs besides its chain range
   const void* c;
-  const Gmm2dConstsPk* cpk;
   const void* kdev;
   void* x;
   long long n_chains;
@@ -730,106 +580,91 @@ struct Launch {  // everything a launch needs besides its chain range
   cudaStream_t st;
 };
 
-template <typename T, int ALG, bool R2, int CPT, int NB, int BLOCK, bool PACK>
-static int launch_one(const Launch& a, long long lo, long long n_launch, int* blocks_per_sm) {
-  auto kern = gmm2d_kernel<T, ALG, R2, CPT, NB, BLOCK, PACK>;
-  if (blocks_per_sm) {
-    PSGLA_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, kern, BLOCK, 0));
-    return PSGLA_OK;
-  }
+template <typename T, int ALG, bool R2, int CPT, int NB, int BLOCK>
+static void launch_one(const Launch& a, long long lo, long long n_launch) {
   const long long threads = (n_launch + CPT - 1) / CPT;
   const unsigned grid = (unsigned)((threads + BLOCK - 1) / BLOCK);
-  kern<<<grid, BLOCK, 0, a.st>>>(*(const Gmm2dConsts<T>*)a.c, *a.cpk, (const Gmm2dComponents<T>*)a.kdev, (T*)a.x, a.n_chains, lo,
-                                 n_launch, a.chain_id0, a.n_steps, a.step0, a.keys, (const T*)a.noise, (T*)a.traj, a.thin);
+  gmm2d_kernel<T, ALG, R2, CPT, NB, BLOCK><<<grid, BLOCK, 0, a.st>>>(
+      *(const Gmm2dConsts<T>*)a.c, (const Gmm2dComponents<T>*)a.kdev, (T*)a.x, a.n_chains, lo, n_launch, a.chain_id0,
+      a.n_steps, a.step0, a.keys, (const T*)a.noise, (T*)a.traj, a.thin);
+}
+
+// Threads that one wave of the full-wave kernel, gmm2d_kernel<T, ALG, R2, 4, 1, 128>, holds on the device.
+template <typename T, int ALG, bool R2>
+static int resident_threads(long long* threads) {
+  int per_sm = 0;
+  PSGLA_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, gmm2d_kernel<T, ALG, R2, 4, 1, 128>, 128, 0));
+  *threads = (long long)num_sms() * (per_sm > 0 ? per_sm : 8) * 128;
   return PSGLA_OK;
 }
 
-// The instantiated geometries.  fp64 and r != 2 keep the plain 128-thread kernels (parity paths, not throughput paths).
+// Full waves of 4 chains per resident thread, then one remainder wave of as few chains per thread (1..4) as still fit in one
+// wave.
 template <typename T, int ALG, bool R2>
-static int launch_geom(const Geom& g, const Launch& a, long long lo, long long n, int* bps) {
-#define PSGLA_GEOM(C_, N_, B_, P_) \
-  if (g.cpt == C_ && g.nb == N_ && g.block == B_ && g.pack == P_) return launch_one<T, ALG, R2, C_, N_, B_, (P_ != 0)>(a, lo, n, bps);
-  PSGLA_GEOM(1, 1, 128, 0)
-  PSGLA_GEOM(2, 1, 128, 0)
-  PSGLA_GEOM(3, 1, 128, 0)
-  PSGLA_GEOM(4, 1, 128, 0)
-  if constexpr (sizeof(T) == 4 && R2) {
-    PSGLA_GEOM(1, 2, 128, 0)
-    PSGLA_GEOM(1, 4, 128, 0)
-    PSGLA_GEOM(2, 2, 128, 0)
-    PSGLA_GEOM(1, 2, 32, 0)
-    PSGLA_GEOM(1, 4, 32, 0)
-    PSGLA_GEOM(2, 2, 32, 0)
-    PSGLA_GEOM(2, 1, 32, 0)
-    PSGLA_GEOM(4, 1, 32, 0)
-    PSGLA_GEOM(1, 4, 64, 0)
-    PSGLA_GEOM(2, 2, 64, 0)
-    PSGLA_GEOM(2, 1, 128, 1)
-    PSGLA_GEOM(4, 1, 128, 1)
-    PSGLA_GEOM(2, 2, 128, 1)
-    PSGLA_GEOM(2, 1, 32, 1)
-    PSGLA_GEOM(2, 2, 32, 1)
-    PSGLA_GEOM(4, 1, 32, 1)
-    PSGLA_GEOM(2, 2, 64, 1)
-    PSGLA_GEOM(4, 1, 64, 1)
+static int launch_waves(const Launch& a, int* launches) {
+  long long resident = 0;
+  const int rc = resident_threads<T, ALG, R2>(&resident);
+  if (rc) return rc;
+  for (long long lo = 0; lo < a.n_chains; ++*launches) {
+    const long long n = std::min(a.n_chains - lo, 4 * resident);
+    const long long cpt = (n + resident - 1) / resident;
+    if (cpt == 1)
+      launch_one<T, ALG, R2, 1, 1, 128>(a, lo, n);
+    else if (cpt == 2)
+      launch_one<T, ALG, R2, 2, 1, 128>(a, lo, n);
+    else if (cpt == 3)
+      launch_one<T, ALG, R2, 3, 1, 128>(a, lo, n);
+    else
+      launch_one<T, ALG, R2, 4, 1, 128>(a, lo, n);
+    lo += n;
   }
-#undef PSGLA_GEOM
-  return set_error(PSGLA_E_UNSUPPORTED, "gmm2d geometry cpt=%d nb=%d block=%d pack=%d is not instantiated", g.cpt, g.nb, g.block,
-                   g.pack);
+  return PSGLA_OK;
 }
 
-// Lean-kernel geometries: "nb,block,minb,pk" (dynamic == 2 in PSGLA_GMM_GEOM: cpt = nb, nb = block, block = minb, pack = pk).
 template <int ALG, int STRUCT>
-static int launch_lean_s(int nb, int block, int minb, int pk, const Launch& a, long long lo, long long n, long long n_rounds,
-                         long long step_lo) {
-  const Gmm2dConsts<float>& c = *(const Gmm2dConsts<float>*)a.c;
-  float2* x = (float2*)a.x + lo;
-  const unsigned long long sub0 = a.chain_id0 + (unsigned long long)lo, pair0 = (unsigned long long)step_lo >> 1;
-#define PSGLA_LEAN(N_, B_, M_, P_)                                                                                          \
-  if (nb == N_ && block == B_ && minb == M_ && pk == P_) {                                                                  \
-    gmm2d_lean_kernel<ALG, STRUCT, N_, B_, M_, P_><<<(unsigned)((n + B_ - 1) / B_), B_, 0, a.st>>>(                           \
-        c, x, (unsigned)n, sub0, pair0, (int)n_rounds, a.keys);                                                             \
-    return PSGLA_OK;                                                                                                        \
-  }
-  PSGLA_LEAN(4, 64, 16, 1)
-  PSGLA_LEAN(4, 64, 16, 0)
-  PSGLA_LEAN(2, 64, 16, 0)
-  PSGLA_LEAN(4, 64, 20, 1)
-  PSGLA_LEAN(4, 64, 24, 0)
-  PSGLA_LEAN(4, 32, 32, 1)
-  PSGLA_LEAN(8, 32, 32, 0)
-  PSGLA_LEAN(1, 64, 16, 2)
-  PSGLA_LEAN(2, 64, 16, 2)
-  PSGLA_LEAN(2, 64, 16, 3)
-  PSGLA_LEAN(4, 64, 16, 2)
-  PSGLA_LEAN(4, 64, 16, 3)
-  PSGLA_LEAN(1, 64, 24, 2)
-  PSGLA_LEAN(2, 64, 24, 2)
-  PSGLA_LEAN(2, 64, 20, 3)
-  PSGLA_LEAN(4, 64, 12, 3)
-  PSGLA_LEAN(4, 64, 12, 2)
-#undef PSGLA_LEAN
-  return set_error(PSGLA_E_UNSUPPORTED, "lean gmm2d geometry nb=%d block=%d minb=%d pk=%d is not instantiated", nb, block, minb, pk);
+static void launch_lean(const Launch& a, long long lo, long long n, long long n_rounds, long long step_lo) {
+  gmm2d_lean_kernel<ALG, STRUCT><<<(unsigned)((n + LEAN_BLOCK - 1) / LEAN_BLOCK), LEAN_BLOCK, 0, a.st>>>(
+      *(const Gmm2dConsts<float>*)a.c, (float2*)a.x + lo, (unsigned)n, a.chain_id0 + (unsigned long long)lo,
+      (unsigned long long)step_lo >> 1, (int)n_rounds, a.keys);
 }
 
+// fp32, r == 2, in-kernel Philox; returns the number of launches.  With a trajectory: one launch of 1-warp blocks of the
+// general kernel (the lean kernel keeps no trajectory).  Without: the lean kernel on the whole rounds of 2 LEAN_NB steps that
+// start on an even step, in chunks of 2^30 chains; the general kernel takes the lead step of an odd step0 and the steps after
+// the last whole round.
 template <int ALG>
-static int launch_lean(int nb, int block, int minb, int pk, const Launch& a, long long lo, long long n, long long n_rounds,
-                       long long step_lo) {
-  int structure = constants_structure(*(const Gmm2dConsts<float>*)a.c);
-  if (const char* e = std::getenv("PSGLA_GMM_STRUCT")) structure = std::min(structure, std::atoi(e));  // A/B: cap the specialisation
-  if (structure == 2) return launch_lean_s<ALG, 2>(nb, block, minb, pk, a, lo, n, n_rounds, step_lo);
-  if (structure == 1) return launch_lean_s<ALG, 1>(nb, block, minb, pk, a, lo, n, n_rounds, step_lo);
-  return launch_lean_s<ALG, 0>(nb, block, minb, pk, a, lo, n, n_rounds, step_lo);
-}
-
-// PSGLA_GMM_GEOM="cpt,nb,block,pack,dynamic" overrides the default policy (A/B runs, scripts/gmm2d_sweep.py).
-static bool geom_from_env(Geom* g) {
-  const char* e = std::getenv("PSGLA_GMM_GEOM");
-  if (!e || !*e) return false;
-  Geom t{4, 1, 128, 0, 0};
-  if (std::sscanf(e, "%d,%d,%d,%d,%d", &t.cpt, &t.nb, &t.block, &t.pack, &t.dynamic) < 1) return false;
-  *g = t;
-  return true;
+static int launch_philox_r2(const Launch& a) {
+  if (a.traj != nullptr) {
+    launch_one<float, ALG, true, 1, 4, 32>(a, 0, a.n_chains);
+    return 1;
+  }
+  const int structure = constants_structure(*(const Gmm2dConsts<float>*)a.c);
+  const long long lead = std::min(a.step0 & 1, a.n_steps);
+  const long long rounds = (a.n_steps - lead) / (2 * LEAN_NB), body = rounds * 2 * LEAN_NB;
+  int launches = 0;
+  if (lead) {
+    Launch b = a;
+    b.n_steps = lead;
+    launch_one<float, ALG, true, 1, 1, 128>(b, 0, a.n_chains);
+    ++launches;
+  }
+  for (long long lo = 0; lo < a.n_chains && rounds > 0; lo += (1ll << 30), ++launches) {
+    const long long n = std::min(a.n_chains - lo, 1ll << 30);
+    if (structure == 2)
+      launch_lean<ALG, 2>(a, lo, n, rounds, a.step0 + lead);
+    else if (structure == 1)
+      launch_lean<ALG, 1>(a, lo, n, rounds, a.step0 + lead);
+    else
+      launch_lean<ALG, 0>(a, lo, n, rounds, a.step0 + lead);
+  }
+  if (lead + body < a.n_steps) {
+    Launch b = a;
+    b.step0 = a.step0 + lead + body;
+    b.n_steps = a.n_steps - lead - body;
+    launch_one<float, ALG, true, 1, 1, 128>(b, 0, a.n_chains);
+    ++launches;
+  }
+  return launches;
 }
 
 static thread_local int g_last_launches = 0;  // launches of this thread's most recent psgla_gmm2d_run (bench bookkeeping)
@@ -841,76 +676,17 @@ static int launch_run(const Folded& f, T* x, long long n_chains, unsigned long l
   Gmm2dConsts<T> c;
   static thread_local Gmm2dComponents<T> k;  // pageable source of the async copy must outlive the call: keep it TLS
   narrow<T>(f, &c, &k);
-  Gmm2dConstsPk cpk;
-  std::memset(&cpk, 0, sizeof(cpk));
-  if constexpr (sizeof(T) == 4) cpk = pack_consts(c);
   Gmm2dComponents<T>* kdev = nullptr;
   if (!R2) {
     int rc = upload_components<T>(k, st, &kdev);
     if (rc) return rc;
   }
-  const Launch a{&c, &cpk, kdev, x, n_chains, chain_id0, n_steps, step0, philox_round_keys(seed), noise, traj, thin, st};
-  constexpr bool fast = sizeof(T) == 4 && R2;
-  Geom g{4, 1, 128, 0, 0};
-  if (fast && noise == nullptr) {
-    g = Geom{PSGLA_GMM_DEFAULT_GEOM};
-    geom_from_env(&g);
-    if (g.dynamic == 2 && traj != nullptr) g = Geom{1, 4, 32, 0, 1};  // the lean kernel keeps no trajectory
-  }
+  const Launch a{&c, kdev, x, n_chains, chain_id0, n_steps, step0, philox_round_keys(seed), noise, traj, thin, st};
   int launches = 0, rc = PSGLA_OK;
-  if (g.dynamic == 2) {
-    if constexpr (fast) {
-      // lean kernel on the whole rounds of 2 nb steps that start on an even step; the general kernel finishes the rest
-      const int nb = g.cpt;
-      long long lead = (step0 & 1) ? 1 : 0;
-      if (lead > n_steps) lead = n_steps;
-      const long long rounds = (n_steps - lead) / (2 * nb), body = rounds * 2 * nb;
-      const Geom rest{1, 1, 128, 0, 1};
-      if (lead) {
-        Launch b = a;
-        b.n_steps = lead;
-        rc = launch_geom<T, ALG, R2>(rest, b, 0, n_chains, nullptr);
-        ++launches;
-      }
-      for (long long lo = 0; lo < n_chains && rc == PSGLA_OK && rounds > 0; lo += (1ll << 30)) {
-        const long long n = n_chains - lo < (1ll << 30) ? n_chains - lo : (1ll << 30);
-        rc = launch_lean<ALG>(nb, g.nb, g.block, g.pack, a, lo, n, rounds, step0 + lead);
-        ++launches;
-      }
-      if (rc == PSGLA_OK && lead + body < n_steps) {
-        Launch b = a;
-        b.step0 = step0 + lead + body;
-        b.n_steps = n_steps - lead - body;
-        rc = launch_geom<T, ALG, R2>(rest, b, 0, n_chains, nullptr);
-        ++launches;
-      }
-    }
-  } else if (g.dynamic) {
-    rc = launch_geom<T, ALG, R2>(g, a, 0, n_chains, nullptr);
-    launches = 1;
-  } else {
-    int per_sm = 0;
-    rc = launch_geom<T, ALG, R2>(g, a, 0, 0, &per_sm);
-    if (rc) return rc;
-    const long long resident = (long long)num_sms() * (per_sm > 0 ? per_sm : 8) * g.block;  // threads one wave holds
-    long long lo = 0;
-    while (lo < n_chains && rc == PSGLA_OK) {
-      const long long left = n_chains - lo;
-      Geom w = g;
-      long long n = (long long)g.cpt * resident;
-      if (left < n) {  // remainder wave: as few chains per thread as still fit in one wave (pairs stay pairs)
-        const int step = g.pack ? 2 : 1;
-        w.cpt = (int)((left + resident - 1) / resident);
-        w.cpt = (w.cpt + step - 1) / step * step;
-        if (w.cpt < g.cpt && w.nb * w.cpt < g.nb * g.cpt && !g.pack) w.nb = 1;
-        n = left;
-        if (launch_geom<T, ALG, R2>(w, a, 0, 0, &per_sm) != PSGLA_OK) w = g;  // not instantiated: the full geometry, partly idle
-      }
-      rc = launch_geom<T, ALG, R2>(w, a, lo, n, nullptr);
-      lo += n;
-      ++launches;
-    }
-  }
+  if (sizeof(T) == 4 && R2 && noise == nullptr)
+    launches = launch_philox_r2<ALG>(a);
+  else
+    rc = launch_waves<T, ALG, R2>(a, &launches);
   if (rc) return rc;
   g_last_launches = launches;
   PSGLA_CUDA_TRY(cudaGetLastError());

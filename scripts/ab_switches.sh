@@ -9,6 +9,3 @@ run() {  # run VAR=value "k expression" files...
 run PSGLA_CONV_FUSE2=0 "dncnn_forward or psgla_replay or reference_fixture or fused_layer" tests/test_image_gpu.py
 run PSGLA_FUSE_PRE=0 "psgla_replay or batched or statistics_only or image_set" tests/test_image_gpu.py
 run PSGLA_BLUR_4PASS=1 "deblur or pnpula" tests/test_image_gpu.py tests/test_torch_stream_gpu.py
-run PSGLA_GMM_GEOM=4,1,128,0,0 "" tests/test_gmm2d_gpu.py tests/test_gmm2d_metric_gpu.py
-run PSGLA_GMM_GEOM=1,4,32,0,1 "" tests/test_gmm2d_gpu.py
-run PSGLA_GMM_STRUCT=0 "" tests/test_gmm2d_gpu.py

@@ -140,30 +140,32 @@ def test_philox_noise_is_standard_normal_and_replayable():
 @pytest.mark.parametrize("alg", ["psgla", "pnp_ula"])
 @pytest.mark.parametrize("name,A", [("symetric_gaussians", np.eye(2)), ("disymmetric_gaussians", np.eye(2)), ("cross", np.eye(2)),
                                     ("symetric_gaussians", np.array([[1.0, 0.3], [-0.2, 0.8]]))])
-def test_lean_kernel_and_every_launch_geometry_equal_the_replayed_stream(name, A, alg, monkeypatch):
-    """The throughput path (csrc/gmm2d.cu: the register-lean one-chain-per-thread kernel with 4 Philox blocks per round, its
-    constants-structure specialisations STRUCT 0 / 1 / 2, the packed FFMA2 variants, the dynamically scheduled and the
-    wave-split launches) must consume exactly the library's Philox stream and do the general kernel's arithmetic: 45 steps
-    from an odd global step (1 lead step + 5 lean rounds of 8 + 4 tail steps) == the replay of the dumped draws, bit for bit."""
+def test_lean_kernel_and_every_launch_geometry_equal_the_replayed_stream(name, A, alg):
+    """Each launch path of csrc/gmm2d.cu must consume exactly the library's Philox stream and do the general kernel's
+    arithmetic: a Philox run == the replay of the dumped draws, bit for bit, in the number of launches its policy makes.
+      fp32, no trajectory: the register-lean one-chain-per-thread kernel with 4 Philox blocks per round and its
+        constants-structure specialisation (STRUCT 2 on the diagonal priors, 1 on `cross`, 0 with a non-diagonal A); 45 steps
+        from the odd global step 3 = 1 lead step + 5 lean rounds of 8 + 4 tail steps, 3 launches;
+      fp32 with a trajectory: one launch of the general kernel in 1-warp blocks (final state and trajectory rows);
+      fp64: occupancy-sized waves of the general kernel.  2 * 10^6 chains are more than 4 per resident thread at any
+        occupancy of its 128-thread blocks (at most 16 per SM), so full waves of 4 chains per thread and a remainder wave run."""
     lib = P._lib.lib()
-    C, n, off = 3000, 45, 3
+    C, n, off, thin = 2_000_003, 45, 3, 16
     z = torch.empty(n, C, 2, device="cuda")
     P._lib.check(lib.psgla_gmm2d_noise(z.data_ptr(), C, 5, n, off, 77, None), "noise")
     D = P.Theorical_MMSE(*P.gaussian_mixt_example(name))
     y = np.array([0.0, -2.0])
     prm = dict(delta=0.3, alpha=2 / 3, epsilon=1.0) if alg == "psgla" else dict(delta=0.1, alpha=1.5, epsilon=0.5)
     kw = dict(y=y, A=A, sigma=1, denoiser=D, n_chains=C, **prm)
-    want, _ = P.run_chains(alg, n, noise=z, **kw)
-    for geom in ("", "4,1,128,0,0", "1,4,32,0,1", "2,2,128,1,1", "4,1,128,1,0", "4,64,16,0,2", "2,64,16,0,2", "8,32,32,0,2",
-                 "4,32,32,1,2"):
-        monkeypatch.setenv("PSGLA_GMM_GEOM", geom)
-        got, _ = P.run_chains(alg, n, seed=77, chain_id0=5, philox_offset=off, **kw)
-        assert torch.equal(got, want), geom
-    monkeypatch.setenv("PSGLA_GMM_GEOM", "")
-    for cap in ("0", "1"):  # the structure specialisation switched off / capped: same bits
-        monkeypatch.setenv("PSGLA_GMM_STRUCT", cap)
-        got, _ = P.run_chains(alg, n, seed=77, chain_id0=5, philox_offset=off, **kw)
-        assert torch.equal(got, want), cap
+    philox = dict(seed=77, chain_id0=5, philox_offset=off)
+    want, want_traj = P.run_chains(alg, n, noise=z, thin=thin, **kw)
+    got, _ = P.run_chains(alg, n, **philox, **kw)
+    assert torch.equal(got, want) and lib.psgla_gmm2d_last_launches() == 3
+    got, traj = P.run_chains(alg, n, thin=thin, **philox, **kw)
+    assert torch.equal(got, want) and torch.equal(traj, want_traj) and lib.psgla_gmm2d_last_launches() == 1
+    want, _ = P.run_chains(alg, n, noise=z, dtype="float64", **kw)
+    got, _ = P.run_chains(alg, n, dtype="float64", **philox, **kw)
+    assert torch.equal(got, want) and lib.psgla_gmm2d_last_launches() >= 2  # every launch but the last is a full wave
 
 
 def test_sharding_and_segmentation_invariance():
