@@ -302,7 +302,7 @@ int psgla_tv_prox_post(const psgla_tv_params* tv, psgla_img_shape shape, const f
 
 /* tcgen05 descriptor self-test (development aid): runs a 128 x 64 x 64 GEMM tile whose A operand starts `row_shift`
  * rows into a 128B-swizzled shared-memory buffer.  mode 0: A from shared memory, shift = descriptor start address;
- * mode 1: same with a base-offset field (kept for reference, wrong on sm_100a); mode 2: A copied to tensor memory.
+ * mode 2: A copied to tensor memory.
  * a_dev: bf16 [136][64], b_dev: bf16 [64][64] (N x K), d_dev: fp32 [128][64]. */
 int psgla_selftest_umma(const void* a_dev, const void* b_dev, float* d_dev, int row_shift, int mode, void* stream);
 /* CTA-pair (cta_group::2) self-test: D[256][64] = A[256][64] B[64][64]^T by one pair of CTAs, A rows split 128 / 128 over

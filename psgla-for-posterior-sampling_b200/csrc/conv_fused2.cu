@@ -16,12 +16,12 @@
 // The intermediate activations are rounded to bf16 exactly as when they travel through global memory, so the result is
 // bit-identical to two conv3x3_ts2_kernel launches (tests/test_image_gpu.py::test_fused_layer_pairs_equal_single_layers).
 // Limits: W <= 256 (the pair holds whole rows, so every halo pixel is on chip) and a single wave of pairs; everything else
-// keeps the per-layer kernels.  PSGLA_CONV_FUSE2=0 disables the path (A/B runs).
+// keeps the per-layer kernels.  PSGLA_CONV_FUSE2=0 disables the path: bench.py times the single-chain iteration with one
+// hidden layer per launch beside the fused one, and tests compare the two bit for bit.
 #include <cuda_bf16.h>
 
 #include <algorithm>
 #include <atomic>
-#include <mutex>
 #include <utility>
 #include <vector>
 
@@ -58,21 +58,7 @@ struct F2Params {
   const uint8_t* weights2;  // second layer: 9 taps, swizzled, all 64 output channels (as ConvParams::weights)
   const float* bias2;
   __nv_bfloat16* out;  // bf16 NHWC [B][H][W][64]
-  long long* trace;  // PSGLA_F2_TRACE=1 (development): 64 clock64 stamps per CTA, see fused2_print_trace
 };
-#define F2_STAMP(k)                                                          \
-  do {                                                                       \
-    if (f.trace) f.trace[(size_t)blockIdx.x * 96 + (k)] = clock64();         \
-  } while (0)
-// wall-clock (ns) stamps in slots 90..: the pipelined timeline across launches (PSGLA_F2_TRACE=2, no synchronisation)
-#define F2_GSTAMP(k)                                                         \
-  do {                                                                       \
-    if (f.trace) {                                                           \
-      unsigned long long g_;                                                 \
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(g_));                 \
-      f.trace[(size_t)blockIdx.x * 96 + (k)] = (long long)g_;                \
-    }                                                                        \
-  } while (0)
 
 // 16 bytes into the shared memory of another CTA of the cluster; the bytes count as a transaction on that CTA's mbarrier
 __device__ __forceinline__ void st_async_v4(uint32_t cluster_addr, const uint4& v, uint32_t mbar_cluster_addr) {
@@ -110,10 +96,6 @@ conv3x3_fused2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_con
   const int lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();
   griddep_launch_dependents();
-  if (threadIdx.x == 0) {
-    F2_STAMP(0);
-    F2_GSTAMP(90);
-  }
 
   // the pair's work item: output rows [y0, y0 + rcur), intermediate rows [m_lo, m_hi], input rows [i_lo, i_hi]
   const ItemCoord c = decode_item(p, blockIdx.x);
@@ -139,8 +121,6 @@ conv3x3_fused2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_con
       mbar_expect_tx(wbar, Cfg::W_BYTES);
       tma_load_3d(smem_w, &tmap_w1, wbar, 0, (int)rank * 32, 0);  // one box: 9 taps x this CTA's 32 rows x 128 B, as they lie
       griddep_wait();
-      F2_STAMP(2);
-      F2_GSTAMP(91);
       for (int q = 0; q < min(n_in, F2_NSTAGE); ++q) {
         mbar_expect_tx(&full[q], Cfg::BOX_BYTES);
         tma_load_4d(ring + q * Cfg::SLOT_BYTES, &tmap, &full[q], 0, c.x0 - 1, i_lo + q, c.b);
@@ -177,7 +157,6 @@ conv3x3_fused2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_con
   __syncthreads();        // this CTA: barriers, the TMEM base address
   cluster_sync_relaxed();  // the pair: both CTAs' barriers exist before any remote arrive / store / multicast commit
   tc_fence_after();
-  if (threadIdx.x == 0) F2_STAMP(1);
   const uint32_t tmem_base = *tmem_ptr_s;
   const uint32_t afull_c = mapa_shared(smem_u32(afull), 0);
   const uint32_t tempty_c = mapa_shared(smem_u32(tempty), 0);
@@ -187,7 +166,7 @@ conv3x3_fused2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_con
   // shared-memory reads and TMEM stores plus four mbarrier operations of ~90 cycles, and passes of one warp set are serial; so
   // where rows wait in line on the critical path -- the first three rows of the launch, the rows the second layer starts
   // with -- the epilogue groups, idle at those moments, each take one (helper_row) and the passes run side by side.
-  auto loader_pass = [&](int q, int q4, int lane_, bool stamp) {
+  auto loader_pass = [&](int q, int q4, int lane_) {
     const int m = q4 * 32 + lane_;
     const uint32_t lane_taddr = tmem_base + ((uint32_t)(q4 * 32) << 16) + TS_A_COL0;
     const uint32_t as = (uint32_t)q % TS_NA;
@@ -196,7 +175,6 @@ conv3x3_fused2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_con
     if (q < n_in) {
       slot = (uint32_t)q % F2_NSTAGE;
       mbar_wait(&full[slot], ((uint32_t)q / F2_NSTAGE) & 1);
-      if (q == 0 && stamp) F2_STAMP(4);
       tile = smem_u32(ring) + slot * Cfg::SLOT_BYTES;
     } else {
       mbar_wait(&mfull[q - n_in], 0);
@@ -204,7 +182,6 @@ conv3x3_fused2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_con
     }
     mbar_wait(&aempty[as], (((uint32_t)q / TS_NA) & 1) ^ 1);
     tc_fence_after();
-    if (stamp) F2_STAMP(32 + q);
 #pragma unroll
     for (int dx = 0; dx < 3; ++dx) {
       uint32_t v[32];
@@ -217,7 +194,6 @@ conv3x3_fused2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_con
     if (lane_ == 0) {
       if (q < n_in) mbar_arrive(&empty[slot]);
       mbar_arrive_remote(afull_c + as * 8u);
-      if (stamp) F2_STAMP(16 + q);
     }
   };
   // rows taken by an epilogue group: input rows 1 and 2 (groups 0 and 1, before their first accumulator), and the third
@@ -228,11 +204,6 @@ conv3x3_fused2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_con
   if (warp == 0) {
     if (lane == 0) {
       // ---------------------------------------------------------------- TMA producer: the rows beyond the first three
-      if (f.trace)  // development: when the first rows land
-        for (int k = 0; k < min(n_in, F2_NSTAGE); ++k) {
-          mbar_wait(&full[k], 0);
-          F2_STAMP(58 + k);
-        }
       for (int q = F2_NSTAGE; q < n_in; ++q) {
         const uint32_t slot = (uint32_t)q % F2_NSTAGE;
         mbar_wait(&empty[slot], (((uint32_t)q / F2_NSTAGE) & 1) ^ 1);
@@ -261,11 +232,10 @@ conv3x3_fused2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_con
       mbar_wait(wbar, 0);
       mbar_wait_cluster(wready, 0);
       tc_fence_after();
-      if (lane == 0) F2_STAMP(3);
       // ONE thread runs the whole issue loop, barrier waits included.  The tensor pipe's queue is shallow: whatever the issuing
-      // thread executes between two MMAs beyond a few dozen cycles is a bubble in the pipe (measured with the stamps below: one
-      // warp-uniform wait / elect / syncwarp boundary per dy group cost 180 cycles per 384 cycles of MMAs), so the loop carries
-      // nothing but try_waits that pass at once in steady state, address adds and the MMAs.
+      // thread executes between two MMAs beyond a few dozen cycles is a bubble in the pipe (measured with clock64 stamps, commit
+      // e803185: one warp-uniform wait / elect / syncwarp boundary per dy group cost 180 cycles per 384 cycles of MMAs), so the
+      // loop carries nothing but try_waits that pass at once in steady state, address adds and the MMAs.
       if (elect_one()) {
         uint32_t T = 0;
         int waited = 0;
@@ -310,10 +280,8 @@ conv3x3_fused2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_con
               accumulate = 1;
               // source row y - 1 is dead once these 12 MMAs retire; after the phase's last output row so are the others
               if ((dy == 0 && y - 1 >= s_lo) || y == o_hi) umma_commit2(&aempty[(uint32_t)q % TS_NA], 3);
-              if (y == o_lo && dy == 2) F2_STAMP(ph ? 8 : 5);
             }
             umma_commit2(&tfull[acc], 3);
-            F2_STAMP(48 + T);
           }
         }
         umma_commit2(done, 3);
@@ -321,13 +289,12 @@ conv3x3_fused2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_con
       __syncwarp();
     }
     mbar_wait(done, 0);
-    if (lane == 0) F2_STAMP(9);
     // both CTAs: no MMA still reads this CTA's shared / tensor memory, no commit is still in flight
   } else if (warp < 6) {
     // ---------------------------------------------------------------- loaders: TMA ring / mid ring -> registers -> TMEM
     const int n_rows = n_in + n_mid;
     for (int q = 0; q < n_rows; ++q)
-      if (!helper_row(q)) loader_pass(q, warp & 3, lane, warp == 2 && lane == 0);
+      if (!helper_row(q)) loader_pass(q, warp & 3, lane);
   } else {
     // ---------------------------------------------------------------- epilogue: 2 groups x 4 warps
     const int ew = warp - 6;
@@ -337,7 +304,7 @@ conv3x3_fused2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_con
       if (i < 2 * NOUT) bias_s[i] = i < NOUT ? p.bias[i] : f.bias2[i - NOUT];
       asm volatile("bar.sync 1, %0;" ::"n"(32 * EPI_WARPS) : "memory");  // the eight epilogue warps only
     }
-    if (1 + grp < n_in) loader_pass(1 + grp, q4, lane, q4 == 0 && lane == 0);
+    if (1 + grp < n_in) loader_pass(1 + grp, q4, lane);
     // phase 1: layer l -> the mid ring (this CTA's 128 pixels, plus its edge pixel into the peer's ring)
     {
       const int mpx = q4 * 32 + lane;       // pixel of the strip
@@ -360,7 +327,6 @@ conv3x3_fused2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_con
         const uint32_t acc = (uint32_t)t % TS_NACC;
         mbar_wait(&tfull[acc], ((uint32_t)t / TS_NACC) & 1);
         tc_fence_after();
-        if (q4 == 0 && lane == 0 && (t == 0 || t == n_mid - 1)) F2_STAMP(t == 0 ? 6 : 7);
         const uint32_t taddr = tmem_base + ((uint32_t)(q4 * 32) << 16) + acc * NOUT;
         uint32_t v[NOUT];
 #pragma unroll
@@ -392,7 +358,7 @@ conv3x3_fused2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_con
         }
       }
     }
-    if (n_mid > 2 && grp == (n_mid & 1)) loader_pass(n_in + 2, q4, lane, q4 == 0 && lane == 0);
+    if (n_mid > 2 && grp == (n_mid & 1)) loader_pass(n_in + 2, q4, lane);
     // phase 2: layer l + 1 -> registers -> global memory, one pixel (128 contiguous bytes) per lane.  No staging box and no TMA
     // store here: with one item per CTA nothing overlaps the store's shared-memory round trip, and plain stores let the CTA
     // retire as soon as they are issued (they are complete when the grid is, which is what the next launch waits for).
@@ -430,14 +396,9 @@ conv3x3_fused2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_con
         }
       }
     }
-    if (q4 == 0 && lane == 0) F2_STAMP(10 + grp);
   }
   tc_fence_before();
   cluster_sync_relaxed();
-  if (threadIdx.x == 0) {
-    F2_STAMP(12);
-    F2_GSTAMP(92);
-  }
   // neither CTA may exit (or free tensor memory) while its partner can still signal, read or write it
   if (warp == 1) {
     tc_fence_after();
@@ -504,7 +465,7 @@ static int fused2_clusters(int* out) {
   return PSGLA_OK;
 }
 
-// PSGLA_CONV_FUSE2=0: per-layer launches everywhere (read per call: tests and A/B scripts switch it inside one process)
+// PSGLA_CONV_FUSE2=0: per-layer launches everywhere (read per call: bench.py and tests switch it inside one process)
 static bool fused2_enabled() {
   const char* e = getenv("PSGLA_CONV_FUSE2");
   return !(e && e[0] == '0');
@@ -530,33 +491,7 @@ int conv64_hidden_fused2(const void* in, void* out, const uint8_t* w1, const flo
   p.strips = 2;
   p.row_blocks = (H + R - 1) / R;
   p.n_items = B * 2 * p.row_blocks;
-  F2Params f{w2, b2, (__nv_bfloat16*)out, nullptr};
-  // Development traces (PSGLA_F2_TRACE): their buffers are process-wide, so a traced launch holds this lock from here to its
-  // return; untraced launches (the product's) never take it.
-  static std::mutex trace_mutex;
-  static long long* trace_dev = nullptr;
-  const char* trace_env = getenv("PSGLA_F2_TRACE");
-  std::unique_lock<std::mutex> trace_lock;
-  if (trace_env != nullptr) trace_lock = std::unique_lock<std::mutex>(trace_mutex);
-  const bool trace = trace_env != nullptr && trace_env[0] == '1';
-  if (trace) {
-    if (!trace_dev) PSGLA_CUDA_TRY(cudaMalloc(&trace_dev, 512 * 96 * sizeof(long long)));
-    PSGLA_CUDA_TRY(cudaMemsetAsync(trace_dev, 0, 512 * 96 * sizeof(long long), st));
-    if (p.n_items <= 512) f.trace = trace_dev;
-  }
-  // PSGLA_F2_TRACE=2: the next 36 launches write their stamps side by side, nothing synchronises in between; after the last
-  // one the wall-clock timeline (entry / previous grid complete / exit of the earliest and latest CTA of each launch) is printed
-  constexpr int kPipeLaunches = 36;
-  static long long* pipe_dev = nullptr;
-  static int pipe_n = 0;
-  const bool pipe = trace_env != nullptr && trace_env[0] == '2' && p.n_items <= 160 && pipe_n < kPipeLaunches;
-  if (pipe) {
-    if (!pipe_dev) {
-      PSGLA_CUDA_TRY(cudaMalloc(&pipe_dev, (size_t)kPipeLaunches * 160 * 96 * sizeof(long long)));
-      PSGLA_CUDA_TRY(cudaMemset(pipe_dev, 0, (size_t)kPipeLaunches * 160 * 96 * sizeof(long long)));
-    }
-    f.trace = pipe_dev + (size_t)pipe_n * 160 * 96;
-  }
+  const F2Params f{w2, b2, (__nv_bfloat16*)out};
   CUtensorMap map, map_w1, map_w2;
   rc = get_act_tensor_map(&map, in, B, H, W, 64, BOX_W);
   if (rc) return rc;
@@ -580,59 +515,6 @@ int conv64_hidden_fused2(const void* in, void* out, const uint8_t* w1, const flo
   cfg.numAttrs = 2;
   PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv3x3_fused2_kernel, map, map_w1, map_w2, p, f));
   *applicable = 1;
-  if (pipe && ++pipe_n == kPipeLaunches) {
-    std::vector<long long> host((size_t)kPipeLaunches * 160 * 96);
-    PSGLA_CUDA_TRY(cudaStreamSynchronize(st));
-    PSGLA_CUDA_TRY(cudaMemcpy(host.data(), pipe_dev, host.size() * sizeof(long long), cudaMemcpyDeviceToHost));
-    long long prev_exit = 0;
-    for (int l = 0; l < kPipeLaunches; ++l) {
-      const long long* h = host.data() + (size_t)l * 160 * 96;
-      long long e_min = 0, e_max = 0, w_min = 0, w_max = 0, x_min = 0, x_max = 0, cyc_max = 0;
-      int slow = 0;
-      for (int cta = 0; cta < p.n_items; ++cta) {
-        const long long e = h[cta * 96 + 90], w = h[cta * 96 + 91], x = h[cta * 96 + 92];
-        if (!e) continue;
-        if (!e_min || e < e_min) e_min = e;
-        if (e > e_max) e_max = e;
-        if (!w_min || w < w_min) w_min = w;
-        if (w > w_max) w_max = w;
-        if (!x_min || x < x_min) x_min = x;
-        if (x > x_max) x_max = x, slow = cta;
-        cyc_max = std::max(cyc_max, h[cta * 96 + 12] - h[cta * 96]);
-      }
-      const long long* hs = h + slow * 96;
-      fprintf(stderr,
-              "f2 pipe launch %2d: period %6lld ns | after the previous launch's last exit: first entry %6lld last entry %6lld, "
-              "grid wait done %6lld .. %6lld, first exit %6lld, last exit (cta %3d) %6lld | that CTA: entry %6lld wait %6lld, cycles "
-              "entry->wait %lld ->rows %lld ->exit %lld\n",
-              l, prev_exit ? x_max - prev_exit : 0, e_min - prev_exit, e_max - prev_exit, w_min - prev_exit, w_max - prev_exit,
-              x_min - prev_exit, slow, x_max - prev_exit, hs[90] - prev_exit, hs[91] - prev_exit, hs[2] - hs[0], hs[4] - hs[0],
-              hs[12] - hs[0]);
-      prev_exit = x_max;
-    }
-  }
-  if (trace && f.trace) {
-    // clock64 stamps (cycles after the CTA's entry): 1 prologue + cluster sync done, 2 previous grid complete, 3 weights of both
-    // CTAs landed, 4 first input row landed, 5 / 8 first MMA of phase 1 / 2 may issue, 6 / 7 first / last intermediate row's
-    // accumulator complete, 9 all MMAs complete, 10 / 11 epilogue groups done (stores complete), 12 final cluster sync
-    std::vector<long long> host(512 * 96);
-    PSGLA_CUDA_TRY(cudaStreamSynchronize(st));
-    PSGLA_CUDA_TRY(cudaMemcpy(host.data(), trace_dev, host.size() * sizeof(long long), cudaMemcpyDeviceToHost));
-    const int ctas[] = {0, 1, p.n_items / 2, p.n_items - 2};
-    for (int cta : ctas) {
-      fprintf(stderr, "f2 trace cta %3d:", cta);
-      for (int k = 1; k <= 12; ++k) fprintf(stderr, " %d:%lld", k, host[cta * 96 + k] ? host[cta * 96 + k] - host[cta * 96] : -1);
-      fprintf(stderr, "\n   loader pass start/end per row:");
-      for (int k = 0; k < 14; ++k)
-        if (host[cta * 96 + 16 + k]) fprintf(stderr, " %lld-%lld", host[cta * 96 + 32 + k] - host[cta * 96], host[cta * 96 + 16 + k] - host[cta * 96]);
-      fprintf(stderr, "\n   first rows landed: %lld %lld %lld", host[cta * 96 + 58] - host[cta * 96], host[cta * 96 + 59] - host[cta * 96],
-              host[cta * 96 + 60] - host[cta * 96]);
-      fprintf(stderr, "\n   issuer, output row issued:");
-      for (int k = 0; k < 10; ++k)
-        if (host[cta * 96 + 48 + k]) fprintf(stderr, " %lld", host[cta * 96 + 48 + k] - host[cta * 96]);
-      fprintf(stderr, "\n");
-    }
-  }
   return PSGLA_OK;
 }
 

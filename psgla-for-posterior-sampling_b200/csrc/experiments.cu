@@ -59,27 +59,13 @@ selftest_umma_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_con
         umma_bf16_ts(tbase, tbase + 64 + k * 8, make_smem_desc(smem_u32(sb) + k * 32, 1024, LAYOUT_SW128, 0), idesc, k > 0);
       umma_commit(&bar[1]);
     }
-  } else if (mode == 3) {
-    // A through tensor memory, copied there by tcgen05.cp (smem -> TMEM, no registers): one 128 x 256 bit copy per K-step from
-    // the row-shifted start address, then the TS MMAs from the same thread (tcgen05.cp and tcgen05.mma execute in issue order)
-    if (threadIdx.x == 0) {
-      mbar_wait(&bar[0], 0);
-      tc_fence_after();
-      const uint32_t a0 = smem_u32(sa) + row_shift * 128;
-      constexpr uint32_t idesc = make_idesc_bf16(128, 64);
-      for (int k = 0; k < 4; ++k) tmem_cp_128x256b(tbase + 64 + k * 8, make_smem_desc(a0 + k * 32, 1024, LAYOUT_SW128, 0));
-      for (int k = 0; k < 4; ++k)
-        umma_bf16_ts(tbase, tbase + 64 + k * 8, make_smem_desc(smem_u32(sb) + k * 32, 1024, LAYOUT_SW128, 0), idesc, k > 0);
-      umma_commit(&bar[1]);
-    }
   } else if (threadIdx.x == 0) {
     mbar_wait(&bar[0], 0);
     tc_fence_after();
     const uint32_t a0 = smem_u32(sa) + row_shift * 128, b0 = smem_u32(sb);
-    const uint32_t boff = mode == 1 ? ((a0 >> 7) & 7) : 0;
     constexpr uint32_t idesc = make_idesc_bf16(128, 64);
     for (int k = 0; k < 4; ++k)
-      umma_bf16(tbase, make_smem_desc(a0 + k * 32, 1024, LAYOUT_SW128, boff),
+      umma_bf16(tbase, make_smem_desc(a0 + k * 32, 1024, LAYOUT_SW128, 0),
                 make_smem_desc(b0 + k * 32, 1024, LAYOUT_SW128, 0), idesc, k > 0);
     umma_commit(&bar[1]);
   }
@@ -102,7 +88,8 @@ selftest_umma_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_con
 
 extern "C" int psgla_selftest_umma(const void* a_dev, const void* b_dev, float* d_dev, int row_shift, int mode,
                                    void* stream) {
-  PSGLA_REQUIRE(a_dev && b_dev && d_dev && row_shift >= 0 && row_shift <= 8, "psgla_selftest_umma: bad argument");
+  PSGLA_REQUIRE(a_dev && b_dev && d_dev && row_shift >= 0 && row_shift <= 8 && (mode == 0 || mode == 2),
+                "psgla_selftest_umma: bad argument");
   PFN_tensorMapEncodeTiled enc = get_tensor_map_encoder();
   if (!enc) return set_error(PSGLA_E_NODEVICE, "cuTensorMapEncodeTiled driver entry point not available");
   CUtensorMap ma, mb;
@@ -188,11 +175,9 @@ selftest_umma2_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_co
     tc_fence_after();
     if (elect_one()) {
       constexpr uint32_t idesc = make_idesc_bf16(256, 64);
-      if (mode == 2)  // one cta_group::2 copy moves each CTA's own 128 rows from its shared memory into its tensor memory
-        for (int k = 0; k < 4; ++k) tmem_cp2_128x256b(tbase + 64 + k * 8, make_smem_desc(smem_u32(sa) + k * 32, 1024, LAYOUT_SW128, 0));
       for (int k = 0; k < 4; ++k) {
         const uint64_t bd = make_smem_desc(smem_u32(sb) + k * 32, 1024, LAYOUT_SW128, 0);
-        if (mode == 0 || mode == 2)
+        if (mode == 0)
           umma_bf16_ts2(tbase, tbase + 64 + k * 8, bd, idesc, k > 0);
         else
           umma_bf16_ss2(tbase, make_smem_desc(smem_u32(sa) + k * 32, 1024, LAYOUT_SW128, 0), bd, idesc, k > 0);
@@ -220,7 +205,7 @@ selftest_umma2_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_co
 }  // namespace psgla
 
 extern "C" int psgla_selftest_umma2(const void* a_dev, const void* b_dev, float* d_dev, int mode, void* stream) {
-  PSGLA_REQUIRE(a_dev && b_dev && d_dev && mode >= 0 && mode <= 2, "psgla_selftest_umma2: bad argument");
+  PSGLA_REQUIRE(a_dev && b_dev && d_dev && mode >= 0 && mode <= 1, "psgla_selftest_umma2: bad argument");
   PFN_tensorMapEncodeTiled enc = get_tensor_map_encoder();
   if (!enc) return set_error(PSGLA_E_NODEVICE, "cuTensorMapEncodeTiled driver entry point not available");
   CUtensorMap ma, mb;
@@ -386,37 +371,7 @@ __global__ void __launch_bounds__(128, 1) mma_rate2_kernel(int n, int iters, lon
       const uint32_t a_lo = (smem_u32(sa) >> 4) | 0x10000u;
       const uint32_t b_lo = (smem_u32(sb) >> 4) | 0x10000u;
       t0 = clock64();
-      if (mode >= 2) {
-        // mode 2: tcgen05.cp only (4 copies of 128 x 256 bit per iteration and CTA); modes 3 / 4: the conv kernel's row -- 12
-        // copies (one input row, three pixel shifts, four K-steps) into an A ring slot and 36 TS MMAs over three slots -- with
-        // the copy feeding this row's last 12 MMAs (3) or a slot no MMA of this row reads (4); mode 5: the 36 MMAs alone
-        for (int it = 0; it < iters; ++it) {
-          if (mode != 5) {
-            const uint32_t slot = (uint32_t)((it + (mode == 4 ? 3 : 2)) & 3) * 96u;
-#pragma unroll
-            for (int dx = 0; dx < (mode == 2 ? 1 : 3); ++dx)
-#pragma unroll
-              for (int k = 0; k < 4; ++k)
-                tmem_cp2_128x256b(tbase + 128 + slot + dx * 32 + k * 8, ((uint64_t)DESC_HI << 32) | (a_lo + (uint32_t)(dx * 8 + k * 2)));
-          }
-          if (mode == 2) continue;
-          const uint32_t d = tbase + (it & 1) * 64;
-          uint32_t accumulate = 0;
-#pragma unroll
-          for (int dy = 0; dy < 3; ++dy) {
-            const uint32_t a_t = tbase + 128 + (uint32_t)((it + dy) & 3) * 96u;
-#pragma unroll
-            for (int dx = 0; dx < 3; ++dx)
-#pragma unroll
-              for (int k = 0; k < 4; ++k) {
-                const uint32_t bl = b_lo + (uint32_t)((((dy * 3 + dx) * 4096) % 16384 + k * 32) >> 4);
-                umma_bf16_ts2(d, a_t + dx * 32 + k * 8, ((uint64_t)DESC_HI << 32) | bl, idesc, accumulate);
-                accumulate = 1;
-              }
-          }
-        }
-      }
-      for (int it = 0; it < (mode >= 2 ? 0 : iters); ++it) {
+      for (int it = 0; it < iters; ++it) {
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
           if (mode == 0)
@@ -442,19 +397,14 @@ __global__ void __launch_bounds__(128, 1) mma_rate2_kernel(int n, int iters, lon
 }  // namespace psgla
 
 extern "C" int psgla_selftest_mma_rate2(int mode, int n, int iters, int n_pairs, long long* cycles_dev, void* stream) {
-  PSGLA_REQUIRE(cycles_dev && mode >= 0 && mode <= 5 && n >= 32 && n <= 256 && n % 32 == 0 && iters > 0 && n_pairs > 0,
+  PSGLA_REQUIRE(cycles_dev && mode >= 0 && mode <= 1 && n >= 32 && n <= 256 && n % 32 == 0 && iters > 0 && n_pairs > 0,
                 "psgla_selftest_mma_rate2: bad argument");
-  PSGLA_REQUIRE(mode < 2 || n == 64, "psgla_selftest_mma_rate2: the conv-row modes are N = 64");
   const int smem = 54 * 1024;
   static std::atomic<unsigned long long> attr_done{0};  // bit d: opted in on device d (a per-device function attribute)
   const unsigned long long dev_bit = 1ull << (current_device() & 63);
   if (!(attr_done.load(std::memory_order_acquire) & dev_bit)) {
     PSGLA_CUDA_TRY(cudaFuncSetAttribute(mma_rate2_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     PSGLA_CUDA_TRY(cudaFuncSetAttribute(mma_rate2_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    PSGLA_CUDA_TRY(cudaFuncSetAttribute(mma_rate2_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    PSGLA_CUDA_TRY(cudaFuncSetAttribute(mma_rate2_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    PSGLA_CUDA_TRY(cudaFuncSetAttribute(mma_rate2_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    PSGLA_CUDA_TRY(cudaFuncSetAttribute(mma_rate2_kernel<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     attr_done.fetch_or(dev_bit, std::memory_order_release);
   }
   cudaLaunchConfig_t cfg{};
@@ -469,14 +419,10 @@ extern "C" int psgla_selftest_mma_rate2(int mode, int n, int iters, int n_pairs,
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  switch (mode) {
-    case 0: PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, mma_rate2_kernel<0>, n, iters, cycles_dev)); break;
-    case 1: PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, mma_rate2_kernel<1>, n, iters, cycles_dev)); break;
-    case 2: PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, mma_rate2_kernel<2>, n, iters, cycles_dev)); break;
-    case 3: PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, mma_rate2_kernel<3>, n, iters, cycles_dev)); break;
-    case 4: PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, mma_rate2_kernel<4>, n, iters, cycles_dev)); break;
-    default: PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, mma_rate2_kernel<5>, n, iters, cycles_dev)); break;
-  }
+  if (mode == 0)
+    PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, mma_rate2_kernel<0>, n, iters, cycles_dev));
+  else
+    PSGLA_CUDA_TRY(cudaLaunchKernelEx(&cfg, mma_rate2_kernel<1>, n, iters, cycles_dev));
   return PSGLA_OK;
 }
 

@@ -9,7 +9,6 @@
 // (the denoiser term of either update is added by the last conv layer's epilogue, csrc/conv_tc.cu).
 #include <cuda_bf16.h>
 
-#include <cstdlib>
 #include <cstring>
 
 #include "common.cuh"
@@ -498,7 +497,7 @@ __device__ __forceinline__ void ata_vpass(float (&hring)[NT][4], const float (&o
 }
 
 // Two blocks per SM (156 registers).  A 96-register build with three resident blocks spills part of the window: 86 us
-// instead of 58 (measured, scripts/blur_sweep.py).
+// instead of 58 (measured with scripts/blur_sweep.py, removed; commit 409bc30 is the last that contains it).
 template <int K2, int C>  // K2 = 2 l: half-width of A^T A;  C: image channels (3 or 1)
 __global__ void __launch_bounds__(ATA_THREADS, 2)
 deblur_ata_kernel(PreArgs a, const Taps2 k, int B, int H, int W, int RH, const float* __restrict__ x,
@@ -904,10 +903,6 @@ static int launch_ata(const PreArgs& a, const Taps2& k, psgla_img_shape s, const
     const long long blocks = (long long)strips * ((s.H + bands * rh - 1) / (bands * rh)) * s.B;
     const long long cost = ((blocks + sms - 1) / sms) * (rh + 2 * K2);
     if (best < 0 || cost < best) best = cost, best_rh = rh;
-  }
-  if (const char* e = std::getenv("PSGLA_ATA_RH")) {  // A/B runs
-    const int v = std::atoi(e);
-    if (v >= 1) best_rh = v;
   }
   const int row_blocks = (s.H + bands * best_rh - 1) / (bands * best_rh);
   PSGLA_REQUIRE(s.B <= 65535 && row_blocks <= 65535, "too many chains / rows for one launch");

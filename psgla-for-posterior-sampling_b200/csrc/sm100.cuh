@@ -335,16 +335,6 @@ __device__ __forceinline__ void tmem_st_32x32b_x32(uint32_t taddr, const uint32_
         "r"(v[27]), "r"(v[28]), "r"(v[29]), "r"(v[30]), "r"(v[31])
       : "memory");
 }
-// shared memory -> TMEM without registers: 128 rows x 256 bit (one K16 bf16 slice of an A operand, 8 columns) from the matrix the
-// descriptor names (same descriptor format and swizzle handling as an MMA operand); asynchronous, ordered with the
-// tcgen05.mma / tcgen05.cp / tcgen05.commit that the same thread issues afterwards.  cta_group::2: each CTA of the pair
-// copies from its own shared memory (same offsets) into its own tensor memory.
-__device__ __forceinline__ void tmem_cp_128x256b(uint32_t taddr, uint64_t sdesc) {
-  asm volatile("tcgen05.cp.cta_group::1.128x256b [%0], %1;" ::"r"(taddr), "l"(sdesc) : "memory");
-}
-__device__ __forceinline__ void tmem_cp2_128x256b(uint32_t taddr, uint64_t sdesc) {
-  asm volatile("tcgen05.cp.cta_group::2.128x256b [%0], %1;" ::"r"(taddr), "l"(sdesc) : "memory");
-}
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ uint4 ld_shared_v4(uint32_t saddr) {
   uint4 v;

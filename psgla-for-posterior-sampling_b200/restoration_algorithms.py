@@ -33,7 +33,6 @@ from __future__ import annotations
 
 import ctypes as C
 import math
-import os
 
 import numpy as np
 import torch
@@ -165,10 +164,8 @@ class _Run:
             self.y = operand(data_grad.y, "the blurred observation y", (Cn,))
             self.mask = None
             # A^T(A x - y) = (A^T A) x - A^T y: A^T y is blurred once here, the iterations run the two-pass A^T A kernel
-            # (PSGLA_BLUR_4PASS=1 keeps the four-pass kernel for A/B runs; half-widths above 4 always take it)
-            self.aty = None
-            if 1 <= data_grad.l <= 4 and os.environ.get("PSGLA_BLUR_4PASS", "0") != "1":
-                self.aty = data_grad.AT(self.y)
+            # (half-widths above 4 take the four-pass kernel: aty = None)
+            self.aty = data_grad.AT(self.y) if 1 <= data_grad.l <= 4 else None
         else:
             self.y = operand(data_grad.y, "the observation y", (1, Cn))
             self.mask = operand(data_grad.mask, "the mask", (1, Cn))
@@ -176,7 +173,7 @@ class _Run:
     def configure(self, pre, gain, base_scale=1.0):
         self.pre_params, self.gain, self.base_scale = pre, float(gain), float(base_scale)
         # the fused next-iteration pre is a conv-epilogue feature: the TV prox runs one pre launch per iteration
-        self.fuse_next_pre = os.environ.get("PSGLA_FUSE_PRE", "1") != "0" and not isinstance(self.den, TVDenoiser)
+        self.fuse_next_pre = not isinstance(self.den, TVDenoiser)
         self._pre_done_for = None
         self._next_params = _lib.PreParams()
 

@@ -7,5 +7,3 @@ run() {  # run VAR=value "k expression" files...
   else env "$setting" python -m pytest -q -m gpu -x "$@" 2>&1 | tail -1; fi
 }
 run PSGLA_CONV_FUSE2=0 "dncnn_forward or psgla_replay or reference_fixture or fused_layer" tests/test_image_gpu.py
-run PSGLA_FUSE_PRE=0 "psgla_replay or batched or statistics_only or image_set" tests/test_image_gpu.py
-run PSGLA_BLUR_4PASS=1 "deblur or pnpula" tests/test_image_gpu.py tests/test_torch_stream_gpu.py

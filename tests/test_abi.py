@@ -77,6 +77,20 @@ def test_product_does_not_import_oracle():
             assert "oracle" not in src.replace("# oracle", ""), f
 
 
+def test_environment_selects_no_kernel_but_the_documented_switches():
+    """The problem alone selects each kernel: the library reads PSGLA_CONV_FUSE2 (per-layer launches, which the bench times
+    beside the fused pairs), PSGLA_CONV_ROWS (a test hook) and PSGLA_VERBOSE (diagnostics), and the package reads none."""
+    names = set()
+    csrc = os.path.join(ROOT, "psgla-for-posterior-sampling_b200", "csrc")
+    for f in os.listdir(csrc):
+        names.update(re.findall(r'getenv\(\s*"(PSGLA_\w*)"', open(os.path.join(csrc, f)).read()))
+    pkg = os.path.join(ROOT, "psgla-for-posterior-sampling_b200")
+    for f in os.listdir(pkg):
+        if f.endswith(".py"):
+            names.update(re.findall(r'os\.(?:environ\b[^"\'\n]*|getenv\(\s*)["\'](PSGLA_\w*)["\']', open(os.path.join(pkg, f)).read()))
+    assert names == {"PSGLA_CONV_FUSE2", "PSGLA_CONV_ROWS", "PSGLA_VERBOSE"}
+
+
 def test_philox_known_answers(built):
     """Random123's kat_vectors for philox4x32-10: the RNG the kernels inline is the published Philox."""
     import ctypes as C

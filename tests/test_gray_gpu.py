@@ -90,14 +90,23 @@ def _assert_channel0(gray, colour, squeeze):
             assert a.shape == want.shape and torch.equal(a, want)
 
 
-def _run(alg, den, dg, init, store, **kw):
+def _run(alg, den, dg, init, store, form=None, **kw):
+    """form "unfused": the stand-alone pre kernel every iteration; "4pass": the four-pass deblurring pre."""
     prm = io_.resolve_params("psgla" if alg == "psgla" else "pnp_ula", s=5.0)
     common = dict(n_iter=9, n_inter=2, n_inter_mmse=2, store=store, **kw)
     if alg == "psgla":
-        return P.psgla(init, dg, den, alpha=torch.tensor(0.9, device="cuda"), lambd=torch.tensor(prm["lambd"], device="cuda"),
-                       sig_float=prm["s"], delta=prm["delta"], **common)
-    pg = P.PriorGrad(den, 1.0, SIG, SIG ** 2)
-    return P.pnpula(init, dg, pg, torch.tensor(1e-5, device="cuda"), torch.tensor(2e-5, device="cuda"), **common)
+        run = P.psgla_run(init, dg, den, alpha=torch.tensor(0.9, device="cuda"), lambd=torch.tensor(prm["lambd"], device="cuda"),
+                          sig_float=prm["s"], delta=prm["delta"], **common)
+    else:
+        pg = P.PriorGrad(den, 1.0, SIG, SIG ** 2)
+        run = P.pnpula_run(init, dg, pg, torch.tensor(1e-5, device="cuda"), torch.tensor(2e-5, device="cuda"), **common)
+    if form == "unfused":
+        run.fuse_next_pre = False
+    elif form == "4pass":
+        run.aty = None
+    for i in range(run.n_iter):
+        run.step(i)
+    return run.finish()
 
 
 # ---------------------------------------------------------------------------------------------- the zero-weight fact
@@ -138,15 +147,11 @@ def test_zero_weights_add_exactly_zero_on_first_and_last_layer(dncnn_pair):
 @pytest.mark.parametrize("problem,form", [("inpainting", "fused"), ("inpainting", "unfused"), ("deblurring", "ata"),
                                           ("deblurring", "4pass")])
 @pytest.mark.parametrize("store", ["all", "stats"])
-def test_gray_equals_channel0_of_embedded_colour_run(family, alg, problem, form, store, dncnn_pair, drunet_pair, monkeypatch):
+def test_gray_equals_channel0_of_embedded_colour_run(family, alg, problem, form, store, dncnn_pair, drunet_pair):
     g1, g3, _ = dncnn_pair if family == "dncnn" else drunet_pair
-    if form == "unfused":
-        monkeypatch.setenv("PSGLA_FUSE_PRE", "0")
-    if form == "4pass":
-        monkeypatch.setenv("PSGLA_BLUR_4PASS", "1")
     H, W = (40, 48) if family == "drunet" else (36, 52)
     dg1, init1, dg3, init3 = _problems(problem, H, W, seed=1)
-    kw = dict(seed=7, n_chains=2, chain_id0=3, rng="philox")
+    kw = dict(seed=7, n_chains=2, chain_id0=3, rng="philox", form=form)
     gray = _run(alg, g1, dg1, init1, store, **kw)
     colour = _run(alg, g3, dg3, init3, store, **kw)
     torch.cuda.synchronize()

@@ -327,20 +327,24 @@ def test_pnp_and_red_gs_against_oracle(gs):
 
 
 @pytest.mark.parametrize("alg", ["psgla", "pnpula"])
-def test_fused_next_pre_is_bit_identical(gs, alg, monkeypatch):
+def test_fused_next_pre_is_bit_identical(gs, alg):
     den, _ = gs
     dg, init, y, mask = _inpaint(3)
     outs = []
-    for fuse in ("1", "0"):
-        monkeypatch.setenv("PSGLA_FUSE_PRE", fuse)
+    for fuse in (True, False):
         if alg == "psgla":
             prm = io_.resolve_params("psgla", den="DRUNet", lambd=25.0)
-            outs.append(P.psgla(init, dg, den, alpha=0.9, lambd=prm["lambd"], sig_float=prm["s"], delta=prm["delta"], n_iter=5,
-                                n_inter=1, n_inter_mmse=2, seed=4, n_chains=2, rng="philox"))
+            run = P.psgla_run(init, dg, den, alpha=0.9, lambd=prm["lambd"], sig_float=prm["s"], delta=prm["delta"], n_iter=5,
+                              n_inter=1, n_inter_mmse=2, seed=4, n_chains=2, rng="philox")
         else:
             prm = io_.resolve_params("pnp_ula", den="DRUNet", s=5.0)
-            outs.append(P.pnpula(init, dg, P.PriorGrad(den, 1.0, prm["s1"], prm["s2"]), prm["delta"], prm["lambd"], n_iter=5,
-                                 n_inter=1, n_inter_mmse=2, seed=4, n_chains=2, rng="philox"))
+            run = P.pnpula_run(init, dg, P.PriorGrad(den, 1.0, prm["s1"], prm["s2"]), prm["delta"], prm["lambd"], n_iter=5,
+                               n_inter=1, n_inter_mmse=2, seed=4, n_chains=2, rng="philox")
+        assert run.fuse_next_pre
+        run.fuse_next_pre = fuse
+        for i in range(run.n_iter):
+            run.step(i)
+        outs.append(run.finish())
     for a, b in zip(outs[0], outs[1]):
         assert len(a) == len(b) and all(torch.equal(u, v) for u, v in zip(a, b))
 

@@ -482,10 +482,10 @@ def test_reference_edge_behaviours(nets, tmp_path):
 @pytest.mark.parametrize("family", ["dncnn", "drunet"])
 @pytest.mark.parametrize("alg,rng,B,H,W", [("psgla", "philox", 3, 40, 56), ("psgla", "torch_cuda", None, 33, 31),
                                            ("pnpula", "philox", 2, 24, 40), ("pnpula", "torch_cuda", None, 64, 64)])
-def test_fused_next_pre_equals_separate_pre_kernel(weights, family, alg, rng, B, H, W, monkeypatch):
+def test_fused_next_pre_equals_separate_pre_kernel(weights, family, alg, rng, B, H, W):
     """Inpainting: the last layer's epilogue evaluates the next iteration's Langevin "pre" on the iterate it has just produced
     (psgla_*_post_next).  Same arithmetic, same noise element: samples and moments must equal, BIT FOR BIT, the run that
-    launches the stand-alone pre kernel every iteration (PSGLA_FUSE_PRE=0)."""
+    launches the stand-alone pre kernel every iteration (run.fuse_next_pre = False)."""
     if family == "drunet":
         if H % 8 or W % 8:
             H, W = (H + 7) // 8 * 8, (W + 7) // 8 * 8
@@ -496,18 +496,22 @@ def test_fused_next_pre_equals_separate_pre_kernel(weights, family, alg, rng, B,
     im = torch.rand(1, 3, H, W, device="cuda")
     dg, init, _, _ = P.make_inpainting(im, prop=0.5, sigma=1.0, seed_ip=0)
 
-    def run():
+    def run(fuse):
         if alg == "psgla":
-            return P.psgla(init, dg, den, alpha=0.8, lambd=5.0, sig_float=2 / 255, delta=(2 / 255) ** 2, n_iter=7, n_inter=2,
-                           n_inter_mmse=2, seed=3, rng=rng, n_chains=B)
-        pg = P.PriorGrad(den, 1.0, 5 / 255, (5 / 255) ** 2)
-        return P.pnpula(init, dg, pg, delta=torch.tensor(1e-5, device="cuda"), lambd=torch.tensor(2e-5, device="cuda"),
-                        n_iter=7, n_inter=2, n_inter_mmse=2, seed=3, rng=rng, n_chains=B)
+            r = P.psgla_run(init, dg, den, alpha=0.8, lambd=5.0, sig_float=2 / 255, delta=(2 / 255) ** 2, n_iter=7, n_inter=2,
+                            n_inter_mmse=2, seed=3, rng=rng, n_chains=B)
+        else:
+            pg = P.PriorGrad(den, 1.0, 5 / 255, (5 / 255) ** 2)
+            r = P.pnpula_run(init, dg, pg, delta=torch.tensor(1e-5, device="cuda"), lambd=torch.tensor(2e-5, device="cuda"),
+                             n_iter=7, n_inter=2, n_inter_mmse=2, seed=3, rng=rng, n_chains=B)
+        assert r.fuse_next_pre
+        r.fuse_next_pre = fuse
+        for i in range(r.n_iter):
+            r.step(i)
+        return r.finish()
 
-    monkeypatch.setenv("PSGLA_FUSE_PRE", "1")
-    a = run()
-    monkeypatch.setenv("PSGLA_FUSE_PRE", "0")
-    b = run()
+    a = run(True)
+    b = run(False)
     torch.cuda.synchronize()
     for la, lb in zip(a, b):
         assert len(la) == len(lb) and len(la) > 0
