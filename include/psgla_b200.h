@@ -300,6 +300,24 @@ int psgla_tv_prox_post(const psgla_tv_params* tv, psgla_img_shape shape, const f
                        float* x_out_dev, float* sample_dev, float* mean_dev, float* mean2_dev, int32_t* iters_dev,
                        void* stream);
 
+/* Convergence diagnostics of a multi-chain run, per element (csrc/mcmc_diag.cu): rank-normalised split-R-hat and bulk / tail
+ * ESS (Vehtari et al. 2021), as arviz's rhat(method="rank"), ess(method="bulk"), ess(method="tail") define them.
+ *   draws_dev   fp32 [n_draws][n_chains][n_elem]: the samplers' own sample buffer ([n_samples][B][C][H][W]), read in place.
+ *   rhat_dev, ess_bulk_dev, ess_tail_dev   fp32 [n_elem].  R-hat = max(bulk, folded-tail) split-R-hat; tail ESS = the smaller
+ *               ESS of the indicators x <= q05, x <= q95.  An element with NaN draws, or whose split chains are each constant
+ *               in a series (W = 0), gets NaN for the statistics of that series.
+ * Each chain is split into two halves (odd n_draws: the middle draw is dropped), so an element has S = 2 n_chains
+ * floor(n_draws / 2) split draws; n_draws >= 4, n_chains >= 1 and S <= PSGLA_MCMC_MAX_DRAWS (one element's draws are sorted
+ * in shared memory).  A longer run is diagnosed after thinning it further (a larger n_inter) or on fewer chains.
+ * ws_dev: psgla_mcmc_diag_workspace_bytes(n_draws, n_chains) bytes (0: out of range), 256-byte aligned.  On return its first
+ * four uint64 hold the SM cycles the call spent, summed over elements, in: loading the draws; sorting them (with the median
+ * and quantiles); ranking and normal scores; chain moments and autocovariances.  Deterministic: an element's results do not
+ * depend on n_elem or on the other elements. */
+#define PSGLA_MCMC_MAX_DRAWS 16384
+size_t psgla_mcmc_diag_workspace_bytes(int64_t n_draws, int64_t n_chains);
+int psgla_mcmc_diag(const float* draws_dev, int64_t n_draws, int64_t n_chains, int64_t n_elem, void* ws_dev, size_t ws_bytes,
+                    float* rhat_dev, float* ess_bulk_dev, float* ess_tail_dev, void* stream);
+
 /* tcgen05 descriptor self-test (development aid): runs a 128 x 64 x 64 GEMM tile whose A operand starts `row_shift`
  * rows into a 128B-swizzled shared-memory buffer.  mode 0: A from shared memory, shift = descriptor start address;
  * mode 2: A copied to tensor memory.

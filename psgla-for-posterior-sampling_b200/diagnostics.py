@@ -1,0 +1,122 @@
+"""Convergence diagnostics of multi-chain image runs, on the device: rank-normalised split-R-hat and bulk / tail ESS per pixel
+(Vehtari, Gelman, Simpson, Carpenter, Buerkner 2021; arviz's rhat(method="rank"), ess(method="bulk"), ess(method="tail")).
+
+    d = psgla_b200.mcmc_diagnostics(run, burn_in=100)      # run = psgla_run(...) / pnpula_run(...) after its steps
+    d["rhat"], d["ess_bulk"], d["ess_tail"]                  # [C, H, W] maps
+    d["rhat_max"], d["frac_rhat_above_1_01"], d["ess_bulk_min"], d["ess_bulk_median"], d["ess_tail_min"]
+
+The kernel (csrc/mcmc_diag.cu) reads the draws where the sampler stored them, [N][M][C][H][W]: a run object is diagnosed in
+place, with no copy.  Limit: S = 2 M floor(N / 2) <= PSGLA_MCMC_MAX_DRAWS = 16 384 split draws per element.
+"""
+from __future__ import annotations
+
+import ctypes as C
+
+import torch
+
+from . import _lib
+
+__all__ = ["mcmc_diagnostics", "MAX_DRAWS"]
+
+MAX_DRAWS = 16384  # PSGLA_MCMC_MAX_DRAWS
+
+
+def _as_draws(draws):
+    """-> (contiguous CUDA fp32 [N, M, E] tensor, map shape [C, H, W], crop (h, w) or None)."""
+    from .restoration_algorithms import _Run
+    if isinstance(draws, _Run):
+        if draws.samples is None:
+            raise ValueError("mcmc_diagnostics needs stored draws: this run has store='stats', which keeps none (run it "
+                             "with store='all')")
+        n = len(draws.Xlist)  # slots written so far
+        x = draws.samples[:n]  # [n, B, C, Hp, Wp], a contiguous view of the run's own buffer
+        return x, tuple(x.shape[2:]), draws.crop
+    if isinstance(draws, (list, tuple)):
+        if len(draws) == 0:
+            raise ValueError("mcmc_diagnostics needs stored draws: Xlist is empty (a store='stats' run keeps none; run it "
+                             "with store='all')")
+        shapes = {tuple(t.shape) for t in draws}
+        if len(shapes) != 1:
+            raise ValueError("the draws of the list have different shapes: %s" % sorted(shapes))
+        for t in draws:
+            _check_tensor(t)
+        x = torch.stack(list(draws))
+        if x.dim() == 3:    # squeezed single grayscale chain [H, W]
+            x = x[:, None, None]
+        elif x.dim() == 4:  # squeezed single chain [C, H, W]
+            x = x[:, None]
+        if x.dim() != 5:
+            raise ValueError("Xlist entries must be [M, C, H, W], [C, H, W] or [H, W], got %s" % (tuple(draws[0].shape),))
+        return x, tuple(x.shape[2:]), None
+    if isinstance(draws, torch.Tensor):
+        _check_tensor(draws)
+        if draws.dim() not in (3, 5):
+            raise ValueError("draws must be [N, M, C, H, W] or [N, M, E], got %s" % (tuple(draws.shape),))
+        return draws, tuple(draws.shape[2:]), None
+    raise TypeError("draws must be a CUDA tensor, a sampler's Xlist or a psgla_run / pnpula_run object")
+
+
+def _check_tensor(t):
+    if not isinstance(t, torch.Tensor):
+        raise TypeError("expected torch tensors, got %s" % type(t).__name__)
+    if not t.is_cuda:
+        raise RuntimeError("mcmc_diagnostics needs CUDA tensors: there is no CPU path")
+    if t.dtype != torch.float32:
+        raise TypeError("draws must be float32 (the samplers' dtype), got %s" % t.dtype)
+
+
+def mcmc_diagnostics(draws, *, burn_in: int = 0) -> dict:
+    """Rank-normalised split-R-hat and bulk / tail ESS of every element of a multi-chain run.
+
+    draws: a CUDA fp32 tensor [N, M, C, H, W] or [N, M, E] (N stored draws of M chains); a sampler's ``Xlist`` (entries
+    [M, C, H, W], or the squeezed single-chain [C, H, W] / [H, W], taken as M = 1); or a ``psgla_run`` / ``pnpula_run`` object,
+    read in place from its sample buffer (the slots written so far).  A DRUNet run padded to multiples of 8 is diagnosed at the
+    padded size and the maps are cropped like its outputs.  burn_in: the first ``burn_in`` draws are dropped.
+
+    Returns a dict: ``rhat``, ``ess_bulk``, ``ess_tail`` -- CUDA fp32 maps [C, H, W] (an [N, M, E] tensor gives [E]) --, and
+    the floats ``rhat_max``, ``frac_rhat_above_1_01``, ``ess_bulk_min``, ``ess_bulk_median``, ``ess_tail_min`` over the
+    elements whose statistic is not NaN (NaN: NaN draws, or an element constant within every split chain; the fraction counts
+    NaN as not above; the median is torch's, the lower middle value for an even count), and the ints ``n_draws``,
+    ``n_chains``.  Stream-ordered on the current stream; reading the scalars synchronises it."""
+    x, map_shape, crop = _as_draws(draws)
+    burn_in = int(burn_in)
+    if burn_in < 0 or burn_in >= x.shape[0]:
+        raise ValueError("burn_in = %d must be in [0, %d) (the number of stored draws)" % (burn_in, x.shape[0]))
+    x = x[burn_in:]
+    if not x.is_contiguous():
+        x = x.contiguous()
+    N, M = int(x.shape[0]), int(x.shape[1])
+    E = x[0, 0].numel()
+    S = 2 * M * (N // 2)
+    if N < 4:
+        raise ValueError("split chains need at least 4 draws after burn-in, got %d" % N)
+    if S > MAX_DRAWS:
+        raise ValueError("%d chains x %d draws give S = %d split draws per element, above the limit of %d: store fewer draws "
+                         "(thin more with a larger n_inter), raise burn_in, or diagnose fewer chains" % (M, N, S, MAX_DRAWS))
+    lib = _lib.lib()
+    with torch.cuda.device(x.device):
+        ws_bytes = lib.psgla_mcmc_diag_workspace_bytes(N, M)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
+        out = torch.empty((3, E), dtype=torch.float32, device=x.device)
+        _lib.check(lib.psgla_mcmc_diag(_lib.ptr(x), N, M, E, _lib.ptr(ws), C.c_size_t(ws_bytes), out[0].data_ptr(),
+                                       out[1].data_ptr(), out[2].data_ptr(), _lib.stream_ptr(x.device)), "psgla_mcmc_diag")
+    maps = out.reshape((3,) + map_shape)
+    if crop is not None:
+        maps = maps[..., :crop[0], :crop[1]]
+    rhat, ess_bulk, ess_tail = maps[0], maps[1], maps[2]
+
+    def finite(t):
+        t = t.reshape(-1)
+        return t[~torch.isnan(t)]
+
+    r, b, t = finite(rhat), finite(ess_bulk), finite(ess_tail)
+    nan = float("nan")
+    return {
+        "rhat": rhat, "ess_bulk": ess_bulk, "ess_tail": ess_tail,
+        "rhat_max": float(r.max()) if r.numel() else nan,
+        "frac_rhat_above_1_01": float((rhat > 1.01).sum()) / rhat.numel(),
+        "ess_bulk_min": float(b.min()) if b.numel() else nan,
+        "ess_bulk_median": float(b.median()) if b.numel() else nan,
+        "ess_tail_min": float(t.min()) if t.numel() else nan,
+        "n_draws": N, "n_chains": M,
+    }
