@@ -79,10 +79,13 @@ inline PhiloxKeys philox_round_keys(uint64_t seed) {
   }
   return r;
 }
+// Rounds FIRST .. 9 of the keyed form: a caller that has computed the first rounds itself (gmm2d_lean_kernel, whose first
+// two rounds are mostly launch or thread constants) finishes the call here.
+template <int FIRST = 0>
 __device__ __forceinline__ void philox4x32_10_keyed(uint32_t& c0, uint32_t& c1, uint32_t& c2, uint32_t& c3,
                                                     const PhiloxKeys& keys) {
 #pragma unroll
-  for (int i = 0; i < 10; ++i) {
+  for (int i = FIRST; i < 10; ++i) {
     const uint64_t p0 = (uint64_t)0xD2511F53u * c0;
     const uint64_t p1 = (uint64_t)0xCD9E8D57u * c2;
     const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ keys.k[2 * i];

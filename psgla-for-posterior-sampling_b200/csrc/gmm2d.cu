@@ -362,16 +362,31 @@ gmm2d_lean_kernel(const Gmm2dConsts<float> c, float2* __restrict__ x, unsigned n
   if (g >= n_launch) return;
   float2 v = x[g];
   float x0 = v.x, x1 = v.y;
-  const unsigned long long sub = sub0 + g;
-  const uint32_t s_lo = (uint32_t)sub, s_hi = (uint32_t)(sub >> 32);
-  unsigned long long pair = pair0;
-  for (int r = 0; r < n_rounds; ++r, pair += LEAN_NB) {
+  // The launch's chain ids share their high word, and so do its counter pairs (launch_lean_body splits where they would not),
+  // so Philox's counter words c1 = pair >> 32 and c3 = chain id >> 32 are launch constants and its first two rounds are
+  // mostly thread constants (T) and launch-uniform values (U):
+  //   round 1: c0' = hi(M1 s_lo) ^ c1 ^ k0 (T), c1' = lo(M1 s_lo) (T), c2' = hi(M0 pair) ^ c3 ^ k1 (U), c3' = lo(M0 pair) (U)
+  //   round 2: M0 c0' (T) and M1 c2' (U)
+  // so per thread and per counter block rounds 1-2 cost one IMAD.WIDE.U32 instead of two (ptxas puts the round-1 U product on
+  // the uniform datapath but keeps the round-2 one on the vector pipe): 17 per block instead of 18.  Same words as
+  // philox4x32_10_keyed from round 0, i.e. bit-identical draws.
+  const uint32_t s_lo = (uint32_t)sub0 + g, s_hi = (uint32_t)(sub0 >> 32), p_hi = (uint32_t)(pair0 >> 32);
+  const uint64_t t1 = (uint64_t)0xCD9E8D57u * s_lo;               // round 1, chain word
+  const uint32_t t1_lo = (uint32_t)t1;
+  const uint64_t t2 = (uint64_t)0xD2511F53u * ((uint32_t)(t1 >> 32) ^ p_hi ^ keys.k[0]);  // round 2, first product
+  const uint32_t t2_hi = (uint32_t)(t2 >> 32), t2_lo = (uint32_t)t2;
+  for (int r = 0; r < n_rounds; ++r) {
     uint32_t w[LEAN_NB][4];  // Philox4x32-10 of counter blocks pair .. pair + LEAN_NB - 1
 #pragma unroll
     for (int b = 0; b < LEAN_NB; ++b) {
-      const unsigned long long pr = pair + b;
-      w[b][0] = (uint32_t)pr, w[b][1] = (uint32_t)(pr >> 32), w[b][2] = s_lo, w[b][3] = s_hi;
-      philox4x32_10_keyed(w[b][0], w[b][1], w[b][2], w[b][3], keys);
+      const uint32_t pr = (uint32_t)pair0 + (uint32_t)(r * LEAN_NB + b);
+      const uint64_t u1 = (uint64_t)0xD2511F53u * pr;                                         // round 1, pair word
+      const uint64_t u2 = (uint64_t)0xCD9E8D57u * ((uint32_t)(u1 >> 32) ^ s_hi ^ keys.k[1]);  // round 2, second product
+      w[b][0] = (uint32_t)(u2 >> 32) ^ t1_lo ^ keys.k[2];
+      w[b][1] = (uint32_t)u2;
+      w[b][2] = t2_hi ^ (uint32_t)u1 ^ keys.k[3];
+      w[b][3] = t2_lo;
+      philox4x32_10_keyed<2>(w[b][0], w[b][1], w[b][2], w[b][3], keys);
     }
     float z[LEAN_NB][4];
 #pragma unroll
@@ -622,16 +637,38 @@ static int launch_waves(const Launch& a, int* launches) {
 }
 
 template <int ALG, int STRUCT>
-static void launch_lean(const Launch& a, long long lo, long long n, long long n_rounds, long long step_lo) {
+static void launch_lean(const Launch& a, long long lo, long long n, long long n_rounds, unsigned long long pair0) {
   gmm2d_lean_kernel<ALG, STRUCT><<<(unsigned)((n + LEAN_BLOCK - 1) / LEAN_BLOCK), LEAN_BLOCK, 0, a.st>>>(
-      *(const Gmm2dConsts<float>*)a.c, (float2*)a.x + lo, (unsigned)n, a.chain_id0 + (unsigned long long)lo,
-      (unsigned long long)step_lo >> 1, (int)n_rounds, a.keys);
+      *(const Gmm2dConsts<float>*)a.c, (float2*)a.x + lo, (unsigned)n, a.chain_id0 + (unsigned long long)lo, pair0,
+      (int)n_rounds, a.keys);
+}
+
+// The lean kernel on chains [lo, lo + n) (one high word of the chain id) for `rounds` rounds from counter pair pair0, in
+// launches within which the pair's high word does not change either (gmm2d_lean_kernel takes both as launch constants).  A
+// round whose LEAN_NB pairs straddle a multiple of 2^32 goes to the general kernel.  Returns the number of launches.
+template <int ALG, int STRUCT>
+static int launch_lean_body(const Launch& a, long long lo, long long n, unsigned long long pair0, long long rounds) {
+  int launches = 0;
+  for (; rounds > 0; ++launches) {
+    const unsigned long long next = ((pair0 >> 32) + 1) << 32;  // the first pair with the next high word
+    const long long fit = (long long)std::min<unsigned long long>((next - pair0) / LEAN_NB, (unsigned long long)rounds);
+    if (fit > 0) {
+      launch_lean<ALG, STRUCT>(a, lo, n, fit, pair0);
+      pair0 += (unsigned long long)fit * LEAN_NB, rounds -= fit;
+    } else {
+      Launch b = a;
+      b.step0 = (long long)(pair0 << 1), b.n_steps = 2 * LEAN_NB;
+      launch_one<float, ALG, true, 1, 1, 128>(b, lo, n);
+      pair0 += LEAN_NB, --rounds;
+    }
+  }
+  return launches;
 }
 
 // fp32, r == 2, in-kernel Philox; returns the number of launches.  With a trajectory: one launch of 1-warp blocks of the
 // general kernel (the lean kernel keeps no trajectory).  Without: the lean kernel on the whole rounds of 2 LEAN_NB steps that
-// start on an even step, in chunks of 2^30 chains; the general kernel takes the lead step of an odd step0 and the steps after
-// the last whole round.
+// start on an even step, in chunks of at most 2^30 chains that do not cross a multiple of 2^32 in the global chain id; the
+// general kernel takes the lead step of an odd step0 and the steps after the last whole round.
 template <int ALG>
 static int launch_philox_r2(const Launch& a) {
   if (a.traj != nullptr) {
@@ -641,6 +678,7 @@ static int launch_philox_r2(const Launch& a) {
   const int structure = constants_structure(*(const Gmm2dConsts<float>*)a.c);
   const long long lead = std::min(a.step0 & 1, a.n_steps);
   const long long rounds = (a.n_steps - lead) / (2 * LEAN_NB), body = rounds * 2 * LEAN_NB;
+  const unsigned long long pair0 = (unsigned long long)(a.step0 + lead) >> 1;
   int launches = 0;
   if (lead) {
     Launch b = a;
@@ -648,14 +686,15 @@ static int launch_philox_r2(const Launch& a) {
     launch_one<float, ALG, true, 1, 1, 128>(b, 0, a.n_chains);
     ++launches;
   }
-  for (long long lo = 0; lo < a.n_chains && rounds > 0; lo += (1ll << 30), ++launches) {
-    const long long n = std::min(a.n_chains - lo, 1ll << 30);
+  for (long long lo = 0, n = 0; lo < a.n_chains && rounds > 0; lo += n) {
+    const unsigned long long id = a.chain_id0 + (unsigned long long)lo, next = ((id >> 32) + 1) << 32;
+    n = (long long)std::min({(unsigned long long)(a.n_chains - lo), 1ull << 30, next - id});
     if (structure == 2)
-      launch_lean<ALG, 2>(a, lo, n, rounds, a.step0 + lead);
+      launches += launch_lean_body<ALG, 2>(a, lo, n, pair0, rounds);
     else if (structure == 1)
-      launch_lean<ALG, 1>(a, lo, n, rounds, a.step0 + lead);
+      launches += launch_lean_body<ALG, 1>(a, lo, n, pair0, rounds);
     else
-      launch_lean<ALG, 0>(a, lo, n, rounds, a.step0 + lead);
+      launches += launch_lean_body<ALG, 0>(a, lo, n, pair0, rounds);
   }
   if (lead + body < a.n_steps) {
     Launch b = a;

@@ -49,6 +49,41 @@ __global__ void __launch_bounds__(256) fp32_rate_kernel(int iters, float seed, f
 }
 
 
+// The FP64-pipe form of a Philox round product's high word (modes 12-14 and 200 + NF): for a = the double with bit pattern
+// {lo word x, hi word 0x43380000} (= 1.5 2^52 + x), fma.rm(a, M 2^-32, 1.5 2^52 - 1.5 2^20 M) = 1.5 2^52 + floor(x M / 2^32)
+// exactly, so the result's low word is mulhi(x, M) and its high word 0x43380000 again (M = 0xD2511F53 here).
+__device__ __forceinline__ uint64_t pair_of(uint32_t lo, uint32_t hi) {
+  uint64_t a;
+  asm("mov.b64 %0, {%1, %2};" : "=l"(a) : "r"(lo), "r"(hi));
+  return a;
+}
+__device__ __forceinline__ uint32_t pair_lo(uint64_t a) {
+  uint32_t lo;
+  asm("mov.b64 {%0, _}, %1;" : "=r"(lo) : "l"(a));
+  return lo;
+}
+__device__ __forceinline__ uint32_t pair_hi(uint64_t a) {
+  uint32_t hi;
+  asm("mov.b64 {_, %0}, %1;" : "=r"(hi) : "l"(a));
+  return hi;
+}
+__device__ __forceinline__ uint64_t mulhi_fp64(uint64_t a) {
+  uint64_t t;
+  asm volatile("fma.rm.f64 %0, %1, 0d3FEA4A23EA600000, 0d4311219440E00000;" : "=l"(t) : "l"(a));
+  return t;
+}
+
+// One round product in that form: the low word x * m by IMAD, the high word by DFMA.RM, and a LOP3 that consumes the high word
+// and writes the next input into the pair's low register.
+__device__ __forceinline__ uint64_t fp64_round_product(uint64_t a, unsigned m) {
+  unsigned lo;
+  asm volatile("mul.lo.u32 %0, %1, %2;" : "=r"(lo) : "r"(pair_lo(a)), "r"(m));
+  const uint64_t t = mulhi_fp64(a);
+  unsigned n;
+  asm volatile("lop3.b32 %0, %1, %2, %3, 0x96;" : "=r"(n) : "r"(pair_lo(t)), "r"(lo), "r"(m));
+  return pair_of(n, pair_hi(t));
+}
+
 // Issue-rate probe of single instruction classes (what bounds the chain kernel's Philox + Box-Muller + sigmoid mix):
 // every thread runs iters x 32 instructions of ONE class in 8 independent dependency chains.
 //   0 IMAD.WIDE.U32 (mul.wide.u32, the Philox round multiply)   1 IMAD.HI.U32 (mul.hi.u32)   2 IMAD (mul.lo.u32)
@@ -58,6 +93,10 @@ __global__ void __launch_bounds__(256) fp32_rate_kernel(int iters, float seed, f
 //      "step", 4 steps per loop round; NF = 19 for mode 11, else 21 / 23 / 26 / 28 / 30 = the FP32 pipe slots per step of the six
 //      (algorithm, constants-structure) specialisations of gmm2d_lean_kernel): what the SM sustains for this instruction mix
 //      when no instruction waits for another -- the measured ceiling the chain kernel is held against
+//   12 DFMA.RM (fma.rm.f64, the high word of a Philox round product on the FP64 pipe, below)   13 IMAD + DFMA.RM + LOP3: that
+//   form of one round product (low word, high word, the XOR that consumes it) -- set against mode 0
+//   14 DFMA.RM + FFMA 1:1
+//   200 + NF: the chain-step MIX with the FP64-pipe multiply (6 MUFU, 9 IMAD, 9 DFMA.RM, 2 MOV, NF FFMA, 10 LOP3, 2 I2FP)
 template <int MODE, int NF = 19>
 __global__ void __launch_bounds__(256) pipe_rate_kernel(int iters, unsigned seed, unsigned* __restrict__ out) {
   unsigned v[8];
@@ -67,6 +106,9 @@ __global__ void __launch_bounds__(256) pipe_rate_kernel(int iters, unsigned seed
     v[j] = seed * 2654435761u + threadIdx.x * 40503u + j;
     f[j] = (float)(v[j] & 1023) * 1e-3f;
   }
+  uint64_t d[8];  // modes 12-14, 20: {x, 0x43380000} pairs
+#pragma unroll
+  for (int j = 0; j < 8; ++j) d[j] = pair_of(v[j], 0x43380000u);
   const unsigned m = 0xD2511F53u + seed;
   const float a = 1.0f + seed * 1e-7f, b = seed * 1e-3f;
   for (int i = 0; i < iters; ++i) {
@@ -108,6 +150,13 @@ __global__ void __launch_bounds__(256) pipe_rate_kernel(int iters, unsigned seed
           float g = f[(j + 1) & 7];
           g = fmaf(g, a, b), g = fmaf(g, a, b), g = fmaf(g, a, b), g = fmaf(g, a, b);
           f[(j + 1) & 7] = g;
+        } else if (MODE == 12) {
+          d[j] = mulhi_fp64(d[j]);
+        } else if (MODE == 13) {
+          d[j] = fp64_round_product(d[j], m);
+        } else if (MODE == 14) {
+          d[j] = mulhi_fp64(d[j]);
+          f[j] = fmaf(f[j], a, b);
         }
       }
     if (MODE == 11) {
@@ -139,10 +188,32 @@ __global__ void __launch_bounds__(256) pipe_rate_kernel(int iters, unsigned seed
 #pragma unroll
       for (int q = 0; q < 3; ++q) v[q] = w[q];
     }
+    if (MODE == 20) {  // as mode 11, each IMAD.WIDE.U32 + LOP3 replaced by IMAD + DFMA.RM + LOP3, plus the kernel's ~2 MOV
+      float e[6];
+#pragma unroll
+      for (int q = 0; q < 6; ++q) e[q] = f[q];
+#pragma unroll
+      for (int st = 0; st < 4; ++st) {
+#pragma unroll
+        for (int q = 0; q < 6; ++q) asm volatile("ex2.approx.ftz.f32 %0, %0;" : "+f"(e[q]));
+#pragma unroll
+        for (int q = 0; q < 9; ++q) d[q % 3] = fp64_round_product(d[q % 3], m);
+#pragma unroll
+        for (int q = 0; q < 2; ++q) asm volatile("mov.b32 %0, %1;" : "=r"(v[4 + q]) : "r"(v[3 + q]));
+#pragma unroll
+        for (int q = 0; q < NF; ++q) asm volatile("fma.rn.f32 %0, %0, %1, %2;" : "+f"(f[6 + (q & 1)]) : "f"(a), "f"(b));
+        float c0, c1;
+        asm volatile("cvt.rn.f32.u32 %0, %1;" : "=f"(c0) : "r"(pair_lo(d[0])));
+        asm volatile("cvt.rn.f32.u32 %0, %1;" : "=f"(c1) : "r"(pair_lo(d[1])));
+        asm volatile("lop3.b32 %0, %0, %1, %2, 0x96;" : "+r"(v[7]) : "r"(__float_as_uint(c0)), "r"(__float_as_uint(c1)));
+      }
+#pragma unroll
+      for (int q = 0; q < 6; ++q) f[q] = e[q];
+    }
   }
   unsigned s = 0;
 #pragma unroll
-  for (int j = 0; j < 8; ++j) s += v[j] + __float_as_uint(f[j]);
+  for (int j = 0; j < 8; ++j) s += v[j] + __float_as_uint(f[j]) + pair_lo(d[j]);
   if (s == 0x12345678u) out[blockIdx.x * blockDim.x + threadIdx.x] = s;
 }
 
@@ -165,7 +236,8 @@ extern "C" int psgla_selftest_fp32_rate(int mode, int iters, int blocks_per_sm, 
 }
 
 extern "C" int psgla_selftest_pipe_rate(int mode, int iters, int blocks_per_sm, void* out_dev, double* ops_out, void* stream) {
-  PSGLA_REQUIRE(((mode >= 0 && mode <= 11) || mode == 121 || mode == 123 || mode == 126 || mode == 128 || mode == 130) && iters > 0 && blocks_per_sm > 0 && blocks_per_sm <= 8 && out_dev != nullptr,
+  const bool mix_nf = mode % 100 == 21 || mode % 100 == 23 || mode % 100 == 26 || mode % 100 == 28 || mode % 100 == 30;
+  PSGLA_REQUIRE(((mode >= 0 && mode <= 14) || ((mode / 100 == 1 || mode / 100 == 2) && mix_nf)) && iters > 0 && blocks_per_sm > 0 && blocks_per_sm <= 8 && out_dev != nullptr,
                 "psgla_selftest_pipe_rate: bad argument");
   const int grid = num_sms() * blocks_per_sm;
   cudaStream_t st = (cudaStream_t)stream;
@@ -187,10 +259,20 @@ extern "C" int psgla_selftest_pipe_rate(int mode, int iters, int blocks_per_sm, 
     case 126: pipe_rate_kernel<11, 26><<<grid, 256, 0, st>>>(iters, 3u, o); break;
     case 128: pipe_rate_kernel<11, 28><<<grid, 256, 0, st>>>(iters, 3u, o); break;
     case 130: pipe_rate_kernel<11, 30><<<grid, 256, 0, st>>>(iters, 3u, o); break;
-    default: pipe_rate_kernel<11><<<grid, 256, 0, st>>>(iters, 3u, o); break;
+    case 11: pipe_rate_kernel<11><<<grid, 256, 0, st>>>(iters, 3u, o); break;
+    case 12: pipe_rate_kernel<12><<<grid, 256, 0, st>>>(iters, 3u, o); break;
+    case 13: pipe_rate_kernel<13><<<grid, 256, 0, st>>>(iters, 3u, o); break;
+    case 14: pipe_rate_kernel<14><<<grid, 256, 0, st>>>(iters, 3u, o); break;
+    case 221: pipe_rate_kernel<20, 21><<<grid, 256, 0, st>>>(iters, 3u, o); break;
+    case 223: pipe_rate_kernel<20, 23><<<grid, 256, 0, st>>>(iters, 3u, o); break;
+    case 226: pipe_rate_kernel<20, 26><<<grid, 256, 0, st>>>(iters, 3u, o); break;
+    case 228: pipe_rate_kernel<20, 28><<<grid, 256, 0, st>>>(iters, 3u, o); break;
+    default: pipe_rate_kernel<20, 30><<<grid, 256, 0, st>>>(iters, 3u, o); break;
   }
   PSGLA_CUDA_TRY(cudaGetLastError());
-  // thread-level instructions of the probed class; mode 11: thread-level "steps" (4 per loop round)
-  if (ops_out) *ops_out = (double)grid * 256.0 * (double)iters * (mode >= 11 ? 4.0 : 32.0);
+  // thread-level instructions of the probed class; mix modes (11, 100 + NF, 200 + NF): thread-level "steps" (4 per loop round)
+  const bool mix = mode == 11 || mode >= 100;
+  if (ops_out) *ops_out = (double)grid * 256.0 * (double)iters * (mix ? 4.0 : 32.0);
   return PSGLA_OK;
 }
+

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Same-box A/B of two builds of libpsgla_b200.so (boxes differ by a few per cent, so two gpurun calls cannot be compared):
    python scripts/ab_lib.py libA.so libB.so [rounds] -- scripts/probe.py [args]
-runs the probe alternately with each library (A B A B ...), one process per run, and prints each run's last line."""
+runs the probe alternately with each library (A B A B ...), one process per run, and prints each run's last stdout line."""
 import os, runpy, subprocess, sys
 
 if sys.argv[1] == "--run":
@@ -18,5 +18,7 @@ else:
     for r in range(rounds):
         for name, lib in zip("AB", libs):
             out = subprocess.run([sys.executable, __file__, "--run", lib] + sys.argv[sep + 1:], capture_output=True, text=True)
-            lines = [l for l in (out.stdout + out.stderr).strip().splitlines() if l.strip()]
+            # the probe's result is its last stdout line (bench.py logs to stderr); a run that printed nothing there shows its
+            # last stderr line instead
+            lines = [l for l in out.stdout.splitlines() if l.strip()] or [l for l in out.stderr.splitlines() if l.strip()]
             print("%s %s: %s" % (name, os.path.basename(lib), lines[-1] if lines else "(no output, rc %d)" % out.returncode), flush=True)
