@@ -318,6 +318,25 @@ size_t psgla_mcmc_diag_workspace_bytes(int64_t n_draws, int64_t n_chains);
 int psgla_mcmc_diag(const float* draws_dev, int64_t n_draws, int64_t n_chains, int64_t n_elem, void* ws_dev, size_t ws_bytes,
                     float* rhat_dev, float* ess_bulk_dev, float* ess_tail_dev, void* stream);
 
+/* The same diagnostics for any S up to 2^31 - 1 split draws per element (csrc/mcmc_diag_large.cu): device-wide, with a radix
+ * sort, tie runs, and autocovariances in rounds of doubling lag blocks instead of one element per CTA in shared memory.  For
+ * 2D chain populations (GMMChains.run(n, thin=k) returns [N][M][2]) and long image runs.  Same input, outputs and NaN rules
+ * as psgla_mcmc_diag; results agree with it to rounding (sums run in a different, equally fixed, order).
+ *   n_draws >= 4, n_chains >= 1, 1 <= n_elem <= 2^31 - 1 and S = 2 n_chains floor(n_draws / 2) <= 2^31 - 1, else
+ *   PSGLA_E_BADARG before any CUDA call, the message naming the argument.
+ * Elements are processed in groups of G = min(n_elem, max(1, floor(2^28 / S)), 65 535).  The workspace,
+ * psgla_mcmc_diag_large_workspace_bytes(n_draws, n_chains, n_elem) bytes (0: out of range), 256-byte aligned, is about
+ * 16 bytes per split draw of a group (sort keys and payloads, ping-pong) plus the lag partials (at most S / 16 + one round's
+ * lags doubles per element) and per-chain moments: about 4.6 GB for groups of 2^28 draws, and for one element of S near 2^31
+ * about 36 GB.  On return its first uint64 words hold: the ns (GPU global timer) spent gathering the draws, sorting them
+ * (with the median and quantiles), computing ranks / normal scores and indicators, chain moments, and lag rounds; then the
+ * lag rounds that had an unfinished element and the lag rounds launched, summed over the three ESS series and the groups.
+ * Stream-ordered; the host does not wait.  Deterministic: an element's results do not depend on n_elem, on its group or on
+ * the other elements. */
+size_t psgla_mcmc_diag_large_workspace_bytes(int64_t n_draws, int64_t n_chains, int64_t n_elem);
+int psgla_mcmc_diag_large(const float* draws_dev, int64_t n_draws, int64_t n_chains, int64_t n_elem, void* ws_dev,
+                          size_t ws_bytes, float* rhat_dev, float* ess_bulk_dev, float* ess_tail_dev, void* stream);
+
 /* tcgen05 descriptor self-test (development aid): runs a 128 x 64 x 64 GEMM tile whose A operand starts `row_shift`
  * rows into a 128B-swizzled shared-memory buffer.  mode 0: A from shared memory, shift = descriptor start address;
  * mode 2: A copied to tensor memory.

@@ -123,6 +123,8 @@ SIGNATURES = {
                                   _vp, _vp, _vp]),
     "psgla_mcmc_diag_workspace_bytes": (_sz, [_i64, _i64]),
     "psgla_mcmc_diag": (_int, [_vp, _i64, _i64, _i64, _vp, _sz, _vp, _vp, _vp, _vp]),
+    "psgla_mcmc_diag_large_workspace_bytes": (_sz, [_i64, _i64, _i64]),
+    "psgla_mcmc_diag_large": (_int, [_vp, _i64, _i64, _i64, _vp, _sz, _vp, _vp, _vp, _vp]),
     "psgla_selftest_umma": (_int, [_vp, _vp, _vp, _int, _int, _vp]),
     "psgla_selftest_umma2": (_int, [_vp, _vp, _vp, _int, _vp]),
     "psgla_convg_layer": (_int, [_int, _int, _int, _int, _int, _int, _vp, _vp, _vp, _vp, _vp, _int, _vp]),

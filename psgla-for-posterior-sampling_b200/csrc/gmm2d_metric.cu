@@ -3,30 +3,20 @@
 // k steps" of sampling_2D.py:38-39,65-66 for a population that never leaves HBM).
 //
 //   project   : keys[p][i] = sortable(theta_p . x_i)                       (one read of the state, P coalesced writes)
-//   sort      : per projection, LSD radix sort of the 32-bit keys, 4 passes of 8 bits:
+//   sort      : per projection, LSD radix sort of the 32-bit keys, 4 passes of 8 bits (radix_sort.cuh, keys only):
 //                 histogram (per tile of 4096 keys) -> exclusive scan over [digit][tile] -> stable scatter, in which each
 //                 warp owns a contiguous slice of the tile and ranks equal digits with __match_any_sync
 //   reduce    : sum_p sum_i (sorted_x[p][i] - sorted_ref[p][i])^2 in double -> sqrt(mean)
 // HBM-bound: 4 passes x (2 reads + 1 write) x 4 B per key; at P = 50, n = 10^6 that is 2.4 GB per evaluation.
-#include "common.cuh"
+#include "radix_sort.cuh"
 
 namespace psgla {
 
 constexpr int SW_MAX_PROJ = 128;
-constexpr int SW_TILE = 4096;  // keys per CTA per pass: 8 warps x 16 rounds x 32 lanes
-constexpr int SW_ROUNDS = SW_TILE / 256;
 
 struct Thetas {
   float t[SW_MAX_PROJ][2];
 };
-
-__device__ __forceinline__ uint32_t float_to_key(float f) {
-  const uint32_t u = __float_as_uint(f);
-  return u ^ ((u >> 31) ? 0xFFFFFFFFu : 0x80000000u);
-}
-__device__ __forceinline__ float key_to_float(uint32_t k) {
-  return __uint_as_float(k ^ ((k >> 31) ? 0x80000000u : 0xFFFFFFFFu));
-}
 
 template <typename T>
 __global__ void __launch_bounds__(256)
@@ -35,97 +25,6 @@ sw_project_kernel(const T* __restrict__ x, long long n, int P, Thetas th, uint32
   if (i >= n) return;
   const float x0 = (float)x[2 * i], x1 = (float)x[2 * i + 1];
   for (int p = 0; p < P; ++p) keys[(long long)p * n + i] = float_to_key(fmaf(th.t[p][0], x0, th.t[p][1] * x1));
-}
-
-__global__ void __launch_bounds__(256)
-sw_hist_kernel(const uint32_t* __restrict__ keys, long long n, int shift, int nb, uint32_t* __restrict__ hist) {
-  __shared__ uint32_t h[256];
-  h[threadIdx.x] = 0;
-  __syncthreads();
-  const int p = blockIdx.y;
-  const long long t0 = (long long)blockIdx.x * SW_TILE;
-  const uint32_t* k = keys + (long long)p * n;
-#pragma unroll 4
-  for (int r = 0; r < SW_ROUNDS; ++r) {
-    const long long i = t0 + r * 256 + threadIdx.x;
-    if (i < n) atomicAdd(&h[(k[i] >> shift) & 255u], 1u);
-  }
-  __syncthreads();
-  hist[((long long)p * 256 + threadIdx.x) * nb + blockIdx.x] = h[threadIdx.x];
-}
-
-// exclusive scan of one projection's [256 digits][nb tiles] counts (digit-major = the order keys land in)
-__global__ void __launch_bounds__(1024)
-sw_scan_kernel(uint32_t* __restrict__ hist, int nb) {
-  __shared__ uint32_t part[1024];
-  const long long L = 256LL * nb;
-  uint32_t* h = hist + (long long)blockIdx.x * L;
-  const long long per = (L + 1023) / 1024;
-  const long long a = threadIdx.x * per, b = (a + per < L) ? a + per : L;
-  uint32_t s = 0;
-  for (long long i = a; i < b; ++i) s += h[i];
-  part[threadIdx.x] = s;
-  __syncthreads();
-  for (int off = 1; off < 1024; off <<= 1) {  // Hillis-Steele inclusive scan of the 1024 partial sums
-    const uint32_t v = threadIdx.x >= off ? part[threadIdx.x - off] : 0u;
-    __syncthreads();
-    part[threadIdx.x] += v;
-    __syncthreads();
-  }
-  uint32_t run = part[threadIdx.x] - s;
-  for (long long i = a; i < b; ++i) {
-    const uint32_t c = h[i];
-    h[i] = run;
-    run += c;
-  }
-}
-
-__global__ void __launch_bounds__(256)
-sw_scatter_kernel(const uint32_t* __restrict__ keys_in, uint32_t* __restrict__ keys_out, long long n, int shift, int nb,
-                  const uint32_t* __restrict__ hist) {
-  __shared__ uint32_t wh[8][256];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  for (int j = threadIdx.x; j < 8 * 256; j += 256) (&wh[0][0])[j] = 0;
-  __syncthreads();
-  const int p = blockIdx.y;
-  const uint32_t* kin = keys_in + (long long)p * n;
-  uint32_t* kout = keys_out + (long long)p * n;
-  const long long w0 = (long long)blockIdx.x * SW_TILE + (long long)warp * (SW_TILE / 8);  // this warp's contiguous slice
-  uint32_t mine[SW_ROUNDS];
-#pragma unroll
-  for (int r = 0; r < SW_ROUNDS; ++r) {
-    const long long i = w0 + r * 32 + lane;
-    mine[r] = i < n ? kin[i] : 0u;
-    if (i < n) atomicAdd(&wh[warp][(mine[r] >> shift) & 255u], 1u);
-  }
-  __syncthreads();
-  {  // digit d: global base of this tile, then the warps' slices in order
-    const int d = threadIdx.x;
-    uint32_t run = hist[((long long)p * 256 + d) * nb + blockIdx.x];
-#pragma unroll
-    for (int w = 0; w < 8; ++w) {
-      const uint32_t c = wh[w][d];
-      wh[w][d] = run;
-      run += c;
-    }
-  }
-  __syncthreads();
-#pragma unroll
-  for (int r = 0; r < SW_ROUNDS; ++r) {
-    const long long i = w0 + r * 32 + lane;
-    const bool valid = i < n;
-    const uint32_t d = valid ? ((mine[r] >> shift) & 255u) : 256u;  // invalid lanes form their own group
-    const uint32_t peers = __match_any_sync(0xffffffffu, d);
-    const uint32_t rank = __popc(peers & ((1u << lane) - 1u));
-    uint32_t base = 0;
-    if (valid) base = wh[warp][d];
-    __syncwarp();
-    if (valid) {
-      kout[base + rank] = mine[r];
-      if (rank == 0) wh[warp][d] = base + __popc(peers);
-    }
-    __syncwarp();
-  }
 }
 
 __global__ void __launch_bounds__(256)
@@ -160,7 +59,7 @@ struct SwLayout {
 };
 static SwLayout sw_layout(long long n, int P) {
   SwLayout l;
-  l.nb = (int)((n + SW_TILE - 1) / SW_TILE);
+  l.nb = radix_tiles(n);
   const size_t kb = ((size_t)P * (size_t)n * 4 + 255) & ~(size_t)255;
   l.keys_a = 0;
   l.keys_b = kb;
@@ -191,14 +90,7 @@ static int sw_sorted_keys(const void* x_dev, int precision, long long n, const f
     sw_project_kernel<float><<<gb, 256, 0, st>>>((const float*)x_dev, n, P, th, a);
   else
     sw_project_kernel<double><<<gb, 256, 0, st>>>((const double*)x_dev, n, P, th, a);
-  for (int pass = 0; pass < 4; ++pass) {
-    sw_hist_kernel<<<dim3(l.nb, P), 256, 0, st>>>(a, n, pass * 8, l.nb, hist);
-    sw_scan_kernel<<<P, 1024, 0, st>>>(hist, l.nb);
-    sw_scatter_kernel<<<dim3(l.nb, P), 256, 0, st>>>(a, b, n, pass * 8, l.nb, hist);
-    uint32_t* t = a;
-    a = b;
-    b = t;
-  }
+  radix_sort_segments(a, b, nullptr, nullptr, n, P, hist, st);
   PSGLA_CUDA_TRY(cudaGetLastError());
   *sorted = a;  // after an even number of passes the result is back in the first buffer
   return PSGLA_OK;

@@ -21,7 +21,7 @@
 #include <cmath>
 #include <cstring>
 
-#include "common.cuh"
+#include "mcmc_diag.cuh"
 
 namespace psgla {
 
@@ -29,46 +29,11 @@ constexpr int DG_THREADS = 1024;
 constexpr int DG_WARPS = DG_THREADS / 32;
 constexpr size_t DG_TABLE_OFFSET = 256;  // workspace: stage cycle counters, then the z table
 
-// Wichura's AS241 (PPND16): the standard normal quantile to about 1e-16 relative.
-__device__ double ppnd16(double p) {
-  const double q = p - 0.5;
-  if (fabs(q) <= 0.425) {
-    const double r = 0.180625 - q * q;
-    const double num = (((((((2509.0809287301226727 * r + 33430.575583588128105) * r + 67265.770927008700853) * r +
-                            45921.953931549871457) * r + 13731.693765509461125) * r + 1971.5909503065514427) * r +
-                         133.14166789178437745) * r + 3.387132872796366608);
-    const double den = (((((((5226.495278852545925 * r + 28729.085735721942674) * r + 39307.89580009271061) * r +
-                            21213.794301586595867) * r + 5394.1960214247511077) * r + 687.1870074920579083) * r +
-                         42.313330701600911252) * r + 1.0);
-    return q * num / den;
-  }
-  double r = sqrt(-log(q < 0 ? p : 1.0 - p));
-  double num, den;
-  if (r <= 5.0) {
-    r -= 1.6;
-    num = (((((((7.7454501427834140764e-4 * r + 0.0227238449892691845833) * r + 0.24178072517745061177) * r +
-               1.27045825245236838258) * r + 3.64784832476320460504) * r + 5.7694972214606914055) * r +
-            4.6303378461565452959) * r + 1.42343711074968357734);
-    den = (((((((1.05075007164441684324e-9 * r + 5.475938084995344946e-4) * r + 0.0151986665636164571966) * r +
-               0.14810397642748007459) * r + 0.68976733498510000455) * r + 1.6763848301838038494) * r +
-            2.05319162663775882187) * r + 1.0);
-  } else {
-    r -= 5.0;
-    num = (((((((2.01033439929228813265e-7 * r + 2.71155556874348757815e-5) * r + 0.0012426609473880784386) * r +
-               0.026532189526576123093) * r + 0.29656057182850489123) * r + 1.7848265399172913358) * r +
-            5.4637849111641143699) * r + 6.6579046435011037772);
-    den = (((((((2.04426310338993978564e-15 * r + 1.4215117583164458887e-7) * r + 1.8463183175100546818e-5) * r +
-               7.868691311456132591e-4) * r + 0.0148753612908506148525) * r + 0.13692988092273580531) * r +
-            0.59983220655588793769) * r + 1.0);
-  }
-  return q < 0 ? -num / den : num / den;
-}
-
 // table[k] = Phi^-1((k / 2 - 3/8) / (S + 1/4)), k = 2r for the (half-)integer average rank r in [1, S]
 __global__ void mcmc_z_table_kernel(int S, float* __restrict__ table) {
   const int k = blockIdx.x * blockDim.x + threadIdx.x;
   if (k > 2 * S) return;
-  table[k] = k < 1 ? 0.f : (float)ppnd16((0.5 * k - 0.375) / (S + 0.25));
+  table[k] = k < 1 ? 0.f : rank_z(k, S);
 }
 
 struct DiagShared {
@@ -128,28 +93,6 @@ __device__ __forceinline__ int upper_bound(const float* a, int n, float v) {
   return lo;
 }
 
-// k-th smallest (0-based) of the union of the sorted arrays a[na] and b[nb]
-__device__ double kth_of_union(const float* a, int na, const float* b, int nb, int k) {
-  int lo = max(0, k + 1 - nb), hi = min(k + 1, na);  // i = how many of the k + 1 smallest come from a
-  while (lo < hi) {
-    const int i = (lo + hi) >> 1, j = k + 1 - i;
-    if (j > 0 && i < na && b[j - 1] > a[i]) lo = i + 1; else hi = i;
-  }
-  const int i = lo, j = k + 1 - lo;
-  const double x = i > 0 ? (double)a[i - 1] : -INFINITY, y = j > 0 ? (double)b[j - 1] : -INFINITY;
-  return fmax(x, y);
-}
-
-// numpy's quantile, method "linear": virtual index (n - 1) q, then numpy's _lerp
-__device__ double quantile_linear(const float* a, int na, const float* b, int nb, double q) {
-  const double h = (double)(na + nb - 1) * q, f = floor(h), t = h - f;
-  const int k = (int)f;
-  const double lo = kth_of_union(a, na, b, nb, k);
-  const double hi = k + 1 < na + nb ? kth_of_union(a, na, b, nb, k + 1) : lo;
-  const double d = hi - lo;
-  return t >= 0.5 ? hi - d * (1.0 - t) : lo + d * t;
-}
-
 // chain index of flat position j of a chain-major [n_chains][n] array, without an integer division
 __device__ __forceinline__ int chain_of(int j, int n, float inv_n) {
   int c = (int)((float)j * inv_n);
@@ -207,23 +150,16 @@ __device__ SeriesStats series_stats(float* ser, int Mp, int n, bool want_ess, Di
   };
   double a1, a2, a3;
   acov3(1, a1, a2, a3);
-  // Geyer's initial positive sequence P_k = rho_2k + rho_2k+1 (rho_0 = 1) made monotone by a running minimum; the loop and
-  // the term added after it are arviz's _ess step for step.  a2 / a3 of the first pass serve the first pair.
-  double even = 1.0, odd = 1.0 - (W - a1) / vp;
-  double p_adj = even + odd, sum_p = 0.0;
-  for (int t = 1; t < n - 3 && even + odd > 0.0; t += 2) {
-    sum_p += p_adj;
-    if (t > 1) {
+  // Geyer's initial positive / monotone sequence (mcmc_diag.cuh); a2 / a3 of the first pass serve the first pair.
+  Geyer g = geyer_start(W, vp, a1);
+  while (geyer_running(g, n)) {
+    if (g.t > 1) {
       double unused;
-      acov3(t + 1, a2, a3, unused);
+      acov3(g.t + 1, a2, a3, unused);
     }
-    even = 1.0 - (W - a2) / vp;
-    odd = 1.0 - (W - a3) / vp;
-    p_adj = fmin(even + odd, p_adj);
+    geyer_step(g, a2, a3);
   }
-  const double last = (even > 0.0 || even + odd >= 0.0) ? even : 0.0;
-  const double tau = fmax(-1.0 + 2.0 * sum_p + last, 1.0 / log10((double)S));
-  r.ess = S / tau;
+  r.ess = geyer_ess(g, S);
   return r;
 }
 

@@ -5,8 +5,13 @@
     d["rhat"], d["ess_bulk"], d["ess_tail"]                  # [C, H, W] maps
     d["rhat_max"], d["frac_rhat_above_1_01"], d["ess_bulk_min"], d["ess_bulk_median"], d["ess_tail_min"]
 
-The kernel (csrc/mcmc_diag.cu) reads the draws where the sampler stored them, [N][M][C][H][W]: a run object is diagnosed in
-place, with no copy.  Limit: S = 2 M floor(N / 2) <= PSGLA_MCMC_MAX_DRAWS = 16 384 split draws per element.
+    d = psgla_b200.mcmc_diagnostics_large(traj, burn_in=b)  # traj = GMMChains.run(n, thin=k): [N, M, 2]
+
+The kernels (csrc/mcmc_diag.cu, csrc/mcmc_diag_large.cu) read the draws where the sampler stored them, [N][M][C][H][W]: a run
+object is diagnosed in place, with no copy.  mcmc_diagnostics sorts one element in shared memory: S = 2 M floor(N / 2) <=
+PSGLA_MCMC_MAX_DRAWS = 16 384 split draws per element.  mcmc_diagnostics_large computes the same statistics device-wide for
+S up to 2^31 - 1 (a 2D population of 10^6 chains x 2 000 draws, an image run with the reference's own thinning), with a
+workspace of about 16 bytes per split draw of a group of elements.
 """
 from __future__ import annotations
 
@@ -16,9 +21,10 @@ import torch
 
 from . import _lib
 
-__all__ = ["mcmc_diagnostics", "MAX_DRAWS"]
+__all__ = ["mcmc_diagnostics", "mcmc_diagnostics_large", "MAX_DRAWS", "MAX_DRAWS_LARGE"]
 
 MAX_DRAWS = 16384  # PSGLA_MCMC_MAX_DRAWS
+MAX_DRAWS_LARGE = 2 ** 31 - 1  # psgla_mcmc_diag_large
 
 
 def _as_draws(draws):
@@ -65,19 +71,8 @@ def _check_tensor(t):
         raise TypeError("draws must be float32 (the samplers' dtype), got %s" % t.dtype)
 
 
-def mcmc_diagnostics(draws, *, burn_in: int = 0) -> dict:
-    """Rank-normalised split-R-hat and bulk / tail ESS of every element of a multi-chain run.
-
-    draws: a CUDA fp32 tensor [N, M, C, H, W] or [N, M, E] (N stored draws of M chains); a sampler's ``Xlist`` (entries
-    [M, C, H, W], or the squeezed single-chain [C, H, W] / [H, W], taken as M = 1); or a ``psgla_run`` / ``pnpula_run`` object,
-    read in place from its sample buffer (the slots written so far).  A DRUNet run padded to multiples of 8 is diagnosed at the
-    padded size and the maps are cropped like its outputs.  burn_in: the first ``burn_in`` draws are dropped.
-
-    Returns a dict: ``rhat``, ``ess_bulk``, ``ess_tail`` -- CUDA fp32 maps [C, H, W] (an [N, M, E] tensor gives [E]) --, and
-    the floats ``rhat_max``, ``frac_rhat_above_1_01``, ``ess_bulk_min``, ``ess_bulk_median``, ``ess_tail_min`` over the
-    elements whose statistic is not NaN (NaN: NaN draws, or an element constant within every split chain; the fraction counts
-    NaN as not above; the median is torch's, the lower middle value for an even count), and the ints ``n_draws``,
-    ``n_chains``.  Stream-ordered on the current stream; reading the scalars synchronises it."""
+def _prepare(draws, burn_in):
+    """-> (contiguous fp32 [N, M, ...] CUDA tensor after burn-in, N, M, E, map shape, crop); the checks both paths share."""
     x, map_shape, crop = _as_draws(draws)
     burn_in = int(burn_in)
     if burn_in < 0 or burn_in >= x.shape[0]:
@@ -86,20 +81,18 @@ def mcmc_diagnostics(draws, *, burn_in: int = 0) -> dict:
     if not x.is_contiguous():
         x = x.contiguous()
     N, M = int(x.shape[0]), int(x.shape[1])
-    E = x[0, 0].numel()
-    S = 2 * M * (N // 2)
     if N < 4:
         raise ValueError("split chains need at least 4 draws after burn-in, got %d" % N)
-    if S > MAX_DRAWS:
-        raise ValueError("%d chains x %d draws give S = %d split draws per element, above the limit of %d: store fewer draws "
-                         "(thin more with a larger n_inter), raise burn_in, or diagnose fewer chains" % (M, N, S, MAX_DRAWS))
-    lib = _lib.lib()
+    return x, N, M, x[0, 0].numel(), map_shape, crop
+
+
+def _run(fn, ws_bytes, x, N, M, E, map_shape, crop, name):
+    """Calls the C-ABI diagnostics ``fn`` and builds the result dict from its [3, E] output."""
     with torch.cuda.device(x.device):
-        ws_bytes = lib.psgla_mcmc_diag_workspace_bytes(N, M)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
         out = torch.empty((3, E), dtype=torch.float32, device=x.device)
-        _lib.check(lib.psgla_mcmc_diag(_lib.ptr(x), N, M, E, _lib.ptr(ws), C.c_size_t(ws_bytes), out[0].data_ptr(),
-                                       out[1].data_ptr(), out[2].data_ptr(), _lib.stream_ptr(x.device)), "psgla_mcmc_diag")
+        _lib.check(fn(_lib.ptr(x), N, M, E, _lib.ptr(ws), C.c_size_t(ws_bytes), out[0].data_ptr(), out[1].data_ptr(),
+                      out[2].data_ptr(), _lib.stream_ptr(x.device)), name)
     maps = out.reshape((3,) + map_shape)
     if crop is not None:
         maps = maps[..., :crop[0], :crop[1]]
@@ -120,3 +113,46 @@ def mcmc_diagnostics(draws, *, burn_in: int = 0) -> dict:
         "ess_tail_min": float(t.min()) if t.numel() else nan,
         "n_draws": N, "n_chains": M,
     }
+
+
+def mcmc_diagnostics(draws, *, burn_in: int = 0) -> dict:
+    """Rank-normalised split-R-hat and bulk / tail ESS of every element of a multi-chain run.
+
+    draws: a CUDA fp32 tensor [N, M, C, H, W] or [N, M, E] (N stored draws of M chains); a sampler's ``Xlist`` (entries
+    [M, C, H, W], or the squeezed single-chain [C, H, W] / [H, W], taken as M = 1); or a ``psgla_run`` / ``pnpula_run`` object,
+    read in place from its sample buffer (the slots written so far).  A DRUNet run padded to multiples of 8 is diagnosed at the
+    padded size and the maps are cropped like its outputs.  burn_in: the first ``burn_in`` draws are dropped.
+
+    Returns a dict: ``rhat``, ``ess_bulk``, ``ess_tail`` -- CUDA fp32 maps [C, H, W] (an [N, M, E] tensor gives [E]) --, and
+    the floats ``rhat_max``, ``frac_rhat_above_1_01``, ``ess_bulk_min``, ``ess_bulk_median``, ``ess_tail_min`` over the
+    elements whose statistic is not NaN (NaN: NaN draws, or an element constant within every split chain; the fraction counts
+    NaN as not above; the median is torch's, the lower middle value for an even count), and the ints ``n_draws``,
+    ``n_chains``.  Stream-ordered on the current stream; reading the scalars synchronises it.  Up to 16 384 split draws per
+    element; mcmc_diagnostics_large takes more."""
+    x, N, M, E, map_shape, crop = _prepare(draws, burn_in)
+    S = 2 * M * (N // 2)
+    if S > MAX_DRAWS:
+        raise ValueError("%d chains x %d draws give S = %d split draws per element, above the limit of %d: store fewer draws "
+                         "(thin more with a larger n_inter), raise burn_in, diagnose fewer chains, or use "
+                         "mcmc_diagnostics_large" % (M, N, S, MAX_DRAWS))
+    lib = _lib.lib()
+    return _run(lib.psgla_mcmc_diag, lib.psgla_mcmc_diag_workspace_bytes(N, M), x, N, M, E, map_shape, crop,
+                "psgla_mcmc_diag")
+
+
+def mcmc_diagnostics_large(draws, *, burn_in: int = 0) -> dict:
+    """mcmc_diagnostics for up to 2^31 - 1 split draws per element (csrc/mcmc_diag_large.cu): the same inputs, definitions and
+    result dict, computed device-wide (radix sort, tie runs, autocovariances in rounds of lags) instead of in one CTA's shared
+    memory.  The 2D trajectory of ``GMMChains.run(n, thin=k)`` ([N, M, 2] fp32) is taken as it is:
+
+        d = psgla_b200.mcmc_diagnostics_large(chains.run(n_steps, thin=k), burn_in=b)   # rhat, ess_bulk, ess_tail: [2]
+
+    The workspace is allocated per call: about 16 bytes per split draw of a group of min(E, 2^28 / S) elements."""
+    x, N, M, E, map_shape, crop = _prepare(draws, burn_in)
+    S = 2 * M * (N // 2)
+    if S > MAX_DRAWS_LARGE:
+        raise ValueError("%d chains x %d draws give S = %d split draws per element, above the limit of 2^31 - 1: thin more, "
+                         "raise burn_in or diagnose fewer chains" % (M, N, S))
+    lib = _lib.lib()
+    return _run(lib.psgla_mcmc_diag_large, lib.psgla_mcmc_diag_large_workspace_bytes(N, M, E), x, N, M, E, map_shape, crop,
+                "psgla_mcmc_diag_large")

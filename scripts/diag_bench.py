@@ -20,7 +20,26 @@ own PnP-ULA thinning would store 10 000, above the diagnostic's limit).  Window 
 they are not measured and the table's 10 would hold 9 090 windows of PnP-ULA's 8 chains).  The DnCNN weights are the
 library's seeded Lipschitz stand-in (lipschitz_dncnn_state_dict(0)), not the reference's checkpoint: the ESS figures
 describe that network's chains.  Reported: sampling wall clock (host clock around the loop, ending in a synchronise), the
-diagnostics after dropping the first 100 stored draws (10 %), and min / median bulk ESS per second of sampling."""
+diagnostics after dropping the first 100 stored draws (10 %), and min / median bulk ESS per second of sampling.
+
+The device-wide path for any S (psgla_mcmc_diag_large, csrc/mcmc_diag_large.cu), under "large":
+  ms, stage_fraction  CUDA events around the call; the call's own GPU-timer split (workspace head): gather / sort (with median
+                      and quantiles) / ranks, normal scores and indicators / chain moments / lag rounds; lag_rounds_run (rounds
+                      with an unfinished element, summed over the three ESS series and the element groups) and launched
+  sort_gb             bytes the radix sort moves: gather (4 read + 8 written), 4 passes x (4 histogram + 8 read + 8 written),
+                      the in-place key conversion (8), per split draw
+  series_gb           bytes the series passes move: 4 series x (ranks or indicators: 4 + 4 read, 4 written; moments: 4 + 4
+                      read, 4 written) per split draw, plus 8 per split draw per lag round run (the series and its lagged
+                      copy), counting every element of a group as unfinished (an upper bound)
+  hbm_fraction        (sort_gb + series_gb) over the measured copy bandwidth, divided by ms
+Cases: (a) one PSGLA and one PnP-ULA cell of BASELINE.json configs[1] (prior symetric_gaussians, y = (0, 0), the GMM_ALGS
+constants of bench.py), 10^6 chains, fp32, Philox noise, 10^4 steps thinned by 10 (1 000 stored draws), the first 200 stored
+draws (2 000 steps) dropped as burn-in: R-hat and bulk / tail ESS per coordinate, and ESS per second against the device time
+of the same 10^4 steps on the throughput path (no trajectory) and of the trajectory-writing run; (b) image PnP-ULA with the
+table's own thinning, n_inter = 10: 10^4 stored draws x 8 chains x 256 x 256 x 3 (a 63 GB sample buffer), S = 72 000 after
+dropping 1 000 stored draws; (c) the synthetic 8 chains x 1 000 draws x 256 x 256 x 3 case through both paths.
+
+    python scripts/diag_bench.py --large-only   # cases (a) - (c) only"""
 import argparse
 import ctypes as C
 import json
@@ -105,6 +124,109 @@ def time_diag(x, reps, copy_gbs):
                 rhat_max=float(out[0][~out[0].isnan()].max()), ess_bulk_median=float(out[1][~out[1].isnan()].median()))
 
 
+def time_diag_large(x, reps, copy_gbs):
+    """x: CUDA fp32 [N, M, E] (contiguous).  psgla_mcmc_diag_large, timed with CUDA events."""
+    N, M, E = x.shape
+    lib = P._lib.lib()
+    ws_bytes = lib.psgla_mcmc_diag_large_workspace_bytes(N, M, E)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
+    out = torch.empty((3, E), dtype=torch.float32, device=x.device)
+    st = P._lib.stream_ptr(x.device)
+
+    def call():
+        P._lib.check(lib.psgla_mcmc_diag_large(x.data_ptr(), N, M, E, ws.data_ptr(), C.c_size_t(ws_bytes), out[0].data_ptr(),
+                                               out[1].data_ptr(), out[2].data_ptr(), st), "psgla_mcmc_diag_large")
+
+    call()
+    ms = []
+    for _ in range(reps):
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        call()
+        e1.record()
+        e1.synchronize()
+        ms.append(e0.elapsed_time(e1))
+    head = ws[:64].cpu().view(torch.int64).tolist()
+    stage = head[:5]
+    t = sorted(ms)[len(ms) // 2]
+    S = 2 * M * (N // 2)
+    groups = -(-E // max(1, min(E, max(1, (1 << 28) // S), 65535)))
+    draws = S * E
+    sort_b = draws * (12 + 4 * 20 + 8)
+    series_b = draws * 4 * 24 + head[5] * 8 * draws / groups
+    r, b, tl = out[0], out[1], out[2]
+    fin = lambda v: v[~v.isnan()]  # noqa: E731
+    return dict(n_draws=N, n_chains=M, n_elem=E, S=S, workspace_gb=ws_bytes / 1e9, ms=t, ms_all=ms,
+                sort_gb=sort_b / 1e9, series_gb=series_b / 1e9,
+                hbm_fraction=(sort_b + series_b) / (copy_gbs * 1e9) / (t * 1e-3),
+                stage_fraction=dict(zip(("gather", "sort", "rank", "moments", "lag_rounds"), (v / sum(stage) for v in stage))),
+                lag_rounds_run=head[5], lag_rounds_launched=head[6],
+                rhat_max=float(fin(r).max()) if fin(r).numel() else None,
+                ess_bulk_median=float(fin(b).median()) if fin(b).numel() else None,
+                ess_tail_min=float(fin(tl).min()) if fin(tl).numel() else None), out
+
+
+def gmm_cell(alg, dev, reps, copy_gbs, n_chains=10 ** 6, n_steps=10 ** 4, thin=10, burn=200):
+    """Case (a): one cell of configs[1] as bench.py sets it up; trajectory diagnosed with psgla_mcmc_diag_large."""
+    import numpy as np
+    prm = dict(psgla=dict(delta=0.3, alpha=2.0 / 3.0, epsilon=1.0), pnp_ula=dict(delta=0.1, alpha=1.5, epsilon=0.5))[alg]
+    mu, Sig, pi = P.gaussian_mixt_example("symetric_gaussians")
+    y = (0.0, 0.0)
+    x0 = torch.tensor(y, dtype=torch.float32, device=dev).repeat(n_chains, 1).contiguous()
+    ch = P.GMMChains(alg, np.array(y), prm["delta"], np.eye(2), 1.0, P.Theorical_MMSE(mu, Sig, pi), prm["alpha"],
+                     prm["epsilon"], n_chains=n_chains, x0=x0, seed=0, dtype="float32", device=dev)
+
+    def timed(thin_):
+        ch.state.copy_(x0)
+        ch.step = 0
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        tr = ch.run(n_steps, thin=thin_)
+        e1.record()
+        e1.synchronize()
+        return e0.elapsed_time(e1) * 1e-3, tr
+
+    timed(0)  # warm-up
+    s_plain = min(timed(0)[0] for _ in range(3))
+    s_traj, traj = timed(thin)
+    timing, out = time_diag_large(traj[burn:].contiguous(), reps, copy_gbs)
+    ess_b, ess_t = out[1].tolist(), out[2].tolist()
+    return dict(case="(a) 2D %s cell, %d chains x %d steps, thin %d, burn-in %d stored draws" % (alg, n_chains, n_steps, thin, burn),
+                alg=alg, steps_s_throughput_path=s_plain, steps_s_trajectory_run=s_traj, rhat=out[0].tolist(), ess_bulk=ess_b,
+                ess_tail=ess_t, ess_bulk_per_s_throughput=[v / s_plain for v in ess_b],
+                ess_bulk_per_s_trajectory=[v / s_traj for v in ess_b], ess_tail_per_s_throughput=[v / s_plain for v in ess_t],
+                **timing)
+
+
+def pnpula_table_thinning(dev, reps, copy_gbs):
+    """Case (b): image PnP-ULA with the table's n_inter = 10 (10^4 stored draws x 8 chains)."""
+    im = P.load_image(os.path.join(ROOT, "tests", "golden", "set3c", "butterfly.png"), device=dev)
+    dg, init, _, _ = P.make_inpainting(im, prop=0.5, sigma=1.0, seed_ip=0)
+    den = P.DnCNN(pretrained=P.lipschitz_dncnn_state_dict(0), device=dev)
+    prm = P.sampler_params("pnp_ula", den="DnCNN")
+    run = P.pnpula_run(init, dg, P.PriorGrad(den, prm["alpha"], prm["s1"], prm["s2"]),
+                       **dict(P.as_pnpula_kwargs(prm, seed=0), n_inter=10, n_inter_mmse=1000), n_chains=8)
+    run.step(0)
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    for i in range(1, run.n_iter):
+        run.step(i)
+    torch.cuda.synchronize()
+    wall = (time.perf_counter() - t0) * run.n_iter / (run.n_iter - 1)
+    run.finish()
+    n = len(run.Xlist)
+    burn = n // 10
+    s = run.samples[burn:n]
+    timing, _ = time_diag_large(s.reshape(s.shape[0], s.shape[1], -1), reps, copy_gbs)
+    d = P.mcmc_diagnostics_large(run, burn_in=burn)
+    del run, s
+    return dict(case="(b) image PnP-ULA, n_inter = 10: %d stored draws x 8 chains x 256x256x3, burn-in %d" % (n, burn),
+                n_iter=prm["N"], sampling_s=wall,
+                **{k: d[k] for k in ("rhat_max", "frac_rhat_above_1_01", "ess_bulk_min", "ess_bulk_median", "ess_tail_min")},
+                ess_bulk_min_per_s=d["ess_bulk_min"] / wall, ess_bulk_median_per_s=d["ess_bulk_median"] / wall,
+                timing=timing)
+
+
 def run_sampler(alg, dev):
     im = P.load_image(os.path.join(ROOT, "tests", "golden", "set3c", "butterfly.png"), device=dev)
     dg, init, _, _ = P.make_inpainting(im, prop=0.5, sigma=1.0, seed_ip=0)
@@ -138,6 +260,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--large-only", action="store_true", help="cases (a) - (c) of the large-S path only")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("diag_bench.py needs a CUDA device")
@@ -146,7 +269,27 @@ def main():
     copy_gbs = copy_bandwidth_gbs(dev)
     res = dict(kind="mcmc_diag", device=torch.cuda.get_device_name(dev), power_limit_w=power_limit(),
                copy_bandwidth_gbs=copy_gbs, weights="lipschitz_dncnn_state_dict(0) (seeded stand-in, not the reference's "
-               "checkpoint)", diag=[], samplers=[])
+               "checkpoint)", diag=[], samplers=[], large=[])
+    x = ar1(1000, 8, 256 * 256 * 3, 0.5, dev, 0)
+    case = "(c) 8 chains x 1000 draws x 256x256x3, synthetic AR(1) rho 0.5"
+    small = time_diag(x, args.reps, copy_gbs)
+    large, out = time_diag_large(x, args.reps, copy_gbs)
+    ref = P.mcmc_diagnostics(x)
+    large["max_abs_diff_vs_small_path"] = {k: float((out[i] - ref[k]).abs().nan_to_num(0).max())
+                                           for i, k in enumerate(("rhat", "ess_bulk", "ess_tail"))}
+    res["large"].append(dict(case=case, small_path=small, **large))
+    print(json.dumps(res["large"][-1]), flush=True)
+    del x, out, ref
+    torch.cuda.empty_cache()
+    for alg in ("psgla", "pnp_ula"):
+        res["large"].append(gmm_cell(alg, dev, args.reps, copy_gbs))
+        print(json.dumps(res["large"][-1]), flush=True)
+        torch.cuda.empty_cache()
+    res["large"].append(pnpula_table_thinning(dev, args.reps, copy_gbs))
+    print(json.dumps(res["large"][-1]), flush=True)
+    torch.cuda.empty_cache()
+    if args.large_only:
+        return finish(res, args)
     x = ar1(1000, 8, 256 * 256 * 3, 0.5, dev, 0)
     res["diag"].append(dict(case="8 chains x 1000 draws x 256x256x3, synthetic AR(1) rho 0.5", **time_diag(x, args.reps, copy_gbs)))
     del x
@@ -163,6 +306,10 @@ def main():
                                 **time_diag(s.reshape(s.shape[0], s.shape[1], -1), args.reps, copy_gbs)))
         del run, s
         torch.cuda.empty_cache()
+    finish(res, args)
+
+
+def finish(res, args):
     line = json.dumps(res, indent=1)
     print(line)
     if args.out:
