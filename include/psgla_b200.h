@@ -441,7 +441,8 @@ int psgla_selftest_fp32_rate(int mode, int iters, int blocks_per_sm, float* out_
  * IMAD.HI.U32, 2 IMAD, 3 LOP3, 4 MUFU.EX2, 5 I2FP, 6 FFMA, 7 MUFU.SIN, 8 IMAD.WIDE + FFMA 1:1, 9 MUFU + IMAD.WIDE 1:1, 10 MUFU + 4
  * FFMA, 11 and 100 + NF (NF = 21, 23, 26, 28, 30): the chain kernel's whole per-step instruction mix with NF FP32 instructions as
  * independent chains, 12 DFMA.RM, 13 IMAD + DFMA.RM + LOP3, 14 DFMA.RM + FFMA 1:1, 200 + NF: the mix with the Philox round
- * products' high words as DFMA.RM on the FP64 pipe); *ops_out = thread-level instructions of the probed class the launch executes (modes 8-10: of the
+ * products' high words as DFMA.RM on the FP64 pipe, 300 + NF: the mix of the chain kernel that reads Philox's launch-uniform
+ * round-2 words from its parameters: 8 IMAD.WIDE.U32 and 9 LOP3 per step); *ops_out = thread-level instructions of the probed class the launch executes (modes 8-10: of the
  * first-named class; mix modes: thread-level "steps"). */
 int psgla_selftest_pipe_rate(int mode, int iters, int blocks_per_sm, void* out_dev, double* ops_out, void* stream);
 

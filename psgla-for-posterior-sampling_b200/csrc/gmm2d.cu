@@ -30,6 +30,18 @@ constexpr int RMAX = PSGLA_GMM_MAX_COMPONENTS;
 // gmm2d_lean_kernel's geometry: 4 Philox counter blocks (8 steps) per round, 64-thread blocks, 16 of them resident per SM.
 constexpr int LEAN_NB = 4, LEAN_BLOCK = 64, LEAN_MINB = 16;
 
+// Philox's launch-uniform words of gmm2d_lean_kernel's counter blocks after round 2 (see the kernel), one entry per round:
+// component b of each vector belongs to counter pair pair0 + r LEAN_NB + b.  Passed BY VALUE as a kernel parameter, so each
+// launch (and each stream: several cells may run at once) carries its own table, read through the uniform datapath.  12 B per
+// counter pair; kernel parameters may take 32 764 B, of which the kernel's other parameters take less than 256.
+struct LeanPairWords {
+  struct Round {
+    uint4 ua, ub, uc;
+  } r[(32764 - 256) / (3 * 16)];  // 677 rounds (5 416 steps) per launch
+};
+constexpr int LEAN_TAB_ROUNDS = sizeof(LeanPairWords) / sizeof(LeanPairWords::Round);
+static_assert(LEAN_NB == 4, "one uint4 per LEAN_NB counter pairs");
+
 template <typename T>
 struct Gmm2dConsts {
   T P[4], q[2];
@@ -355,36 +367,36 @@ static int constants_structure(const Gmm2dConsts<float>& c) {
 // same arithmetic per chain as gmm2d_kernel: bit-identical results.
 template <int ALG, int STRUCT>
 __global__ void __launch_bounds__(LEAN_BLOCK, LEAN_MINB)
-gmm2d_lean_kernel(const Gmm2dConsts<float> c, float2* __restrict__ x, unsigned n_launch, unsigned long long sub0,
-                  unsigned long long pair0, int n_rounds, const PhiloxKeys keys) {
+gmm2d_lean_kernel(const Gmm2dConsts<float> c, float2* __restrict__ x, unsigned n_launch, uint32_t sub0_lo, uint32_t pair0_hi,
+                  int n_rounds, const PhiloxKeys keys, const LeanPairWords tab) {
   static_assert(LEAN_NB % 2 == 0, "Box-Muller packs counter blocks in pairs");
   const unsigned g = blockIdx.x * LEAN_BLOCK + threadIdx.x;
   if (g >= n_launch) return;
   float2 v = x[g];
   float x0 = v.x, x1 = v.y;
-  // The launch's chain ids share their high word, and so do its counter pairs (launch_lean_body splits where they would not),
-  // so Philox's counter words c1 = pair >> 32 and c3 = chain id >> 32 are launch constants and its first two rounds are
-  // mostly thread constants (T) and launch-uniform values (U):
-  //   round 1: c0' = hi(M1 s_lo) ^ c1 ^ k0 (T), c1' = lo(M1 s_lo) (T), c2' = hi(M0 pair) ^ c3 ^ k1 (U), c3' = lo(M0 pair) (U)
+  // The launch's chain ids share their high word s_hi, and so do its counter pairs (launch_lean_body splits where they would
+  // not), so Philox's counter words c1 = pair >> 32 and c3 = s_hi are launch constants and its first two rounds are thread
+  // constants (T) and values that depend only on the counter pair and the launch (U):
+  //   round 1: c0' = hi(M1 s_lo) ^ c1 ^ k0 (T), c1' = lo(M1 s_lo) (T), c2' = hi(M0 pair) ^ s_hi ^ k1 (U), c3' = lo(M0 pair) (U)
   //   round 2: M0 c0' (T) and M1 c2' (U)
-  // so per thread and per counter block rounds 1-2 cost one IMAD.WIDE.U32 instead of two (ptxas puts the round-1 U product on
-  // the uniform datapath but keeps the round-2 one on the vector pipe): 17 per block instead of 18.  Same words as
-  // philox4x32_10_keyed from round 0, i.e. bit-identical draws.
-  const uint32_t s_lo = (uint32_t)sub0 + g, s_hi = (uint32_t)(sub0 >> 32), p_hi = (uint32_t)(pair0 >> 32);
+  // The host computes the U words after round 2 (ua = hi(M1 c2') ^ k2, ub = lo(M1 c2'), uc = c3' ^ k3) into `tab`, so per
+  // thread and per counter block rounds 1-2 cost no IMAD.WIDE.U32 and two LOP3: 16 per block, the floor for rounds 3-10.  Same
+  // words as philox4x32_10_keyed from round 0, i.e. bit-identical draws.
+  const uint32_t s_lo = sub0_lo + g;
   const uint64_t t1 = (uint64_t)0xCD9E8D57u * s_lo;               // round 1, chain word
   const uint32_t t1_lo = (uint32_t)t1;
-  const uint64_t t2 = (uint64_t)0xD2511F53u * ((uint32_t)(t1 >> 32) ^ p_hi ^ keys.k[0]);  // round 2, first product
+  const uint64_t t2 = (uint64_t)0xD2511F53u * ((uint32_t)(t1 >> 32) ^ pair0_hi ^ keys.k[0]);  // round 2, first product
   const uint32_t t2_hi = (uint32_t)(t2 >> 32), t2_lo = (uint32_t)t2;
   for (int r = 0; r < n_rounds; ++r) {
-    uint32_t w[LEAN_NB][4];  // Philox4x32-10 of counter blocks pair .. pair + LEAN_NB - 1
+    const uint4 ua = tab.r[r].ua, ub = tab.r[r].ub, uc = tab.r[r].uc;
+    const uint32_t wa[LEAN_NB] = {ua.x, ua.y, ua.z, ua.w}, wb[LEAN_NB] = {ub.x, ub.y, ub.z, ub.w},
+                   wc[LEAN_NB] = {uc.x, uc.y, uc.z, uc.w};
+    uint32_t w[LEAN_NB][4];  // Philox4x32-10 of counter blocks pair0 + r LEAN_NB .. + LEAN_NB - 1
 #pragma unroll
     for (int b = 0; b < LEAN_NB; ++b) {
-      const uint32_t pr = (uint32_t)pair0 + (uint32_t)(r * LEAN_NB + b);
-      const uint64_t u1 = (uint64_t)0xD2511F53u * pr;                                         // round 1, pair word
-      const uint64_t u2 = (uint64_t)0xCD9E8D57u * ((uint32_t)(u1 >> 32) ^ s_hi ^ keys.k[1]);  // round 2, second product
-      w[b][0] = (uint32_t)(u2 >> 32) ^ t1_lo ^ keys.k[2];
-      w[b][1] = (uint32_t)u2;
-      w[b][2] = t2_hi ^ (uint32_t)u1 ^ keys.k[3];
+      w[b][0] = wa[b] ^ t1_lo;
+      w[b][1] = wb[b];
+      w[b][2] = t2_hi ^ wc[b];
       w[b][3] = t2_lo;
       philox4x32_10_keyed<2>(w[b][0], w[b][1], w[b][2], w[b][3], keys);
     }
@@ -578,8 +590,9 @@ static int upload_components(const Gmm2dComponents<T>& k, cudaStream_t st, Gmm2d
 // Launch policy.  The kernel is issue-bound and its warps do identical work, but the SM's warp arbiter is not fair: of the
 // warps resident on a scheduler some finish long before others (ncu: 5.4 of 8 warps active on average over a launch whose
 // grid is exactly one resident wave), and what they leave behind is an under-filled tail.  So the fp32, r == 2 Philox path,
-// the throughput path, is ONE launch of small blocks, many more blocks than fit: the hardware block scheduler back-fills
-// every slot a finished warp frees, so all SMs stay full until the population is exhausted and the tail is one short block.
+// the throughput path, runs all its chains in each launch (one per LEAN_TAB_ROUNDS rounds, launch_lean_body) as small blocks,
+// many more blocks than fit: the hardware block scheduler back-fills every slot a finished warp frees, so all SMs stay full
+// until the population is exhausted and the tail is one short block.
 // The other paths (fp64, replay, r != 2: parity paths, not throughput paths) keep the round-1 policy: occupancy-sized waves.
 struct Launch {  // everything a launch needs besides its chain range
   const void* c;
@@ -636,22 +649,43 @@ static int launch_waves(const Launch& a, int* launches) {
   return PSGLA_OK;
 }
 
+// Philox words of a counter block after round 2 that depend only on the counter pair and the chain id's high word (the U
+// words of gmm2d_lean_kernel), with the kernel's arithmetic.
+static void lean_pair_words(const PhiloxKeys& keys, uint32_t pair_lo, uint32_t sub_hi, uint32_t* ua, uint32_t* ub,
+                            uint32_t* uc) {
+  const uint64_t u1 = (uint64_t)0xD2511F53u * pair_lo;                                      // round 1, pair word
+  const uint64_t u2 = (uint64_t)0xCD9E8D57u * ((uint32_t)(u1 >> 32) ^ sub_hi ^ keys.k[1]);  // round 2, second product
+  *ua = (uint32_t)(u2 >> 32) ^ keys.k[2];
+  *ub = (uint32_t)u2;
+  *uc = (uint32_t)u1 ^ keys.k[3];
+}
+
 template <int ALG, int STRUCT>
 static void launch_lean(const Launch& a, long long lo, long long n, long long n_rounds, unsigned long long pair0) {
+  static thread_local LeanPairWords tab;  // copied into the launch's parameters at the launch
+  const unsigned long long sub0 = a.chain_id0 + (unsigned long long)lo;
+  for (long long r = 0; r < n_rounds; ++r) {
+    uint32_t ua[LEAN_NB], ub[LEAN_NB], uc[LEAN_NB];
+    for (int b = 0; b < LEAN_NB; ++b)
+      lean_pair_words(a.keys, (uint32_t)pair0 + (uint32_t)(r * LEAN_NB + b), (uint32_t)(sub0 >> 32), &ua[b], &ub[b], &uc[b]);
+    tab.r[r] = {{ua[0], ua[1], ua[2], ua[3]}, {ub[0], ub[1], ub[2], ub[3]}, {uc[0], uc[1], uc[2], uc[3]}};
+  }
   gmm2d_lean_kernel<ALG, STRUCT><<<(unsigned)((n + LEAN_BLOCK - 1) / LEAN_BLOCK), LEAN_BLOCK, 0, a.st>>>(
-      *(const Gmm2dConsts<float>*)a.c, (float2*)a.x + lo, (unsigned)n, a.chain_id0 + (unsigned long long)lo, pair0,
-      (int)n_rounds, a.keys);
+      *(const Gmm2dConsts<float>*)a.c, (float2*)a.x + lo, (unsigned)n, (uint32_t)sub0, (uint32_t)(pair0 >> 32), (int)n_rounds,
+      a.keys, tab);
 }
 
 // The lean kernel on chains [lo, lo + n) (one high word of the chain id) for `rounds` rounds from counter pair pair0, in
-// launches within which the pair's high word does not change either (gmm2d_lean_kernel takes both as launch constants).  A
-// round whose LEAN_NB pairs straddle a multiple of 2^32 goes to the general kernel.  Returns the number of launches.
+// launches within which the pair's high word does not change either (gmm2d_lean_kernel takes both as launch constants) and
+// of at most LEAN_TAB_ROUNDS rounds (what its table of pair words holds).  A round whose LEAN_NB pairs straddle a multiple of
+// 2^32 goes to the general kernel.  Returns the number of launches.
 template <int ALG, int STRUCT>
 static int launch_lean_body(const Launch& a, long long lo, long long n, unsigned long long pair0, long long rounds) {
   int launches = 0;
   for (; rounds > 0; ++launches) {
     const unsigned long long next = ((pair0 >> 32) + 1) << 32;  // the first pair with the next high word
-    const long long fit = (long long)std::min<unsigned long long>((next - pair0) / LEAN_NB, (unsigned long long)rounds);
+    const long long fit =
+        (long long)std::min<unsigned long long>({(next - pair0) / LEAN_NB, (unsigned long long)rounds, LEAN_TAB_ROUNDS});
     if (fit > 0) {
       launch_lean<ALG, STRUCT>(a, lo, n, fit, pair0);
       pair0 += (unsigned long long)fit * LEAN_NB, rounds -= fit;

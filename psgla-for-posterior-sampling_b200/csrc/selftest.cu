@@ -97,6 +97,9 @@ __device__ __forceinline__ uint64_t fp64_round_product(uint64_t a, unsigned m) {
 //   form of one round product (low word, high word, the XOR that consumes it) -- set against mode 0
 //   14 DFMA.RM + FFMA 1:1
 //   200 + NF: the chain-step MIX with the FP64-pipe multiply (6 MUFU, 9 IMAD, 9 DFMA.RM, 2 MOV, NF FFMA, 10 LOP3, 2 I2FP)
+//   300 + NF: the chain-step MIX of gmm2d_lean_kernel with its pair words from the launch's parameter table (6 MUFU,
+//      8 IMAD.WIDE, NF FFMA, 9 LOP3, 2 I2FP and 3 uniform constant loads (LDCU) per 4 steps)
+__constant__ unsigned pipe_rate_table[64];  // never written: zeros; what mode 21's LDCU reads
 template <int MODE, int NF = 19>
 __global__ void __launch_bounds__(256) pipe_rate_kernel(int iters, unsigned seed, unsigned* __restrict__ out) {
   unsigned v[8];
@@ -188,6 +191,36 @@ __global__ void __launch_bounds__(256) pipe_rate_kernel(int iters, unsigned seed
 #pragma unroll
       for (int q = 0; q < 3; ++q) v[q] = w[q];
     }
+    if (MODE == 21) {  // as mode 11 with 8 IMAD.WIDE.U32 + LOP3 and the 9th LOP3, one of them reading a uniform constant load
+      float e[6];
+      unsigned w[3];
+#pragma unroll
+      for (int q = 0; q < 6; ++q) e[q] = f[q];
+#pragma unroll
+      for (int q = 0; q < 3; ++q) w[q] = v[q];
+#pragma unroll
+      for (int st = 0; st < 4; ++st) {
+        const unsigned u = st < 3 ? pipe_rate_table[(i & 15) + 16 * st] : m;  // loop-uniform index: LDCU
+#pragma unroll
+        for (int q = 0; q < 6; ++q) asm volatile("ex2.approx.ftz.f32 %0, %0;" : "+f"(e[q]));
+#pragma unroll
+        for (int q = 0; q < 8; ++q) {
+          unsigned long long p;
+          asm volatile("mul.wide.u32 %0, %1, %2;" : "=l"(p) : "r"(w[q % 3]), "r"(m));
+          asm volatile("lop3.b32 %0, %1, %2, %3, 0x96;" : "=r"(w[q % 3]) : "r"((unsigned)(p >> 32)), "r"((unsigned)p), "r"(q ? m : u));
+        }
+#pragma unroll
+        for (int q = 0; q < NF; ++q) asm volatile("fma.rn.f32 %0, %0, %1, %2;" : "+f"(f[6 + (q & 1)]) : "f"(a), "f"(b));
+        float c0, c1;
+        asm volatile("cvt.rn.f32.u32 %0, %1;" : "=f"(c0) : "r"(w[0]));
+        asm volatile("cvt.rn.f32.u32 %0, %1;" : "=f"(c1) : "r"(w[1]));
+        asm volatile("lop3.b32 %0, %0, %1, %2, 0x96;" : "+r"(v[7]) : "r"(__float_as_uint(c0)), "r"(__float_as_uint(c1)));  // the 9th LOP3
+      }
+#pragma unroll
+      for (int q = 0; q < 6; ++q) f[q] = e[q];
+#pragma unroll
+      for (int q = 0; q < 3; ++q) v[q] = w[q];
+    }
     if (MODE == 20) {  // as mode 11, each IMAD.WIDE.U32 + LOP3 replaced by IMAD + DFMA.RM + LOP3, plus the kernel's ~2 MOV
       float e[6];
 #pragma unroll
@@ -237,7 +270,7 @@ extern "C" int psgla_selftest_fp32_rate(int mode, int iters, int blocks_per_sm, 
 
 extern "C" int psgla_selftest_pipe_rate(int mode, int iters, int blocks_per_sm, void* out_dev, double* ops_out, void* stream) {
   const bool mix_nf = mode % 100 == 21 || mode % 100 == 23 || mode % 100 == 26 || mode % 100 == 28 || mode % 100 == 30;
-  PSGLA_REQUIRE(((mode >= 0 && mode <= 14) || ((mode / 100 == 1 || mode / 100 == 2) && mix_nf)) && iters > 0 && blocks_per_sm > 0 && blocks_per_sm <= 8 && out_dev != nullptr,
+  PSGLA_REQUIRE(((mode >= 0 && mode <= 14) || (mode / 100 >= 1 && mode / 100 <= 3 && mix_nf)) && iters > 0 && blocks_per_sm > 0 && blocks_per_sm <= 8 && out_dev != nullptr,
                 "psgla_selftest_pipe_rate: bad argument");
   const int grid = num_sms() * blocks_per_sm;
   cudaStream_t st = (cudaStream_t)stream;
@@ -267,10 +300,16 @@ extern "C" int psgla_selftest_pipe_rate(int mode, int iters, int blocks_per_sm, 
     case 223: pipe_rate_kernel<20, 23><<<grid, 256, 0, st>>>(iters, 3u, o); break;
     case 226: pipe_rate_kernel<20, 26><<<grid, 256, 0, st>>>(iters, 3u, o); break;
     case 228: pipe_rate_kernel<20, 28><<<grid, 256, 0, st>>>(iters, 3u, o); break;
-    default: pipe_rate_kernel<20, 30><<<grid, 256, 0, st>>>(iters, 3u, o); break;
+    case 230: pipe_rate_kernel<20, 30><<<grid, 256, 0, st>>>(iters, 3u, o); break;
+    case 321: pipe_rate_kernel<21, 21><<<grid, 256, 0, st>>>(iters, 3u, o); break;
+    case 323: pipe_rate_kernel<21, 23><<<grid, 256, 0, st>>>(iters, 3u, o); break;
+    case 326: pipe_rate_kernel<21, 26><<<grid, 256, 0, st>>>(iters, 3u, o); break;
+    case 328: pipe_rate_kernel<21, 28><<<grid, 256, 0, st>>>(iters, 3u, o); break;
+    default: pipe_rate_kernel<21, 30><<<grid, 256, 0, st>>>(iters, 3u, o); break;
   }
   PSGLA_CUDA_TRY(cudaGetLastError());
-  // thread-level instructions of the probed class; mix modes (11, 100 + NF, 200 + NF): thread-level "steps" (4 per loop round)
+  // thread-level instructions of the probed class; mix modes (11, 100 + NF, 200 + NF, 300 + NF): thread-level "steps" (4 per
+  // loop round)
   const bool mix = mode == 11 || mode >= 100;
   if (ops_out) *ops_out = (double)grid * 256.0 * (double)iters * (mix ? 4.0 : 32.0);
   return PSGLA_OK;

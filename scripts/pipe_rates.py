@@ -13,9 +13,11 @@ import psgla_b200 as P  # noqa: E402
 NAMES = ["IMAD.WIDE.U32", "IMAD.HI.U32", "IMAD (lo)", "LOP3", "MUFU.EX2", "I2FP.F32.U32", "FFMA", "MUFU.SIN (+FMUL.RZ)",
          "IMAD.WIDE + FFMA 1:1", "MUFU.EX2 + IMAD.WIDE 1:1", "MUFU.EX2 + 4 FFMA", "chain-step mix (6M 9W 19F 10L 2C)",
          "DFMA.RM", "IMAD + DFMA.RM + LOP3", "DFMA.RM + FFMA 1:1"]
-# the chain-step mix with the integer Philox multiply (100 + NF) and with the FP64-pipe one (200 + NF), NF = FP32 slots per step
+# the chain-step mix with the integer Philox multiply (100 + NF), with the FP64-pipe one (200 + NF) and with the round-2 pair
+# words from the launch's parameter table (300 + NF: 8 IMAD.WIDE, 9 LOP3), NF = FP32 slots per step
 MIXES = [(100 + nf, "mix, IMAD.WIDE form, NF = %d" % nf) for nf in (21, 23, 26, 28, 30)] + \
-        [(200 + nf, "mix, FP64-pipe form, NF = %d" % nf) for nf in (21, 23, 26, 28, 30)]
+        [(200 + nf, "mix, FP64-pipe form, NF = %d" % nf) for nf in (21, 23, 26, 28, 30)] + \
+        [(300 + nf, "mix, 8 IMAD.WIDE + LDCU, NF = %d" % nf) for nf in (21, 23, 26, 28, 30)]
 lib = P._lib.lib()
 scratch = torch.empty(148 * 8 * 256, dtype=torch.float32, device="cuda")
 sms = torch.cuda.get_device_properties(0).multi_processor_count
