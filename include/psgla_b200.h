@@ -337,6 +337,32 @@ size_t psgla_mcmc_diag_large_workspace_bytes(int64_t n_draws, int64_t n_chains, 
 int psgla_mcmc_diag_large(const float* draws_dev, int64_t n_draws, int64_t n_chains, int64_t n_elem, void* ws_dev,
                           size_t ws_bytes, float* rhat_dev, float* ess_bulk_dev, float* ess_tail_dev, void* stream);
 
+/* Posterior summary per element on the engine of psgla_mcmc_diag_large (csrc/mcmc_summary.cu), as arviz's published
+ * functions define it.  With A the K = n_draws n_chains draws of an element (the middle draws of odd n_draws included):
+ *   mean_dev, sd_dev            fp64 mean and sd (divisor K - 1) of A
+ *   ess_mean_dev, mcse_mean_dev Geyer ESS of the raw draws in split-chain order (_ess_mean, not rank-normalised); sd / sqrt(ESS)
+ *   quantiles_dev               numpy's quantile of A at probs_host[i], method "linear"               [n_probs][n_elem]
+ *   ess_quantiles_dev           Geyer ESS of the indicator x <= quantile (_ess_quantile)              [n_probs][n_elem]
+ *   mcse_quantiles_dev          _mcse_quantile: half the distance between the sorted draws at the 0.1586553 / 0.8413447
+ *                               quantiles of Beta(ESS p + 1, ESS (1 - p) + 1), times K, minus 1, rounded half to even
+ *   hdi_low_dev, hdi_high_dev   the narrowest window (a_i, a_{i+k}) of sorted A, k = floor(hdi_prob K); ties: the smaller i
+ * All fp32 [n_elem] unless stated.  NaN draws give NaN for every output of the element; a series whose within-chain variance
+ * is 0 gives NaN for its ESS and MCSE.  Same input layout, ranges and error codes as psgla_mcmc_diag_large; also
+ * PSGLA_E_BADARG for n_probs outside 1..PSGLA_MCMC_MAX_PROBS or a probability or hdi_prob not in the open interval (0, 1),
+ * before any CUDA call.  Workspace: psgla_mcmc_summary_workspace_bytes(...) bytes (0: out of range), 256-byte aligned; the
+ * large path's plus, per element of a group, the quantiles, ESS slots, HDI partials and, for odd n_draws, the merged sorted
+ * draws (4 B per draw).  Its head holds psgla_mcmc_diag_large's words (gather, sort with quantiles, series, moments, lag
+ * rounds, round counts over the 1 + n_probs series), then at word 9 the ns of the HDI scan, at word 10 of the Beta
+ * quantiles and outputs, at word 11 of the merge of odd n_draws; word 12 counts the incomplete-beta evaluations of the Beta
+ * quantiles, word 13 their continued-fraction terms, word 14 the most terms one (element, probability) pair ran.  Stream-ordered; deterministic: an element's results do not depend on n_elem, on its group or on
+ * the other elements. */
+#define PSGLA_MCMC_MAX_PROBS 8
+size_t psgla_mcmc_summary_workspace_bytes(int64_t n_draws, int64_t n_chains, int64_t n_elem, int n_probs);
+int psgla_mcmc_summary(const float* draws_dev, int64_t n_draws, int64_t n_chains, int64_t n_elem, const double* probs_host,
+                       int n_probs, double hdi_prob, void* ws_dev, size_t ws_bytes, float* mean_dev, float* sd_dev,
+                       float* mcse_mean_dev, float* ess_mean_dev, float* quantiles_dev, float* mcse_quantiles_dev,
+                       float* ess_quantiles_dev, float* hdi_low_dev, float* hdi_high_dev, void* stream);
+
 /* tcgen05 descriptor self-test (development aid): runs a 128 x 64 x 64 GEMM tile whose A operand starts `row_shift`
  * rows into a 128B-swizzled shared-memory buffer.  mode 0: A from shared memory, shift = descriptor start address;
  * mode 2: A copied to tensor memory.

@@ -10,7 +10,7 @@ from . import dist  # noqa: F401
 from . import metrics  # noqa: F401
 from . import image_set  # noqa: F401
 from .image_set import load_image, run_image_set  # noqa: F401
-from .diagnostics import mcmc_diagnostics, mcmc_diagnostics_large  # noqa: F401
+from .diagnostics import mcmc_diagnostics, mcmc_diagnostics_large, mcmc_summary  # noqa: F401
 from .metrics import posterior_summary, psnr_ssim  # noqa: F401
 from .denoisers import (DRUNET_KEYS, GSDRUNET_KEYS, DRUNet, DnCNN, GSDRUNet, TVDenoiser, lipschitz_dncnn_state_dict,  # noqa: F401
                         random_dncnn_state_dict, random_drunet_state_dict, random_gsdrunet_state_dict,  # noqa: F401

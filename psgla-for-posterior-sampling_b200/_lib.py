@@ -125,6 +125,9 @@ SIGNATURES = {
     "psgla_mcmc_diag": (_int, [_vp, _i64, _i64, _i64, _vp, _sz, _vp, _vp, _vp, _vp]),
     "psgla_mcmc_diag_large_workspace_bytes": (_sz, [_i64, _i64, _i64]),
     "psgla_mcmc_diag_large": (_int, [_vp, _i64, _i64, _i64, _vp, _sz, _vp, _vp, _vp, _vp]),
+    "psgla_mcmc_summary_workspace_bytes": (_sz, [_i64, _i64, _i64, _int]),
+    "psgla_mcmc_summary": (_int, [_vp, _i64, _i64, _i64, C.POINTER(C.c_double), _int, C.c_double, _vp, _sz, _vp, _vp, _vp,
+                                  _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "psgla_selftest_umma": (_int, [_vp, _vp, _vp, _int, _int, _vp]),
     "psgla_selftest_umma2": (_int, [_vp, _vp, _vp, _int, _vp]),
     "psgla_convg_layer": (_int, [_int, _int, _int, _int, _int, _int, _vp, _vp, _vp, _vp, _vp, _int, _vp]),

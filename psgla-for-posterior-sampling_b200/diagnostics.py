@@ -7,11 +7,20 @@
 
     d = psgla_b200.mcmc_diagnostics_large(traj, burn_in=b)  # traj = GMMChains.run(n, thin=k): [N, M, 2]
 
-The kernels (csrc/mcmc_diag.cu, csrc/mcmc_diag_large.cu) read the draws where the sampler stored them, [N][M][C][H][W]: a run
+and the posterior summary with its Monte Carlo standard errors (arviz's _mcse_mean, _mcse_quantile, _ess_mean,
+_ess_quantile, _hdi), with the calibration check against a ground truth:
+
+    s = psgla_b200.mcmc_summary(run, burn_in=100, probs=(0.05, 0.5, 0.95), hdi_prob=0.94, truth=x_true)
+    s["mean"], s["sd"], s["mcse_mean"], s["ess_mean"], s["hdi_low"], s["hdi_high"]   # [C, H, W] maps
+    s["quantiles"], s["mcse_quantiles"], s["ess_quantiles"]                          # [P, C, H, W]
+    s["coverage_hdi"], s["frac_truth_below"]                                        # with truth=
+
+The kernels (csrc/mcmc_diag.cu, csrc/mcmc_diag_large.cu, csrc/mcmc_summary.cu) read the draws where the sampler stored them, [N][M][C][H][W]: a run
 object is diagnosed in place, with no copy.  mcmc_diagnostics sorts one element in shared memory: S = 2 M floor(N / 2) <=
 PSGLA_MCMC_MAX_DRAWS = 16 384 split draws per element.  mcmc_diagnostics_large computes the same statistics device-wide for
 S up to 2^31 - 1 (a 2D population of 10^6 chains x 2 000 draws, an image run with the reference's own thinning), with a
-workspace of about 16 bytes per split draw of a group of elements.
+workspace of about 16 bytes per split draw of a group of elements.  mcmc_summary runs on the engine of
+mcmc_diagnostics_large, with the same inputs and limits.
 """
 from __future__ import annotations
 
@@ -21,10 +30,11 @@ import torch
 
 from . import _lib
 
-__all__ = ["mcmc_diagnostics", "mcmc_diagnostics_large", "MAX_DRAWS", "MAX_DRAWS_LARGE"]
+__all__ = ["mcmc_diagnostics", "mcmc_diagnostics_large", "mcmc_summary", "MAX_DRAWS", "MAX_DRAWS_LARGE", "MAX_PROBS"]
 
 MAX_DRAWS = 16384  # PSGLA_MCMC_MAX_DRAWS
 MAX_DRAWS_LARGE = 2 ** 31 - 1  # psgla_mcmc_diag_large
+MAX_PROBS = 8  # PSGLA_MCMC_MAX_PROBS
 
 
 def _as_draws(draws):
@@ -84,6 +94,13 @@ def _prepare(draws, burn_in):
     if N < 4:
         raise ValueError("split chains need at least 4 draws after burn-in, got %d" % N)
     return x, N, M, x[0, 0].numel(), map_shape, crop
+
+
+def _check_large(N, M):
+    S = 2 * M * (N // 2)
+    if S > MAX_DRAWS_LARGE:
+        raise ValueError("%d chains x %d draws give S = %d split draws per element, above the limit of 2^31 - 1: thin more, "
+                         "raise burn_in or diagnose fewer chains" % (M, N, S))
 
 
 def _run(fn, ws_bytes, x, N, M, E, map_shape, crop, name):
@@ -149,10 +166,92 @@ def mcmc_diagnostics_large(draws, *, burn_in: int = 0) -> dict:
 
     The workspace is allocated per call: about 16 bytes per split draw of a group of min(E, 2^28 / S) elements."""
     x, N, M, E, map_shape, crop = _prepare(draws, burn_in)
-    S = 2 * M * (N // 2)
-    if S > MAX_DRAWS_LARGE:
-        raise ValueError("%d chains x %d draws give S = %d split draws per element, above the limit of 2^31 - 1: thin more, "
-                         "raise burn_in or diagnose fewer chains" % (M, N, S))
+    _check_large(N, M)
     lib = _lib.lib()
     return _run(lib.psgla_mcmc_diag_large, lib.psgla_mcmc_diag_large_workspace_bytes(N, M, E), x, N, M, E, map_shape, crop,
                 "psgla_mcmc_diag_large")
+
+
+def _open_unit(v, name):
+    v = float(v)
+    if not 0.0 < v < 1.0:  # NaN fails too
+        raise ValueError("%s = %r must be in the open interval (0, 1)" % (name, v))
+    return v
+
+
+def mcmc_summary(draws, *, burn_in: int = 0, probs=(0.05, 0.5, 0.95), hdi_prob: float = 0.94, truth=None) -> dict:
+    """Posterior summary of every element of a multi-chain run with its Monte Carlo standard errors, on the device
+    (csrc/mcmc_summary.cu, on the engine of mcmc_diagnostics_large), as arviz's published functions define it.  With A the
+    N M draws of an element after burn-in (the middle draws of odd N included) and split chains as in mcmc_diagnostics:
+
+      mean, sd          fp64 mean and sd (ddof 1) of A
+      ess_mean          Geyer ESS of the raw draws in split-chain order (arviz's _ess_mean: not rank-normalised)
+      mcse_mean         sd / sqrt(ess_mean): the Monte Carlo error of the MMSE estimate
+      quantiles[i]      np.quantile(A, probs[i]) (method "linear")
+      ess_quantiles[i]  Geyer ESS of the indicator x <= quantiles[i] (_ess_quantile; at 0.05 / 0.95 the tail ESS's series)
+      mcse_quantiles[i] _mcse_quantile: half the distance between the sorted draws at the Beta(ess p + 1, ess (1 - p) + 1)
+                        quantiles 0.1586553 / 0.8413447 of the draw ranks
+      hdi_low, hdi_high the narrowest interval holding floor(hdi_prob N M) + 1 sorted draws (_hdi; ties: the lowest)
+
+    draws: as mcmc_diagnostics_large (a run object read in place, an Xlist, [N, M, C, H, W] or [N, M, E]); a padded DRUNet
+    run's maps are cropped like its outputs.  probs: 1 to 8 probabilities in (0, 1); hdi_prob in (0, 1).
+
+    Returns a dict of CUDA fp32 maps ``mean``, ``sd``, ``mcse_mean``, ``ess_mean``, ``hdi_low``, ``hdi_high`` (the map shape)
+    and ``quantiles``, ``mcse_quantiles``, ``ess_quantiles`` ([P, *map]); ``probs``, ``hdi_prob``, ``n_draws``, ``n_chains``;
+    the floats ``mcse_mean_max`` and ``mcse_quantiles_max`` (a list, one per p) over the elements where they are not NaN.
+    NaN draws make every output of their element NaN; a series constant within every split chain gives NaN for its ESS and
+    MCSE.  ``truth`` (the ground truth at the map shape) adds ``coverage_hdi``, the fraction of the elements with an HDI
+    (not NaN) that hold it, and ``frac_truth_below`` (one per p), the fraction of the elements with a quantile that it does not
+    exceed: for calibrated intervals these approach hdi_prob and p.  Stream-ordered on the current stream; the scalars
+    synchronise it."""
+    x, N, M, E, map_shape, crop = _prepare(draws, burn_in)
+    _check_large(N, M)
+    probs = tuple(_open_unit(p, "probs[%d]" % i) for i, p in enumerate(probs))
+    if not 1 <= len(probs) <= MAX_PROBS:
+        raise ValueError("probs must hold 1 to %d probabilities, got %d" % (MAX_PROBS, len(probs)))
+    hdi_prob = _open_unit(hdi_prob, "hdi_prob")
+    P = len(probs)
+    lib = _lib.lib()
+    ws_bytes = lib.psgla_mcmc_summary_workspace_bytes(N, M, E, P)
+    with torch.cuda.device(x.device):
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
+        out = torch.empty((6 + 3 * P, E), dtype=torch.float32, device=x.device)
+        maps6, per_p = out[:6], out[6:].reshape(3, P, E)
+        _lib.check(lib.psgla_mcmc_summary(
+            _lib.ptr(x), N, M, E, (C.c_double * P)(*probs), P, hdi_prob, _lib.ptr(ws), C.c_size_t(ws_bytes),
+            *[maps6[i].data_ptr() for i in range(4)], *[per_p[i].data_ptr() for i in range(3)], maps6[4].data_ptr(),
+            maps6[5].data_ptr(), _lib.stream_ptr(x.device)), "psgla_mcmc_summary")
+    maps6 = maps6.reshape((6,) + map_shape)
+    per_p = per_p.reshape((3, P) + map_shape)
+    if crop is not None:
+        maps6, per_p = maps6[..., :crop[0], :crop[1]], per_p[..., :crop[0], :crop[1]]
+    mean, sd, mcse_mean, ess_mean, hdi_low, hdi_high = maps6
+    quantiles, mcse_quantiles, ess_quantiles = per_p
+
+    def finite_max(t):
+        t = t.reshape(-1)
+        t = t[~torch.isnan(t)]
+        return float(t.max()) if t.numel() else float("nan")
+
+    res = {
+        "mean": mean, "sd": sd, "mcse_mean": mcse_mean, "ess_mean": ess_mean, "hdi_low": hdi_low, "hdi_high": hdi_high,
+        "quantiles": quantiles, "mcse_quantiles": mcse_quantiles, "ess_quantiles": ess_quantiles,
+        "probs": probs, "hdi_prob": hdi_prob, "n_draws": N, "n_chains": M,
+        "mcse_mean_max": finite_max(mcse_mean), "mcse_quantiles_max": [finite_max(t) for t in mcse_quantiles],
+    }
+    if truth is not None:
+        if not isinstance(truth, torch.Tensor):
+            raise TypeError("truth must be a torch tensor, got %s" % type(truth).__name__)
+        if tuple(truth.shape) != tuple(mean.shape):
+            raise ValueError("truth has shape %s; the summary maps have shape %s" % (tuple(truth.shape), tuple(mean.shape)))
+        t = truth.to(device=mean.device, dtype=torch.float32)
+        ok = ~torch.isnan(hdi_low)
+        n_ok = int(ok.sum())
+        res["coverage_hdi"] = (float(((hdi_low <= t) & (t <= hdi_high) & ok).sum()) / n_ok) if n_ok else float("nan")
+        below = []
+        for q in quantiles:
+            okq = ~torch.isnan(q)
+            n_q = int(okq.sum())
+            below.append(float(((t <= q) & okq).sum()) / n_q if n_q else float("nan"))
+        res["frac_truth_below"] = below
+    return res
